@@ -24,6 +24,10 @@ roofline algorithmic bytes of one frame (SURVEY.md 8d formula over the kernel's 
 cpu_baseline  the unmodified reference (oracle/_ref) on all host cores, on a bounded sample of the same
          frame (full-width row bands), rays of the sample counted by the oracle restatement.
 config.other_workloads  the other GPU configurations of BASELINE.json (C2, C4, C5) on the same GPU, 3 frames each.
+
+--dump-outputs DIR writes the frame of the last timed step (what a caller of the timed path receives) to
+DIR/frame.npy as float32 (H, W, 3); the scene, camera and lights are seeded, so two builds can be compared output for
+output.  The benchmark runs the library as it was built and writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -37,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the tree
 
 WORKLOAD = "C3"
 SCENE_DIR = os.environ.get("MTB_SCENE_DIR", "/tmp/mtb_scenes")
@@ -363,7 +368,6 @@ def _run_ours(args):
     import torch.distributed as dist
 
     from mythtracer_b200 import Light, MythTracer, MTB_FLAG_COUNT_WORK, MTB_FLAG_HYBRID, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE, MTB_FLAG_WAVEFRONT, tiles
-    from mythtracer_b200 import build as mtb_build
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -378,8 +382,6 @@ def _run_ours(args):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
 
-    if rank == 0:
-        mtb_build.build()
     if world > 1:
         dist.barrier()
     files, cfg = (load_workload() if rank == 0 else (None, None))
@@ -519,7 +521,13 @@ def _run_ours(args):
     elapsed_ms = ev0.elapsed_time(ev1)
     kernel_ms_mean = sum(a.elapsed_time(b) for a, b in k_events) / len(k_events)
     counters = mt.read_counters()
-    frame_sha = hashlib.sha256(read_frame(last_ptr).tobytes()).hexdigest() if rank == 0 else None
+    frame = read_frame(last_ptr) if rank == 0 else None
+    frame_sha = hashlib.sha256(frame.tobytes()).hexdigest() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        # 1920 x 1080 x 3 float32 = 25 MB: the whole frame, exact (uint8 values)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "frame.npy"), frame.reshape(H, W, 3).astype(np.float32))
+        log("bench.py: wrote the last timed frame to %s" % os.path.join(args.dump_outputs, "frame.npy"))
     t = torch.tensor([elapsed_ms, float(counters["rays"]), float(launches), kernel_ms_mean], dtype=torch.float64, device=dev)
     kernel_ms_max = kernel_ms_mean
     kernel_ms_ranks = [kernel_ms_mean]
@@ -687,7 +695,10 @@ def main():
     ap.add_argument("--pipeline", default=os.environ.get("MTB_PIPELINE", "auto"), choices=["auto", "mega", "wavefront", "hybrid", "queue"])
     ap.add_argument("--gather", default=os.environ.get("MTB_GATHER", "peer"), choices=["peer", "nccl"],
                     help="N > 1 under torchrun: direct peer stores into rank 0's frame (default) or an NCCL gather (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR/frame.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_ours(args)
