@@ -157,7 +157,21 @@ class MythTracer {
     if (rc != MTB_OK) fprintf(stderr, "error: %s\n", mtb_last_error(ctx));
     return rc == MTB_OK;
   }
+  // Batches (mtb_render_batch): cams.size() whole frames in one launch per device, written view-major to `out`
+  // (cams.size() * w * h * 3 bytes).  lights: one light list per view, all of the same length; nullptr = scene.lights
+  // for every view.  RayTraceBatchAsync returns once the batch is queued (`out` pinned, from AllocFrames; Wait joins).
+  bool RayTraceBatch(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
+                     uint8_t *out) {
+    return RenderBatch(image_width, image_height, cams, lights, out, true);
+  }
+  bool RayTraceBatchAsync(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
+                          uint8_t *pinned_out) {
+    return RenderBatch(image_width, image_height, cams, lights, pinned_out, false);
+  }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
+  static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
+    return static_cast<uint8_t *>(mtb_host_alloc((size_t)image_width * image_height * 3 * (size_t)n_frames));
+  }
   static uint8_t *AllocFrame(int image_width, int image_height) {
     return static_cast<uint8_t *>(mtb_host_alloc((size_t)image_width * image_height * 3));
   }
@@ -168,6 +182,51 @@ class MythTracer {
   mtb_stats last_stats{};
 
  private:
+  bool RenderBatch(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
+                   uint8_t *out, bool synchronous) {
+    if (!was_scene_finalized) {
+      puts("Finalizing tree.");
+      if (!scene.tree.Finalize(&scene.materials, &scene.textures)) return false;
+      was_scene_finalized = true;
+    }
+    mtb_context *ctx = scene.tree.context();
+    std::vector<mtb_camera> mcams;
+    for (const Camera &c : cams) mcams.push_back(c.AsMtb());
+    std::vector<Light> flat;
+    int32_t n_lights = 0;
+    if (lights == nullptr) {
+      if (mtb_set_lights(ctx, reinterpret_cast<const mtb_light *>(scene.lights.data()), (int32_t)scene.lights.size()) != MTB_OK) {
+        return false;
+      }
+    } else {
+      if (lights->size() != cams.size()) {
+        fprintf(stderr, "error: %zu light sets for %zu cameras (one per view)\n", lights->size(), cams.size());
+        return false;
+      }
+      n_lights = lights->empty() ? 0 : (int32_t)lights->front().size();
+      for (const std::vector<Light> &ls : *lights) {
+        if ((int32_t)ls.size() != n_lights) {
+          fputs("error: every view needs the same number of lights\n", stderr);
+          return false;
+        }
+        flat.insert(flat.end(), ls.begin(), ls.end());
+      }
+      flat.resize(flat.size() + 1);  // (non-NULL even with no lights: n_lights = 0 is not "the scene's lights")
+    }
+    const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
+    mtb_stats stats;
+    const int rc = synchronous ? mtb_render_batch(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
+                                                  max_recursion_level, out, &stats)
+                               : mtb_render_batch_async(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
+                                                        max_recursion_level, out);
+    if (rc != MTB_OK) {
+      fprintf(stderr, "error: %s\n", mtb_last_error(ctx));
+      return false;
+    }
+    if (synchronous) last_stats = stats;
+    return true;
+  }
+
   Scene scene;
   bool was_scene_finalized = false;
   int max_recursion_level = MAX_RECURSION_LEVEL;

@@ -236,6 +236,25 @@ int mtb_wait(mtb_context *ctx);
 void *mtb_host_alloc(size_t bytes);
 void mtb_host_free(void *p);
 
+/* Batches: N whole frames of one scene, one camera and one light set per view, in one launch per device (an orbit, a
+ * camera path, a light sweep, many small views: a 480x270 frame is less than one wave of the B200, a batch of them
+ * fills the machine).  Always the per-pixel megakernel: the pipeline bits (MTB_FLAG_WAVEFRONT, _QUEUE, _HYBRID,
+ * _MEGAKERNEL) are ignored; MTB_FLAG_COUNT_WORK and the traversal flags apply as for a single frame.  The bytes of view
+ * v equal those of mtb_render_chunk with cams[v] and view v's lights.  A batch leaves the state of the single-frame
+ * path alone (the context's lights, the automatic pipeline choice, the tile order).  With several devices, device g
+ * renders a contiguous range of the views (counts differ by at most one) and copies them to their slice of rgb_out;
+ * there is no gather.  The partition must be (0, 1).
+ *
+ * rgb_out: HOST, n_views * image_h * image_w * 3 bytes, view-major.  lights: n_views * n_lights entries
+ * (view v uses lights[v*n_lights .. +n_lights)); NULL = every view uses the context's lights (mtb_set_lights)
+ * and n_lights is ignored.  n_views: 1..65535.  stats (nullable): summed over views; kernel_ms = slowest device. */
+int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
+                     int32_t n_lights, int image_w, int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats);
+/* Same, returns once queued (rgb_out pinned, from mtb_host_alloc; mtb_wait joins), like mtb_render_chunk_async.
+ * cams and lights may be reused as soon as the call returns. */
+int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
+                           int32_t n_lights, int image_w, int image_h, int max_depth, uint8_t *rgb_out);
+
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the
  * context has one device.  This is the entry bench.py times for the HBM-resident figure. */

@@ -79,6 +79,7 @@ EXPORTED_SYMBOLS = [
     "mtb_scene_triangle_nodes", "mtb_scene_bvh", "mtb_set_flags", "mtb_set_partition", "mtb_render_chunk",
     "mtb_render_chunk_device", "mtb_render_chunk_async", "mtb_wait", "mtb_host_alloc", "mtb_host_free", "mtb_read_counters", "mtb_launch_count", "mtb_pipeline_in_use", "mtb_intersect_rays", "mtb_camera_sensor", "mtb_version",
     "mtb_frame_create", "mtb_frame_open", "mtb_frame_release", "mtb_frame_read", "mtb_load_timing", "mtb_hybrid_share",
+    "mtb_render_batch", "mtb_render_batch_async",
 ]
 
 
@@ -130,6 +131,8 @@ def load_library():
     lib.mtb_set_partition.argtypes = [vp, i32, i32]
     lib.mtb_render_chunk.argtypes = [vp, vp] + [i32] * 7 + [vp, vp, vp, vp]
     lib.mtb_render_chunk_device.argtypes = [vp, vp] + [i32] * 7 + [vp, vp, vp]
+    lib.mtb_render_batch.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, vp, vp]
+    lib.mtb_render_batch_async.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, vp]
     lib.mtb_read_counters.argtypes = [vp, vp]
     lib.mtb_pipeline_in_use.argtypes = [vp, vp, vp]
     lib.mtb_launch_count.argtypes = [vp]
@@ -459,6 +462,44 @@ class MythTracer:
             res["line_no"] = dbg["line_no"]
             res["points"] = dbg["point"]
         res["stats"] = {k: stats[k].item() for k in STATS_DTYPE.names}
+        self.last_stats = res["stats"]
+        return res
+
+    def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None):
+        """mtb_render_batch: len(cameras) whole frames in one launch per device, at depth self.max_depth.
+
+        lights: None (every view uses GetScene().lights) or one list of Light per view, all of the same length.
+        Returns dict(rgb=uint8[n, height, width, 3], stats) with the stats summed over the views."""
+        cams = [c if isinstance(c, Camera) else Camera.from_tuple(c) for c in cameras]
+        if not cams:
+            raise MythTracerError("render_batch: no cameras")
+        cam_arr = np.zeros(len(cams), CAMERA_DTYPE)
+        for i, c in enumerate(cams):
+            cam_arr[i] = c.as_array()
+        light_arr, n_lights = None, 0
+        if lights is None:
+            self._push_lights()
+        else:
+            lights = list(lights)
+            if len(lights) != len(cams):
+                raise MythTracerError("render_batch: %d light sets for %d cameras (one per view)" % (len(lights), len(cams)))
+            sizes = {len(ls) for ls in lights}
+            if len(sizes) != 1:
+                raise MythTracerError("render_batch: every view needs the same number of lights (got %s)" % sorted(sizes))
+            n_lights = sizes.pop()
+            # (n_lights = 0 still passes a non-NULL array: no lights at all, not "the scene's lights")
+            light_arr = _lights_array([l for ls in lights for l in ls]) if n_lights else np.zeros(1, LIGHT_DTYPE)
+        shape = (len(cams), height, width, 3)
+        if out is None:
+            rgb = np.zeros(shape, np.uint8)
+        else:
+            if out.shape != shape or out.dtype != np.uint8 or not out.flags["C_CONTIGUOUS"]:
+                raise MythTracerError("render_batch: out must be a C-contiguous uint8 array of shape %s" % (shape,))
+            rgb = out
+        stats = np.zeros((), STATS_DTYPE)
+        self._check(self._lib.mtb_render_batch(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
+                                               self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch")
+        res = {"rgb": rgb, "stats": {k: stats[k].item() for k in STATS_DTYPE.names}}
         self.last_stats = res["stats"]
         return res
 

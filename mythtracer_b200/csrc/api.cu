@@ -111,6 +111,12 @@ struct DeviceState {
   cudaEvent_t ev_split = nullptr, ev_mega_done = nullptr, ev_wf_done = nullptr;  // (timed: they steer the split)
   float hybrid_share = 0.30f;     // share of the frame's rays that goes through the wavefront; steered frame by frame
   bool hybrid_timed = false;      // the three events above were recorded by the previous hybrid frame
+  // batch launches (RenderBatchImpl): view records, per-view lights and the views' frames of this device, and the
+  // events that time them (the single-frame events steer the automatic pipeline choice and are left alone)
+  DeviceBuffer<mtb::ViewRec> batch_views;
+  DeviceBuffer<mtb_light> batch_lights;
+  DeviceBuffer<uint8_t> batch_rgb;
+  cudaEvent_t ev_batch_start = nullptr, ev_batch_stop = nullptr;
   // intersect scratch
   DeviceBuffer<double> q_origins, q_dirs, q_t, q_point;
   DeviceBuffer<int32_t> q_tri;
@@ -147,6 +153,10 @@ struct DeviceState {
     nodes.Free(); slots.Free(); shade.Free(); bvh.Free(); gnodes.Free(); gslots.Free(); list_order.Free(); slot_node.Free(); leaf_ref.Free(); ref_slot.Free(); materials.Free();
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
     counters.Free(); tile_cost.Free(); tile_order.Free(); heavy_k.Free();
+    batch_views.Free(); batch_lights.Free(); batch_rgb.Free();
+    if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
+    if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
+    ev_batch_start = ev_batch_stop = nullptr;
     if (hybrid_stream != nullptr) cudaStreamDestroy(hybrid_stream);
     hybrid_stream = nullptr;
     if (ev_split != nullptr) cudaEventDestroy(ev_split);
@@ -998,6 +1008,159 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
   return MTB_OK;
 }
 
+// A batch: n_views whole frames of one scene, one camera and one light set per view.  Always the megakernel, in one
+// launch per device (grid = tiles of a view x views of the device): the pipeline choice, the cost-aware tile order, the
+// hybrid split and the strip interleave are all single-frame machinery and none of their state is read or written.
+// lights == NULL: every view uses the context's lights.  Device g renders a contiguous range of views; the counts
+// differ by at most one.
+int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
+                    int image_h, int max_depth, uint8_t *rgb_host, mtb_stats *stats, bool synchronous) {
+  const auto wall0 = std::chrono::steady_clock::now();
+  if (ctx == nullptr) return MTB_ERR_ARG;
+  if (ctx->dev.empty()) {
+    ctx->err = "host-only context: no CUDA device to render on (there is no CPU fallback)";
+    return MTB_ERR_CUDA;
+  }
+  if (!ctx->has_scene) {
+    ctx->err = "no scene uploaded";
+    return MTB_ERR_ARG;
+  }
+  if (cams == nullptr || rgb_host == nullptr) {
+    ctx->err = cams == nullptr ? "cams is NULL" : "rgb_out is NULL";
+    return MTB_ERR_ARG;
+  }
+  if (n_views < 1 || n_views > 65535) {
+    ctx->err = "n_views must be in 1..65535 (one grid row per view)";
+    return MTB_ERR_ARG;
+  }
+  if (lights != nullptr && n_lights < 0) {
+    ctx->err = "n_lights must be >= 0";
+    return MTB_ERR_ARG;
+  }
+  if (image_w <= 0 || image_h <= 0 || max_depth < 0 || max_depth > MTB_MAX_RAY_DEPTH) {
+    ctx->err = "bad render arguments";
+    return MTB_ERR_ARG;
+  }
+  if (ctx->part_index != 0 || ctx->part_count != 1) {
+    ctx->err = "a batch renders whole views: the partition must be (0, 1)";
+    return MTB_ERR_ARG;
+  }
+  const size_t npx = (size_t)image_w * image_h;
+  const bool debug_build = (ctx->flags & MTB_FLAG_COUNT_WORK) != 0;
+  const int n_dev = (int)ctx->dev.size();
+  const int tiles_x = (image_w + 7) / 8, tiles_per_view = tiles_x * ((image_h + 7) / 8);
+
+  // per-view records and the views' lights, view-major (the context's lights repeated when the caller passes none)
+  const int32_t nl = lights != nullptr ? n_lights : (int32_t)ctx->lights.size();
+  std::vector<mtb::ViewRec> views((size_t)n_views);
+  std::vector<mtb_light> view_lights((size_t)n_views * nl);
+  for (int32_t v = 0; v < n_views; v++) {
+    mtb::ComputeSensor(cams[v], image_w, image_h, views[(size_t)v].sensor);
+    for (int a = 0; a < 3; a++) views[(size_t)v].origin[a] = cams[v].origin[a];
+    const mtb_light *src = lights != nullptr ? lights + (size_t)v * nl : ctx->lights.data();
+    if (nl > 0) std::copy(src, src + nl, view_lights.begin() + (size_t)v * nl);
+  }
+
+  mtb::RenderParams rp;
+  memset(&rp, 0, sizeof(rp));
+  rp.image_w = rp.chunk_w = image_w;
+  rp.image_h = rp.chunk_h = image_h;
+  rp.max_depth = max_depth;
+  rp.tiles_x = tiles_x;
+  rp.strip_stride = 1;
+
+  // Where the pixels go: a single device stores straight into a mapped pinned rgb_host (RenderImpl's rule); otherwise
+  // every device renders into its own frames and copies its views to their slice of rgb_host.
+  uint8_t *host_direct = nullptr;
+  if (n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
+    MTB_CUDA(ctx, cudaSetDevice(ctx->dev[0].device));
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer != nullptr) {
+      host_direct = static_cast<uint8_t *>(attr.devicePointer);
+    }
+    cudaGetLastError();  // (an unregistered pointer is not an error here)
+  }
+
+  auto launch_on_device = [&](int g) -> int {
+    DeviceState &d = ctx->dev[(size_t)g];
+    const int first = g * (n_views / n_dev) + std::min(g, n_views % n_dev);
+    const int count = n_views / n_dev + (g < n_views % n_dev ? 1 : 0);
+    if (count == 0) return MTB_OK;
+    MTB_CUDA(ctx, cudaSetDevice(d.device));
+    cudaStream_t s = d.stream;
+    if (d.ev_batch_start == nullptr) {
+      MTB_CUDA(ctx, cudaEventCreate(&d.ev_batch_start));
+      MTB_CUDA(ctx, cudaEventCreate(&d.ev_batch_stop));
+    }
+    // Everything below is ordered on d.stream: a batch queued behind another one overwrites the records only after the
+    // earlier launch has read them.  A buffer that has to grow is freed and reallocated, so the earlier work that may
+    // still read it is waited for first.
+    const size_t n_rgb = host_direct != nullptr ? 0 : (size_t)count * npx * 3;
+    const size_t n_lt = (size_t)count * nl;
+    if ((size_t)count > d.batch_views.count || n_lt > d.batch_lights.count || n_rgb > d.batch_rgb.count) {
+      MTB_CUDA(ctx, cudaStreamSynchronize(s));
+    }
+    MTB_CUDA(ctx, d.batch_views.Upload(views.data() + first, (size_t)count, s));
+    MTB_CUDA(ctx, d.batch_lights.Upload(view_lights.data() + (size_t)first * nl, n_lt, s));
+    if (n_rgb > 0) MTB_CUDA(ctx, d.batch_rgb.Reserve(n_rgb));
+    mtb::DeviceScene sc = d.scene;
+    sc.lights = d.batch_lights.ptr;
+    sc.n_lights = nl;
+    mtb::RenderParams p = rp;
+    p.rgb = host_direct != nullptr ? host_direct + (size_t)first * npx * 3 : d.batch_rgb.ptr;
+    MTB_CUDA(ctx, d.counters.Reserve(mtb::kNumCounters));
+    p.counters = d.counters.ptr;
+    if (stats != nullptr || synchronous) {
+      MTB_CUDA(ctx, cudaMemsetAsync(d.counters.ptr, 0, mtb::kNumCounters * sizeof(unsigned long long), s));
+    }
+    MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_start, s));
+    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, debug_build, s);
+    ctx->launches++;
+    MTB_CUDA(ctx, cudaGetLastError());
+    MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_stop, s));
+    if (host_direct == nullptr) {
+      MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first * npx * 3, d.batch_rgb.ptr, (size_t)count * npx * 3, cudaMemcpyDeviceToHost, s));
+    }
+    return MTB_OK;
+  };
+  if (n_dev == 1) {
+    const int rc = launch_on_device(0);
+    if (rc != MTB_OK) return rc;
+  } else {
+    std::vector<int> rcs((size_t)n_dev, MTB_OK);
+    std::vector<std::thread> workers;
+    for (int g = 0; g < n_dev; g++) workers.emplace_back([&, g]() { rcs[(size_t)g] = launch_on_device(g); });
+    for (std::thread &t : workers) t.join();
+    for (int rc : rcs) {
+      if (rc != MTB_OK) return rc;
+    }
+  }
+  if (!synchronous && stats == nullptr) return MTB_OK;
+
+  unsigned long long total[mtb::kNumCounters];
+  memset(total, 0, sizeof(total));
+  double kernel_ms = 0.0;
+  for (int g = 0; g < n_dev && g < n_views; g++) {
+    DeviceState &d = ctx->dev[(size_t)g];
+    MTB_CUDA(ctx, cudaSetDevice(d.device));
+    MTB_CUDA(ctx, cudaStreamSynchronize(d.stream));
+    if (stats == nullptr) continue;
+    unsigned long long c[mtb::kNumCounters];
+    MTB_CUDA(ctx, cudaMemcpy(c, d.counters.ptr, sizeof(c), cudaMemcpyDeviceToHost));
+    for (int i = 0; i < mtb::kNumCounters; i++) total[i] += c[i];
+    float ms = 0.f;
+    MTB_CUDA(ctx, cudaEventElapsedTime(&ms, d.ev_batch_start, d.ev_batch_stop));
+    if (ms > kernel_ms) kernel_ms = ms;  // devices run concurrently: the batch takes the slowest
+  }
+  if (stats != nullptr) {
+    memset(stats, 0, sizeof(*stats));
+    FillStats(total, stats);
+    stats->kernel_ms = kernel_ms;
+    stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
+  }
+  return MTB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1326,6 +1489,16 @@ int mtb_render_chunk_async(mtb_context *ctx, const mtb_camera *cam, int image_w,
   }
   return RenderImpl(ctx, cam, image_w, image_h, chunk_x, chunk_y, chunk_w, chunk_h, max_depth, rgb_out, nullptr, nullptr,
                     nullptr, nullptr, nullptr, false);
+}
+
+int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
+                     int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, max_depth, rgb_out, stats, true);
+}
+
+int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
+                           int image_w, int image_h, int max_depth, uint8_t *rgb_out) {
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, max_depth, rgb_out, nullptr, false);
 }
 
 int mtb_wait(mtb_context *ctx) {

@@ -70,6 +70,13 @@ struct RenderParams {
   const uint32_t *run_if;
 };
 
+// One view of a batch launch (LaunchRenderMegaBatch): its camera as Camera::GetSensor leaves it (ComputeSensor on the
+// host).  The lights of view v are DeviceScene::lights[v * n_lights ..] of the scene copy the batch launch passes.
+struct ViewRec {
+  double sensor[9];  // start_point, delta_scanline, delta_pixel
+  double origin[3];
+};
+
 struct IntersectParams {
   int64_t n;
   const double *origins, *dirs;
@@ -143,6 +150,11 @@ void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles,
                           cudaStream_t stream);
 // One 8x8 tile per 64-thread block; n_blocks = tiles of the launch (rp.tiles_x in units of 8 pixels).
 void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_blocks, bool debug_build, cudaStream_t stream);
+// n_views whole frames in one launch: grid (tiles_per_view, n_views), camera of view v = views[v] (device memory), its
+// lights sc.lights + v * sc.n_lights, its pixels rp.rgb + v * chunk_w * chunk_h * 3.  rp.strip_first = 0,
+// rp.strip_stride = 1, and tile_order / tile_cost / heavy_k / run_if / taps / dbg NULL.
+void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views, bool debug_build,
+                           cudaStream_t stream);
 void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, int mode, cudaStream_t stream);  // mode 0: one ray per thread, 1: two rays per lane (Trace2), 2: chain (TraceChain), 3: two calls
 
 }  // namespace mtb
