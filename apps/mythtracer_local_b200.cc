@@ -2,10 +2,13 @@
 // (SURVEY.md section 8 f3): orbiting camera, lights re-set every frame, raw RGB24 frames to
 // anim/dump_%05i.raw.  The model path, resolution and frame range are arguments instead of constants.
 //
-//   mythtracer_local_b200 scene.obj [width height first_frame last_frame out_dir frames_per_call]
+//   mythtracer_local_b200 scene.obj [width height first_frame last_frame out_dir frames_per_call samples_per_axis]
 //
 // frames_per_call N > 1 renders N consecutive frames per batch call (one launch for all of them: a 480x270 frame alone
 // is less than one wave of the B200); the files and their bytes are the same as with N = 1, the default.
+// samples_per_axis s = 2, 4 or 8 writes anti-aliased frames (s x s samples per pixel, averaged on the device) of the
+// same width x height; they always go through the batch path, with N frames per call.  s = 1, the default, is the
+// reference's one ray per pixel.
 #include <sys/stat.h>
 #include <sys/types.h>
 
@@ -49,7 +52,7 @@ bool WriteFrame(const char *out_dir, int number, const uint8_t *pixels, size_t f
 // frames_per_call > 1: `per_call` consecutive frames per batch call (the last batch may be partial), into two pinned
 // batch buffers in rotation: batch k is written to disk while batch k+1 renders.  Every frame uses the same rig, so
 // the views take the scene's lights.
-int RenderBatches(MythTracer &mt, int W, int H, int first, int last, const char *out_dir, int per_call) {
+int RenderBatches(MythTracer &mt, int W, int H, int first, int last, const char *out_dir, int per_call, int samples_per_axis) {
   SetRig(mt);
   std::vector<int> numbers;
   std::vector<Camera> cams;
@@ -75,7 +78,7 @@ int RenderBatches(MythTracer &mt, int W, int H, int first, int last, const char 
     const size_t count = std::min(cams.size() - begin, (size_t)per_call);
     const std::vector<Camera> batch(cams.begin() + (long)begin, cams.begin() + (long)(begin + count));
     printf("Rendering %zu frames.\n", count);
-    if (!mt.RayTraceBatchAsync(W, H, batch, nullptr, bufs[calls & 1])) return 1;
+    if (!mt.RayTraceBatchAsync(W, H, samples_per_axis, batch, nullptr, bufs[calls & 1])) return 1;
     if (pending_count > 0 && !write_batch(pending_begin, pending_count, bufs[(calls + 1) & 1])) return 1;  // overlaps the render
     if (!mt.Wait()) return 1;
     pending_begin = begin;
@@ -95,15 +98,20 @@ int RenderBatches(MythTracer &mt, int W, int H, int first, int last, const char 
 
 int main(int argc, char **argv) {
   if (argc < 2) {
-    puts("usage: mythtracer_local_b200 scene.obj [width height first_frame last_frame out_dir frames_per_call]");
+    puts("usage: mythtracer_local_b200 scene.obj [width height first_frame last_frame out_dir frames_per_call samples_per_axis]");
     return 1;
   }
   const int W = argc > 2 ? atoi(argv[2]) : 1920 / 4, H = argc > 3 ? atoi(argv[3]) : 1080 / 4;
   const int first = argc > 4 ? atoi(argv[4]) : 74, last = argc > 5 ? atoi(argv[5]) : 180;
   const char *out_dir = argc > 6 ? argv[6] : "anim";
   const int per_call = argc > 7 ? atoi(argv[7]) : 1;
+  const int samples = argc > 8 ? atoi(argv[8]) : 1;
   if (per_call < 1) {
     puts("frames_per_call must be >= 1");
+    return 1;
+  }
+  if (samples != 1 && samples != 2 && samples != 4 && samples != 8) {
+    puts("samples_per_axis must be 1, 2, 4 or 8");
     return 1;
   }
   printf("Creating %s/ directory\n", out_dir);
@@ -115,7 +123,7 @@ int main(int argc, char **argv) {
   const AABB aabb = mt.GetScene()->tree.GetAABB();
   printf("%f %f %f x %f %f %f\n", aabb.min.v[0], aabb.min.v[1], aabb.min.v[2], aabb.max.v[0], aabb.max.v[1], aabb.max.v[2]);
 
-  if (per_call > 1) return RenderBatches(mt, W, H, first, last, out_dir, per_call);
+  if (per_call > 1 || samples > 1) return RenderBatches(mt, W, H, first, last, out_dir, per_call, samples);
 
   // Two pinned frames in rotation: while frame k+1 renders (queued without waiting), frame k is written to disk.
   uint8_t *frames[2] = {MythTracer::AllocFrame(W, H), MythTracer::AllocFrame(W, H)};

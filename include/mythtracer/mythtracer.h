@@ -162,11 +162,21 @@ class MythTracer {
   // for every view.  RayTraceBatchAsync returns once the batch is queued (`out` pinned, from AllocFrames; Wait joins).
   bool RayTraceBatch(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
                      uint8_t *out) {
-    return RenderBatch(image_width, image_height, cams, lights, out, true);
+    return RenderBatch(image_width, image_height, 1, cams, lights, out, true);
   }
   bool RayTraceBatchAsync(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
                           uint8_t *pinned_out) {
-    return RenderBatch(image_width, image_height, cams, lights, pinned_out, false);
+    return RenderBatch(image_width, image_height, 1, cams, lights, pinned_out, false);
+  }
+  // Anti-aliased batches (mtb_render_batch_ss): samples_per_axis s = 1, 2, 4 or 8; every output pixel is the rounded
+  // mean of the s x s pixels of the same view rendered at (s*w) x (s*h).  `out` holds cams.size() * w * h * 3 bytes.
+  bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
+                     const std::vector<std::vector<Light>> *lights, uint8_t *out) {
+    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, out, true);
+  }
+  bool RayTraceBatchAsync(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
+                          const std::vector<std::vector<Light>> *lights, uint8_t *pinned_out) {
+    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, pinned_out, false);
   }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
   static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
@@ -182,8 +192,8 @@ class MythTracer {
   mtb_stats last_stats{};
 
  private:
-  bool RenderBatch(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
-                   uint8_t *out, bool synchronous) {
+  bool RenderBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
+                   const std::vector<std::vector<Light>> *lights, uint8_t *out, bool synchronous) {
     if (!was_scene_finalized) {
       puts("Finalizing tree.");
       if (!scene.tree.Finalize(&scene.materials, &scene.textures)) return false;
@@ -215,10 +225,11 @@ class MythTracer {
     }
     const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
     mtb_stats stats;
-    const int rc = synchronous ? mtb_render_batch(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
-                                                  max_recursion_level, out, &stats)
-                               : mtb_render_batch_async(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
-                                                        max_recursion_level, out);
+    // (samples_per_axis = 1: mtb_render_batch_ss is mtb_render_batch)
+    const int rc = synchronous ? mtb_render_batch_ss(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
+                                                     samples_per_axis, max_recursion_level, out, &stats)
+                               : mtb_render_batch_ss_async(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width,
+                                                           image_height, samples_per_axis, max_recursion_level, out);
     if (rc != MTB_OK) {
       fprintf(stderr, "error: %s\n", mtb_last_error(ctx));
       return false;

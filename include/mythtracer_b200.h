@@ -255,6 +255,24 @@ int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, 
 int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
                            int32_t n_lights, int image_w, int image_h, int max_depth, uint8_t *rgb_out);
 
+/* Supersampled (anti-aliased) batches: as mtb_render_batch, with s = samples_per_axis samples per axis of every
+ * output pixel.  With F the frame mtb_render_batch renders for the same view at (s*image_w) x (s*image_h), output
+ * pixel (x, y) channel c of a view is
+ *     (sum over i, j in 0..s-1 of F[s*y + j][s*x + i][c] + s*s/2) / (s*s)      (integer division)
+ * the mean of the reference's own quantised samples at its own sensor positions (no jitter), rounded half up.  The
+ * means are formed in the kernel: no high-resolution frame is stored and there is no second kernel.
+ *
+ * samples_per_axis: 1, 2, 4 or 8 (anything else: MTB_ERR_ARG); 1 is exactly mtb_render_batch.  s*image_w and
+ * s*image_h: at most 65536.  rgb_out: HOST, n_views * image_h * image_w * 3 bytes (output pixels), view-major.
+ * stats: those of the (s*image_w) x (s*image_h) batch (rays and, under MTB_FLAG_COUNT_WORK, every work counter). */
+int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
+                        int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out,
+                        mtb_stats *stats);
+/* Same, returns once queued (rgb_out pinned, from mtb_host_alloc; mtb_wait joins). */
+int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
+                              int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                              uint8_t *rgb_out);
+
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the
  * context has one device.  This is the entry bench.py times for the HBM-resident figure. */

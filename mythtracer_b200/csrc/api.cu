@@ -1012,9 +1012,11 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 // launch per device (grid = tiles of a view x views of the device): the pipeline choice, the cost-aware tile order, the
 // hybrid split and the strip interleave are all single-frame machinery and none of their state is read or written.
 // lights == NULL: every view uses the context's lights.  Device g renders a contiguous range of views; the counts
-// differ by at most one.
+// differ by at most one.  ss > 1 (samples per axis, 2, 4 or 8): every view is traced on the (ss*W) x (ss*H) sample grid,
+// exactly as a batch of that size, and the kernel writes the W x H block means; everything else is as for ss = 1.
+constexpr int64_t kMaxSampleSide = 65536;  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
 int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
-                    int image_h, int max_depth, uint8_t *rgb_host, mtb_stats *stats, bool synchronous) {
+                    int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_stats *stats, bool synchronous) {
   const auto wall0 = std::chrono::steady_clock::now();
   if (ctx == nullptr) return MTB_ERR_ARG;
   if (ctx->dev.empty()) {
@@ -1041,21 +1043,30 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     ctx->err = "bad render arguments";
     return MTB_ERR_ARG;
   }
+  if (ss != 1 && ss != 2 && ss != 4 && ss != 8) {
+    ctx->err = "samples_per_axis must be 1, 2, 4 or 8 (the samples of an output pixel then lie in one 8x8 tile)";
+    return MTB_ERR_ARG;
+  }
+  if (ss > 1 && ((int64_t)image_w * ss > kMaxSampleSide || (int64_t)image_h * ss > kMaxSampleSide)) {
+    ctx->err = "the sample grid (samples_per_axis * image_w x samples_per_axis * image_h) must be at most 65536 on a side";
+    return MTB_ERR_ARG;
+  }
   if (ctx->part_index != 0 || ctx->part_count != 1) {
     ctx->err = "a batch renders whole views: the partition must be (0, 1)";
     return MTB_ERR_ARG;
   }
-  const size_t npx = (size_t)image_w * image_h;
+  const size_t npx = (size_t)image_w * image_h;  // output pixels of a view
+  const int grid_w = image_w * ss, grid_h = image_h * ss;  // its sample grid (the view itself when ss = 1)
   const bool debug_build = (ctx->flags & MTB_FLAG_COUNT_WORK) != 0;
   const int n_dev = (int)ctx->dev.size();
-  const int tiles_x = (image_w + 7) / 8, tiles_per_view = tiles_x * ((image_h + 7) / 8);
+  const int tiles_x = (grid_w + 7) / 8, tiles_per_view = tiles_x * ((grid_h + 7) / 8);
 
   // per-view records and the views' lights, view-major (the context's lights repeated when the caller passes none)
   const int32_t nl = lights != nullptr ? n_lights : (int32_t)ctx->lights.size();
   std::vector<mtb::ViewRec> views((size_t)n_views);
   std::vector<mtb_light> view_lights((size_t)n_views * nl);
   for (int32_t v = 0; v < n_views; v++) {
-    mtb::ComputeSensor(cams[v], image_w, image_h, views[(size_t)v].sensor);
+    mtb::ComputeSensor(cams[v], grid_w, grid_h, views[(size_t)v].sensor);
     for (int a = 0; a < 3; a++) views[(size_t)v].origin[a] = cams[v].origin[a];
     const mtb_light *src = lights != nullptr ? lights + (size_t)v * nl : ctx->lights.data();
     if (nl > 0) std::copy(src, src + nl, view_lights.begin() + (size_t)v * nl);
@@ -1063,16 +1074,18 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
 
   mtb::RenderParams rp;
   memset(&rp, 0, sizeof(rp));
-  rp.image_w = rp.chunk_w = image_w;
-  rp.image_h = rp.chunk_h = image_h;
+  rp.image_w = rp.chunk_w = grid_w;
+  rp.image_h = rp.chunk_h = grid_h;
   rp.max_depth = max_depth;
   rp.tiles_x = tiles_x;
   rp.strip_stride = 1;
 
   // Where the pixels go: a single device stores straight into a mapped pinned rgb_host (RenderImpl's rule); otherwise
-  // every device renders into its own frames and copies its views to their slice of rgb_host.
+  // every device renders into its own frames and copies its views to their slice of rgb_host.  Supersampled views always
+  // take the second way: their epilogue stores single bytes, and a direct store of those into mapped host memory has
+  // not been measured against the copy (which moves 1/ss^2 of the samples' bytes).
   uint8_t *host_direct = nullptr;
-  if (n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
+  if (ss == 1 && n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
     MTB_CUDA(ctx, cudaSetDevice(ctx->dev[0].device));
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer != nullptr) {
@@ -1114,7 +1127,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
       MTB_CUDA(ctx, cudaMemsetAsync(d.counters.ptr, 0, mtb::kNumCounters * sizeof(unsigned long long), s));
     }
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_start, s));
-    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, debug_build, s);
+    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, debug_build, s);
     ctx->launches++;
     MTB_CUDA(ctx, cudaGetLastError());
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_stop, s));
@@ -1493,12 +1506,22 @@ int mtb_render_chunk_async(mtb_context *ctx, const mtb_camera *cam, int image_w,
 
 int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                      int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, max_depth, rgb_out, stats, true);
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, stats, true);
 }
 
 int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, max_depth, rgb_out, nullptr, false);
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, false);
+}
+
+int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
+                        int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, stats, true);
+}
+
+int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
+                              int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, false);
 }
 
 int mtb_wait(mtb_context *ctx) {

@@ -153,8 +153,11 @@ void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_block
 // n_views whole frames in one launch: grid (tiles_per_view, n_views), camera of view v = views[v] (device memory), its
 // lights sc.lights + v * sc.n_lights, its pixels rp.rgb + v * chunk_w * chunk_h * 3.  rp.strip_first = 0,
 // rp.strip_stride = 1, and tile_order / tile_cost / heavy_k / run_if / taps / dbg NULL.
-void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views, bool debug_build,
-                           cudaStream_t stream);
+// samples_per_axis s = 2, 4 or 8: supersampled views.  rp.chunk_w x rp.chunk_h (and views[v].sensor) describe the
+// s*W x s*H sample grid, tiles_per_view counts its tiles, and view v's W x H output pixels (each the rounded mean of
+// its s x s samples) go to rp.rgb + v * W * H * 3.  s = 1: the plain batch above.
+void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
+                           int samples_per_axis, bool debug_build, cudaStream_t stream);
 void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, int mode, cudaStream_t stream);  // mode 0: one ray per thread, 1: two rays per lane (Trace2), 2: chain (TraceChain), 3: two calls
 
 }  // namespace mtb

@@ -86,14 +86,82 @@ __device__ __forceinline__ uint8_t *ViewFrame(const RenderParams &rp) {
   return BATCH ? rp.rgb + (size_t)blockIdx.y * rp.chunk_w * rp.chunk_h * 3 : rp.rgb;
 }
 
+// Supersampled batch (SS = 2, 4, 8 samples per axis): the tile is a tile of the (SS*W) x (SS*H) sample grid (rp.chunk_w
+// x rp.chunk_h), every thread traces one sample exactly as a pixel of that frame, and the epilogue writes the
+// (8/SS)^2 output pixels of the tile, each the rounded mean of its SS x SS quantised samples, to view-major W x H frames.
+// W = chunk_w / SS: the sample grid's sides are multiples of SS, so an output pixel inside the frame has all its samples
+// live, and its SS x SS block never straddles a tile (SS divides 8).
+//
+// SS = 2 and 4: a warp (8x4 samples) holds whole blocks, so the sum stays warp-level like the plain epilogue.
+// SS = 8: the one output pixel of a tile spans both warps.  Each warp reduces its 32 samples with shuffles; the warp
+// that finishes first leaves its partial sums in shared memory and exits, the last one adds them and stores the pixel.
+// A block barrier there instead holds the first warp's slot until the other is done: 1.3 % more kernel time for 16 C3
+// views at 240x135 (B200, DESIGN.md section 13).
+template <int SS>
+__device__ __forceinline__ void SupersampleEpilogue(const RenderParams &rp, const unsigned char *s_rgb, int tile_id, int strip,
+                                                    unsigned *s_ss8) {
+  const int out_w = rp.chunk_w / SS, out_h = rp.chunk_h / SS;
+  uint8_t *frame = rp.rgb + (size_t)blockIdx.y * out_w * out_h * 3;
+  const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  if constexpr (SS == 8) {
+    // the tile is one output pixel, and every sample of it is live (tiles_x = W, 8 rows of tiles per output row)
+    const unsigned char *mine = s_rgb + threadIdx.x * 3;
+    unsigned r = mine[0], g = mine[1], b = mine[2];
+    for (int off = 16; off > 0; off >>= 1) {
+      r += __shfl_down_sync(0xffffffffu, r, off);
+      g += __shfl_down_sync(0xffffffffu, g, off);
+      b += __shfl_down_sync(0xffffffffu, b, off);
+    }
+    // s_ss8: [0] warps done (zeroed before the trace), [1 + 3 * warp ..] that warp's three sums
+    volatile unsigned *part = s_ss8 + 1;
+    if (lane == 0u) {
+      part[warp * 3 + 0] = r;
+      part[warp * 3 + 1] = g;
+      part[warp * 3 + 2] = b;
+      __threadfence_block();
+      if (atomicAdd(s_ss8, 1u) == 1u) {  // the other warp's sums are in place
+        __threadfence_block();
+        const unsigned o = (warp ^ 1u) * 3;
+        uint8_t *dst = frame + (size_t)tile_id * 3;  // tile (x, y) = output pixel (x, y): tiles_x = out_w
+        dst[0] = (uint8_t)((r + part[o + 0] + 32u) >> 6);
+        dst[1] = (uint8_t)((g + part[o + 1] + 32u) >> 6);
+        dst[2] = (uint8_t)((b + part[o + 2] + 32u) >> 6);
+      }
+    }
+  } else {
+    // this warp's 8x4 samples = (8/SS) x (4/SS) output pixels; one lane per output channel
+    constexpr int kCols = kTile / SS, kRows = 4 / SS;
+    if (lane >= (unsigned)(kCols * kRows * 3)) return;
+    const int k = (int)lane / 3, c = (int)lane % 3, i = k % kCols, j = k / kCols;
+    const int ox = (tile_id % rp.tiles_x) * kCols + i, oy = (strip * kTile + (int)warp * 4) / SS + j;
+    if (ox >= out_w || oy >= out_h) return;
+    const unsigned char *src = s_rgb + warp * (4 * kTile * 3) + (j * SS * kTile + i * SS) * 3 + c;
+    unsigned sum = 0;
+#pragma unroll
+    for (int a = 0; a < SS; a++) {
+#pragma unroll
+      for (int b = 0; b < SS; b++) sum += src[(a * kTile + b) * 3];
+    }
+    frame[((size_t)oy * out_w + ox) * 3 + c] = (uint8_t)((sum + SS * SS / 2) / (SS * SS));
+  }
+}
+
 // BATCH: grid (tiles per view, views), block b of row v renders tile b of view v in scanline order; the camera comes from
 // views[v] and the pixels go to rp.rgb + v * chunk_w * chunk_h * 3.  A batch launch passes NULL for tile_order,
 // tile_cost, heavy_k, run_if and the taps / debug planes.  Without BATCH, `views` is unused and every `BATCH ? :`
-// folds away: the single-view kernels compile to the code they had before the batch form existed.
-template <bool DBG, bool BATCH>
+// folds away: the single-view kernels compile to the code they had before the batch form existed.  SS > 1 (BATCH only):
+// the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.
+template <bool DBG, bool BATCH, int SS>
 __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(DeviceScene sc, RenderParams rp, const ViewRec *views) {
+  static_assert(SS == 1 || (BATCH && (SS == 2 || SS == 4 || SS == 8)), "supersampling is a batch form with 2, 4 or 8 samples per axis");
   MTB_DECLARE_FAST_CTX(kBlockThreads);
-  __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3];
+  // (SS = 8: 7 more words behind the samples for the epilogue's counter and partial sums)
+  __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3 + (SS == 8 ? 7 * 4 : 0)];
+  unsigned *const s_ss8 = reinterpret_cast<unsigned *>(s_rgb + kTile * kTile * 3);
+  if constexpr (SS == 8) {
+    if (threadIdx.x == 0) s_ss8[0] = 0u;
+    __syncthreads();  // (both warps start together: unlike a barrier after the trace, this holds nobody's slot)
+  }
   // repair launch of a wavefront frame whose queues did not overflow: nothing to do
   if (rp.run_if != nullptr && __ldg(rp.run_if) == 0u) return;
   // hybrid frame: the leading (most expensive) tiles of the order belong to the wavefront pipeline
@@ -400,7 +468,9 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
 #else
   __syncwarp();
 #endif
-  {
+  if constexpr (SS > 1) {
+    SupersampleEpilogue<SS>(rp, s_rgb, tile_id, strip, s_ss8);
+  } else {
     const int px0 = (tile_id % rp.tiles_x) * kTile, py0 = strip * kTile + (int)(threadIdx.x >> 5) * 4;
     const unsigned lane = threadIdx.x & 31u;
     const unsigned char *half = s_rgb + (threadIdx.x >> 5) * (4 * kTile * 3);
@@ -696,20 +766,31 @@ void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles,
 void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_blocks, bool debug_build, cudaStream_t stream) {
   if (n_blocks <= 0) return;
   if (debug_build) {
-    RenderMega<true, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr);
+    RenderMega<true, false, 1><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr);
   } else {
-    RenderMega<false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr);
+    RenderMega<false, false, 1><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr);
   }
 }
 
-void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views, bool debug_build,
-                           cudaStream_t stream) {
+template <int SS>
+void LaunchBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const dim3 &grid, bool debug_build, cudaStream_t stream) {
+  if (debug_build) {
+    RenderMega<true, true, SS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views);
+  } else {
+    RenderMega<false, true, SS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views);
+  }
+}
+
+void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
+                           int samples_per_axis, bool debug_build, cudaStream_t stream) {
   if (tiles_per_view <= 0 || n_views <= 0) return;
   const dim3 grid((unsigned)tiles_per_view, (unsigned)n_views);
-  if (debug_build) {
-    RenderMega<true, true><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views);
-  } else {
-    RenderMega<false, true><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views);
+  switch (samples_per_axis) {
+    case 1: LaunchBatch<1>(sc, rp, views, grid, debug_build, stream); break;
+    case 2: LaunchBatch<2>(sc, rp, views, grid, debug_build, stream); break;
+    case 4: LaunchBatch<4>(sc, rp, views, grid, debug_build, stream); break;
+    case 8: LaunchBatch<8>(sc, rp, views, grid, debug_build, stream); break;
+    default: break;  // (the host API admits 1, 2, 4 and 8 only)
   }
 }
 

@@ -1,11 +1,13 @@
-"""Compares the SASS of the single-view megakernel of two source trees, ignoring symbol names.
+"""Compares the SASS of the megakernel of two source trees, ignoring symbol names.
 
     python tools/sass_compare.py OLD_TREE [NEW_TREE]      (NEW_TREE defaults to this repository)
 
 Compiles csrc/megakernel.cu of both trees for sm_100a with the library's flags (no GPU needed), dumps the SASS with
-cuobjdump and compares the instruction listings of RenderMega<DBG> (a tree from before the batch form) or
-RenderMega<DBG, false> (a tree with it), for DBG = false and true.  Also prints ptxas' registers / stack / spill figures
-of every RenderMega instantiation.  Exit status 0 when the listings are identical.
+cuobjdump and compares the instruction listings of RenderMega<DBG, BATCH> (RenderMega<DBG, BATCH, 1> in a tree with
+the supersampled batch) for DBG and BATCH = false and true.  A tree from before the batch form only has the single-view
+kernel, RenderMega<DBG>, which is then compared with BATCH = false alone.  Also prints ptxas' registers / stack / spill
+figures of every RenderMega instantiation, the supersampled ones (SS = 2, 4, 8) included.  Exit status 0 when the
+listings are identical.
 """
 import os
 import re
@@ -46,11 +48,13 @@ def _functions(sass):
     return funcs
 
 
-def _single_view(funcs, dbg):
+def _instantiation(funcs, dbg, batch):
+    """(name, code) of RenderMega<dbg, batch> (<dbg, batch, 1>; <dbg> stands for <dbg, false>), or None."""
+    patterns = [r"RenderMegaILb%dELb%dE(Li1E)?EEv" % (dbg, batch)] + ([r"RenderMegaILb%dEEEv" % dbg] if not batch else [])
     for name, code in funcs.items():
-        if re.search(r"RenderMegaILb%dEEEv" % dbg, name) or re.search(r"RenderMegaILb%dELb0EEEv" % dbg, name):
+        if any(re.search(p, name) for p in patterns):
             return name, code
-    raise SystemExit("no single-view RenderMega<%d> in the listing" % dbg)
+    return None
 
 
 def main():
@@ -67,16 +71,26 @@ def main():
         for name, fig in _ptxas_figures(log).items():
             print("%s %s %s" % (label, re.search(r"RenderMega\w*?E(?=EvN)", name).group(0), fig))
     old_f, new_f = _functions(old_sass), _functions(new_sass)
-    for dbg in (0, 1):
-        (on, oc), (nn, nc) = _single_view(old_f, dbg), _single_view(new_f, dbg)
-        equal = oc == nc
-        same &= equal
-        print("RenderMega<DBG=%d> single view: %d vs %d instructions, %s" % (dbg, len(oc), len(nc), "identical" if equal else "DIFFERENT"))
-        if not equal:
-            for i, (a, b) in enumerate(zip(oc, nc)):
-                if a != b:
-                    print("  first difference at instruction %d: %s | %s" % (i, a, b))
-                    break
+    for batch in (0, 1):
+        for dbg in (0, 1):
+            old, new = _instantiation(old_f, dbg, batch), _instantiation(new_f, dbg, batch)
+            if new is None:
+                raise SystemExit("no RenderMega<%d, %d> in the listing of %s" % (dbg, batch, new_tree))
+            if old is None:
+                if not batch:
+                    raise SystemExit("no single-view RenderMega<%d> in the listing of %s" % (dbg, old_tree))
+                print("RenderMega<DBG=%d, BATCH=1>: not in %s" % (dbg, old_tree))
+                continue
+            (on, oc), (nn, nc) = old, new
+            equal = oc == nc
+            same &= equal
+            print("RenderMega<DBG=%d, BATCH=%d>: %d vs %d instructions, %s" % (dbg, batch, len(oc), len(nc),
+                                                                             "identical" if equal else "DIFFERENT"))
+            if not equal:
+                for i, (a, b) in enumerate(zip(oc, nc)):
+                    if a != b:
+                        print("  first difference at instruction %d: %s | %s" % (i, a, b))
+                        break
     sys.exit(0 if same else 1)
 
 
