@@ -119,18 +119,18 @@ typedef struct {
 
 #define MTB_FLAG_COUNT_WORK 1u   /* fill the n_* work counters (counting kernels) */
 #define MTB_FLAG_NO_LIST_BVH 2u  /* scan every node list linearly, like the reference (A/B measurements) */
-/* Pipeline choice.  With none of the three bits set the library decides at run time: on the first frames of a
+/* Pipeline choice.  With none of the pipeline bits set the library decides at run time: on the first frames of a
  * given geometry (chunk size, partition, depth, light count) it times the per-pixel megakernel (second frame, once
- * its cost-aware tile order is warm), the wavefront pipeline (fourth frame, once its buffers exist) and the hybrid
- * split (frames 5 to 12, while the split settles; the last one is timed) and keeps the fastest from frame 13 on.  All three produce identical bytes, so the
- * choice is invisible in the output (DESIGN.md section 6). */
-#define MTB_FLAG_WAVEFRONT 4u    /* force the wavefront pipeline */
+ * its cost-aware tile order is warm) and the queue pipeline (fourth frame, once its buffers exist) and keeps the
+ * faster from frame 5 on.  Both produce identical bytes, so the choice is invisible in the output (DESIGN.md
+ * section 6). */
 #define MTB_FLAG_MEGAKERNEL 16u  /* force the per-pixel megakernel */
 #define MTB_FLAG_QUEUE 8192u     /* force the queue pipeline: the wavefront as ONE persistent kernel over a single device-side ray queue (all levels) */
-#define MTB_FLAG_HYBRID 2048u    /* force hybrid frames: the tiles that were most expensive in the previous frame go through the wavefront, the rest through the megakernel, concurrently */
+#define MTB_FLAG_WAVEFRONT 4u    /* the same as MTB_FLAG_QUEUE: the queue pipeline is the wavefront's only form */
 #define MTB_FLAG_EXACT_OCTREE 128u /* every regular ray walks the octree in the reference's recursion order (no certified fast traversal) */
-/* Retired A/B forms of round 1 (all bit-identical, all measured slower on B200; DESIGN.md section 5 keeps the
- * numbers).  The bits are still accepted and ignored, so callers that set them keep working. */
+/* Retired forms (all bit-identical, all measured slower on B200; DESIGN.md sections 5 and 6 keep the numbers).  The
+ * bits are still accepted and ignored, so callers that set them keep working. */
+#define MTB_FLAG_HYBRID 2048u     /* was: hybrid frames, the most expensive tiles through the level-by-level wavefront, the rest through the megakernel */
 #define MTB_FLAG_RAY_SORT 8u      /* was: wavefront, counting-sort every queue by origin cell + direction octant */
 #define MTB_FLAG_PACKING 256u     /* was: megakernel, block-level ray packing on 16x8 tiles */
 #define MTB_FLAG_RESUME 1024u     /* was: megakernel, suspendable walks */
@@ -238,7 +238,7 @@ void mtb_host_free(void *p);
 
 /* Batches: N whole frames of one scene, one camera and one light set per view, in one launch per device (an orbit, a
  * camera path, a light sweep, many small views: a 480x270 frame is less than one wave of the B200, a batch of them
- * fills the machine).  Always the per-pixel megakernel: the pipeline bits (MTB_FLAG_WAVEFRONT, _QUEUE, _HYBRID,
+ * fills the machine).  Always the per-pixel megakernel: the pipeline bits (MTB_FLAG_WAVEFRONT, _QUEUE,
  * _MEGAKERNEL) are ignored; MTB_FLAG_COUNT_WORK and the traversal flags apply as for a single frame.  The bytes of view
  * v equal those of mtb_render_chunk with cams[v] and view v's lights.  A batch leaves the state of the single-frame
  * path alone (the context's lights, the automatic pipeline choice, the tile order).  With several devices, device g
@@ -298,12 +298,11 @@ int mtb_frame_read(mtb_context *ctx, const void *d_ptr, size_t offset, size_t by
  * read; synchronises every device of the context and resets the counters. */
 int mtb_read_counters(mtb_context *ctx, mtb_stats *stats);
 
-/* Pipeline in use on device 0: 0 = megakernel, 1 = wavefront (level by level; only when forced), 2 = hybrid,
- * 3 = queue pipeline (the wavefront candidate of the automatic choice), -1 = still measuring; the timed megakernel /
- * queue-pipeline frames (ms) of the automatic choice are returned when the pointers are non-NULL. */
+/* Pipeline in use on device 0: 0 = megakernel, 3 = queue pipeline, -1 = still measuring (codes 1 and 2 belonged to
+ * retired pipelines); the timed megakernel / queue-pipeline frames (ms) of the automatic choice are returned when the
+ * pointers are non-NULL. */
 int mtb_pipeline_in_use(const mtb_context *ctx, float *mega_ms, float *wavefront_ms);
-/* Hybrid frames: the share of the frame's rays that currently goes through the wavefront on device 0 (steered frame by
- * frame from the measured times of the two halves). */
+/* Retired with hybrid frames: always 0.0f.  Kept so that callers built against earlier versions still link. */
 float mtb_hybrid_share(const mtb_context *ctx);
 /* Number of kernels of this library launched on this context so far (bench.py's gpu_launches). */
 uint64_t mtb_launch_count(const mtb_context *ctx);

@@ -32,7 +32,7 @@ LIB_PATH = os.environ.get("MTB_LIB_PATH", os.path.join(HERE, "libmythtracer_b200
 MTB_OK = 0
 MTB_FLAG_COUNT_WORK = 1
 MTB_FLAG_NO_LIST_BVH = 2
-MTB_FLAG_WAVEFRONT = 4
+MTB_FLAG_WAVEFRONT = 4  # the same as MTB_FLAG_QUEUE
 MTB_FLAG_RAY_SORT = 8
 MTB_FLAG_MEGAKERNEL = 16
 MTB_FLAG_NO_TILE_ORDER = 32
@@ -41,7 +41,7 @@ MTB_FLAG_EXACT_OCTREE = 128
 MTB_FLAG_PACKING = 256
 MTB_FLAG_WARP_SYNC = 512
 MTB_FLAG_RESUME = 1024
-MTB_FLAG_HYBRID = 2048
+MTB_FLAG_HYBRID = 2048  # retired: accepted and ignored
 MTB_FLAG_DEVICE_BVH = 4096
 MTB_FLAG_QUEUE = 8192
 MTB_FLAG_PAIR_RAYS = 16384
@@ -142,8 +142,6 @@ def load_library():
     lib.mtb_intersect_rays.argtypes = [vp, i64, vp, vp, vp, vp, vp, vp]
     lib.mtb_camera_sensor.argtypes = [vp, i32, i32, vp]
     lib.mtb_wait.argtypes = [vp]
-    lib.mtb_hybrid_share.argtypes = [vp]
-    lib.mtb_hybrid_share.restype = ctypes.c_float
     lib.mtb_load_timing.argtypes = [vp, vp]
     lib.mtb_frame_create.argtypes = [vp, ctypes.c_size_t, ctypes.POINTER(vp), vp]
     lib.mtb_frame_open.argtypes = [vp, vp, ctypes.POINTER(vp)]
@@ -566,14 +564,15 @@ class MythTracer:
         return out
 
     def pipeline_in_use(self):
-        """('mega' | 'wavefront' | 'hybrid' | 'queue' | 'measuring', mega_ms, queue_ms) on device 0."""
+        """('mega' | 'queue' | 'measuring', mega_ms, queue_ms) on device 0."""
         a, b = ctypes.c_float(0), ctypes.c_float(0)
         rc = self._lib.mtb_pipeline_in_use(self._ctx, ctypes.cast(ctypes.byref(a), ctypes.c_void_p),
                                            ctypes.cast(ctypes.byref(b), ctypes.c_void_p))
-        return {0: "mega", 1: "wavefront", 2: "hybrid", 3: "queue"}.get(rc, "measuring"), a.value, b.value
+        return {0: "mega", 3: "queue"}.get(rc, "measuring"), a.value, b.value
 
     def hybrid_share(self) -> float:
-        return float(self._lib.mtb_hybrid_share(self._ctx))
+        """Retired with hybrid frames: always 0.0."""
+        return 0.0
 
     def launch_count(self) -> int:
         return int(self._lib.mtb_launch_count(self._ctx))

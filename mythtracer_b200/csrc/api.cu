@@ -100,17 +100,11 @@ struct DeviceState {
   DeviceBuffer<int32_t> tile_order;
   long long tile_signature = -1;  // geometry the costs were recorded for
   // run-time choice between the two pipelines (flags without a pipeline bit): both are timed once per
-  // geometry (megakernel with a warm tile order, then wavefront) and the faster one is kept
+  // geometry (megakernel with a warm tile order, then the queue pipeline) and the faster one is kept
   long long tune_signature = -1;
-  int tune_stage = 0;           // see RenderImpl
-  float tune_ms[3] = {0.f, 0.f, 0.f};  // megakernel, wavefront, hybrid
-  int tune_choice = 0;                 // 0 megakernel, 1 wavefront, 2 hybrid
-  // hybrid frames: the most expensive tiles go through the wavefront while the megakernel renders the rest
-  DeviceBuffer<int32_t> heavy_k;
-  cudaStream_t hybrid_stream = nullptr;
-  cudaEvent_t ev_split = nullptr, ev_mega_done = nullptr, ev_wf_done = nullptr;  // (timed: they steer the split)
-  float hybrid_share = 0.30f;     // share of the frame's rays that goes through the wavefront; steered frame by frame
-  bool hybrid_timed = false;      // the three events above were recorded by the previous hybrid frame
+  int tune_stage = 0;              // see RenderImpl
+  float tune_ms[2] = {0.f, 0.f};   // megakernel, queue pipeline
+  bool tune_queue = false;         // the decision: the queue pipeline (else the megakernel)
   // batch launches (RenderBatchImpl): view records, per-view lights and the views' frames of this device, and the
   // events that time them (the single-frame events steer the automatic pipeline choice and are left alone)
   DeviceBuffer<mtb::ViewRec> batch_views;
@@ -121,71 +115,32 @@ struct DeviceState {
   DeviceBuffer<double> q_origins, q_dirs, q_t, q_point;
   DeviceBuffer<int32_t> q_tri;
   // wavefront pipeline state (wavefront.cu)
-  DeviceBuffer<double> wf_rq_o[2], wf_rq_d[2], wf_rq_coef[2];
-  DeviceBuffer<unsigned long long> wf_rq_path[2];
-  DeviceBuffer<int32_t> wf_rq_pixel[2];
-  DeviceBuffer<unsigned char> wf_rq_inobj[2];
-  DeviceBuffer<double> wf_act_point, wf_act_normal, wf_act_surface, wf_act_reflected, wf_act_dir, wf_sh_power;
-  DeviceBuffer<uint32_t> wf_sh_flags;
-  DeviceBuffer<double> wf_act_color;
-  DeviceBuffer<int32_t> wf_act_refl, wf_act_refr, wf_act_mtl, wf_act_pixel;
+  DeviceBuffer<double> wf_act_point, wf_act_dir, wf_act_color, wf_act_coef;
+  DeviceBuffer<int32_t> wf_act_refl, wf_act_refr, wf_act_mtl, wf_act_pixel, wf_act_info;
   DeviceBuffer<unsigned long long> wf_act_path;
-  cudaStream_t wf_stream2 = nullptr;             // shadow / light kernels (side stream 0)
-  cudaStream_t wf_side[3] = {nullptr, nullptr, nullptr};  // further side streams: the shadow kernels of different levels are independent
-  cudaEvent_t wf_ev_side[4] = {nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t wf_ev_level[MTB_MAX_RAY_DEPTH + 2] = {};  // level L traced (main stream)
-  cudaEvent_t wf_ev_lit = nullptr;               // all lights folded (second stream)
-  DeviceBuffer<uint32_t> wf_level_n, wf_ctrl;
-  DeviceBuffer<double> wf_act_coef;       // queue pipeline (WfQueue)
-  DeviceBuffer<int32_t> wf_act_info;
-  DeviceBuffer<uint32_t> wf_act_ready, wf_qctl;
-  uint32_t wf_epoch = 0;                  // frame number of the queue pipeline: act_ready[id] == epoch marks a complete entry
+  DeviceBuffer<uint32_t> wf_ctrl, wf_act_ready, wf_qctl;
+  uint32_t wf_epoch = 0;                  // frame number: act_ready[id] == epoch marks a complete entry
   DeviceBuffer<unsigned long long> wf_work;
-  // pinned; written by WfCommit at the end of every frame (level counts, overflow flag, frame sequence number) and read
-  // by the host at the START of the next frame only: grid sizes and queue capacities follow the scene with one frame
-  // of delay and without a single host read-back while a frame is in flight
+  // pinned; written by WfCommit at the end of every frame (overflow flag, frame sequence number) and read by the host
+  // at the START of the next frame only: the table capacity follows the scene with one frame of delay and without a
+  // single host read-back while a frame is in flight
   uint32_t *wf_host = nullptr;
   uint32_t wf_seen_sequence = 0;
-  int wf_queue_factor = 2, wf_act_factor = 6;  // capacities in units of the pixel-slot count; doubled after an overflow
+  int wf_act_factor = 6;  // activation table capacity in units of the pixel-slot count; doubled after an overflow
   mtb::WfBuffers wf{};
 
   void FreeAll() {
     nodes.Free(); slots.Free(); shade.Free(); bvh.Free(); gnodes.Free(); gslots.Free(); list_order.Free(); slot_node.Free(); leaf_ref.Free(); ref_slot.Free(); materials.Free();
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
-    counters.Free(); tile_cost.Free(); tile_order.Free(); heavy_k.Free();
+    counters.Free(); tile_cost.Free(); tile_order.Free();
     batch_views.Free(); batch_lights.Free(); batch_rgb.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
     if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
     ev_batch_start = ev_batch_stop = nullptr;
-    if (hybrid_stream != nullptr) cudaStreamDestroy(hybrid_stream);
-    hybrid_stream = nullptr;
-    if (ev_split != nullptr) cudaEventDestroy(ev_split);
-    if (ev_mega_done != nullptr) cudaEventDestroy(ev_mega_done);
-    if (ev_wf_done != nullptr) cudaEventDestroy(ev_wf_done);
-    ev_split = ev_mega_done = ev_wf_done = nullptr; q_origins.Free(); q_dirs.Free(); q_t.Free(); q_point.Free(); q_tri.Free();
-    for (int k = 0; k < 2; k++) {
-      wf_rq_o[k].Free(); wf_rq_d[k].Free(); wf_rq_coef[k].Free(); wf_rq_path[k].Free(); wf_rq_pixel[k].Free();
-      wf_rq_inobj[k].Free();
-    }
-    wf_act_point.Free(); wf_act_normal.Free(); wf_act_surface.Free(); wf_act_reflected.Free(); wf_act_dir.Free();
-    wf_sh_power.Free(); wf_sh_flags.Free(); wf_act_color.Free(); wf_act_refl.Free(); wf_act_refr.Free();
-    wf_act_mtl.Free(); wf_act_pixel.Free(); wf_act_path.Free(); wf_level_n.Free(); wf_ctrl.Free(); wf_work.Free(); wf_act_coef.Free(); wf_act_info.Free(); wf_act_ready.Free(); wf_qctl.Free();
-    if (wf_stream2 != nullptr) cudaStreamDestroy(wf_stream2);
-    wf_stream2 = nullptr;
-    for (cudaStream_t &st : wf_side) {
-      if (st != nullptr) cudaStreamDestroy(st);
-      st = nullptr;
-    }
-    for (cudaEvent_t &e : wf_ev_side) {
-      if (e != nullptr) cudaEventDestroy(e);
-      e = nullptr;
-    }
-    for (cudaEvent_t &e : wf_ev_level) {
-      if (e != nullptr) cudaEventDestroy(e);
-      e = nullptr;
-    }
-    if (wf_ev_lit != nullptr) cudaEventDestroy(wf_ev_lit);
-    wf_ev_lit = nullptr;
+    q_origins.Free(); q_dirs.Free(); q_t.Free(); q_point.Free(); q_tri.Free();
+    wf_act_point.Free(); wf_act_dir.Free(); wf_act_color.Free(); wf_act_coef.Free(); wf_act_refl.Free(); wf_act_refr.Free();
+    wf_act_mtl.Free(); wf_act_pixel.Free(); wf_act_info.Free(); wf_act_path.Free(); wf_ctrl.Free(); wf_act_ready.Free(); wf_qctl.Free();
+    wf_work.Free();
     if (wf_host != nullptr) cudaFreeHost(wf_host);
     wf_host = nullptr;
   }
@@ -507,210 +462,81 @@ int GatherStrips(mtb_context *ctx, const StripPlan &plan, int owner, int chunk_w
   return MTB_OK;
 }
 
-// Sizes the wavefront buffers for `slots` pixel slots and the current light count.
-int EnsureWavefront(mtb_context *ctx, DeviceState *d, int slots, int n_lights) {
-  const size_t qcap = (size_t)slots * d->wf_queue_factor;
+// One frame (this device's strips) through the wavefront pipeline: one persistent kernel takes every activation of
+// every level from a single device-side ray queue (wavefront.cu, WfQueue), then the per-pixel fold.  Four launches and
+// the repair launch, nothing read back.  If the activation table overflows, the RenderMega launch queued at the end
+// renders the same tiles instead (same bytes); the host sees the overflow flag at the start of a later frame and
+// doubles the table.
+int RunWavefrontQueue(mtb_context *ctx, DeviceState *d, const mtb::RenderParams &p, int n_blocks, bool debug_build, cudaStream_t s) {
+  const int slots = n_blocks * 64;
+  if (slots <= 0) return MTB_OK;
+  // feedback of the frames completed so far (pinned memory written by WfCommit; a frame still in flight simply is not
+  // in it yet)
+  if (d->wf_host != nullptr) {
+    const uint32_t seq = d->wf_host[mtb::kWfHostSequence];
+    if (seq != d->wf_seen_sequence) {
+      d->wf_seen_sequence = seq;
+      if (d->wf_host[mtb::kWfHostOverflow] != 0u) d->wf_act_factor *= 2;
+    }
+  }
   const size_t acap = (size_t)slots * d->wf_act_factor;
-  if (qcap > 0x7fffffffull / 4 || acap > 0x7fffffffull / 4) {
+  if (acap > 0x7fffffffull / 4) {
     ctx->err = "wavefront buffers exceed the 32-bit index range";
     return MTB_ERR_LIMIT;
   }
-  for (int k = 0; k < 2; k++) {
-    MTB_CUDA(ctx, d->wf_rq_o[k].Reserve(qcap * 3));
-    MTB_CUDA(ctx, d->wf_rq_d[k].Reserve(qcap * 3));
-    MTB_CUDA(ctx, d->wf_rq_coef[k].Reserve(qcap));
-    MTB_CUDA(ctx, d->wf_rq_path[k].Reserve(qcap));
-    MTB_CUDA(ctx, d->wf_rq_pixel[k].Reserve(qcap));
-    MTB_CUDA(ctx, d->wf_rq_inobj[k].Reserve(qcap));
-    d->wf.rq_o[k] = d->wf_rq_o[k].ptr;
-    d->wf.rq_d[k] = d->wf_rq_d[k].ptr;
-    d->wf.rq_coef[k] = d->wf_rq_coef[k].ptr;
-    d->wf.rq_path[k] = d->wf_rq_path[k].ptr;
-    d->wf.rq_pixel[k] = d->wf_rq_pixel[k].ptr;
-    d->wf.rq_inobj[k] = d->wf_rq_inobj[k].ptr;
-  }
-  const size_t nl = (size_t)(n_lights > 0 ? n_lights : 1);
+  const uint32_t *ready_before = d->wf_act_ready.ptr;
   MTB_CUDA(ctx, d->wf_act_point.Reserve(acap * 3));
-  MTB_CUDA(ctx, d->wf_act_normal.Reserve(acap * 3));
-  MTB_CUDA(ctx, d->wf_act_surface.Reserve(acap * 3));
-  MTB_CUDA(ctx, d->wf_act_reflected.Reserve(acap * 3));
   MTB_CUDA(ctx, d->wf_act_dir.Reserve(acap * 3));
-  MTB_CUDA(ctx, d->wf_sh_power.Reserve(acap * 3 * nl));
-  MTB_CUDA(ctx, d->wf_sh_flags.Reserve(acap * nl));
   MTB_CUDA(ctx, d->wf_act_color.Reserve(acap * 3));
+  MTB_CUDA(ctx, d->wf_act_coef.Reserve(acap));
   MTB_CUDA(ctx, d->wf_act_refl.Reserve(acap));
   MTB_CUDA(ctx, d->wf_act_refr.Reserve(acap));
   MTB_CUDA(ctx, d->wf_act_mtl.Reserve(acap));
   MTB_CUDA(ctx, d->wf_act_pixel.Reserve(acap));
+  MTB_CUDA(ctx, d->wf_act_info.Reserve(acap));
   MTB_CUDA(ctx, d->wf_act_path.Reserve(acap));
-  if (d->wf_stream2 == nullptr) {
-    MTB_CUDA(ctx, cudaStreamCreateWithFlags(&d->wf_stream2, cudaStreamNonBlocking));
-    for (cudaStream_t &st : d->wf_side) MTB_CUDA(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    for (cudaEvent_t &e : d->wf_ev_side) MTB_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    for (cudaEvent_t &e : d->wf_ev_level) MTB_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    MTB_CUDA(ctx, cudaEventCreateWithFlags(&d->wf_ev_lit, cudaEventDisableTiming));
-  }
-  MTB_CUDA(ctx, d->wf_level_n.Reserve(MTB_MAX_RAY_DEPTH + 2));
+  MTB_CUDA(ctx, d->wf_act_ready.Reserve(acap));
+  MTB_CUDA(ctx, d->wf_qctl.Reserve(mtb::kQWords));
   MTB_CUDA(ctx, d->wf_ctrl.Reserve(2));
   MTB_CUDA(ctx, d->wf_work.Reserve(mtb::kNumCounters));
   if (d->wf_host == nullptr) {
     MTB_CUDA(ctx, cudaMallocHost(reinterpret_cast<void **>(&d->wf_host), mtb::kWfHostWords * sizeof(uint32_t)));
     memset(d->wf_host, 0, mtb::kWfHostWords * sizeof(uint32_t));
   }
-  d->wf.act_point = d->wf_act_point.ptr;
-  d->wf.act_normal = d->wf_act_normal.ptr;
-  d->wf.act_surface = d->wf_act_surface.ptr;
-  d->wf.act_reflected = d->wf_act_reflected.ptr;
-  d->wf.act_dir = d->wf_act_dir.ptr;
-  d->wf.sh_power = d->wf_sh_power.ptr;
-  d->wf.sh_flags = d->wf_sh_flags.ptr;
-  d->wf.act_color = d->wf_act_color.ptr;
-  d->wf.act_refl = d->wf_act_refl.ptr;
-  d->wf.act_refr = d->wf_act_refr.ptr;
-  d->wf.act_mtl = d->wf_act_mtl.ptr;
-  d->wf.act_pixel = d->wf_act_pixel.ptr;
-  d->wf.act_path = d->wf_act_path.ptr;
-  d->wf.level_n = d->wf_level_n.ptr;
-  d->wf.ctrl = d->wf_ctrl.ptr;
-  d->wf.work = d->wf_work.ptr;
-  d->wf.queue_cap = (int32_t)qcap;
-  d->wf.act_cap = (int32_t)acap;
-  return MTB_OK;
-}
-
-// One frame (this device's strips / its share of a hybrid frame) through the wavefront pipeline: every kernel of
-// every level is enqueued at once, nothing is read back.  How many rays a level holds is only known on the device;
-// the grids are sized from the counts of the last completed frame of the same size (+25 %), else from the capacity
-// bound, and the kernels loop grid-strided over the real count.  If a queue overflows, the kernels of the remaining
-// levels exit at once and the RenderMega launch queued at the end renders the same tiles instead (same bytes); the
-// host sees the overflow flag at the start of the next frame and doubles the queues.
-int RunWavefront(mtb_context *ctx, DeviceState *d, const mtb::RenderParams &p, int n_blocks, bool debug_build,
-                 cudaStream_t s) {
-  const int slots = n_blocks * 64;
-  if (slots <= 0) return MTB_OK;
-  // feedback of the frames completed so far (pinned memory written by WfCommit; a frame still in flight simply is not
-  // in it yet)
-  long long hint[MTB_MAX_RAY_DEPTH + 2];
-  bool have_hint = false;
-  if (d->wf_host != nullptr) {
-    const uint32_t seq = d->wf_host[mtb::kWfHostSequence];
-    if (seq != d->wf_seen_sequence) {
-      d->wf_seen_sequence = seq;
-      if (d->wf_host[mtb::kWfHostOverflow] != 0u) {
-        d->wf_queue_factor *= 2;
-        d->wf_act_factor *= 2;
-      }
-    }
-    if (seq != 0u && d->wf_host[mtb::kWfHostOverflow] == 0u && d->wf_host[0] == (uint32_t)slots) {
-      have_hint = true;
-      for (int l = 0; l <= MTB_MAX_RAY_DEPTH + 1; l++) hint[l] = (long long)d->wf_host[l];
-    }
-  }
-  const int rc = EnsureWavefront(ctx, d, slots, d->scene.n_lights);
-  if (rc != MTB_OK) return rc;
-  long long expect[MTB_MAX_RAY_DEPTH + 2];
-  for (int level = 0; level <= p.max_depth; level++) {
-    long long bound = level >= 24 ? (long long)d->wf.queue_cap : std::min<long long>((long long)d->wf.queue_cap, (long long)slots << level);
-    expect[level] = have_hint ? std::min(bound, hint[level] + hint[level] / 4 + 2048) : bound;
-  }
-  expect[0] = slots;
-  // Side streams: the shadow walks + Phong sums of level L only depend on the trace of level L, so the levels'
-  // side kernels go round-robin over four streams and overlap each other as well as the deeper traces (on a small
-  // share of a frame - one of 8 GPUs - every one of them is latency-bound and they were the critical path when
-  // serialised on one stream).
-  cudaStream_t side[4] = {d->wf_stream2, d->wf_side[0], d->wf_side[1], d->wf_side[2]};
-  mtb::LaunchWfBegin(d->wf, slots, s);
-  // they must not start before earlier work on the main stream (previous frame, taps memset, WfBegin)
-  MTB_CUDA(ctx, cudaEventRecord(d->wf_ev_lit, s));
-  for (cudaStream_t st : side) MTB_CUDA(ctx, cudaStreamWaitEvent(st, d->wf_ev_lit, 0));
-  for (int level = 0; level <= p.max_depth; level++) {
-    // critical path (main stream): trace the level and queue its children
-    mtb::LaunchWfTrace(d->scene, p, d->wf, level, expect[level], debug_build, s);
-    MTB_CUDA(ctx, cudaEventRecord(d->wf_ev_level[level], s));
-    // side branch: shadow walks and the Phong sums of this level
-    cudaStream_t s2 = side[level & 3];
-    MTB_CUDA(ctx, cudaStreamWaitEvent(s2, d->wf_ev_level[level], 0));
-    mtb::LaunchWfShadow(d->scene, p, d->wf, level, expect[level], debug_build, s2);
-    mtb::LaunchWfLight(d->scene, p, d->wf, level, expect[level], s2);
-    ctx->launches += 2u + (d->scene.n_lights > 0 ? 1u : 0u);
-  }
-  // join: the folds need every level's colours
-  for (int k = 0; k < 4; k++) {
-    MTB_CUDA(ctx, cudaEventRecord(d->wf_ev_side[k], side[k]));
-    MTB_CUDA(ctx, cudaStreamWaitEvent(s, d->wf_ev_side[k], 0));
-  }
-  for (int level = p.max_depth - 1; level >= 0; level--) {
-    mtb::LaunchWfFold(d->scene, d->wf, level, expect[level], s);
-    ctx->launches++;
-  }
-  mtb::LaunchWfResolve(p, d->wf, slots, s);
-  mtb::LaunchWfCommit(d->wf, p.counters, d->wf_host, s);
-  // the repair launch: a no-op (its blocks read one word and exit) unless a queue overflowed
-  mtb::RenderParams repair = p;
-  repair.run_if = d->wf.ctrl;
-  repair.mega_part = 1;
-  mtb::LaunchRenderMega(d->scene, repair, n_blocks, debug_build, s);
-  ctx->launches += 4u;  // WfBegin, WfResolve, WfCommit, repair
-  MTB_CUDA(ctx, cudaGetLastError());
-  return MTB_OK;
-}
-
-// One frame through the queue pipeline: one persistent kernel takes every activation of every level from a single
-// device-side ray queue (wavefront.cu, WfQueue), then the per-pixel fold.  Four launches, nothing read back; overflow
-// of the activation table is handled like in RunWavefront (repair launch, larger tables next frame).
-int RunWavefrontQueue(mtb_context *ctx, DeviceState *d, const mtb::RenderParams &p, int n_blocks, bool debug_build, cudaStream_t s) {
-  const int slots = n_blocks * 64;
-  if (slots <= 0) return MTB_OK;
-  if (d->wf_host != nullptr) {
-    const uint32_t seq = d->wf_host[mtb::kWfHostSequence];
-    if (seq != d->wf_seen_sequence) {
-      d->wf_seen_sequence = seq;
-      if (d->wf_host[mtb::kWfHostOverflow] != 0u) {
-        d->wf_queue_factor *= 2;
-        d->wf_act_factor *= 2;
-      }
-    }
-  }
-  const int rc = EnsureWavefront(ctx, d, slots, d->scene.n_lights);
-  if (rc != MTB_OK) return rc;
-  const size_t acap = (size_t)d->wf.act_cap;
-  const uint32_t *ready_before = d->wf_act_ready.ptr;
-  MTB_CUDA(ctx, d->wf_act_coef.Reserve(acap));
-  MTB_CUDA(ctx, d->wf_act_info.Reserve(acap));
-  MTB_CUDA(ctx, d->wf_act_ready.Reserve(acap));
-  MTB_CUDA(ctx, d->wf_qctl.Reserve(mtb::kQWords));
   if (d->wf_act_ready.ptr != ready_before || d->wf_epoch == 0xffffffffu) {
     MTB_CUDA(ctx, cudaMemsetAsync(d->wf_act_ready.ptr, 0, d->wf_act_ready.count * sizeof(uint32_t), s));
     d->wf_epoch = 0;
   }
   d->wf_epoch++;
+  d->wf.act_point = d->wf_act_point.ptr;
+  d->wf.act_dir = d->wf_act_dir.ptr;
+  d->wf.act_color = d->wf_act_color.ptr;
   d->wf.act_coef = d->wf_act_coef.ptr;
+  d->wf.act_refl = d->wf_act_refl.ptr;
+  d->wf.act_refr = d->wf_act_refr.ptr;
+  d->wf.act_mtl = d->wf_act_mtl.ptr;
+  d->wf.act_pixel = d->wf_act_pixel.ptr;
   d->wf.act_info = d->wf_act_info.ptr;
+  d->wf.act_path = d->wf_act_path.ptr;
   d->wf.act_ready = d->wf_act_ready.ptr;
   d->wf.qctl = d->wf_qctl.ptr;
+  d->wf.ctrl = d->wf_ctrl.ptr;
+  d->wf.work = d->wf_work.ptr;
+  d->wf.act_cap = (int32_t)acap;
   mtb::LaunchWfQueueBegin(d->wf, slots, s);
   mtb::LaunchWfQueue(d->scene, p, d->wf, slots, d->wf_epoch, d->sm_count, debug_build, s);
   mtb::LaunchWfResolveTree(d->scene, p, d->wf, slots, s);
   mtb::LaunchWfCommit(d->wf, p.counters, d->wf_host, s);
+  // the repair launch: a no-op (its blocks read one word and exit) unless the table overflowed
   mtb::RenderParams repair = p;
   repair.run_if = d->wf.ctrl;
-  repair.mega_part = 1;
   mtb::LaunchRenderMega(d->scene, repair, n_blocks, debug_build, s);
   ctx->launches += 5u;
   MTB_CUDA(ctx, cudaGetLastError());
   return MTB_OK;
 }
 
-// Hybrid frames: which tiles go through the wavefront.  The megakernel's critical path is its most expensive pixel
-// (a serial chain of up to ~80 rays), the wavefront's is one ray per level but it pays ~1.3x the instructions, so the
-// most expensive tiles of the previous frame go to the wavefront and the rest to the megakernel, concurrently.  How
-// much is not a constant: round 1 used two fixed rules picked from a table measured on C3; now the share of the
-// frame's rays that the wavefront gets is STEERED - both halves are timed with events, and the share moves a step
-// towards whichever half finished first (no host wait: the events of the previous frame are only read if they have
-// completed).  At most half of the tiles can go to the wavefront (its queues are sized for that).
-constexpr int kTuneDecided = 13;  // frames 5..12 of a new geometry are hybrid frames
-constexpr float kHybridShareMin = 0.02f, kHybridShareMax = 0.90f, kHybridShareStep = 0.04f;
-int HybridMaxTiles(int tiles) { return tiles / 2; }
+constexpr int kTuneDecided = 5;  // frames 1..4 of a new geometry measure the two pipelines
 
 // Core of both render entry points.  d_rgb_user: device-0 buffer to leave the pixels in (may be NULL when
 // rgb_host is given); user_stream: stream of device 0 to enqueue on (NULL = context stream).
@@ -788,7 +614,7 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
     p.strip_first = owner;
     // Where the pixels go.  Device 0: the caller's device buffer, or the context's frame.  Other devices: straight
     // into device 0's frame through its peer mapping when there is one (RenderMega leaves whole tile rows as aligned
-    // 8-byte stores, WfResolve likewise) - the in-box BlitWorkChunk (main_net_master.cc:223-236) costs no copy then -
+    // 8-byte stores, WfResolveTree likewise) - the in-box BlitWorkChunk (main_net_master.cc:223-236) costs no copy then -
     // else into an own frame that device 0 gathers with one pitched peer copy.
     if (g == 0) {
       p.rgb = rgb_target;
@@ -819,35 +645,25 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
     // a peer's scratch frame must not be overwritten while device 0 still gathers the previous one
     if (g > 0) MTB_CUDA(ctx, cudaStreamWaitEvent(s, ctx->dev[0].ev_gathered, 0));
     bool wavefront = (ctx->flags & (MTB_FLAG_WAVEFRONT | MTB_FLAG_QUEUE)) != 0;
-    bool queue = (ctx->flags & MTB_FLAG_QUEUE) != 0;  // the wavefront as one persistent kernel over a ray queue
-    bool hybrid = (ctx->flags & MTB_FLAG_HYBRID) != 0 && !wavefront;
-    if ((ctx->flags & (MTB_FLAG_WAVEFRONT | MTB_FLAG_QUEUE | MTB_FLAG_MEGAKERNEL | MTB_FLAG_HYBRID)) == 0 && blocks > 0) {
+    if ((ctx->flags & (MTB_FLAG_WAVEFRONT | MTB_FLAG_QUEUE | MTB_FLAG_MEGAKERNEL)) == 0 && blocks > 0) {
       // automatic: measure both pipelines on the first frames of this geometry, then keep the faster
       const long long tsig = ((long long)chunk_w << 42) ^ ((long long)chunk_h << 24) ^ ((long long)owner << 12) ^
                              ((long long)plan.owners << 6) ^ ((long long)max_depth << 1) ^ ((long long)d.scene.n_lights << 50);
       if (tsig != d.tune_signature) {
         d.tune_signature = tsig;
         d.tune_stage = 0;
-      } else if (d.tune_stage == 2 || d.tune_stage == 4 || d.tune_stage == kTuneDecided - 1) {
+      } else if (d.tune_stage == 2 || d.tune_stage == 4) {
         // the previous frame was a timed one: harvest it
         float ms = 0.f;
         if (cudaEventSynchronize(d.ev_stop) == cudaSuccess && cudaEventElapsedTime(&ms, d.ev_start, d.ev_stop) == cudaSuccess) {
-          d.tune_ms[d.tune_stage == 2 ? 0 : (d.tune_stage == 4 ? 1 : 2)] = ms;
+          d.tune_ms[d.tune_stage == 2 ? 0 : 1] = ms;
         }
-        if (d.tune_stage == kTuneDecided - 1) {
-          d.tune_choice = 0;
-          if (d.tune_ms[1] < d.tune_ms[d.tune_choice]) d.tune_choice = 1;
-          if (d.tune_ms[2] < d.tune_ms[d.tune_choice]) d.tune_choice = 2;
-        }
+        if (d.tune_stage == 4) d.tune_queue = d.tune_ms[1] < d.tune_ms[0];
       }
       if (d.tune_stage < kTuneDecided) d.tune_stage++;
       // stage now: 1 = megakernel (cold tile order), 2 = megakernel (timed), 3 = queue pipeline (cold: buffers are
-      // allocated), 4 = queue pipeline (timed), 5 .. kTuneDecided - 1 = hybrid (the split settles; the last one is
-      // timed), kTuneDecided = decided.  (The wavefront candidate is its queue form: measured faster than the
-      // level-by-level form at every share of the C3 frame, DESIGN.md section 6.)
-      wavefront = d.tune_stage == 3 || d.tune_stage == 4 || (d.tune_stage == kTuneDecided && d.tune_choice == 1);
-      queue = wavefront;
-      hybrid = (d.tune_stage >= 5 && d.tune_stage < kTuneDecided) || (d.tune_stage == kTuneDecided && d.tune_choice == 2);
+      // allocated), 4 = queue pipeline (timed), kTuneDecided = decided
+      wavefront = d.tune_stage == 3 || d.tune_stage == 4 || (d.tune_stage == kTuneDecided && d.tune_queue);
     }
     if (ctx->l2_persist_mb > 0 && d.l2_window_stream != s) {
       ApplyL2Window(ctx, &d, s);
@@ -861,7 +677,7 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
         MTB_CUDA(ctx, cudaMemsetAsync(d.sig_shadow.ptr, 0, npx * 8, s));
         MTB_CUDA(ctx, cudaMemsetAsync(d.n_rays.ptr, 0, npx * 4, s));
       }
-      const int wrc = queue ? RunWavefrontQueue(ctx, &d, p, blocks, debug_build, s) : RunWavefront(ctx, &d, p, blocks, debug_build, s);
+      const int wrc = RunWavefrontQueue(ctx, &d, p, blocks, debug_build, s);
       if (wrc != MTB_OK) return wrc;
     } else {
       const int mblocks = blocks;
@@ -872,65 +688,18 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
         MTB_CUDA(ctx, d.tile_cost.Reserve((size_t)mblocks));
         MTB_CUDA(ctx, d.tile_order.Reserve((size_t)mblocks));
         p.tile_cost = d.tile_cost.ptr;
-        const bool split = hybrid && mblocks >= 64;
-        if (split) MTB_CUDA(ctx, d.heavy_k.Reserve(1));
-        if (split && d.hybrid_timed && d.ev_wf_done != nullptr && cudaEventQuery(d.ev_wf_done) == cudaSuccess &&
-            cudaEventQuery(d.ev_mega_done) == cudaSuccess) {
-          // steer the split with the previous hybrid frame: the half that took longer gives up work
-          float t_mega = 0.f, t_wf = 0.f;
-          if (cudaEventElapsedTime(&t_mega, d.ev_split, d.ev_mega_done) == cudaSuccess &&
-              cudaEventElapsedTime(&t_wf, d.ev_split, d.ev_wf_done) == cudaSuccess) {
-            if (t_wf > t_mega * 1.04f) d.hybrid_share -= kHybridShareStep;
-            if (t_mega > t_wf * 1.04f) d.hybrid_share += kHybridShareStep;
-            d.hybrid_share = std::min(kHybridShareMax, std::max(kHybridShareMin, d.hybrid_share));
-          }
-          cudaGetLastError();
-        }
         if (signature == d.tile_signature) {
-          mtb::LaunchBuildTileOrder(d.tile_cost.ptr, d.tile_order.ptr, mblocks, split ? d.heavy_k.ptr : nullptr, HybridMaxTiles(mblocks),
-                                    (unsigned)(d.hybrid_share * 65536.0f), s);
+          mtb::LaunchBuildTileOrder(d.tile_cost.ptr, d.tile_order.ptr, mblocks, s);
           ctx->launches++;
           p.tile_order = d.tile_order.ptr;
-          if (split) p.heavy_k = d.heavy_k.ptr;
         } else {
           MTB_CUDA(ctx, cudaMemsetAsync(d.tile_cost.ptr, 0, (size_t)mblocks * sizeof(uint32_t), s));
           d.tile_signature = signature;
-          d.hybrid_timed = false;
         }
       }
-      if (p.heavy_k != nullptr) {
-        // Hybrid frame.  The megakernel's critical path is its most expensive pixel (a serial chain of up to ~80
-        // rays), the wavefront's is one ray per level but it pays ~1.3x the instructions: so the tiles that were
-        // the most expensive in the previous frame (the first *heavy_k of the launch order, at most 1/8 of the tiles)
-        // go through the wavefront while the megakernel renders the rest on a second stream.  Both write their own
-        // pixels of the same buffers; the bytes do not depend on the split.
-        if (d.hybrid_stream == nullptr) {
-          MTB_CUDA(ctx, cudaStreamCreateWithFlags(&d.hybrid_stream, cudaStreamNonBlocking));
-          MTB_CUDA(ctx, cudaEventCreate(&d.ev_split));
-          MTB_CUDA(ctx, cudaEventCreate(&d.ev_mega_done));
-          MTB_CUDA(ctx, cudaEventCreate(&d.ev_wf_done));
-        }
-        if (want_taps) {  // the wavefront kernels accumulate the taps with atomics
-          MTB_CUDA(ctx, cudaMemsetAsync(d.sig_hits.ptr, 0, npx * 8, s));
-          MTB_CUDA(ctx, cudaMemsetAsync(d.sig_shadow.ptr, 0, npx * 8, s));
-          MTB_CUDA(ctx, cudaMemsetAsync(d.n_rays.ptr, 0, npx * 4, s));
-        }
-        MTB_CUDA(ctx, cudaEventRecord(d.ev_split, s));
-        MTB_CUDA(ctx, cudaStreamWaitEvent(d.hybrid_stream, d.ev_split, 0));
-        mtb::LaunchRenderMega(d.scene, p, mblocks, debug_build, d.hybrid_stream);
-        ctx->launches++;
-        MTB_CUDA(ctx, cudaGetLastError());
-        MTB_CUDA(ctx, cudaEventRecord(d.ev_mega_done, d.hybrid_stream));
-        const int wrc = RunWavefront(ctx, &d, p, HybridMaxTiles(mblocks), debug_build, s);
-        if (wrc != MTB_OK) return wrc;
-        MTB_CUDA(ctx, cudaEventRecord(d.ev_wf_done, s));
-        d.hybrid_timed = true;
-        MTB_CUDA(ctx, cudaStreamWaitEvent(s, d.ev_mega_done, 0));
-      } else {
-        mtb::LaunchRenderMega(d.scene, p, mblocks, debug_build, s);
-        if (mblocks > 0) ctx->launches++;
-        MTB_CUDA(ctx, cudaGetLastError());
-      }
+      mtb::LaunchRenderMega(d.scene, p, mblocks, debug_build, s);
+      if (mblocks > 0) ctx->launches++;
+      MTB_CUDA(ctx, cudaGetLastError());
     }
     MTB_CUDA(ctx, cudaEventRecord(d.ev_stop, s));
     return MTB_OK;
@@ -1009,8 +778,8 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 }
 
 // A batch: n_views whole frames of one scene, one camera and one light set per view.  Always the megakernel, in one
-// launch per device (grid = tiles of a view x views of the device): the pipeline choice, the cost-aware tile order, the
-// hybrid split and the strip interleave are all single-frame machinery and none of their state is read or written.
+// launch per device (grid = tiles of a view x views of the device): the pipeline choice, the cost-aware tile order and
+// the strip interleave are all single-frame machinery and none of their state is read or written.
 // lights == NULL: every view uses the context's lights.  Device g renders a contiguous range of views; the counts
 // differ by at most one.  ss > 1 (samples per axis, 2, 4 or 8): every view is traced on the (ss*W) x (ss*H) sample grid,
 // exactly as a batch of that size, and the kernel writes the W x H block means; everything else is as for ss = 1.
@@ -1237,9 +1006,8 @@ int mtb_create(mtb_context **out, const int *devices, int n_devices) {
     ctx->no_host_store = hs != nullptr && hs[0] == '1';
     const char *l2 = getenv("MTB_L2_PERSIST_MB");
     ctx->l2_persist_mb = l2 != nullptr ? atoi(l2) : 0;
-    const char *qf = getenv("MTB_WF_QUEUE_FACTOR"), *af = getenv("MTB_WF_ACT_FACTOR");
+    const char *af = getenv("MTB_WF_ACT_FACTOR");
     for (DeviceState &d : ctx->dev) {
-      if (qf != nullptr && atoi(qf) >= 1) d.wf_queue_factor = atoi(qf);
       if (af != nullptr && atoi(af) >= 1) d.wf_act_factor = atoi(af);
     }
   }
@@ -1564,15 +1332,13 @@ int mtb_pipeline_in_use(const mtb_context *ctx, float *mega_ms, float *wavefront
   const DeviceState &d = ctx->dev[0];
   if (mega_ms != nullptr) *mega_ms = d.tune_ms[0];
   if (wavefront_ms != nullptr) *wavefront_ms = d.tune_ms[1];
-  if ((ctx->flags & MTB_FLAG_QUEUE) != 0) return 3;
-  if ((ctx->flags & MTB_FLAG_WAVEFRONT) != 0) return 1;
-  if ((ctx->flags & MTB_FLAG_HYBRID) != 0) return 2;
+  if ((ctx->flags & (MTB_FLAG_WAVEFRONT | MTB_FLAG_QUEUE)) != 0) return 3;
   if ((ctx->flags & MTB_FLAG_MEGAKERNEL) != 0) return 0;
   if (d.tune_stage < kTuneDecided) return -1;
-  return d.tune_choice == 1 ? 3 : d.tune_choice;
+  return d.tune_queue ? 3 : 0;
 }
 
-float mtb_hybrid_share(const mtb_context *ctx) { return ctx == nullptr || ctx->dev.empty() ? 0.0f : ctx->dev[0].hybrid_share; }
+float mtb_hybrid_share(const mtb_context *) { return 0.0f; }
 
 int mtb_read_counters(mtb_context *ctx, mtb_stats *stats) {
   if (ctx == nullptr || stats == nullptr) return MTB_ERR_ARG;

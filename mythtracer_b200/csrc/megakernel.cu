@@ -148,7 +148,7 @@ __device__ __forceinline__ void SupersampleEpilogue(const RenderParams &rp, cons
 
 // BATCH: grid (tiles per view, views), block b of row v renders tile b of view v in scanline order; the camera comes from
 // views[v] and the pixels go to rp.rgb + v * chunk_w * chunk_h * 3.  A batch launch passes NULL for tile_order,
-// tile_cost, heavy_k, run_if and the taps / debug planes.  Without BATCH, `views` is unused and every `BATCH ? :`
+// tile_cost, run_if and the taps / debug planes.  Without BATCH, `views` is unused and every `BATCH ? :`
 // folds away: the single-view kernels compile to the code they had before the batch form existed.  SS > 1 (BATCH only):
 // the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.
 template <bool DBG, bool BATCH, int SS>
@@ -162,10 +162,8 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
     if (threadIdx.x == 0) s_ss8[0] = 0u;
     __syncthreads();  // (both warps start together: unlike a barrier after the trace, this holds nobody's slot)
   }
-  // repair launch of a wavefront frame whose queues did not overflow: nothing to do
+  // repair launch of a wavefront frame whose activation table did not overflow: nothing to do
   if (rp.run_if != nullptr && __ldg(rp.run_if) == 0u) return;
-  // hybrid frame: the leading (most expensive) tiles of the order belong to the wavefront pipeline
-  if (rp.heavy_k != nullptr && (((int)blockIdx.x < __ldg(rp.heavy_k)) != (rp.mega_part == 1))) return;
   unsigned long long cnt_store[DBG ? kNumCounters : 1];
   unsigned long long *cnt = cnt_store;
   if (DBG) {
@@ -664,24 +662,13 @@ __global__ void __launch_bounds__(64) IntersectChainKernel(DeviceScene sc, Inter
 }
 
 // Counting sort of the tiles by cost bucket (log2 of the ray count, most expensive first).  One block.
-// heavy_k (nullable): receives how many leading tiles of the order - the most expensive ones - together carry
-// `heavy_share_q16` / 65536 of the frame's rays (whole buckets, then part of the next one), at most k_max tiles: the
-// wavefront's side of a hybrid frame.
-__global__ void __launch_bounds__(1024) BuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles, int32_t *heavy_k, int k_max,
-                                                       unsigned heavy_share_q16) {
+__global__ void __launch_bounds__(1024) BuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles) {
   __shared__ unsigned hist[33];
   __shared__ unsigned offset[33];
-  // (32-bit sums: 64-bit shared-memory atomics are CAS loops - with all tiles in two or three buckets they made this
-  // one-block kernel take 570 us per frame, 6 % of a C3 frame; a device's share of a frame stays far below 2^32 rays)
   // Every warp counts into its own copy (atomics on one address are serialised; 1024 threads on two or three hot
   // buckets took 33 us in round 1).
-  __shared__ unsigned bucket_cost[33];
-  __shared__ unsigned long long total;
-  __shared__ unsigned w_hist[32][33], w_cost[32][33];
-  for (int i = threadIdx.x; i < 32 * 33; i += blockDim.x) {
-    (&w_hist[0][0])[i] = 0;
-    (&w_cost[0][0])[i] = 0;
-  }
+  __shared__ unsigned w_hist[32][33];
+  for (int i = threadIdx.x; i < 32 * 33; i += blockDim.x) (&w_hist[0][0])[i] = 0;
   __syncthreads();
   // warp w owns the contiguous tiles [w * chunk, (w + 1) * chunk): inside a bucket the launch order then stays in
   // tile order, i.e. blocks that run at the same time render neighbouring tiles
@@ -692,23 +679,12 @@ __global__ void __launch_bounds__(1024) BuildTileOrder(uint32_t *tile_cost, int3
     const unsigned c = tile_cost[t];
     const int b = c == 0u ? 0 : 32 - __clz((int)c);
     atomicAdd(&w_hist[warp][b], 1u);
-    atomicAdd(&w_cost[warp][b], c);
   }
   __syncthreads();
   if (threadIdx.x < 33) {
-    unsigned h = 0, c = 0;
-    for (int w = 0; w < 32; w++) {
-      h += w_hist[w][threadIdx.x];
-      c += w_cost[w][threadIdx.x];
-    }
+    unsigned h = 0;
+    for (int w = 0; w < 32; w++) h += w_hist[w][threadIdx.x];
     hist[threadIdx.x] = h;
-    bucket_cost[threadIdx.x] = c;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned long long sum = 0;
-    for (int b = 0; b <= 32; b++) sum += bucket_cost[b];
-    total = sum;
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -716,23 +692,6 @@ __global__ void __launch_bounds__(1024) BuildTileOrder(uint32_t *tile_cost, int3
     for (int b = 32; b >= 0; b--) {
       offset[b] = run;
       run += hist[b];
-    }
-    if (heavy_k != nullptr) {
-      const unsigned long long want = (total >> 16) * heavy_share_q16 + (((total & 0xffffull) * heavy_share_q16) >> 16);
-      unsigned long long got = 0;
-      int k = 0;
-      for (int b = 32; b >= 1 && got < want; b--) {
-        if (hist[b] == 0u) continue;
-        if (got + (unsigned long long)bucket_cost[b] <= want) {
-          got += (unsigned long long)bucket_cost[b];
-          k += (int)hist[b];
-        } else {  // part of this bucket (its tiles cost within a factor of two of each other)
-          const unsigned long long per_tile = (unsigned long long)bucket_cost[b] / hist[b] + 1ull;
-          k += (int)((want - got) / per_tile);
-          got = want;
-        }
-      }
-      *heavy_k = k < k_max ? k : k_max;
     }
   }
   __syncthreads();
@@ -756,10 +715,9 @@ __global__ void __launch_bounds__(1024) BuildTileOrder(uint32_t *tile_cost, int3
 
 }  // namespace
 
-void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles, int32_t *heavy_k, int k_max, unsigned heavy_share_q16,
-                          cudaStream_t stream) {
+void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles, cudaStream_t stream) {
   if (n_tiles <= 0) return;
-  BuildTileOrder<<<1, 1024, 0, stream>>>(tile_cost, tile_order, n_tiles, heavy_k, k_max, heavy_share_q16);
+  BuildTileOrder<<<1, 1024, 0, stream>>>(tile_cost, tile_order, n_tiles);
 }
 
 // n_blocks = number of 8x8 tiles of the launch.

@@ -1,44 +1,24 @@
-// Wavefront pipeline: the recursive TraceRayWorker (mythtracer.cc:13-228) as an iterative, level-by-level
-// sequence of kernels over ray queues in HBM.
+// Wavefront pipeline (the queue pipeline): the recursive TraceRayWorker (mythtracer.cc:13-228) as activations taken
+// from ONE device-side ray queue by a persistent kernel, then a per-pixel fold.  Four kernels per frame:
 //
-//   level L:  WfTrace       one thread per queued ray: OctTree::IntersectRay, hit point, interpolated normal,
-//                           surface colour, reflected direction (mythtracer.cc:18-76) -> activation record; then, in
-//                           the same kernel, the reflection / refraction children of the hit are appended to the queue
-//                           of level L+1 with a warp-aggregated (ballot + prefix count) slot allocation
-//                           (mythtracer.cc:181-225).  Whether a child exists does not depend on the lights.
-//     side streams:
-//             WfShadow      one thread per (hit, light): the whole shadow walk through transparent surfaces
-//                           (mythtracer.cc:86-156); lights are independent of each other, only the order in
-//                           which their terms are summed matters, and that order is kept by WfLight
-//             WfLight       one thread per hit: Phong sum over the lights in scene order (mythtracer.cc:78-178)
-//   The trace chain of the levels is the critical path (each link ends with the slowest ray of its level); the
-//   shadow / light kernels of level L only need level L's activation records, so they run on side streams and fill
-//   the machine while the chain advances.
-//   finally:  WfFold        deepest level first: parent += child * Refl, then parent += (child * Tf) * Tr --
-//                           the same two additions, in the same order, as the recursion performs on return
-//             WfResolve     V3DtoRGB (mythtracer.cc:235-241) into the chunk-local RGB24 buffer
-//             WfCommit      work counters of the frame -> the context's counters
+//   WfQueueBegin   resets the queue, the overflow flag and the frame's work counters
+//   WfQueue        traces every activation of every level, queues its reflection / refraction children, walks its
+//                  shadow segments and sums its Phong terms (mythtracer.cc:13-178)
+//   WfResolveTree  per pixel: parent += child * Refl, then parent += (child * Tf) * Tr -- the same two additions, in the
+//                  same order, as the recursion performs on return -- and V3DtoRGB (mythtracer.cc:235-241)
+//   WfCommit       work counters of the frame -> the context's counters; overflow flag -> pinned host words
 //
-// Nothing is read back to the host while a frame is in flight (round 1 read one counter per level): how many rays
-// a level holds is a device-side number (WfBuffers::level_n), every kernel sizes its own loop from it, and the host
-// only chooses grid sizes - from the previous frame's counts when it has them, else from the capacity bound.  A
-// queue that overflows sets WfBuffers::ctrl[0]; every later kernel of the frame then exits at once and a RenderMega
-// launch that is always queued behind the frame (RenderParams::run_if) renders the same pixels instead - both
-// pipelines produce the same bytes - while the host enlarges the queues for the next frame.
+// Nothing is read back to the host while a frame is in flight.  An activation table that overflows sets
+// WfBuffers::ctrl[0]; every warp then leaves, and a RenderMega launch that is always queued behind the frame
+// (RenderParams::run_if) renders the same pixels instead - both pipelines produce the same bytes - while the host
+// enlarges the table for the next frame.
 //
 // Because every activation keeps its own colour and the fold replays the reference's additions in the
 // reference's order, the result is bit-identical to the megakernel (and to the reference, up to pow()).
-#include <cstdlib>
-
 #include "device_core.cuh"
 
 namespace mtb {
 namespace {
-
-constexpr int kWfBlock = 128;
-#ifndef MTB_WF_MIN_BLOCKS
-#define MTB_WF_MIN_BLOCKS 8  // measured on B200 (C3): 1 -> 107 ms, 4 -> 90, 6 -> 79, 8 -> 70 (64 registers, 32 warps/SM)
-#endif
 
 __device__ __forceinline__ void Store3(double *p, const D3 &v) {
   p[0] = v.x;
@@ -62,402 +42,12 @@ __device__ __forceinline__ void FlushCounters(unsigned long long *cnt, unsigned 
   }
 }
 
-// Rays queued for `level` and the activation id of its first ray (activations are numbered level by level).
-struct LevelRange {
-  int n, base;
-};
-__device__ __forceinline__ LevelRange WfLevel(const WfBuffers &wf, int level) {
-  LevelRange r;
-  r.base = 0;
-  for (int k = 0; k < level; k++) r.base += (int)wf.level_n[k];
-  r.n = (int)wf.level_n[level];
-  return r;
-}
-
-// Sub-warp packing.  A warp runs as long as its slowest ray and serialises what its lanes do differently,
-// so a level with few rays (deep levels, or a small share of the frame on one of 8 GPUs) finishes sooner
-// when its rays are spread over more, emptier warps: only the first `lanes` lanes of each warp get a ray.
-// The loops below are warp-uniform: a warp handles items [first, first + lanes), then advances by the grid.
-struct WarpSpan {
-  long long first, step;
-  int lane;
-};
-__device__ __forceinline__ WarpSpan WfSpan(int lanes) {
-  WarpSpan s;
-  const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  s.lane = (int)(threadIdx.x & 31u);
-  s.first = warp * lanes;
-  s.step = (((long long)gridDim.x * blockDim.x) >> 5) * lanes;
-  return s;
-}
-
 // ---------------------------------------------------------------------------------------------------
-// WfTrace
+// WfQueue: ONE persistent kernel for all levels
 // ---------------------------------------------------------------------------------------------------
-// Pixel slot -> tile of this launch.  Hybrid frames (rp.heavy_k): slot >> 6 is a position in the launch order and
-// only the first *heavy_k positions belong to the wavefront (-1 beyond them).
-__device__ __forceinline__ int WfTileOfSlot(const RenderParams &rp, int slot) {
-  const int pos = slot >> 6;
-  if (rp.heavy_k == nullptr) return pos;
-  if (pos >= __ldg(rp.heavy_k)) return -1;
-  return __ldg(rp.tile_order + pos);
-}
-
-// What a tile cost, for the next frame's launch order and split (the megakernel does the same per block).
-__device__ __forceinline__ void WfChargeTile(const RenderParams &rp, int pixel, unsigned rays) {
-  if (rp.tile_cost == nullptr || rays == 0u || pixel < 0) return;
-  const int px = pixel % rp.chunk_w, py = pixel / rp.chunk_w;
-  const int local_strip = ((py >> 3) - rp.strip_first) / rp.strip_stride;
-  atomicAdd(rp.tile_cost + local_strip * rp.tiles_x + (px >> 3), rays);
-}
-
-// First kernel of a frame: level 0 holds one ray per pixel slot, nothing else is queued, no overflow, no work yet.
-__global__ void WfBegin(WfBuffers wf, int slots) {
-  const int i = (int)threadIdx.x;
-  if (i <= MTB_MAX_RAY_DEPTH + 1) wf.level_n[i] = i == 0 ? (uint32_t)slots : 0u;
-  if (i < 2) wf.ctrl[i] = 0u;
-  if (i < kNumCounters) wf.work[i] = 0ull;
-}
-
-template <bool DBG>
-__global__ void __launch_bounds__(kWfBlock, MTB_WF_MIN_BLOCKS) WfTrace(DeviceScene sc, RenderParams rp, WfBuffers wf, int level, int lanes) {
-  MTB_DECLARE_FAST_CTX(kWfBlock);
-  if (wf.ctrl[0] != 0u) return;  // an earlier level overflowed: the frame is rendered by the repair launch
-  const LevelRange lr = WfLevel(wf, level);
-  const int n = lr.n < wf.queue_cap ? lr.n : wf.queue_cap, act_base = lr.base;
-  unsigned long long cnt_store[DBG ? kNumCounters : 1];
-  unsigned long long *cnt = cnt_store;
-  if (DBG) {
-    for (int k = 0; k < kNumCounters; k++) cnt[k] = 0;
-  }
-  unsigned traced = 0;
-  const int q = level & 1, qn = q ^ 1;
-  const WarpSpan span = WfSpan(lanes);
-  for (long long first = span.first; first < n; first += span.step) {
-    // i: position in the level's queue; activation id = act_base + i
-    const int i = (int)first + span.lane;
-    const bool mine = span.lane < lanes && i < n;
-    bool do_reflect = false, do_refract = false, in_object = false;
-    double coef = 1.0, refl = 0.0;
-    D3 P = Mk(0.0, 0.0, 0.0), child_refl = Mk(0.0, 0.0, 0.0), d = Mk(0.0, 0.0, 0.0);
-    int pixel = -1;
-    unsigned long long path = 1ull;
-    const int act = act_base + i;
-    if (mine) {
-      D3 o;
-      bool live = true;
-      if (level == 0) {
-        // 8x8 pixel tiles (a warp = 8x4 pixels) of this launch's strips, as in RenderMega; in a hybrid frame the
-        // slots are the first *heavy_k tiles of the launch order
-        const int tile = WfTileOfSlot(rp, i), t = i & 63;
-        const int strip = rp.strip_first + (tile / rp.tiles_x) * rp.strip_stride;
-        const int px = (tile % rp.tiles_x) * 8 + (t & 7);
-        const int py = strip * 8 + (t >> 3);
-        live = tile >= 0 && px < rp.chunk_w && py < rp.chunk_h;
-        pixel = live ? py * rp.chunk_w + px : -1;
-        const D3 start = Load3(rp.sensor), d_scan = Load3(rp.sensor + 3), d_pixel = Load3(rp.sensor + 6);
-        o = Load3(rp.origin);
-        d = Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px))));
-        if (live) Count<DBG>(cnt, kPrimary);
-      } else {
-        o = Load3(wf.rq_o[q] + (size_t)i * 3);
-        d = Load3(wf.rq_d[q] + (size_t)i * 3);
-        pixel = wf.rq_pixel[q][i];
-        path = wf.rq_path[q][i];
-        coef = wf.rq_coef[q][i];
-        in_object = wf.rq_inobj[q][i] != 0;
-      }
-      wf.act_refl[act] = -1;
-      wf.act_refr[act] = -1;
-      wf.act_pixel[act] = pixel;
-      wf.act_path[act] = path;
-      int act_mtl = -2;
-      D3 color = Mk(0.0, 0.0, 0.0);
-      if (live) {
-        double t = 0.0;
-        const int slot = Trace<DBG>(sc, o, d, CUDART_INF, &t, cnt, fctx);
-        traced++;
-        if (rp.n_rays != nullptr) atomicAdd(rp.n_rays + pixel, 1u);
-        WfChargeTile(rp, pixel, 1u);
-        if (slot < 0) {
-          if (level == 0 && rp.dbg != nullptr) {
-            mtb_debug *dbg = rp.dbg + pixel;
-            dbg->line_no = -1;
-            dbg->pad_ = 0;
-            dbg->point[0] = dbg->point[1] = dbg->point[2] = CUDART_NAN;
-          }
-        } else {
-          const ShadeRec *sh = sc.shade + slot;
-          const SlotRec *sr = sc.slots + slot;
-          P = Add(o, MulS(d, t));
-          const int line_no = __ldg(&sh->line_no);
-          if (level == 0 && rp.dbg != nullptr) {
-            mtb_debug *dbg = rp.dbg + pixel;
-            dbg->line_no = line_no;
-            dbg->pad_ = 0;
-            dbg->point[0] = P.x;
-            dbg->point[1] = P.y;
-            dbg->point[2] = P.z;
-          }
-          if (rp.sig_hits != nullptr) {
-            atomicAdd(reinterpret_cast<unsigned long long *>(rp.sig_hits) + pixel, Mix64(path, 1ull, (unsigned long long)(long long)line_no));
-          }
-          Count<DBG>(cnt, kShade);
-          const D3 v0 = Load3(sr->vert), v1 = Load3(sr->vert + 3), v2 = Load3(sr->vert + 6);
-          const BaryWeights w = Barycentric(v0, v1, v2, P);
-          D3 normal = DivS(Add(Add(MulS(Load3(sh->normal), w.n0), MulS(Load3(sh->normal + 3), w.n1)), MulS(Load3(sh->normal + 6), w.n2)), w.n);
-          const D3 towards_camera = Neg(d);
-          double normal_ray_dot = Dot(towards_camera, normal);
-          if (normal_ray_dot < 0.0) {
-            normal = Neg(normal);
-            normal_ray_dot = Dot(towards_camera, normal);
-          }
-          const int material = __ldg(&sh->material);
-          if (material < 0) {  // mythtracer.cc:49-52
-            normal_ray_dot = (normal_ray_dot + 1.0) * 0.5;
-            color = Mk(normal_ray_dot, normal_ray_dot, normal_ray_dot);
-          } else {
-            const mtb_material *m = sc.materials + material;
-            D3 surface = Load3(m->ambient);
-            const int tex = m->texture;
-            if (tex >= 0) {
-              const double u = (sh->uv[0] * w.n0 + sh->uv[2] * w.n1 + sh->uv[4] * w.n2) / w.n;
-              const double v = (sh->uv[1] * w.n0 + sh->uv[3] * w.n1 + sh->uv[5] * w.n2) / w.n;
-              surface = MulV(surface, SampleTexture(sc.tex_atlas, tex, sc.texture_dim[tex], u, v));
-            }
-            child_refl = Sub(d, MulS(normal, 2 * Dot(normal, d)));
-            act_mtl = material;
-            Store3(wf.act_point + (size_t)act * 3, P);
-            Store3(wf.act_normal + (size_t)act * 3, normal);
-            Store3(wf.act_surface + (size_t)act * 3, surface);
-            Store3(wf.act_reflected + (size_t)act * 3, child_refl);
-            Store3(wf.act_dir + (size_t)act * 3, d);
-            if (level < rp.max_depth) {
-              refl = m->reflectance;
-              do_reflect = refl > 0.0 && coef > 0.01 && !in_object;  // mythtracer.cc:181-184
-              do_refract = m->transparency > 0.0;                    // mythtracer.cc:192
-            }
-          }
-        }
-      }
-      wf.act_mtl[act] = act_mtl;
-      Store3(wf.act_color + (size_t)act * 3, color);
-    }
-    // ---- children of the warp's hits -> queue of the next level: warp ballots + prefix counts, one atomic per
-    // warp.  The warp's reflection children are stored first, then its refraction children, so that neighbouring
-    // queue entries (= the lanes of a warp in the next level) are rays of the same kind from neighbouring pixels ----
-    __syncwarp();
-    const unsigned refl_mask = __ballot_sync(0xffffffffu, do_reflect);
-    const unsigned refr_mask = __ballot_sync(0xffffffffu, do_refract);
-    const unsigned n_refl = (unsigned)__popc(refl_mask), n_refr = (unsigned)__popc(refr_mask);
-    const unsigned total = n_refl + n_refr;
-    if (total == 0u) continue;
-    const unsigned below = (1u << span.lane) - 1u;
-    unsigned base = 0;
-    if (span.lane == 0) base = atomicAdd(wf.level_n + level + 1, total);
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if (do_reflect || do_refract) {
-      const int next_base = act_base + lr.n;
-      if (base + total > (unsigned)wf.queue_cap || (long long)next_base + base + total > (long long)wf.act_cap) {
-        wf.ctrl[0] = 1u;  // overflow: this frame is rendered by the repair launch, the next one gets larger queues
-      } else {
-        if (do_reflect) {
-          const unsigned pos = base + (unsigned)__popc(refl_mask & below);
-          Count<DBG>(cnt, kReflect);
-          Store3(wf.rq_o[qn] + (size_t)pos * 3, Add(P, MulS(child_refl, 0.0001)));  // mythtracer.cc:70-75
-          Store3(wf.rq_d[qn] + (size_t)pos * 3, child_refl);
-          wf.rq_coef[qn][pos] = coef * refl;
-          wf.rq_path[qn][pos] = path * 2ull;
-          wf.rq_pixel[qn][pos] = pixel;
-          wf.rq_inobj[qn][pos] = in_object ? 1 : 0;
-          wf.act_refl[act] = next_base + (int)pos;
-        }
-        if (do_refract) {
-          const unsigned pos = base + n_refl + (unsigned)__popc(refr_mask & below);
-          Count<DBG>(cnt, kRefract);
-          const D3 rdir = Normalized(d);                                       // mythtracer.cc:208-212
-          Store3(wf.rq_o[qn] + (size_t)pos * 3, Add(P, MulS(rdir, 0.00001)));  // mythtracer.cc:214-218
-          Store3(wf.rq_d[qn] + (size_t)pos * 3, rdir);
-          wf.rq_coef[qn][pos] = coef;
-          wf.rq_path[qn][pos] = path * 2ull + 1ull;
-          wf.rq_pixel[qn][pos] = pixel;
-          wf.rq_inobj[qn][pos] = in_object ? 0 : 1;
-          wf.act_refr[act] = next_base + (int)pos;
-        }
-      }
-    }
-  }
-  FlushCounters<DBG>(cnt, wf.work, traced);
-}
-
-// ---------------------------------------------------------------------------------------------------
-// WfShadow: thread = (light, activation).  Light-major task order keeps the rays of a warp aimed at one light.
-// ---------------------------------------------------------------------------------------------------
-template <bool DBG>
-__global__ void __launch_bounds__(kWfBlock, MTB_WF_MIN_BLOCKS) WfShadow(DeviceScene sc, RenderParams rp, WfBuffers wf, int level, int lanes) {
-  MTB_DECLARE_FAST_CTX(kWfBlock);
-  if (wf.ctrl[0] != 0u) return;
-  const LevelRange lr = WfLevel(wf, level);
-  const int n = lr.n < wf.queue_cap ? lr.n : wf.queue_cap;
-  const long long tasks = (long long)n * sc.n_lights;
-  unsigned long long cnt_store[DBG ? kNumCounters : 1];
-  unsigned long long *cnt = cnt_store;
-  if (DBG) {
-    for (int k = 0; k < kNumCounters; k++) cnt[k] = 0;
-  }
-  unsigned traced = 0;
-  const WarpSpan span = WfSpan(lanes);
-  for (long long first = span.first; first < tasks; first += span.step) {
-    const long long task = first + span.lane;
-    if (span.lane >= lanes || task >= tasks) continue;
-    const int li = (int)(task / n);
-    const int act = lr.base + (int)(task - (long long)li * n);
-    if (wf.act_mtl[act] < 0) continue;
-    const D3 P = Load3(wf.act_point + (size_t)act * 3);
-    const D3 lpos = Load3(sc.lights[li].position);
-    const D3 ldir = Normalized(Sub(lpos, P));
-    D3 power = Mk(1.0, 1.0, 1.0);
-    bool in_shadow = false, through = false;
-    unsigned segments = 0;
-    D3 seg_start = P;
-    for (;;) {  // mythtracer.cc:94-156
-      const D3 to = Add(seg_start, MulS(ldir, 0.00001));
-      const double light_distance = Dist(seg_start, lpos);
-      double t = 0.0;
-      Count<DBG>(cnt, kShadow);
-      const int slot = Trace<DBG>(sc, to, ldir, light_distance, &t, cnt, fctx);
-      segments++;
-      if (slot < 0) break;
-      if (t > light_distance) break;
-      const int smtl = __ldg(&sc.shade[slot].material);
-      const double str = smtl >= 0 ? __ldg(&sc.materials[smtl].transparency) : 0.0;
-      if (str == 0.0) {
-        power = Mk(0.0, 0.0, 0.0);
-        in_shadow = true;
-        break;
-      }
-      if (!through) power = MulV(power, MulS(Load3(sc.materials[smtl].transmission_filter), str));
-      through = !through;
-      seg_start = Add(Add(to, MulS(ldir, t)), MulS(ldir, 0.0000001));
-      if (SqrDist(P, seg_start) > SqrDist(P, lpos)) break;
-      if (power.x <= 0.001 && power.y <= 0.001 && power.z <= 0.001) {
-        power = Mk(0.0, 0.0, 0.0);
-        in_shadow = true;
-        break;
-      }
-    }
-    traced += segments;
-    Store3(wf.sh_power + ((size_t)li * wf.act_cap + act) * 3, power);
-    wf.sh_flags[(size_t)li * wf.act_cap + act] = (in_shadow ? 1u : 0u) | (segments << 1);
-    if (rp.n_rays != nullptr) atomicAdd(rp.n_rays + wf.act_pixel[act], segments);
-    WfChargeTile(rp, wf.act_pixel[act], segments);
-  }
-  FlushCounters<DBG>(cnt, wf.work, traced);
-}
-
-// ---------------------------------------------------------------------------------------------------
-// WfLight: Phong sum over the lights in scene order (mythtracer.cc:78-178)
-// ---------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kWfBlock) WfLight(DeviceScene sc, RenderParams rp, WfBuffers wf, int level) {
-  if (wf.ctrl[0] != 0u) return;
-  const LevelRange lr = WfLevel(wf, level);
-  const int n = lr.n < wf.queue_cap ? lr.n : wf.queue_cap;
-  for (int k = (int)(blockIdx.x * blockDim.x + threadIdx.x); k < n; k += (int)(gridDim.x * blockDim.x)) {
-    const int act = lr.base + k;
-    const int material = wf.act_mtl[act];
-    if (material < 0) continue;
-    const mtb_material *m = sc.materials + material;
-    const D3 P = Load3(wf.act_point + (size_t)act * 3);
-    const D3 normal = Load3(wf.act_normal + (size_t)act * 3);
-    const D3 surface = Load3(wf.act_surface + (size_t)act * 3);
-    const D3 reflected = Load3(wf.act_reflected + (size_t)act * 3);
-    const D3 m_d = Load3(wf.act_dir + (size_t)act * 3);
-    const unsigned long long path = wf.act_path[act];
-    D3 color = Mk(0.0, 0.0, 0.0);
-    unsigned long long sig = 0;
-    for (int li = 0; li < sc.n_lights; li++) {
-      const mtb_light *lt = sc.lights + li;
-      const D3 ldir = Normalized(Sub(Load3(lt->position), P));
-      const D3 lamb = Load3(lt->ambient);
-      color = Add(color, MulV(lamb, surface));
-      D3 power = Load3(wf.sh_power + ((size_t)li * wf.act_cap + act) * 3);
-      const unsigned flags = wf.sh_flags[(size_t)li * wf.act_cap + act];
-      const bool in_shadow = (flags & 1u) != 0u;
-      sig += Mix64(path, 2ull + (unsigned long long)li, (unsigned long long)flags);
-      power.x = SMax(power.x, lamb.x);
-      power.y = SMax(power.y, lamb.y);
-      power.z = SMax(power.z, lamb.z);
-      color = Add(color, MulV(MulV(MulS(MulV(Load3(m->diffuse), surface), Dot(normal, ldir)), Load3(lt->diffuse)), power));
-      if (!in_shadow) {
-        const double refl_dot = Dot(Neg(m_d), reflected);
-        if (refl_dot > 0) {
-          color = Add(color, MulV(MulS(MulV(Load3(m->specular), surface), pow(refl_dot, m->specular_exp)), Load3(lt->specular)));
-        }
-      }
-    }
-    if (rp.sig_shadow != nullptr && sc.n_lights > 0) {
-      atomicAdd(reinterpret_cast<unsigned long long *>(rp.sig_shadow) + wf.act_pixel[act], sig);
-    }
-    Store3(wf.act_color + (size_t)act * 3, color);
-  }
-}
-
-// parent += child * Refl ; parent += (child * Tf) * Tr   (mythtracer.cc:185-189, 220-224)
-__global__ void __launch_bounds__(256) WfFold(DeviceScene sc, WfBuffers wf, int level) {
-  if (wf.ctrl[0] != 0u) return;
-  const LevelRange lr = WfLevel(wf, level);
-  const int n = lr.n < wf.queue_cap ? lr.n : wf.queue_cap;
-  for (int k = (int)(blockIdx.x * blockDim.x + threadIdx.x); k < n; k += (int)(gridDim.x * blockDim.x)) {
-    const int a = lr.base + k;
-    const int rc = wf.act_refl[a], tc = wf.act_refr[a];
-    if (rc < 0 && tc < 0) continue;
-    const mtb_material *m = sc.materials + wf.act_mtl[a];
-    D3 color = Load3(wf.act_color + (size_t)a * 3);
-    if (rc >= 0) color = Add(color, MulS(Load3(wf.act_color + (size_t)rc * 3), m->reflectance));
-    if (tc >= 0) color = Add(color, MulS(MulV(Load3(wf.act_color + (size_t)tc * 3), Load3(m->transmission_filter)), m->transparency));
-    Store3(wf.act_color + (size_t)a * 3, color);
-  }
-}
-
-// One thread = 8 bytes of a tile row (a row of 8 pixels = 24 bytes = the 24 consecutive doubles of act_color that
-// belong to slots tile * 64 + row * 8 + 0..7): the frame may be the peer-mapped frame of another GPU, where one
-// aligned 8-byte store per thread is what the link likes (RenderMega writes its tiles the same way).
-__global__ void __launch_bounds__(256) WfResolve(RenderParams rp, WfBuffers wf, int n_slots) {
-  if (wf.ctrl[0] != 0u) return;
-  const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);  // (tile position, row, segment)
-  const int pos = i / 24, row = (i % 24) / 3, seg = i % 3;
-  if (pos * 64 >= n_slots) return;
-  // same slot -> pixel mapping as level 0 of WfTrace (the level-0 queue itself has been reused by now)
-  const int tile = WfTileOfSlot(rp, pos * 64);
-  if (tile < 0) return;
-  const int strip = rp.strip_first + (tile / rp.tiles_x) * rp.strip_stride;
-  const int px0 = (tile % rp.tiles_x) * 8, py = strip * 8 + row;
-  if (py >= rp.chunk_h) return;
-  const double *c = wf.act_color + ((size_t)pos * 64 + (size_t)row * 8) * 3 + seg * 8;
-  unsigned char b[8];
-#pragma unroll
-  for (int k = 0; k < 8; k++) b[k] = QuantizeChannel(c[k]);
-  unsigned char *out = rp.rgb + ((size_t)py * rp.chunk_w + px0) * 3 + seg * 8;
-  if (px0 + 8 <= rp.chunk_w && (rp.chunk_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rp.rgb) & 7u) == 0u) {
-    uint2 v;
-    v.x = (unsigned)b[0] | ((unsigned)b[1] << 8) | ((unsigned)b[2] << 16) | ((unsigned)b[3] << 24);
-    v.y = (unsigned)b[4] | ((unsigned)b[5] << 8) | ((unsigned)b[6] << 16) | ((unsigned)b[7] << 24);
-    *reinterpret_cast<uint2 *>(out) = v;
-  } else {
-    const int valid = (rp.chunk_w - px0) * 3 - seg * 8;  // bytes of this segment that lie inside the chunk
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      if (k < valid) out[k] = b[k];
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------
-// Queue pipeline: ONE persistent kernel for all levels
-// ---------------------------------------------------------------------------------------------------
-// The level-by-level pipeline above pays, per level, one kernel boundary on its critical path (a level's trace kernel
-// ends with its slowest ray before the first ray of the next level starts) and writes the whole shading context of
-// every activation to HBM for the shadow / light kernels.  Here a task is ONE ACTIVATION from beginning to end:
+// A kernel per level would pay one kernel boundary per level on its critical path (a level's trace kernel ends with
+// its slowest ray before the first ray of the next level starts) and write the whole shading context of every
+// activation to HBM for separate shadow / light kernels.  Here a task is ONE ACTIVATION from beginning to end:
 // a warp takes up to 32 consecutive entries of a single ray queue (entry id = activation id; ids below `slots` are
 // the primary rays), traces them, shades the hits, appends their reflection / refraction children to the queue
 // (warp ballots + prefix counts, one atomic per warp) and publishes them BEFORE it walks its own shadow segments -
@@ -513,7 +103,6 @@ __device__ __forceinline__ void St3q(double *p, const D3 &v) {
 
 __global__ void WfQueueBegin(WfBuffers wf, int slots) {
   const int i = (int)threadIdx.x;
-  if (i <= MTB_MAX_RAY_DEPTH + 1) wf.level_n[i] = i == 0 ? (uint32_t)slots : 0u;
   if (i < 2) wf.ctrl[i] = 0u;
   if (i < kNumCounters) wf.work[i] = 0ull;
   if (i < kQWords) wf.qctl[i] = (i == kQTail || i == kQPending) ? (uint32_t)slots : 0u;
@@ -611,12 +200,12 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_QUEUE_MIN_BLOCKS) WfQueue(D
     D3 o = Mk(0.0, 0.0, 0.0), d = Mk(0.0, 0.0, 0.0);
     if (mine) {
       if (act < slots) {
-        // 8x8 pixel tiles (a warp = 8x4 pixels) of this launch's strips, as in RenderMega / WfTrace level 0
-        const int tile = WfTileOfSlot(rp, act), t = act & 63;
+        // 8x8 pixel tiles (a warp = 8x4 pixels) of this launch's strips, as in RenderMega
+        const int tile = act >> 6, t = act & 63;
         const int strip = rp.strip_first + (tile / rp.tiles_x) * rp.strip_stride;
         const int px = (tile % rp.tiles_x) * 8 + (t & 7);
         const int py = strip * 8 + (t >> 3);
-        live = tile >= 0 && px < rp.chunk_w && py < rp.chunk_h;
+        live = px < rp.chunk_w && py < rp.chunk_h;
         st.pixel = live ? py * rp.chunk_w + px : -1;
         const D3 start = Load3(rp.sensor), d_scan = Load3(rp.sensor + 3), d_pixel = Load3(rp.sensor + 6);
         o = Load3(rp.origin);
@@ -901,7 +490,6 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_QUEUE_MIN_BLOCKS) WfQueue(D
         traced += st.rays;
         if (lit && rp.sig_shadow != nullptr && sc.n_lights > 0) atomicAdd(reinterpret_cast<unsigned long long *>(rp.sig_shadow) + st.pixel, st.sig);
         if (rp.n_rays != nullptr) atomicAdd(rp.n_rays + st.pixel, st.rays);
-        WfChargeTile(rp, st.pixel, st.rays);
       }
     }
   }
@@ -914,9 +502,8 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_QUEUE_MIN_BLOCKS) WfQueue(D
 __global__ void __launch_bounds__(kBlockThreads) WfResolveTree(DeviceScene sc, RenderParams rp, WfBuffers wf, int slots) {
   __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3];
   if (wf.ctrl[0] != 0u) return;
-  const int pos = (int)blockIdx.x, root = pos * 64 + (int)threadIdx.x;
-  const int tile = WfTileOfSlot(rp, pos * 64);
-  if (tile < 0 || root >= slots) return;
+  const int tile = (int)blockIdx.x, root = tile * 64 + (int)threadIdx.x;
+  if (root >= slots) return;
   const int strip = rp.strip_first + (tile / rp.tiles_x) * rp.strip_stride;
   const int tx = (int)(threadIdx.x & 7u), ty = (int)(threadIdx.x >> 3);
   const int px = (tile % rp.tiles_x) * kTile + tx, py = strip * kTile + ty;
@@ -991,14 +578,13 @@ __global__ void __launch_bounds__(kBlockThreads) WfResolveTree(DeviceScene sc, R
 }
 
 // Last kernel of a frame.  The work counters of a frame that overflowed are dropped (the repair launch counts its
-// own rays); host_copy (pinned, nullable) receives level_n[] and the overflow flag for the next frame's grid sizes
-// and queue capacities - written by the device, never waited for by the host.
+// own rays); host_copy (pinned, nullable) receives the overflow flag for the next frame's table capacity - written by
+// the device, never waited for by the host.
 __global__ void WfCommit(WfBuffers wf, unsigned long long *global, uint32_t *host_copy) {
   const int i = (int)threadIdx.x;
   const bool overflow = wf.ctrl[0] != 0u;
   if (!overflow && global != nullptr && i < kNumCounters && wf.work[i] != 0ull) atomicAdd(global + i, wf.work[i]);
   if (host_copy != nullptr) {
-    if (i <= MTB_MAX_RAY_DEPTH + 1) host_copy[i] = wf.level_n[i];
     if (i == 0) host_copy[kWfHostOverflow] = overflow ? 1u : 0u;
     __syncwarp();
     __threadfence_system();
@@ -1007,72 +593,6 @@ __global__ void WfCommit(WfBuffers wf, unsigned long long *global, uint32_t *hos
 }
 
 }  // namespace
-
-// Lanes per warp for a queue of `n` items: full warps once the queue fills the machine (148 SMs x 32
-// resident warps), otherwise the largest power of two that still spreads it over all warp slots.
-static int PackLanes(long long n) {
-  static const int min_lanes = []() {
-    const char *env = getenv("MTB_WF_MIN_LANES");  // development knob (A/B of the packing)
-    const int v = env != nullptr ? atoi(env) : 4;
-    return v >= 1 && v <= 32 ? v : 4;
-  }();
-  const long long slots = 148LL * 32;
-  int lanes = 32;
-  while (lanes > min_lanes && n < slots * lanes) lanes >>= 1;
-  return lanes;
-}
-
-// Blocks for `items` loop items at `lanes` items per warp, at most what `bound` items need; never zero (the real
-// item count is read on the device, the loops are grid-strided).
-static int BlocksFor(long long items, long long bound, int lanes, int block) {
-  if (items > bound) items = bound;
-  if (items < 1) items = 1;
-  const long long warps = (items + lanes - 1) / lanes;
-  long long blocks = (warps * 32 + block - 1) / block;
-  if (blocks > 0x3fffffff) blocks = 0x3fffffff;
-  return (int)blocks;
-}
-
-void LaunchWfBegin(const WfBuffers &wf, int slots, cudaStream_t stream) { WfBegin<<<1, 32, 0, stream>>>(wf, slots); }
-
-// `expect`: how many rays the level is expected to hold (previous frame, with headroom; or the capacity bound)
-void LaunchWfTrace(const DeviceScene &sc, const RenderParams &rp, const WfBuffers &wf, int level, long long expect, bool debug_build,
-                   cudaStream_t stream) {
-  const int lanes = level == 0 ? 32 : PackLanes(expect);  // level 0 maps warps to 8x4 pixel tiles
-  const int blocks = BlocksFor(expect, wf.queue_cap, lanes, kWfBlock);
-  if (debug_build) {
-    WfTrace<true><<<blocks, kWfBlock, 0, stream>>>(sc, rp, wf, level, lanes);
-  } else {
-    WfTrace<false><<<blocks, kWfBlock, 0, stream>>>(sc, rp, wf, level, lanes);
-  }
-}
-
-void LaunchWfShadow(const DeviceScene &sc, const RenderParams &rp, const WfBuffers &wf, int level, long long expect, bool debug_build,
-                    cudaStream_t stream) {
-  if (sc.n_lights <= 0) return;
-  const long long tasks = expect * sc.n_lights;
-  const int lanes = PackLanes(tasks);
-  const int blocks = BlocksFor(tasks, (long long)wf.queue_cap * sc.n_lights, lanes, kWfBlock);
-  if (debug_build) {
-    WfShadow<true><<<blocks, kWfBlock, 0, stream>>>(sc, rp, wf, level, lanes);
-  } else {
-    WfShadow<false><<<blocks, kWfBlock, 0, stream>>>(sc, rp, wf, level, lanes);
-  }
-}
-
-void LaunchWfLight(const DeviceScene &sc, const RenderParams &rp, const WfBuffers &wf, int level, long long expect, cudaStream_t stream) {
-  WfLight<<<BlocksFor(expect, wf.queue_cap, 32, kWfBlock), kWfBlock, 0, stream>>>(sc, rp, wf, level);
-}
-
-void LaunchWfFold(const DeviceScene &sc, const WfBuffers &wf, int level, long long expect, cudaStream_t stream) {
-  WfFold<<<BlocksFor(expect, wf.queue_cap, 32, 256), 256, 0, stream>>>(sc, wf, level);
-}
-
-void LaunchWfResolve(const RenderParams &rp, const WfBuffers &wf, int n_slots, cudaStream_t stream) {
-  if (n_slots <= 0) return;
-  const int threads = (n_slots / 64) * 24;
-  WfResolve<<<(threads + 255) / 256, 256, 0, stream>>>(rp, wf, n_slots);
-}
 
 void LaunchWfQueueBegin(const WfBuffers &wf, int slots, cudaStream_t stream) { WfQueueBegin<<<1, 32, 0, stream>>>(wf, slots); }
 

@@ -6,8 +6,8 @@ tests/golden/make_golden_full.py in the build container with oracle/_ref):
 * C2 (textured, 720p), C4 (2 M triangles incl. the room-spanning sticks that the scene BVH references through
   several pre-split pieces) and C5 (4K, depth 8, 4 lights, 160 M rays): the whole frame as well.
 
-Plus the paths that only matter at scale: a wavefront frame whose queues overflow (repaired on the device, taps and
-counters exact), and frames shared between processes (tiles stored straight into another process's frame).
+Plus the paths that only matter at scale: a queue-pipeline frame whose activation table overflows (repaired on the
+device, taps and counters exact), and frames shared between processes (tiles stored straight into another process's frame).
 """
 import hashlib
 import multiprocessing as mp
@@ -61,9 +61,8 @@ def _compare(got_rgb, got_line_no, z, what):
 
 
 def test_c3_full_frame_equals_the_reference(product_lib, scene_dir):
-    """Every pixel of the 1920x1080 C3 frame against the reference's own render: megakernel, wavefront (level by level),
-    queue pipeline, hybrid."""
-    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_HYBRID, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE, MTB_FLAG_WAVEFRONT
+    """Every pixel of the 1920x1080 C3 frame against the reference's own render: megakernel and queue pipeline."""
+    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     z, files, cfg = _golden("C3", scene_dir)
     W, H = cfg["width"], cfg["height"]
     assert len(z["rows"]) == H
@@ -71,9 +70,9 @@ def test_c3_full_frame_equals_the_reference(product_lib, scene_dir):
     assert mt.LoadObj(files.obj_path), mt.last_error()
     mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
     shas = set()
-    for name, flags, frames in (("megakernel", MTB_FLAG_MEGAKERNEL, 2), ("wavefront", MTB_FLAG_WAVEFRONT, 2), ("queue", MTB_FLAG_QUEUE, 2), ("hybrid", MTB_FLAG_HYBRID, 3)):
+    for name, flags in (("megakernel", MTB_FLAG_MEGAKERNEL), ("queue", MTB_FLAG_QUEUE)):
         mt.set_flags(flags)
-        for frame in range(frames):  # (later frames: warm tile order / hybrid split / grids sized from the last frame)
+        for frame in range(2):  # (the second frame: warm tile order)
             got = mt.render_chunk(files.camera, W, H, 0, 0, W, H, debug=True)
         differing = _compare(got["rgb"], got["line_no"], z, "C3 " + name)
         assert _sha(got["line_no"]) == str(z["line_no_sha256"])
@@ -127,11 +126,10 @@ def test_c4_c5_full_frames_equal_the_reference(product_lib, scene_dir, name):
 
 
 def test_wavefront_queue_overflow_is_repaired_on_the_device(product_lib, oracle_mod, scene_dir, monkeypatch):
-    """Queues sized for one ray per pixel overflow at the first bounce of a reflective + transparent scene: the frame
-    must still be exact in every tap and counter (the repair launch renders it), and the queues must have grown by
-    the time a later frame goes through the wavefront kernels themselves."""
-    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_COUNT_WORK, MTB_FLAG_QUEUE, MTB_FLAG_WAVEFRONT
-    monkeypatch.setenv("MTB_WF_QUEUE_FACTOR", "1")
+    """An activation table sized for one ray per pixel overflows at the first bounce of a reflective + transparent
+    scene: the frame must still be exact in every tap and counter (the repair launch renders it), and the table must
+    have grown by the time a later frame goes through the queue pipeline's kernels themselves."""
+    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_COUNT_WORK, MTB_FLAG_QUEUE
     monkeypatch.setenv("MTB_WF_ACT_FACTOR", "1")
     files, cfg = scenes.config_scene("C1", scene_dir)
     w, h = 200, 120
@@ -139,7 +137,7 @@ def test_wavefront_queue_overflow_is_repaired_on_the_device(product_lib, oracle_
     orc.set_lights(files.lights)
     cpu = orc.render(files.camera, w, h, depth=4, taps=True)
     assert cpu["stats"]["reflect"] + cpu["stats"]["refract"] > 0
-    for flags in (MTB_FLAG_WAVEFRONT, MTB_FLAG_WAVEFRONT | MTB_FLAG_COUNT_WORK, MTB_FLAG_QUEUE, MTB_FLAG_QUEUE | MTB_FLAG_COUNT_WORK):
+    for flags in (MTB_FLAG_QUEUE, MTB_FLAG_QUEUE | MTB_FLAG_COUNT_WORK):
         mt = MythTracer(max_depth=4, flags=flags)
         assert mt.LoadObj(files.obj_path), mt.last_error()
         mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]

@@ -17,7 +17,7 @@ MAX_RGB_FRACTION = 1e-5
 
 
 def _tracer(product_lib, depth, flags=0, devices=None):
-    """flags without a pipeline bit: force the megakernel (small test frames would auto-select the wavefront)."""
+    """flags without a pipeline bit: force the megakernel (small test frames would auto-select the queue pipeline)."""
     from mythtracer_b200 import MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT, MythTracer
     from mythtracer_b200 import MTB_FLAG_QUEUE
     if not flags & (MTB_FLAG_WAVEFRONT | MTB_FLAG_MEGAKERNEL | MTB_FLAG_QUEUE):
@@ -72,7 +72,7 @@ def test_c1_full_frame(product_lib, oracle_mod, scene_dir):
     fast = mt.render_chunk(files.camera, w, h, 0, 0, w, h)
     assert np.array_equal(fast["rgb"], gpu["rgb"])
     assert fast["stats"]["rays"] == cpu["stats"]["rays"]
-    mt.set_flags(0)  # automatic choice (wavefront at this size): same bytes
+    mt.set_flags(0)  # automatic choice: same bytes
     auto = mt.render_chunk(files.camera, w, h, 0, 0, w, h)
     assert np.array_equal(auto["rgb"], gpu["rgb"]) and auto["stats"]["rays"] == cpu["stats"]["rays"]
 
@@ -307,11 +307,11 @@ def test_golden_fixtures_on_gpu(product_lib):
 
 def test_multi_device_context(product_lib, scene_dir):
     """In-process multi-GPU: strips interleaved over the devices of one context, gathered by peer copies;
-    the frame must be byte-identical to the single-GPU frame."""
+    the frame must be byte-identical to the single-GPU frame, through either pipeline."""
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
-    from mythtracer_b200 import Light
+    from mythtracer_b200 import Light, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     files, cfg = scenes.config_scene("C1", scene_dir)
     W, H = 320, 243
     one = _tracer(product_lib, 2)
@@ -319,60 +319,15 @@ def test_multi_device_context(product_lib, scene_dir):
     one.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
     ref = one.render_chunk(files.camera, W, H, 0, 0, W, H, debug=True, taps=True)
     n = min(torch.cuda.device_count(), 8)
-    many = _tracer(product_lib, 2, devices=list(range(n)))
-    assert many.LoadObj(files.obj_path)
-    many.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
-    got = many.render_chunk(files.camera, W, H, 0, 0, W, H, debug=True, taps=True)
-    for k in ("rgb", "line_no", "points", "n_rays", "sig_hits", "sig_shadow"):
-        assert np.array_equal(got[k], ref[k], equal_nan=(k == "points")), k
-    assert got["stats"]["rays"] == ref["stats"]["rays"]
-
-
-@pytest.mark.parametrize("name,scale,w,h", [("C1", 1.0, 320, 240), ("C2", 0.3, 256, 144)])
-def test_wavefront_pipeline_parity(product_lib, oracle_mod, scene_dir, name, scale, w, h):
-    """The wavefront pipeline (MTB_FLAG_WAVEFRONT) against the oracle, every tap, and against the megakernel."""
-    from mythtracer_b200 import MTB_FLAG_COUNT_WORK, MTB_FLAG_WAVEFRONT
-    files, cfg = scenes.config_scene(name, scene_dir, scale)
-    mt, orc = _load_pair(product_lib, oracle_mod, files, cfg["depth"], MTB_FLAG_WAVEFRONT | MTB_FLAG_COUNT_WORK)
-    gpu = mt.render_chunk(files.camera, w, h, 0, 0, w, h, debug=True, taps=True)
-    cpu = orc.render(files.camera, w, h, depth=cfg["depth"], taps=True)
-    _assert_render_equal(gpu, cpu, name + " wavefront")
-    from mythtracer_b200 import MTB_FLAG_MEGAKERNEL
-    mt.set_flags(MTB_FLAG_WAVEFRONT)
-    fast = mt.render_chunk(files.camera, w, h, 0, 0, w, h)
-    mt.set_flags(MTB_FLAG_MEGAKERNEL)
-    mega = mt.render_chunk(files.camera, w, h, 0, 0, w, h)
-    assert np.array_equal(fast["rgb"], mega["rgb"]) and np.array_equal(fast["rgb"], gpu["rgb"])
-    assert fast["stats"]["rays"] == mega["stats"]["rays"] == cpu["stats"]["rays"]
-
-
-def test_wavefront_depths_lights_lattice_and_tiles(product_lib, oracle_mod, scene_dir):
-    from mythtracer_b200 import Light, MTB_FLAG_WAVEFRONT
-    files, cfg = scenes.config_scene("C1", scene_dir)
-    mt, orc = _load_pair(product_lib, oracle_mod, files, 5, MTB_FLAG_WAVEFRONT)
-    w, h = 160, 120
-    for depth, n_lights in [(0, 1), (2, 0), (5, 4), (8, 2)]:
-        lights = scenes.LIGHT_RIG[:n_lights]
-        mt.max_depth = depth
-        mt.GetScene().lights = [Light.from_tuple(l) for l in lights]
-        orc.set_lights(lights)
-        gpu = mt.render_chunk(files.camera, w, h, 0, 0, w, h, debug=True, taps=True)
-        cpu = orc.render(files.camera, w, h, depth=depth, taps=True)
-        _assert_render_equal(gpu, cpu, "wavefront depth %d lights %d" % (depth, n_lights))
-    # a clipped WorkChunk tile with odd sizes
-    mt.max_depth = 3
-    gpu = mt.render_chunk(files.camera, 333, 211, 100, 37, 77, 45, debug=True, taps=True)
-    cpu = orc.render(files.camera, 333, 211, chunk=(100, 37, 77, 45), depth=3, taps=True)
-    _assert_render_equal(gpu, cpu, "wavefront tile")
-    path, cam, lights = scenes.lattice_scene(scene_dir)
-    mt2 = _tracer(product_lib, 5, MTB_FLAG_WAVEFRONT)
-    assert mt2.LoadObj(path)
-    mt2.GetScene().lights = [Light.from_tuple(l) for l in lights]
-    orc2 = oracle_mod.Oracle.from_obj(path)
-    orc2.set_lights(lights)
-    gpu = mt2.render_chunk(cam, 65, 49, 0, 0, 65, 49, debug=True, taps=True)
-    cpu = orc2.render(cam, 65, 49, depth=5, taps=True)
-    _assert_render_equal(gpu, cpu, "wavefront lattice")
+    for flags in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE):
+        many = _tracer(product_lib, 2, flags, devices=list(range(n)))
+        assert many.LoadObj(files.obj_path)
+        many.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
+        got = many.render_chunk(files.camera, W, H, 0, 0, W, H, debug=True, taps=True)
+        for k in ("rgb", "line_no", "points", "n_rays", "sig_hits", "sig_shadow"):
+            assert np.array_equal(got[k], ref[k], equal_nan=(k == "points")), (flags, k)
+        assert got["stats"]["rays"] == ref["stats"]["rays"]
+        many.close()
 
 
 @pytest.mark.parametrize("name,scale,w,h", [("C1", 1.0, 320, 240), ("C2", 0.3, 256, 144)])
@@ -425,11 +380,11 @@ def test_queue_pipeline_depths_lights_lattice_and_tiles(product_lib, oracle_mod,
 
 def test_megakernel_launch_forms(product_lib, oracle_mod, scene_dir):
     """The megakernel against the oracle, every tap: the plain and the counting build, with and without the
-    cost-aware tile order, with the retired round-1 flag bits set (accepted and ignored) -- on a full frame, a
+    cost-aware tile order, with the retired flag bits set (accepted and ignored) -- on a full frame, a
     clipped odd-sized tile (rows that cannot leave the block as aligned 8-byte stores), a partitioned render and
-    two consecutive frames (warm tile order)."""
-    from mythtracer_b200 import (MTB_FLAG_COUNT_WORK, MTB_FLAG_MEGAKERNEL, MTB_FLAG_NO_TILE_ORDER, MTB_FLAG_PACKING,
-                                 MTB_FLAG_PERSISTENT, MTB_FLAG_RESUME, MTB_FLAG_WARP_SYNC)
+    two consecutive frames (warm tile order).  MTB_FLAG_WAVEFRONT is the queue pipeline."""
+    from mythtracer_b200 import (MTB_FLAG_COUNT_WORK, MTB_FLAG_HYBRID, MTB_FLAG_MEGAKERNEL, MTB_FLAG_NO_TILE_ORDER, MTB_FLAG_PACKING,
+                                 MTB_FLAG_PERSISTENT, MTB_FLAG_QUEUE, MTB_FLAG_RESUME, MTB_FLAG_WARP_SYNC, MTB_FLAG_WAVEFRONT)
     files, cfg = scenes.config_scene("C2", scene_dir, 0.3)
     mt, orc = _load_pair(product_lib, oracle_mod, files, cfg["depth"], MTB_FLAG_MEGAKERNEL)
     w, h = 250, 141
@@ -437,7 +392,7 @@ def test_megakernel_launch_forms(product_lib, oracle_mod, scene_dir):
     cpu_tile = orc.render(files.camera, 333, 211, chunk=(100, 37, 77, 45), depth=cfg["depth"], taps=True)
     cpu_w8 = orc.render(files.camera, 256, 100, chunk=(0, 0, 256, 100), depth=cfg["depth"], taps=True)
     for flags in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_MEGAKERNEL | MTB_FLAG_COUNT_WORK, MTB_FLAG_MEGAKERNEL | MTB_FLAG_NO_TILE_ORDER,
-                  MTB_FLAG_MEGAKERNEL | MTB_FLAG_PACKING | MTB_FLAG_PERSISTENT | MTB_FLAG_RESUME | MTB_FLAG_WARP_SYNC):
+                  MTB_FLAG_MEGAKERNEL | MTB_FLAG_PACKING | MTB_FLAG_PERSISTENT | MTB_FLAG_RESUME | MTB_FLAG_WARP_SYNC | MTB_FLAG_HYBRID):
         mt.set_flags(flags)
         for frame in range(2):
             gpu = mt.render_chunk(files.camera, w, h, 0, 0, w, h, debug=True, taps=True)
@@ -458,16 +413,25 @@ def test_megakernel_launch_forms(product_lib, oracle_mod, scene_dir):
         rows = np.arange(h)
         own0 = ((rows // 8) % 2) == 0
         assert np.array_equal(parts[0][own0], full[own0]) and np.array_equal(parts[1][~own0], full[~own0])
+    assert mt.pipeline_in_use()[0] == "mega" and mt.hybrid_share() == 0.0
+    outs = {}
+    for flags in (MTB_FLAG_QUEUE, MTB_FLAG_WAVEFRONT):
+        mt.set_flags(flags)
+        outs[flags] = mt.render_chunk(files.camera, w, h, 0, 0, w, h, debug=True, taps=True)
+        assert mt.pipeline_in_use()[0] == "queue"
+        _assert_render_equal(outs[flags], cpu, "flags %d" % flags)
+    for k in ("rgb", "line_no", "n_rays", "sig_hits", "sig_shadow"):
+        assert np.array_equal(outs[MTB_FLAG_WAVEFRONT][k], outs[MTB_FLAG_QUEUE][k]), k
 
 
-@pytest.mark.parametrize("pipeline", ["mega", "wavefront"])
+@pytest.mark.parametrize("pipeline", ["mega", "queue"])
 def test_textured_light_terms_in_isolation(product_lib, oracle_mod, scene_dir, pipeline):
     """Ambient-only, diffuse-only and specular-only lights on the textured scene, both pipelines: each Phong
     term (mythtracer.cc:83-84,163-167,169-177) is compared on its own, so a wrong surface colour cannot hide
     behind the other terms.  (A register-capped build of the megakernel once lost one bilinear tap here.)"""
-    from mythtracer_b200 import Light, MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT
+    from mythtracer_b200 import Light, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     files, cfg = scenes.config_scene("C2", scene_dir, 0.1)
-    flags = MTB_FLAG_MEGAKERNEL if pipeline == "mega" else MTB_FLAG_WAVEFRONT
+    flags = MTB_FLAG_MEGAKERNEL if pipeline == "mega" else MTB_FLAG_QUEUE
     mt, orc = _load_pair(product_lib, oracle_mod, files, 2, flags)
     w, h = 200, 112
     pos = (200.0, 100.0, 160.0)
@@ -481,9 +445,9 @@ def test_textured_light_terms_in_isolation(product_lib, oracle_mod, scene_dir, p
         _assert_render_equal(gpu, cpu, "%s terms %s" % (pipeline, (amb, dif, spe)))
 
 
-def test_automatic_pipeline_choice(product_lib, oracle_mod, scene_dir):
-    """flags = 0: the library times the megakernel, the wavefront and the hybrid split on the first frames of a
-    geometry and keeps the fastest; every one of those frames must carry the same bytes (the choice is invisible in
+def test_automatic_pipeline_choice_decides_at_frame_5(product_lib, oracle_mod, scene_dir):
+    """flags = 0: the library times the megakernel and the queue pipeline on the first four frames of a geometry and
+    keeps the faster from frame 5 on; every one of those frames must carry the same bytes (the choice is invisible in
     the output)."""
     from mythtracer_b200 import Light, MythTracer
     files, cfg = scenes.config_scene("C1", scene_dir)
@@ -495,17 +459,15 @@ def test_automatic_pipeline_choice(product_lib, oracle_mod, scene_dir):
     w, h = 320, 240
     cpu = orc.render(files.camera, w, h, depth=cfg["depth"])
     states = []
-    for _ in range(15):
+    for _ in range(8):
         out = mt.render_chunk(files.camera, w, h, 0, 0, w, h)
         assert np.array_equal(out["rgb"], cpu["rgb"])
         assert out["stats"]["rays"] == cpu["stats"]["rays"]
         states.append(mt.pipeline_in_use()[0])
-    assert states[0] == "measuring" and states[10] == "measuring" and states[-1] in ("mega", "queue", "hybrid")
-    assert 0.0 < mt.hybrid_share() < 1.0
+    assert states[:4] == ["measuring"] * 4 and states[4] in ("mega", "queue") and len(set(states[4:])) == 1
     _, mega_ms, wf_ms = mt.pipeline_in_use()
     assert mega_ms > 0 and wf_ms > 0
-    if states[-1] != "hybrid":
-        assert states[-1] == ("queue" if wf_ms < mega_ms else "mega")
+    assert states[-1] == ("queue" if wf_ms < mega_ms else "mega")
     # a different geometry starts measuring again
     mt.render_chunk(files.camera, w, h, 0, 0, w // 2, h)
     assert mt.pipeline_in_use()[0] == "measuring"
@@ -541,12 +503,12 @@ def test_c4_stress_scene_tiles(product_lib, oracle_mod, scene_dir):
 def test_c5_4k_depth8_four_lights_tiles(product_lib, oracle_mod, scene_dir):
     """BASELINE config C5: the 500 k-triangle interior at 3840x2160, 4 lights, depth 8 -- tiles against the oracle
     with both pipelines."""
-    from mythtracer_b200 import MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT
+    from mythtracer_b200 import MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     files, cfg = scenes.config_scene("C5", scene_dir)
     assert len(files.lights) == 4 and cfg["depth"] == 8
     mt, orc = _pair_from_loader(product_lib, oracle_mod, files, cfg["depth"], files.lights)
     W, H = cfg["width"], cfg["height"]
-    for flags, (cx, cy, cw, ch) in [(MTB_FLAG_MEGAKERNEL, (1800, 1100, 96, 64)), (MTB_FLAG_WAVEFRONT, (2600, 1500, 80, 48))]:
+    for flags, (cx, cy, cw, ch) in [(MTB_FLAG_MEGAKERNEL, (1800, 1100, 96, 64)), (MTB_FLAG_QUEUE, (2600, 1500, 80, 48))]:
         mt.set_flags(flags)
         gpu = mt.render_chunk(files.camera, W, H, cx, cy, cw, ch, debug=True, taps=True)
         cpu = orc.render(files.camera, W, H, chunk=(cx, cy, cw, ch), depth=cfg["depth"], taps=True)
@@ -556,7 +518,7 @@ def test_c5_4k_depth8_four_lights_tiles(product_lib, oracle_mod, scene_dir):
 def test_edge_scenes(product_lib, oracle_mod, scene_dir):
     """Empty scene, a single triangle, zero-area and needle triangles, all triangles in one unsplit node, a ray
     batch of size 0 -- both pipelines."""
-    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT
+    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     from mythtracer_b200.api import MTL_DTYPE, TRI_DTYPE
     cam = (0.3, 0.4, -6.0, 2.0, 5.0, 1.0, 70.0)
     lights = [(1.0, 5.0, -4.0, 0.2, 0.2, 0.2, 1.0, 1.0, 1.0, 0.8, 0.8, 0.8)]
@@ -583,7 +545,7 @@ def test_edge_scenes(product_lib, oracle_mod, scene_dir):
         orc = oracle_mod.Oracle(tris, mtl, [])
         orc.set_lights(lights)
         cpu = orc.render(cam, 96, 64, depth=4, taps=True)
-        for flags in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT):
+        for flags in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE):
             mt = MythTracer(max_depth=4, flags=flags)
             mt.upload(tris, mtl)
             mt.GetScene().lights = [Light.from_tuple(l) for l in lights]
@@ -597,13 +559,13 @@ def test_fast_traversal_and_exact_octree_agree(product_lib, oracle_mod, scene_di
     """Regular rays are answered by the certified fast traversal (scene BVH, DESIGN.md section 4) by default and
     by the exact octree recursion under MTB_FLAG_EXACT_OCTREE.  Both against the oracle, every tap, both pipelines,
     on C1 (full frame), textured C2 and a C3 tile; the counters must show which traversal ran."""
-    from mythtracer_b200 import MTB_FLAG_COUNT_WORK, MTB_FLAG_EXACT_OCTREE, MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT
+    from mythtracer_b200 import MTB_FLAG_COUNT_WORK, MTB_FLAG_EXACT_OCTREE, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     for name, scale, (W, H), chunk in [("C1", 1.0, (320, 240), (0, 0, 320, 240)), ("C2", 0.3, (320, 180), (0, 0, 320, 180)),
                                         ("C3", 0.2, (1920, 1080), (900, 500, 128, 64))]:
         files, cfg = scenes.config_scene(name, scene_dir, scale)
         mt, orc = _load_pair(product_lib, oracle_mod, files, cfg["depth"], MTB_FLAG_MEGAKERNEL)
         cpu = orc.render(files.camera, W, H, chunk=chunk, depth=cfg["depth"], taps=True)
-        for pipe in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT):
+        for pipe in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE):
             for exact in (0, MTB_FLAG_EXACT_OCTREE):
                 mt.set_flags(pipe | exact | MTB_FLAG_COUNT_WORK)
                 gpu = mt.render_chunk(files.camera, W, H, *chunk, debug=True, taps=True)
@@ -623,7 +585,7 @@ def test_ambiguous_hits_fall_back_to_the_exact_recursion(product_lib, oracle_mod
     """Coincident triangles (exact ties in t: the reference's list order decides, octtree.cc:186-195), triangles that
     differ by 1e-13 (hits inside each other's error bound) and a grazing, ill-conditioned triangle: the fast
     traversal must declare these rays ambiguous and the exact recursion must give the reference's answer."""
-    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_COUNT_WORK, MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT
+    from mythtracer_b200 import Light, MythTracer, MTB_FLAG_COUNT_WORK, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     from mythtracer_b200.api import MTL_DTYPE, TRI_DTYPE
     cam = (0.3, 0.4, -6.0, 2.0, 5.0, 1.0, 70.0)
     lights = [(1.0, 5.0, -4.0, 0.2, 0.2, 0.2, 1.0, 1.0, 1.0, 0.8, 0.8, 0.8)]
@@ -648,7 +610,7 @@ def test_ambiguous_hits_fall_back_to_the_exact_recursion(product_lib, oracle_mod
     orc = oracle_mod.Oracle(tris, mtl, [])
     orc.set_lights(lights)
     cpu = orc.render(cam, 128, 96, depth=3, taps=True)
-    for flags in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT):
+    for flags in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE):
         mt = MythTracer(max_depth=3, flags=flags | MTB_FLAG_COUNT_WORK)
         mt.upload(tris, mtl)
         mt.GetScene().lights = [Light.from_tuple(l) for l in lights]
@@ -671,7 +633,7 @@ def test_fast_traversal_equals_exact_octree_at_full_size(product_lib, scene_dir)
     the same bytes and the same taps (hit ids, hit points, per-pixel ray counts, secondary-hit and shadow-decision
     signatures) on the whole C3 frame (22.5 M rays), on a 4K band of C5 (depth 8, 4 lights) and on a tile of the C4
     stress scene; the number of rays that needed the exact recursion is reported by the counters."""
-    from mythtracer_b200 import MTB_FLAG_COUNT_WORK, MTB_FLAG_EXACT_OCTREE, MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT
+    from mythtracer_b200 import MTB_FLAG_COUNT_WORK, MTB_FLAG_EXACT_OCTREE, MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE
     for name, chunk in [("C3", None), ("C5", (0, 1000, 3840, 96)), ("C4", (800, 500, 160, 64))]:
         files, cfg = scenes.config_scene(name, scene_dir)
         W, H = cfg["width"], cfg["height"]
@@ -681,7 +643,7 @@ def test_fast_traversal_equals_exact_octree_at_full_size(product_lib, scene_dir)
         assert mt.LoadObj(files.obj_path), mt.last_error()
         mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
         exact = mt.render_chunk(files.camera, W, H, *chunk, debug=True, taps=True)
-        for pipe in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_WAVEFRONT):
+        for pipe in (MTB_FLAG_MEGAKERNEL, MTB_FLAG_QUEUE):
             mt.set_flags(pipe | MTB_FLAG_COUNT_WORK)
             fast = mt.render_chunk(files.camera, W, H, *chunk, debug=True, taps=True)
             for k in ("rgb", "line_no", "points", "n_rays", "sig_hits", "sig_shadow"):
@@ -691,49 +653,6 @@ def test_fast_traversal_equals_exact_octree_at_full_size(product_lib, scene_dir)
             assert st["n_fast"] + st["n_fallback"] + st["n_literal"] == st["rays"]
             assert st["n_fallback"] < 1e-4 * st["rays"], "%s: %d rays fell back" % (name, st["n_fallback"])
         mt.close()
-
-
-def test_hybrid_frames(product_lib, oracle_mod, scene_dir):
-    """MTB_FLAG_HYBRID: from the second frame of a geometry on, the tiles that were most expensive in the previous
-    frame go through the wavefront pipeline while the megakernel renders the rest.  Every frame must carry the same
-    bytes and taps as the oracle's, whatever the split; also with a partition and with the counting build."""
-    from mythtracer_b200 import MTB_FLAG_COUNT_WORK, MTB_FLAG_HYBRID
-    files, cfg = scenes.config_scene("C2", scene_dir, 0.3)
-    mt, orc = _load_pair(product_lib, oracle_mod, files, cfg["depth"], MTB_FLAG_HYBRID)
-    w, h = 250, 141
-    cpu = orc.render(files.camera, w, h, depth=cfg["depth"], taps=True)
-    for flags in (MTB_FLAG_HYBRID, MTB_FLAG_HYBRID | MTB_FLAG_COUNT_WORK):
-        mt.set_flags(flags)
-        for frame in range(4):
-            gpu = mt.render_chunk(files.camera, w, h, 0, 0, w, h, debug=True, taps=True)
-            _assert_render_equal(gpu, cpu, "hybrid flags %d frame %d" % (flags, frame))
-    assert mt.pipeline_in_use()[0] == "hybrid"
-    full = gpu["rgb"].copy()
-    for rank in range(2):
-        mt.set_partition(rank, 2)
-        for frame in range(3):
-            part = mt.render_chunk(files.camera, w, h, 0, 0, w, h)["rgb"]
-        rows = np.arange(h)
-        own = ((rows // 8) % 2) == rank
-        assert np.array_equal(part[own], full[own])
-    mt.set_partition(0, 1)
-    # the full-size frame: same bytes as the megakernel alone, over several frames (the split follows the costs)
-    files, cfg = scenes.config_scene("C3", scene_dir)
-    from mythtracer_b200 import Light, MTB_FLAG_MEGAKERNEL
-    mt = _tracer(product_lib, cfg["depth"], MTB_FLAG_MEGAKERNEL)
-    assert mt.LoadObj(files.obj_path)
-    mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
-    W, H = cfg["width"], cfg["height"]
-    ref = mt.render_chunk(files.camera, W, H, 0, 0, W, H, taps=True)
-    mt.set_flags(MTB_FLAG_HYBRID)
-    shares = []
-    for frame in range(6):  # (the share of the frame that goes to the wavefront is steered from frame to frame)
-        got = mt.render_chunk(files.camera, W, H, 0, 0, W, H, taps=True)
-        shares.append(mt.hybrid_share())
-        for k in ("rgb", "n_rays", "sig_hits", "sig_shadow"):
-            assert np.array_equal(got[k], ref[k]), "C3 hybrid frame %d: %s" % (frame, k)
-        assert got["stats"]["rays"] == ref["stats"]["rays"]
-    assert len(set(shares)) > 1, "the split must move"
 
 
 def test_sibling_entry_tie_on_the_device(product_lib, oracle_mod):

@@ -4,10 +4,10 @@ about as long as one alone, the kernels of a share do not fill the machine (deve
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
-from mythtracer_b200 import MythTracer, Light, scenegen, MTB_FLAG_WAVEFRONT, tiles
+from mythtracer_b200 import MythTracer, Light, scenegen, tiles
 world = int(sys.argv[1]) if len(sys.argv) > 1 else 16
-mode = sys.argv[2] if len(sys.argv) > 2 else "wf"
-flags = {"wf": MTB_FLAG_WAVEFRONT, "mega": 16, "hybrid": 2048, "auto": 0}[mode]
+mode = sys.argv[2] if len(sys.argv) > 2 else "queue"
+flags = {"queue": 8192, "mega": 16, "auto": 0}[mode]
 files, cfg = scenegen.generate_config("C3", "/tmp/mtb_scenes")
 W, H = cfg["width"], cfg["height"]
 mts, streams, bufs = [], [], []

@@ -2,7 +2,7 @@
 import sys, os, time, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
-from mythtracer_b200 import MythTracer, Light, scenegen, MTB_FLAG_COUNT_WORK, MTB_FLAG_NO_LIST_BVH, MTB_FLAG_WAVEFRONT
+from mythtracer_b200 import MythTracer, Light, scenegen, MTB_FLAG_COUNT_WORK, MTB_FLAG_NO_LIST_BVH
 
 names = sys.argv[1].split(",") if len(sys.argv) > 1 else ["C1", "C2", "C3"]
 modes = sys.argv[2].split(",") if len(sys.argv) > 2 else ["bvh"]
@@ -10,7 +10,7 @@ out = []
 for name in names:
     files, cfg = scenegen.generate_config(name, "/tmp/mtb_scenes")
     for mode in modes:
-        base_flags = {"bvh": 16, "nobvh": MTB_FLAG_NO_LIST_BVH | 16, "wf": MTB_FLAG_WAVEFRONT, "wfsort": MTB_FLAG_WAVEFRONT | 8, "auto": 0, "noorder": 16 | 32, "persist": 16 | 64, "exact": 16 | 128, "pack": 16 | 256, "sync": 16 | 512, "resume": 16 | 1024, "hybrid": 2048, "wfexact": 4 | 128, "devbvh": 16 | 4096, "queue": 8192}.get(mode, 0)
+        base_flags = {"bvh": 16, "nobvh": MTB_FLAG_NO_LIST_BVH | 16, "auto": 0, "noorder": 16 | 32, "persist": 16 | 64, "exact": 16 | 128, "pack": 16 | 256, "sync": 16 | 512, "resume": 16 | 1024, "devbvh": 16 | 4096, "queue": 8192}.get(mode, 0)
         mt = MythTracer(max_depth=cfg["depth"], flags=base_flags)
         t0 = time.time(); assert mt.LoadObj(files.obj_path); t_load = time.time() - t0
         mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
