@@ -162,21 +162,35 @@ class MythTracer {
   // for every view.  RayTraceBatchAsync returns once the batch is queued (`out` pinned, from AllocFrames; Wait joins).
   bool RayTraceBatch(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
                      uint8_t *out) {
-    return RenderBatch(image_width, image_height, 1, cams, lights, out, true);
+    return RenderBatch(image_width, image_height, 1, cams, lights, out, nullptr, true);
   }
   bool RayTraceBatchAsync(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
                           uint8_t *pinned_out) {
-    return RenderBatch(image_width, image_height, 1, cams, lights, pinned_out, false);
+    return RenderBatch(image_width, image_height, 1, cams, lights, pinned_out, nullptr, false);
   }
   // Anti-aliased batches (mtb_render_batch_ss): samples_per_axis s = 1, 2, 4 or 8; every output pixel is the rounded
   // mean of the s x s pixels of the same view rendered at (s*w) x (s*h).  `out` holds cams.size() * w * h * 3 bytes.
   bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
                      const std::vector<std::vector<Light>> *lights, uint8_t *out) {
-    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, out, true);
+    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, out, nullptr, true);
   }
   bool RayTraceBatchAsync(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
                           const std::vector<std::vector<Light>> *lights, uint8_t *pinned_out) {
-    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, pinned_out, false);
+    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, pinned_out, nullptr, false);
+  }
+  // The same batch with the batch form of WorkChunk::output_debug (mtb_render_batch_debug): *debug_out is resized to
+  // cams.size() * (s*h) * (s*w) entries, view-major, the primary hit of every sample of every view (for s = 1, of every
+  // pixel): entry (x, y) of view v is what RayTrace(WorkChunk*) leaves for pixel (x, y) of an (s*w) x (s*h) frame.
+  bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
+                     const std::vector<std::vector<Light>> *lights, uint8_t *out, std::vector<PerPixelDebugInfo> *debug_out) {
+    // (other sizes are refused by the call before it writes anything; debug_out == nullptr: the overload above)
+    mtb_debug *dbg = nullptr;
+    if (debug_out != nullptr && (samples_per_axis == 1 || samples_per_axis == 2 || samples_per_axis == 4 || samples_per_axis == 8) &&
+        image_width > 0 && image_height > 0) {
+      debug_out->resize(cams.size() * (size_t)(samples_per_axis * image_height) * (size_t)(samples_per_axis * image_width));
+      dbg = reinterpret_cast<mtb_debug *>(debug_out->data());
+    }
+    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, out, dbg, true);
   }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
   static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
@@ -193,7 +207,7 @@ class MythTracer {
 
  private:
   bool RenderBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
-                   const std::vector<std::vector<Light>> *lights, uint8_t *out, bool synchronous) {
+                   const std::vector<std::vector<Light>> *lights, uint8_t *out, mtb_debug *dbg, bool synchronous) {
     if (!was_scene_finalized) {
       puts("Finalizing tree.");
       if (!scene.tree.Finalize(&scene.materials, &scene.textures)) return false;
@@ -225,9 +239,9 @@ class MythTracer {
     }
     const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
     mtb_stats stats;
-    // (samples_per_axis = 1: mtb_render_batch_ss is mtb_render_batch)
-    const int rc = synchronous ? mtb_render_batch_ss(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
-                                                     samples_per_axis, max_recursion_level, out, &stats)
+    // (samples_per_axis = 1: mtb_render_batch_ss is mtb_render_batch; dbg = NULL: mtb_render_batch_debug is mtb_render_batch_ss)
+    const int rc = synchronous ? mtb_render_batch_debug(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
+                                                        samples_per_axis, max_recursion_level, out, dbg, nullptr, &stats)
                                : mtb_render_batch_ss_async(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width,
                                                            image_height, samples_per_axis, max_recursion_level, out);
     if (rc != MTB_OK) {

@@ -80,7 +80,8 @@ typedef struct {
   double point[3]; /* NaN on a miss */
 } mtb_debug;
 
-/* Optional per-pixel decision taps (device-computed; used by the parity tests, see oracle/mt_oracle.h). */
+/* Optional per-pixel decision taps (device-computed; used by the parity tests, see oracle/mt_oracle.h).  The sizes
+ * below are those of mtb_render_chunk; mtb_render_batch_debug takes n_views * (s*image_h) * (s*image_w) entries. */
 typedef struct {
   uint64_t *sig_hits;   /* chunk_w*chunk_h, may be NULL */
   uint64_t *sig_shadow; /* chunk_w*chunk_h, may be NULL */
@@ -272,6 +273,22 @@ int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_view
 int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
                               int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
                               uint8_t *rgb_out);
+
+/* Batches with per-pixel planes: mtb_render_batch_ss (synchronous), which also returns for every view what
+ * mtb_render_chunk returns for a frame besides its bytes: the PerPixelDebugInfo of the primary hit (line_no and point,
+ * -1 / NaN on a miss; WorkChunk::output_debug) and the taps.  The planes live on each view's sample grid, of
+ * (s*image_w) x (s*image_h) entries: entry (x, y) of view v is exactly what mtb_render_chunk writes for pixel (x, y)
+ * of an (s*image_w) x (s*image_h) frame rendered with cams[v] and view v's lights.  For s = 1 that is the view itself;
+ * for s > 1 they are the planes of the samples (no per-output-pixel aggregate is formed).
+ *
+ * dbg_out and each pointer of taps (and taps itself) may be NULL; each non-NULL one is a HOST array of
+ * n_views * (s*image_h) * (s*image_w) entries, view-major and row-major.  With every plane NULL the call is
+ * mtb_render_batch_ss.  rgb_out and stats are those of the same call without planes, byte for byte.  Arguments,
+ * limits and the partition rule are those of mtb_render_batch_ss.  With several devices every device copies the
+ * planes of its own views; there is no gather.  The single-frame path's debug and tap buffers are not used. */
+int mtb_render_batch_debug(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights,
+                           int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                           uint8_t *rgb_out, mtb_debug *dbg_out, const mtb_taps *taps, mtb_stats *stats);
 
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the

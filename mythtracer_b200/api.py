@@ -79,7 +79,7 @@ EXPORTED_SYMBOLS = [
     "mtb_scene_triangle_nodes", "mtb_scene_bvh", "mtb_set_flags", "mtb_set_partition", "mtb_render_chunk",
     "mtb_render_chunk_device", "mtb_render_chunk_async", "mtb_wait", "mtb_host_alloc", "mtb_host_free", "mtb_read_counters", "mtb_launch_count", "mtb_pipeline_in_use", "mtb_intersect_rays", "mtb_camera_sensor", "mtb_version",
     "mtb_frame_create", "mtb_frame_open", "mtb_frame_release", "mtb_frame_read", "mtb_load_timing", "mtb_hybrid_share",
-    "mtb_render_batch", "mtb_render_batch_async", "mtb_render_batch_ss", "mtb_render_batch_ss_async",
+    "mtb_render_batch", "mtb_render_batch_async", "mtb_render_batch_ss", "mtb_render_batch_ss_async", "mtb_render_batch_debug",
 ]
 
 
@@ -135,6 +135,7 @@ def load_library():
     lib.mtb_render_batch_async.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, vp]
     lib.mtb_render_batch_ss.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp]
     lib.mtb_render_batch_ss_async.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp]
+    lib.mtb_render_batch_debug.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp]
     lib.mtb_read_counters.argtypes = [vp, vp]
     lib.mtb_pipeline_in_use.argtypes = [vp, vp, vp]
     lib.mtb_launch_count.argtypes = [vp]
@@ -465,18 +466,26 @@ class MythTracer:
         self.last_stats = res["stats"]
         return res
 
-    def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None, samples_per_axis: int = 1):
+    def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None, samples_per_axis: int = 1,
+                     debug: bool = False, taps: bool = False):
         """mtb_render_batch: len(cameras) whole frames in one launch per device, at depth self.max_depth.
 
         lights: None (every view uses GetScene().lights) or one list of Light per view, all of the same length.
         samples_per_axis: 1, 2, 4 or 8.  s > 1 renders anti-aliased views through mtb_render_batch_ss: each output pixel
         is the rounded mean of the s x s pixels of the same view rendered at (s*width) x (s*height).
         Returns dict(rgb=uint8[n, height, width, 3], stats) with the stats summed over the views (those of the
-        s*width x s*height samples)."""
+        s*width x s*height samples).
+
+        debug / taps: also return the planes render_chunk returns (through mtb_render_batch_debug): debug, line_no and
+        points, and sig_hits, sig_shadow and n_rays, each of shape (n, s*height, s*width) - one entry per sample, entry
+        (x, y) of view v being that of pixel (x, y) of view v rendered by render_chunk at (s*width) x (s*height)."""
         ss = samples_per_axis
         if isinstance(ss, bool) or not isinstance(ss, (int, np.integer)) or ss not in (1, 2, 4, 8):
             raise MythTracerError("render_batch: samples_per_axis must be 1, 2, 4 or 8 (got %r)" % (ss,))
         ss = int(ss)
+        for name, flag in (("debug", debug), ("taps", taps)):
+            if not isinstance(flag, (bool, np.bool_)):
+                raise MythTracerError("render_batch: %s must be True or False (got %r)" % (name, flag))
         cams = [c if isinstance(c, Camera) else Camera.from_tuple(c) for c in cameras]
         if not cams:
             raise MythTracerError("render_batch: no cameras")
@@ -504,13 +513,32 @@ class MythTracer:
                 raise MythTracerError("render_batch: out must be a C-contiguous uint8 array of shape %s" % (shape,))
             rgb = out
         stats = np.zeros((), STATS_DTYPE)
-        if ss == 1:
+        res = {}
+        if debug or taps:
+            plane = (len(cams), ss * height, ss * width)
+            dbg = np.zeros(plane, DEBUG_DTYPE) if debug else None
+            tap_ptr = None
+            if taps:
+                res["sig_hits"] = np.zeros(plane, np.uint64)
+                res["sig_shadow"] = np.zeros(plane, np.uint64)
+                res["n_rays"] = np.zeros(plane, np.uint32)
+                tap_struct = _TapsStruct(res["sig_hits"].ctypes.data, res["sig_shadow"].ctypes.data, res["n_rays"].ctypes.data)
+                tap_ptr = ctypes.cast(ctypes.pointer(tap_struct), ctypes.c_void_p)
+            self._check(self._lib.mtb_render_batch_debug(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
+                                                         ss, self.max_depth, _ptr(rgb), _ptr(dbg), tap_ptr, _ptr(stats)),
+                        "mtb_render_batch_debug")
+            if debug:
+                res["debug"] = dbg
+                res["line_no"] = dbg["line_no"]
+                res["points"] = dbg["point"]
+        elif ss == 1:
             self._check(self._lib.mtb_render_batch(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
                                                    self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch")
         else:
             self._check(self._lib.mtb_render_batch_ss(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
                                                       ss, self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch_ss")
-        res = {"rgb": rgb, "stats": {k: stats[k].item() for k in STATS_DTYPE.names}}
+        res["rgb"] = rgb
+        res["stats"] = {k: stats[k].item() for k in STATS_DTYPE.names}
         self.last_stats = res["stats"]
         return res
 

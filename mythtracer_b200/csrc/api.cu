@@ -105,11 +105,15 @@ struct DeviceState {
   int tune_stage = 0;              // see RenderImpl
   float tune_ms[2] = {0.f, 0.f};   // megakernel, queue pipeline
   bool tune_queue = false;         // the decision: the queue pipeline (else the megakernel)
-  // batch launches (RenderBatchImpl): view records, per-view lights and the views' frames of this device, and the
-  // events that time them (the single-frame events steer the automatic pipeline choice and are left alone)
+  // batch launches (RenderBatchImpl): view records, per-view lights and the views' frames of this device, the debug and
+  // tap planes of those views (only when a batch asks for them), and the events that time them (the single-frame
+  // events steer the automatic pipeline choice and are left alone)
   DeviceBuffer<mtb::ViewRec> batch_views;
   DeviceBuffer<mtb_light> batch_lights;
   DeviceBuffer<uint8_t> batch_rgb;
+  DeviceBuffer<mtb_debug> batch_dbg;
+  DeviceBuffer<uint64_t> batch_sig_hits, batch_sig_shadow;
+  DeviceBuffer<uint32_t> batch_n_rays;
   cudaEvent_t ev_batch_start = nullptr, ev_batch_stop = nullptr;
   // intersect scratch
   DeviceBuffer<double> q_origins, q_dirs, q_t, q_point;
@@ -133,7 +137,7 @@ struct DeviceState {
     nodes.Free(); slots.Free(); shade.Free(); bvh.Free(); gnodes.Free(); gslots.Free(); list_order.Free(); slot_node.Free(); leaf_ref.Free(); ref_slot.Free(); materials.Free();
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
     counters.Free(); tile_cost.Free(); tile_order.Free();
-    batch_views.Free(); batch_lights.Free(); batch_rgb.Free();
+    batch_views.Free(); batch_lights.Free(); batch_rgb.Free(); batch_dbg.Free(); batch_sig_hits.Free(); batch_sig_shadow.Free(); batch_n_rays.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
     if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
     ev_batch_start = ev_batch_stop = nullptr;
@@ -783,9 +787,12 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 // lights == NULL: every view uses the context's lights.  Device g renders a contiguous range of views; the counts
 // differ by at most one.  ss > 1 (samples per axis, 2, 4 or 8): every view is traced on the (ss*W) x (ss*H) sample grid,
 // exactly as a batch of that size, and the kernel writes the W x H block means; everything else is as for ss = 1.
+// dbg_host / taps (nullable, HOST): the per-pixel debug info and taps of every view on its sample grid, view-major; each
+// device copies the planes of its own views.
 constexpr int64_t kMaxSampleSide = 65536;  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
 int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
-                    int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_stats *stats, bool synchronous) {
+                    int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps, mtb_stats *stats,
+                    bool synchronous) {
   const auto wall0 = std::chrono::steady_clock::now();
   if (ctx == nullptr) return MTB_ERR_ARG;
   if (ctx->dev.empty()) {
@@ -826,6 +833,10 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
   }
   const size_t npx = (size_t)image_w * image_h;  // output pixels of a view
   const int grid_w = image_w * ss, grid_h = image_h * ss;  // its sample grid (the view itself when ss = 1)
+  const size_t gpx = (size_t)grid_w * grid_h;              // entries of each of its debug / tap planes
+  uint64_t *const hits_host = taps != nullptr ? taps->sig_hits : nullptr;
+  uint64_t *const shadow_host = taps != nullptr ? taps->sig_shadow : nullptr;
+  uint32_t *const rays_host = taps != nullptr ? taps->n_rays : nullptr;
   const bool debug_build = (ctx->flags & MTB_FLAG_COUNT_WORK) != 0;
   const int n_dev = (int)ctx->dev.size();
   const int tiles_x = (grid_w + 7) / 8, tiles_per_view = tiles_x * ((grid_h + 7) / 8);
@@ -879,7 +890,11 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     // still read it is waited for first.
     const size_t n_rgb = host_direct != nullptr ? 0 : (size_t)count * npx * 3;
     const size_t n_lt = (size_t)count * nl;
-    if ((size_t)count > d.batch_views.count || n_lt > d.batch_lights.count || n_rgb > d.batch_rgb.count) {
+    const size_t n_plane = (size_t)count * gpx;
+    auto grows = [n_plane](const void *host, size_t have) { return host != nullptr && n_plane > have; };
+    if ((size_t)count > d.batch_views.count || n_lt > d.batch_lights.count || n_rgb > d.batch_rgb.count ||
+        grows(dbg_host, d.batch_dbg.count) || grows(hits_host, d.batch_sig_hits.count) || grows(shadow_host, d.batch_sig_shadow.count) ||
+        grows(rays_host, d.batch_n_rays.count)) {
       MTB_CUDA(ctx, cudaStreamSynchronize(s));
     }
     MTB_CUDA(ctx, d.batch_views.Upload(views.data() + first, (size_t)count, s));
@@ -888,8 +903,24 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     mtb::DeviceScene sc = d.scene;
     sc.lights = d.batch_lights.ptr;
     sc.n_lights = nl;
-    mtb::RenderParams p = rp;
+    mtb::RenderParams p = rp;  // (planes NULL unless this batch asks for them)
     p.rgb = host_direct != nullptr ? host_direct + (size_t)first * npx * 3 : d.batch_rgb.ptr;
+    if (dbg_host != nullptr) {
+      MTB_CUDA(ctx, d.batch_dbg.Reserve(n_plane));
+      p.dbg = d.batch_dbg.ptr;
+    }
+    if (hits_host != nullptr) {
+      MTB_CUDA(ctx, d.batch_sig_hits.Reserve(n_plane));
+      p.sig_hits = d.batch_sig_hits.ptr;
+    }
+    if (shadow_host != nullptr) {
+      MTB_CUDA(ctx, d.batch_sig_shadow.Reserve(n_plane));
+      p.sig_shadow = d.batch_sig_shadow.ptr;
+    }
+    if (rays_host != nullptr) {
+      MTB_CUDA(ctx, d.batch_n_rays.Reserve(n_plane));
+      p.n_rays = d.batch_n_rays.ptr;
+    }
     MTB_CUDA(ctx, d.counters.Reserve(mtb::kNumCounters));
     p.counters = d.counters.ptr;
     if (stats != nullptr || synchronous) {
@@ -903,6 +934,11 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     if (host_direct == nullptr) {
       MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first * npx * 3, d.batch_rgb.ptr, (size_t)count * npx * 3, cudaMemcpyDeviceToHost, s));
     }
+    const size_t at = (size_t)first * gpx;
+    if (dbg_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(dbg_host + at, p.dbg, n_plane * sizeof(mtb_debug), cudaMemcpyDeviceToHost, s));
+    if (hits_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(hits_host + at, p.sig_hits, n_plane * 8, cudaMemcpyDeviceToHost, s));
+    if (shadow_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(shadow_host + at, p.sig_shadow, n_plane * 8, cudaMemcpyDeviceToHost, s));
+    if (rays_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(rays_host + at, p.n_rays, n_plane * 4, cudaMemcpyDeviceToHost, s));
     return MTB_OK;
   };
   if (n_dev == 1) {
@@ -1274,22 +1310,29 @@ int mtb_render_chunk_async(mtb_context *ctx, const mtb_camera *cam, int image_w,
 
 int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                      int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, stats, true);
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, false);
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                         int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, stats, true);
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                               int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, false);
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+}
+
+int mtb_render_batch_debug(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
+                           int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_debug *dbg_out,
+                           const mtb_taps *taps, mtb_stats *stats) {
+  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
+                         true);
 }
 
 int mtb_wait(mtb_context *ctx) {

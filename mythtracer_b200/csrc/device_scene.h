@@ -123,8 +123,9 @@ void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles,
 // One 8x8 tile per 64-thread block; n_blocks = tiles of the launch (rp.tiles_x in units of 8 pixels).
 void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_blocks, bool debug_build, cudaStream_t stream);
 // n_views whole frames in one launch: grid (tiles_per_view, n_views), camera of view v = views[v] (device memory), its
-// lights sc.lights + v * sc.n_lights, its pixels rp.rgb + v * chunk_w * chunk_h * 3.  rp.strip_first = 0,
-// rp.strip_stride = 1, and tile_order / tile_cost / run_if / taps / dbg NULL.
+// lights sc.lights + v * sc.n_lights, its pixels rp.rgb + v * chunk_w * chunk_h * 3, its debug / tap entries (each
+// plane nullable) rp.dbg / sig_hits / sig_shadow / n_rays + v * chunk_w * chunk_h.  rp.strip_first = 0,
+// rp.strip_stride = 1, and tile_order / tile_cost / run_if NULL.
 // samples_per_axis s = 2, 4 or 8: supersampled views.  rp.chunk_w x rp.chunk_h (and views[v].sensor) describe the
 // s*W x s*H sample grid, tiles_per_view counts its tiles, and view v's W x H output pixels (each the rounded mean of
 // its s x s samples) go to rp.rgb + v * W * H * 3.  s = 1: the plain batch above.

@@ -85,6 +85,12 @@ template <bool BATCH>
 __device__ __forceinline__ uint8_t *ViewFrame(const RenderParams &rp) {
   return BATCH ? rp.rgb + (size_t)blockIdx.y * rp.chunk_w * rp.chunk_h * 3 : rp.rgb;
 }
+// ... and the entry of pixel (px, py) in its debug and tap planes (view-major planes of chunk_w x chunk_h entries: for a
+// supersampled batch, the sample grid).
+template <bool BATCH>
+__device__ __forceinline__ size_t PlaneIndex(const RenderParams &rp, int px, int py) {
+  return (BATCH ? (size_t)blockIdx.y * rp.chunk_w * rp.chunk_h : 0) + (size_t)py * rp.chunk_w + px;
+}
 
 // Supersampled batch (SS = 2, 4, 8 samples per axis): the tile is a tile of the (SS*W) x (SS*H) sample grid (rp.chunk_w
 // x rp.chunk_h), every thread traces one sample exactly as a pixel of that frame, and the epilogue writes the
@@ -148,7 +154,8 @@ __device__ __forceinline__ void SupersampleEpilogue(const RenderParams &rp, cons
 
 // BATCH: grid (tiles per view, views), block b of row v renders tile b of view v in scanline order; the camera comes from
 // views[v] and the pixels go to rp.rgb + v * chunk_w * chunk_h * 3.  A batch launch passes NULL for tile_order,
-// tile_cost, run_if and the taps / debug planes.  Without BATCH, `views` is unused and every `BATCH ? :`
+// tile_cost and run_if; its debug and tap planes (NULL unless the caller asked for them) are view-major, view v's entries
+// start at v * chunk_w * chunk_h (PlaneIndex).  Without BATCH, `views` is unused and every `BATCH ? :`
 // folds away: the single-view kernels compile to the code they had before the batch form existed.  SS > 1 (BATCH only):
 // the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.
 template <bool DBG, bool BATCH, int SS>
@@ -297,7 +304,7 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         // ---- result of a primary / reflection / refraction ray (mythtracer.cc:13-76) ----
         if (slot < 0) {
           if (st.level == 0 && rp.dbg != nullptr) {
-            mtb_debug *dbg = rp.dbg + (size_t)py * rp.chunk_w + px;
+            mtb_debug *dbg = rp.dbg + PlaneIndex<BATCH>(rp, px, py);
             dbg->line_no = -1;
             dbg->pad_ = 0;
             dbg->point[0] = dbg->point[1] = dbg->point[2] = CUDART_NAN;
@@ -310,7 +317,7 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
           const D3 P = Add(Ld3(st.m_o), MulS(m_d, t));
           const int line_no = __ldg(&sh->line_no);
           if (st.level == 0 && rp.dbg != nullptr) {
-            mtb_debug *dbg = rp.dbg + (size_t)py * rp.chunk_w + px;
+            mtb_debug *dbg = rp.dbg + PlaneIndex<BATCH>(rp, px, py);
             dbg->line_no = line_no;
             dbg->pad_ = 0;
             dbg->point[0] = P.x;
@@ -448,7 +455,7 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
       out[0] = QuantizeChannel(ret.x);
       out[1] = QuantizeChannel(ret.y);
       out[2] = QuantizeChannel(ret.z);
-      const size_t pix = (size_t)py * rp.chunk_w + px;
+      const size_t pix = PlaneIndex<BATCH>(rp, px, py);
       if (rp.sig_hits != nullptr) rp.sig_hits[pix] = st.sig_hits;
       if (rp.sig_shadow != nullptr) rp.sig_shadow[pix] = st.sig_shadow;
       n_rays = st.n_rays;

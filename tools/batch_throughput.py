@@ -1,7 +1,7 @@
 """Throughput of batches (mtb_render_batch) against one call per frame, on the C3 scene (two lights, depth 5) and its
 orbit yaw = C3 yaw + 2 degrees * k.
 
-    python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3] [--supersample]
+    python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3] [--supersample | --debug-planes]
 
 480x270, 64 frames: (a) one render_chunk per frame, megakernel forced; (b) one render_chunk per frame, automatic
 pipeline choice (after the 13 frames it needs to decide); (c) render_batch in batches of 1, 4, 16, 64.
@@ -20,6 +20,12 @@ are read in the same run.  Prints one JSON document (and writes it to --out).
 at s*W x s*H plus the block mean in numpy (frames/s end to end).  Per mode: median kernel_ms per call over --reps calls,
 Mrays/s, frames/s, and whether every view equals the block mean of the 1920x1080 views.  Then the work per ray of each
 mode from the counting build (not timed).
+
+--debug-planes measures batches that also return per-pixel planes (render_batch(..., debug=True / taps=True)): 64 C3
+views at 480x270 and 8 at 1920x1080, each with neither, with debug, with taps and with both, against one
+render_chunk(debug=True) per frame (megakernel).  Per mode: median kernel_ms per call (summed over the calls of a
+pass for render_chunk), frames/s end to end, Mrays/s and the bytes copied back per view; whether the RGB equals that of
+the batch without planes, and whether the planes of the first and the last view equal render_chunk's.
 """
 import argparse
 import hashlib
@@ -182,10 +188,67 @@ def supersample(mt, files, cfg, reps):
     return dict(shape="C3 orbit, %d views" % n, modes=recs, work_per_ray=work)
 
 
+PLANE_KEYS = ("debug", "sig_hits", "sig_shadow", "n_rays")
+
+
+def debug_planes(mt, files, cfg, reps):
+    """The --debug-planes measurements (see the module docstring)."""
+    groups = []
+    for w, h, n in ((480, 270, 64), (cfg["width"], cfg["height"], 8)):
+        cams = _orbit(files.camera, n)
+        recs, rgb0 = [], None
+        for debug, taps in ((False, False), (True, False), (False, True), (True, True)):
+            last = {}
+
+            def call():
+                last.update(mt.render_batch(cams, w, h, debug=debug, taps=taps))
+                return last["stats"]
+            walls, kms, rays = _timed_calls(call, reps)
+            if rgb0 is None:
+                rgb0 = last["rgb"].copy()
+            per_view = w * h * (3 + (32 if debug else 0) + (20 if taps else 0))
+            name = "render_batch %d x %dx%d, %s" % (n, w, h, {(False, False): "no planes", (True, False): "debug", (False, True): "taps",
+                                                           (True, True): "debug + taps"}[(debug, taps)])
+            rec = _ss_record(name, n, w, h, 1, walls, kms, rays, None)
+            del rec["equals_block_mean_of_1080p"]
+            rec.update(debug=debug, taps=taps, bytes_copied_per_view=per_view, rgb_equals_no_planes=bool(np.array_equal(last["rgb"], rgb0)))
+            if debug or taps:
+                same = True
+                for v in (0, n - 1):
+                    single = mt.render_chunk(cams[v], w, h, 0, 0, w, h, debug=True, taps=True)
+                    same &= all(last[k][v].tobytes() == single[k].tobytes() for k in PLANE_KEYS if k in last)
+                rec["planes_equal_render_chunk"] = bool(same)
+            recs.append(rec)
+
+        def singles():
+            kms, nr = 0.0, 0
+            for cam in cams:
+                st = mt.render_chunk(cam, w, h, 0, 0, w, h, debug=True)["stats"]
+                kms += st["kernel_ms"]
+                nr += st["rays"]
+            return dict(kernel_ms=kms, rays=nr)
+        walls, kms, rays = _timed_calls(singles, reps)
+        rec = _ss_record("render_chunk(debug=True) x %d, %dx%d" % (n, w, h), n, w, h, 1, walls, kms, rays, None)
+        del rec["equals_block_mean_of_1080p"]
+        rec.update(debug=True, taps=False, bytes_copied_per_view=w * h * (3 + 32))
+        recs.append(rec)
+        groups.append(dict(shape="C3 orbit, %d views at %dx%d" % (n, w, h), modes=recs))
+    return groups
+
+
 def _group(title, w, h, recs):
     first = recs[0]["frame_sha256"]
     same = all(r["frame_sha256"] == first for r in recs)
     return dict(shape=title, width=w, height=h, frames_identical_across_modes=same, modes=recs)
+
+
+def _emit(doc, out):
+    text = json.dumps(doc, indent=1)
+    print(text)
+    if out:
+        os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
+        with open(out, "w") as f:
+            f.write(text + "\n")
 
 
 def main():
@@ -194,6 +257,7 @@ def main():
     ap.add_argument("--out", default=None)
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--supersample", action="store_true")
+    ap.add_argument("--debug-planes", action="store_true")
     args = ap.parse_args()
     devices = [int(x) for x in args.devices.split(",")]
     files, cfg = scenegen.generate_config("C3", os.environ.get("MTB_SCENE_DIR", "/tmp/mtb_scenes"))
@@ -205,15 +269,19 @@ def main():
     assert mt.LoadObj(files.obj_path), mt.last_error()
     mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]
 
+    if args.debug_planes:
+        doc["debug_planes"] = debug_planes(mt, files, cfg, args.reps)
+        mt.close()
+        _emit(doc, args.out)
+        modes = [r for g in doc["debug_planes"] for r in g["modes"]]
+        if not all(r.get("rgb_equals_no_planes", True) and r.get("planes_equal_render_chunk", True) for r in modes):
+            sys.exit("a batch with planes differs from the batch without planes or from render_chunk")
+        return
+
     if args.supersample:
         doc["supersample"] = supersample(mt, files, cfg, args.reps)
         mt.close()
-        text = json.dumps(doc, indent=1)
-        print(text)
-        if args.out:
-            os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-            with open(args.out, "w") as f:
-                f.write(text + "\n")
+        _emit(doc, args.out)
         if not all(r["equals_block_mean_of_1080p"] is not False for r in doc["supersample"]["modes"]):
             sys.exit("a supersampled mode differs from the block means of the 1080p views")
         return
@@ -277,12 +345,7 @@ def main():
         doc["groups"].append(_group("480x270 x 64 on devices %s" % args.devices, w, h, recs))
         many.close()
 
-    text = json.dumps(doc, indent=1)
-    print(text)
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write(text + "\n")
+    _emit(doc, args.out)
     if not all(g["frames_identical_across_modes"] for g in doc["groups"]):
         sys.exit("frames differ between modes")
 
