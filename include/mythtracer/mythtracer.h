@@ -162,21 +162,21 @@ class MythTracer {
   // for every view.  RayTraceBatchAsync returns once the batch is queued (`out` pinned, from AllocFrames; Wait joins).
   bool RayTraceBatch(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
                      uint8_t *out) {
-    return RenderBatch(image_width, image_height, 1, cams, lights, out, nullptr, true);
+    return RenderBatch(image_width, image_height, 1, 1, cams, lights, out, nullptr, true);
   }
   bool RayTraceBatchAsync(int image_width, int image_height, const std::vector<Camera> &cams, const std::vector<std::vector<Light>> *lights,
                           uint8_t *pinned_out) {
-    return RenderBatch(image_width, image_height, 1, cams, lights, pinned_out, nullptr, false);
+    return RenderBatch(image_width, image_height, 1, 1, cams, lights, pinned_out, nullptr, false);
   }
   // Anti-aliased batches (mtb_render_batch_ss): samples_per_axis s = 1, 2, 4 or 8; every output pixel is the rounded
   // mean of the s x s pixels of the same view rendered at (s*w) x (s*h).  `out` holds cams.size() * w * h * 3 bytes.
   bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
                      const std::vector<std::vector<Light>> *lights, uint8_t *out) {
-    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, out, nullptr, true);
+    return RenderBatch(image_width, image_height, samples_per_axis, 1, cams, lights, out, nullptr, true);
   }
   bool RayTraceBatchAsync(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
                           const std::vector<std::vector<Light>> *lights, uint8_t *pinned_out) {
-    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, pinned_out, nullptr, false);
+    return RenderBatch(image_width, image_height, samples_per_axis, 1, cams, lights, pinned_out, nullptr, false);
   }
   // The same batch with the batch form of WorkChunk::output_debug (mtb_render_batch_debug): *debug_out is resized to
   // cams.size() * (s*h) * (s*w) entries, view-major, the primary hit of every sample of every view (for s = 1, of every
@@ -190,7 +190,19 @@ class MythTracer {
       debug_out->resize(cams.size() * (size_t)(samples_per_axis * image_height) * (size_t)(samples_per_axis * image_width));
       dbg = reinterpret_cast<mtb_debug *>(debug_out->data());
     }
-    return RenderBatch(image_width, image_height, samples_per_axis, cams, lights, out, dbg, true);
+    return RenderBatch(image_width, image_height, samples_per_axis, 1, cams, lights, out, dbg, true);
+  }
+  // Accumulated batches (mtb_render_batch_accum): every output view is the rounded mean of all subframes * s * s
+  // samples of its `subframes` sub-frames (motion blur: a camera path over the shutter interval; soft shadows: jittered
+  // positions on an area light).  cams (and *lights) hold `subframes` entries per output view, output-major; `out` holds
+  // cams.size() / subframes * w * h * 3 bytes.  subframes = 1: the overloads above.
+  bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
+                     const std::vector<std::vector<Light>> *lights, uint8_t *out) {
+    return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, out, nullptr, true);
+  }
+  bool RayTraceBatchAsync(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
+                          const std::vector<std::vector<Light>> *lights, uint8_t *pinned_out) {
+    return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, pinned_out, nullptr, false);
   }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
   static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
@@ -206,7 +218,7 @@ class MythTracer {
   mtb_stats last_stats{};
 
  private:
-  bool RenderBatch(int image_width, int image_height, int samples_per_axis, const std::vector<Camera> &cams,
+  bool RenderBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
                    const std::vector<std::vector<Light>> *lights, uint8_t *out, mtb_debug *dbg, bool synchronous) {
     if (!was_scene_finalized) {
       puts("Finalizing tree.");
@@ -239,11 +251,24 @@ class MythTracer {
     }
     const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
     mtb_stats stats;
-    // (samples_per_axis = 1: mtb_render_batch_ss is mtb_render_batch; dbg = NULL: mtb_render_batch_debug is mtb_render_batch_ss)
-    const int rc = synchronous ? mtb_render_batch_debug(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
-                                                        samples_per_axis, max_recursion_level, out, dbg, nullptr, &stats)
-                               : mtb_render_batch_ss_async(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width,
-                                                           image_height, samples_per_axis, max_recursion_level, out);
+    int rc;
+    if (subframes != 1) {
+      if (subframes < 1 || cams.size() % (size_t)subframes != 0) {
+        fprintf(stderr, "error: %zu cameras are not a whole number of output views of %d subframes\n", cams.size(), subframes);
+        return false;
+      }
+      const int32_t n_out = (int32_t)(cams.size() / (size_t)subframes);
+      rc = synchronous ? mtb_render_batch_accum(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
+                                                max_recursion_level, out, &stats)
+                       : mtb_render_batch_accum_async(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height,
+                                                      samples_per_axis, max_recursion_level, out);
+    } else {
+      // (samples_per_axis = 1: mtb_render_batch_ss is mtb_render_batch; dbg = NULL: mtb_render_batch_debug is mtb_render_batch_ss)
+      rc = synchronous ? mtb_render_batch_debug(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
+                                                samples_per_axis, max_recursion_level, out, dbg, nullptr, &stats)
+                       : mtb_render_batch_ss_async(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,
+                                                   samples_per_axis, max_recursion_level, out);
+    }
     if (rc != MTB_OK) {
       fprintf(stderr, "error: %s\n", mtb_last_error(ctx));
       return false;

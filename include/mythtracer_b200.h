@@ -290,6 +290,31 @@ int mtb_render_batch_debug(mtb_context *ctx, const mtb_camera *cams, int32_t n_v
                            int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
                            uint8_t *rgb_out, mtb_debug *dbg_out, const mtb_taps *taps, mtb_stats *stats);
 
+/* Accumulated batches (motion blur, soft shadows from area lights): every output view is the mean of k = subframes
+ * sub-frames, each with its own camera and light set.  Sub-frame u = v*k + j (j < k) of output view v uses cams[u]
+ * and lights[u*n_lights .. +n_lights).  With F_u the frame mtb_render_batch renders for sub-frame u at
+ * (s*image_w) x (s*image_h), s = samples_per_axis, output pixel (x, y) channel c of view v is
+ *     (sum over j < k, a, b < s of F_{v*k+j}[s*y + b][s*x + a][c] + k*s*s/2) / (k*s*s)      (integer division)
+ * the rounded-half-up mean of all k*s*s quantised samples (not a mean of per-sub-frame means).  The sums are formed
+ * on the device in integers, so the bytes depend neither on the order in which the sub-frames finish nor on the
+ * number of devices.  k = 1 is exactly mtb_render_batch_ss.  The library chooses no sub-frames itself: a camera path
+ * over the shutter interval gives motion blur, jittered positions on an area light give soft shadows.
+ *
+ * cams: n_out * subframes entries, output-major.  lights: n_out * subframes * n_lights entries, or NULL (every
+ * sub-frame uses the context's lights).  rgb_out: HOST, n_out * image_h * image_w * 3 bytes, view-major.
+ * subframes >= 1, n_out >= 1 and n_out * subframes <= 65535 (one grid row per sub-frame), else MTB_ERR_ARG; every
+ * other argument rule is that of mtb_render_batch_ss.  stats (nullable): those of the n_out * subframes sub-frames at
+ * (s*image_w) x (s*image_h) (rays and, under MTB_FLAG_COUNT_WORK, every work counter).  With several devices, device g
+ * renders a contiguous range of output views with all their sub-frames; there is no gather.  There are no debug or
+ * tap planes of accumulated views: mtb_render_batch_debug returns those of the sub-frames. */
+int mtb_render_batch_accum(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
+                           int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out,
+                           mtb_stats *stats);
+/* Same, returns once queued (rgb_out pinned, from mtb_host_alloc; mtb_wait joins). */
+int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes,
+                                 const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis,
+                                 int max_depth, uint8_t *rgb_out);
+
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the
  * context has one device.  This is the entry bench.py times for the HBM-resident figure. */

@@ -80,6 +80,7 @@ EXPORTED_SYMBOLS = [
     "mtb_render_chunk_device", "mtb_render_chunk_async", "mtb_wait", "mtb_host_alloc", "mtb_host_free", "mtb_read_counters", "mtb_launch_count", "mtb_pipeline_in_use", "mtb_intersect_rays", "mtb_camera_sensor", "mtb_version",
     "mtb_frame_create", "mtb_frame_open", "mtb_frame_release", "mtb_frame_read", "mtb_load_timing", "mtb_hybrid_share",
     "mtb_render_batch", "mtb_render_batch_async", "mtb_render_batch_ss", "mtb_render_batch_ss_async", "mtb_render_batch_debug",
+    "mtb_render_batch_accum", "mtb_render_batch_accum_async",
 ]
 
 
@@ -136,6 +137,8 @@ def load_library():
     lib.mtb_render_batch_ss.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp]
     lib.mtb_render_batch_ss_async.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp]
     lib.mtb_render_batch_debug.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp]
+    lib.mtb_render_batch_accum.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp]
+    lib.mtb_render_batch_accum_async.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp]
     lib.mtb_read_counters.argtypes = [vp, vp]
     lib.mtb_pipeline_in_use.argtypes = [vp, vp, vp]
     lib.mtb_launch_count.argtypes = [vp]
@@ -467,7 +470,7 @@ class MythTracer:
         return res
 
     def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None, samples_per_axis: int = 1,
-                     debug: bool = False, taps: bool = False):
+                     debug: bool = False, taps: bool = False, subframes: int = 1):
         """mtb_render_batch: len(cameras) whole frames in one launch per device, at depth self.max_depth.
 
         lights: None (every view uses GetScene().lights) or one list of Light per view, all of the same length.
@@ -478,17 +481,32 @@ class MythTracer:
 
         debug / taps: also return the planes render_chunk returns (through mtb_render_batch_debug): debug, line_no and
         points, and sig_hits, sig_shadow and n_rays, each of shape (n, s*height, s*width) - one entry per sample, entry
-        (x, y) of view v being that of pixel (x, y) of view v rendered by render_chunk at (s*width) x (s*height)."""
+        (x, y) of view v being that of pixel (x, y) of view v rendered by render_chunk at (s*width) x (s*height).
+
+        subframes: k >= 1.  k > 1 renders accumulated views (motion blur, soft shadows) through mtb_render_batch_accum:
+        cameras (and lights, if given) hold k sub-frames per output view, output-major, and output view v is the
+        rounded mean of all k*s*s samples of sub-frames v*k .. v*k + k-1.  rgb then has shape (len(cameras) / k,
+        height, width, 3) and the stats are those of the sub-frames.  debug and taps are refused with k > 1: render the
+        sub-frames with render_batch(..., debug=True) for their planes."""
         ss = samples_per_axis
         if isinstance(ss, bool) or not isinstance(ss, (int, np.integer)) or ss not in (1, 2, 4, 8):
             raise MythTracerError("render_batch: samples_per_axis must be 1, 2, 4 or 8 (got %r)" % (ss,))
         ss = int(ss)
+        k = subframes
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1:
+            raise MythTracerError("render_batch: subframes must be an int >= 1 (got %r)" % (k,))
+        k = int(k)
         for name, flag in (("debug", debug), ("taps", taps)):
             if not isinstance(flag, (bool, np.bool_)):
                 raise MythTracerError("render_batch: %s must be True or False (got %r)" % (name, flag))
+        if k > 1 and (debug or taps):
+            raise MythTracerError("render_batch: debug and taps are not available with subframes > 1 (there is no plane of an "
+                                  "accumulated view; render the sub-frames with debug=True / taps=True)")
         cams = [c if isinstance(c, Camera) else Camera.from_tuple(c) for c in cameras]
         if not cams:
             raise MythTracerError("render_batch: no cameras")
+        if len(cams) % k != 0:
+            raise MythTracerError("render_batch: %d cameras are not a whole number of output views of %d subframes" % (len(cams), k))
         cam_arr = np.zeros(len(cams), CAMERA_DTYPE)
         for i, c in enumerate(cams):
             cam_arr[i] = c.as_array()
@@ -505,7 +523,8 @@ class MythTracer:
             n_lights = sizes.pop()
             # (n_lights = 0 still passes a non-NULL array: no lights at all, not "the scene's lights")
             light_arr = _lights_array([l for ls in lights for l in ls]) if n_lights else np.zeros(1, LIGHT_DTYPE)
-        shape = (len(cams), height, width, 3)
+        n_out = len(cams) // k
+        shape = (n_out, height, width, 3)
         if out is None:
             rgb = np.zeros(shape, np.uint8)
         else:
@@ -531,6 +550,9 @@ class MythTracer:
                 res["debug"] = dbg
                 res["line_no"] = dbg["line_no"]
                 res["points"] = dbg["point"]
+        elif k > 1:
+            self._check(self._lib.mtb_render_batch_accum(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height,
+                                                         ss, self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch_accum")
         elif ss == 1:
             self._check(self._lib.mtb_render_batch(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
                                                    self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch")

@@ -114,6 +114,8 @@ struct DeviceState {
   DeviceBuffer<mtb_debug> batch_dbg;
   DeviceBuffer<uint64_t> batch_sig_hits, batch_sig_shadow;
   DeviceBuffer<uint32_t> batch_n_rays;
+  // accumulated batches: the channel sums of this device's output views and the arrival counters of their tiles
+  DeviceBuffer<uint32_t> batch_sum, batch_arrive;
   cudaEvent_t ev_batch_start = nullptr, ev_batch_stop = nullptr;
   // intersect scratch
   DeviceBuffer<double> q_origins, q_dirs, q_t, q_point;
@@ -138,6 +140,7 @@ struct DeviceState {
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
     counters.Free(); tile_cost.Free(); tile_order.Free();
     batch_views.Free(); batch_lights.Free(); batch_rgb.Free(); batch_dbg.Free(); batch_sig_hits.Free(); batch_sig_shadow.Free(); batch_n_rays.Free();
+    batch_sum.Free(); batch_arrive.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
     if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
     ev_batch_start = ev_batch_stop = nullptr;
@@ -789,10 +792,13 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 // exactly as a batch of that size, and the kernel writes the W x H block means; everything else is as for ss = 1.
 // dbg_host / taps (nullable, HOST): the per-pixel debug info and taps of every view on its sample grid, view-major; each
 // device copies the planes of its own views.
+// subframes k > 1 (accumulated views, no planes): cams and lights hold k sub-frames per output view, output-major, and
+// output view v is the rounded mean of the k * ss * ss samples of sub-frames v*k .. v*k + k-1; n_out counts output
+// views.  Device g renders a contiguous range of output views with all their sub-frames.  k = 1: n_out views as above.
 constexpr int64_t kMaxSampleSide = 65536;  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
-int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
-                    int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps, mtb_stats *stats,
-                    bool synchronous) {
+int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
+                    int image_w, int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps,
+                    mtb_stats *stats, bool synchronous) {
   const auto wall0 = std::chrono::steady_clock::now();
   if (ctx == nullptr) return MTB_ERR_ARG;
   if (ctx->dev.empty()) {
@@ -807,10 +813,19 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     ctx->err = cams == nullptr ? "cams is NULL" : "rgb_out is NULL";
     return MTB_ERR_ARG;
   }
-  if (n_views < 1 || n_views > 65535) {
+  if (subframes < 1) {
+    ctx->err = "subframes must be >= 1";
+    return MTB_ERR_ARG;
+  }
+  if (subframes == 1 && (n_out < 1 || n_out > 65535)) {
     ctx->err = "n_views must be in 1..65535 (one grid row per view)";
     return MTB_ERR_ARG;
   }
+  if (subframes > 1 && (n_out < 1 || (int64_t)n_out * subframes > 65535)) {
+    ctx->err = "n_out must be >= 1 and n_out * subframes at most 65535 (one grid row per sub-frame)";
+    return MTB_ERR_ARG;
+  }
+  const int32_t k = subframes, n_views = n_out * subframes;  // n_views: the sub-frames (the views themselves when k = 1)
   if (lights != nullptr && n_lights < 0) {
     ctx->err = "n_lights must be >= 0";
     return MTB_ERR_ARG;
@@ -840,6 +855,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
   const bool debug_build = (ctx->flags & MTB_FLAG_COUNT_WORK) != 0;
   const int n_dev = (int)ctx->dev.size();
   const int tiles_x = (grid_w + 7) / 8, tiles_per_view = tiles_x * ((grid_h + 7) / 8);
+  const bool accum = k > 1;
 
   // per-view records and the views' lights, view-major (the context's lights repeated when the caller passes none)
   const int32_t nl = lights != nullptr ? n_lights : (int32_t)ctx->lights.size();
@@ -865,7 +881,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
   // take the second way: their epilogue stores single bytes, and a direct store of those into mapped host memory has
   // not been measured against the copy (which moves 1/ss^2 of the samples' bytes).
   uint8_t *host_direct = nullptr;
-  if (ss == 1 && n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
+  if (ss == 1 && !accum && n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
     MTB_CUDA(ctx, cudaSetDevice(ctx->dev[0].device));
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer != nullptr) {
@@ -876,9 +892,10 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
 
   auto launch_on_device = [&](int g) -> int {
     DeviceState &d = ctx->dev[(size_t)g];
-    const int first = g * (n_views / n_dev) + std::min(g, n_views % n_dev);
-    const int count = n_views / n_dev + (g < n_views % n_dev ? 1 : 0);
-    if (count == 0) return MTB_OK;
+    const int first_out = g * (n_out / n_dev) + std::min(g, n_out % n_dev);
+    const int count_out = n_out / n_dev + (g < n_out % n_dev ? 1 : 0);
+    if (count_out == 0) return MTB_OK;
+    const int first = first_out * k, count = count_out * k;  // this device's sub-frames
     MTB_CUDA(ctx, cudaSetDevice(d.device));
     cudaStream_t s = d.stream;
     if (d.ev_batch_start == nullptr) {
@@ -888,13 +905,14 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     // Everything below is ordered on d.stream: a batch queued behind another one overwrites the records only after the
     // earlier launch has read them.  A buffer that has to grow is freed and reallocated, so the earlier work that may
     // still read it is waited for first.
-    const size_t n_rgb = host_direct != nullptr ? 0 : (size_t)count * npx * 3;
+    const size_t n_rgb = host_direct != nullptr ? 0 : (size_t)count_out * npx * 3;
     const size_t n_lt = (size_t)count * nl;
     const size_t n_plane = (size_t)count * gpx;
+    const size_t n_sum = accum ? (size_t)count_out * npx * 3 : 0, n_arrive = accum ? (size_t)count_out * tiles_per_view * 2 : 0;
     auto grows = [n_plane](const void *host, size_t have) { return host != nullptr && n_plane > have; };
     if ((size_t)count > d.batch_views.count || n_lt > d.batch_lights.count || n_rgb > d.batch_rgb.count ||
         grows(dbg_host, d.batch_dbg.count) || grows(hits_host, d.batch_sig_hits.count) || grows(shadow_host, d.batch_sig_shadow.count) ||
-        grows(rays_host, d.batch_n_rays.count)) {
+        grows(rays_host, d.batch_n_rays.count) || n_sum > d.batch_sum.count || n_arrive > d.batch_arrive.count) {
       MTB_CUDA(ctx, cudaStreamSynchronize(s));
     }
     MTB_CUDA(ctx, d.batch_views.Upload(views.data() + first, (size_t)count, s));
@@ -905,6 +923,16 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
     sc.n_lights = nl;
     mtb::RenderParams p = rp;  // (planes NULL unless this batch asks for them)
     p.rgb = host_direct != nullptr ? host_direct + (size_t)first * npx * 3 : d.batch_rgb.ptr;
+    mtb::AccumParams acc{nullptr, nullptr, k};
+    if (accum) {
+      // (cleared on the stream before every launch: a call queued behind another one of a different shape starts from 0)
+      MTB_CUDA(ctx, d.batch_sum.Reserve(n_sum));
+      MTB_CUDA(ctx, d.batch_arrive.Reserve(n_arrive));
+      MTB_CUDA(ctx, cudaMemsetAsync(d.batch_sum.ptr, 0, n_sum * sizeof(uint32_t), s));
+      MTB_CUDA(ctx, cudaMemsetAsync(d.batch_arrive.ptr, 0, n_arrive * sizeof(uint32_t), s));
+      acc.sum = d.batch_sum.ptr;
+      acc.arrive = d.batch_arrive.ptr;
+    }
     if (dbg_host != nullptr) {
       MTB_CUDA(ctx, d.batch_dbg.Reserve(n_plane));
       p.dbg = d.batch_dbg.ptr;
@@ -927,12 +955,12 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
       MTB_CUDA(ctx, cudaMemsetAsync(d.counters.ptr, 0, mtb::kNumCounters * sizeof(unsigned long long), s));
     }
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_start, s));
-    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, debug_build, s);
+    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, acc, debug_build, s);
     ctx->launches++;
     MTB_CUDA(ctx, cudaGetLastError());
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_stop, s));
     if (host_direct == nullptr) {
-      MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first * npx * 3, d.batch_rgb.ptr, (size_t)count * npx * 3, cudaMemcpyDeviceToHost, s));
+      MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first_out * npx * 3, d.batch_rgb.ptr, (size_t)count_out * npx * 3, cudaMemcpyDeviceToHost, s));
     }
     const size_t at = (size_t)first * gpx;
     if (dbg_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(dbg_host + at, p.dbg, n_plane * sizeof(mtb_debug), cudaMemcpyDeviceToHost, s));
@@ -958,7 +986,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, c
   unsigned long long total[mtb::kNumCounters];
   memset(total, 0, sizeof(total));
   double kernel_ms = 0.0;
-  for (int g = 0; g < n_dev && g < n_views; g++) {
+  for (int g = 0; g < n_dev && g < n_out; g++) {
     DeviceState &d = ctx->dev[(size_t)g];
     MTB_CUDA(ctx, cudaSetDevice(d.device));
     MTB_CUDA(ctx, cudaStreamSynchronize(d.stream));
@@ -1310,29 +1338,41 @@ int mtb_render_chunk_async(mtb_context *ctx, const mtb_camera *cam, int image_w,
 
 int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                      int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
+  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                         int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
+  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                               int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_debug(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_debug *dbg_out,
                            const mtb_taps *taps, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
+  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
                          true);
+}
+
+int mtb_render_batch_accum(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
+                           int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
+  return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
+                         stats, true);
+}
+
+int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
+                                 int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
+  return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
+                         nullptr, false);
 }
 
 int mtb_wait(mtb_context *ctx) {

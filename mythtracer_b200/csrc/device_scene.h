@@ -71,6 +71,14 @@ struct ViewRec {
   double origin[3];
 };
 
+// Accumulated batch (LaunchRenderMegaBatch with subframes k > 1): grid row u is sub-frame u of output view u / k.
+// Both arrays cover the output views of the launch and are zero when it starts.
+struct AccumParams {
+  uint32_t *sum;       // per output view: W x H x 3 sums of the k * s * s quantised samples of each output channel
+  uint32_t *arrive;    // per output view, tile of the sample grid and warp half: warps that have added their sums
+  int32_t subframes;   // k; 1: no accumulation (sum and arrive unused)
+};
+
 struct IntersectParams {
   int64_t n;
   const double *origins, *dirs;
@@ -129,8 +137,12 @@ void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_block
 // samples_per_axis s = 2, 4 or 8: supersampled views.  rp.chunk_w x rp.chunk_h (and views[v].sensor) describe the
 // s*W x s*H sample grid, tiles_per_view counts its tiles, and view v's W x H output pixels (each the rounded mean of
 // its s x s samples) go to rp.rgb + v * W * H * 3.  s = 1: the plain batch above.
+// acc.subframes k > 1: accumulated views.  n_views counts sub-frames (a multiple of k); sub-frame u is traced exactly as
+// view u above, and output view v = u / k (W x H, at rp.rgb + v * W * H * 3) is the rounded mean of the k * s * s
+// samples of its sub-frames, summed in acc.sum (zeroed by the caller, with acc.arrive, before the launch).  The planes
+// must be NULL.  k = 1: the batches above.
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
-                           int samples_per_axis, bool debug_build, cudaStream_t stream);
+                           int samples_per_axis, const AccumParams &acc, bool debug_build, cudaStream_t stream);
 void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, int mode, cudaStream_t stream);  // mode 0: one ray per thread, 1: two rays per lane (Trace2), 2: chain (TraceChain), 3: two calls
 
 }  // namespace mtb

@@ -152,15 +152,109 @@ __device__ __forceinline__ void SupersampleEpilogue(const RenderParams &rp, cons
   }
 }
 
+// Accumulated batch (ACC, SS = 1, 2, 4, 8): block row u traces sub-frame u of output view v = u / k exactly as view u of
+// a batch, and the output pixel is the rounded mean of all k * SS * SS quantised samples of its k sub-frames.  Every
+// warp adds the per-output-channel sums of its half tile (formed as SupersampleEpilogue forms them; SS = 8: by the
+// warp that finishes second, for the whole tile) into acc.sum of view v, fences, and bumps the arrival counter of
+// (v, tile, warp half).  The warp whose arrival is the k-th reads the completed sums from L2 and stores the bytes.  The
+// sums are integers, so the bytes do not depend on the order in which the sub-frames finish.  No block barrier after
+// the trace, for the reason of the plain epilogue.
+template <int SS>
+__device__ __forceinline__ void AccumulateEpilogue(const RenderParams &rp, const AccumParams &acc, const unsigned char *s_rgb, int tile_id,
+                                                   int strip, unsigned *s_ss8) {
+  const int out_w = rp.chunk_w / SS, out_h = rp.chunk_h / SS;
+  const unsigned view = blockIdx.y / (unsigned)acc.subframes;
+  const size_t view_base = (size_t)view * out_w * out_h * 3;
+  uint32_t *const sum = acc.sum + view_base;
+  uint8_t *const frame = rp.rgb + view_base;
+  const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  const unsigned n = (unsigned)acc.subframes * (SS * SS);
+  uint32_t *const arrive = acc.arrive + ((size_t)view * gridDim.x + tile_id) * 2;
+  if constexpr (SS == 8) {
+    // as SupersampleEpilogue: the warp that finishes second holds the tile's (= the output pixel's) three sums in lane 0
+    const unsigned char *mine = s_rgb + threadIdx.x * 3;
+    unsigned r = mine[0], g = mine[1], b = mine[2];
+    for (int off = 16; off > 0; off >>= 1) {
+      r += __shfl_down_sync(0xffffffffu, r, off);
+      g += __shfl_down_sync(0xffffffffu, g, off);
+      b += __shfl_down_sync(0xffffffffu, b, off);
+    }
+    volatile unsigned *part = s_ss8 + 1;
+    if (lane != 0u) return;
+    part[warp * 3 + 0] = r;
+    part[warp * 3 + 1] = g;
+    part[warp * 3 + 2] = b;
+    __threadfence_block();
+    if (atomicAdd(s_ss8, 1u) != 1u) return;
+    __threadfence_block();
+    const unsigned o = (warp ^ 1u) * 3;
+    uint32_t *dst = sum + (size_t)tile_id * 3;  // tile (x, y) = output pixel (x, y)
+    atomicAdd(dst + 0, r + part[o + 0]);
+    atomicAdd(dst + 1, g + part[o + 1]);
+    atomicAdd(dst + 2, b + part[o + 2]);
+    __threadfence();
+    if (atomicAdd(arrive, 1u) != (unsigned)acc.subframes - 1u) return;
+    __threadfence();
+    for (int c = 0; c < 3; c++) frame[(size_t)tile_id * 3 + c] = (uint8_t)((__ldcg(dst + c) + n / 2) / n);
+  } else {
+    // the output channels this lane owns: SS = 1, the 3 of its own pixel; SS = 2, 4, one of the warp's (8/SS) x (4/SS)
+    // output pixels (lane = 3 * pixel + channel)
+    constexpr int kPer = SS == 1 ? 3 : 1;
+    long long at = -1;  // this lane's first channel in the view's sums; -1: none
+    unsigned val[kPer];
+    if constexpr (SS == 1) {
+      const int tx = (int)(threadIdx.x & 7u), ty = (int)(threadIdx.x >> 3);
+      const int px = (tile_id % rp.tiles_x) * kTile + tx, py = strip * kTile + ty;
+      if (px < out_w && py < out_h) {
+        at = ((long long)py * out_w + px) * 3;
+        const unsigned char *src = s_rgb + ((ty * kTile) + tx) * 3;
+        for (int c = 0; c < 3; c++) val[c] = src[c];
+      }
+    } else {
+      constexpr int kCols = kTile / SS, kRows = 4 / SS;
+      if (lane < (unsigned)(kCols * kRows * 3)) {
+        const int k = (int)lane / 3, c = (int)lane % 3, i = k % kCols, j = k / kCols;
+        const int ox = (tile_id % rp.tiles_x) * kCols + i, oy = (strip * kTile + (int)warp * 4) / SS + j;
+        if (ox < out_w && oy < out_h) {
+          at = ((long long)oy * out_w + ox) * 3 + c;
+          const unsigned char *src = s_rgb + warp * (4 * kTile * 3) + (j * SS * kTile + i * SS) * 3 + c;
+          unsigned s = 0;
+#pragma unroll
+          for (int a = 0; a < SS; a++) {
+#pragma unroll
+            for (int b = 0; b < SS; b++) s += src[(a * kTile + b) * 3];
+          }
+          val[0] = s;
+        }
+      }
+    }
+    if (at >= 0) {
+      for (int c = 0; c < kPer; c++) atomicAdd(sum + at + c, val[c]);
+    }
+    __threadfence();
+    __syncwarp();
+    unsigned last = 0u;
+    if (lane == 0u) last = atomicAdd(arrive + warp, 1u) == (unsigned)acc.subframes - 1u ? 1u : 0u;
+    if (__shfl_sync(0xffffffffu, last, 0) == 0u) return;
+    __threadfence();
+    if (at >= 0) {
+      for (int c = 0; c < kPer; c++) frame[at + c] = (uint8_t)((__ldcg(sum + at + c) + n / 2) / n);
+    }
+  }
+}
+
 // BATCH: grid (tiles per view, views), block b of row v renders tile b of view v in scanline order; the camera comes from
 // views[v] and the pixels go to rp.rgb + v * chunk_w * chunk_h * 3.  A batch launch passes NULL for tile_order,
 // tile_cost and run_if; its debug and tap planes (NULL unless the caller asked for them) are view-major, view v's entries
 // start at v * chunk_w * chunk_h (PlaneIndex).  Without BATCH, `views` is unused and every `BATCH ? :`
 // folds away: the single-view kernels compile to the code they had before the batch form existed.  SS > 1 (BATCH only):
-// the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.
-template <bool DBG, bool BATCH, int SS>
-__global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(DeviceScene sc, RenderParams rp, const ViewRec *views) {
+// the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.  ACC (BATCH only): the
+// accumulated batch, see AccumulateEpilogue; `acc` is unused without it.
+template <bool DBG, bool BATCH, int SS, bool ACC>
+__global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(DeviceScene sc, RenderParams rp, const ViewRec *views,
+                                                                                 AccumParams acc) {
   static_assert(SS == 1 || (BATCH && (SS == 2 || SS == 4 || SS == 8)), "supersampling is a batch form with 2, 4 or 8 samples per axis");
+  static_assert(!ACC || BATCH, "accumulation is a batch form");
   MTB_DECLARE_FAST_CTX(kBlockThreads);
   // (SS = 8: 7 more words behind the samples for the epilogue's counter and partial sums)
   __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3 + (SS == 8 ? 7 * 4 : 0)];
@@ -473,7 +567,9 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
 #else
   __syncwarp();
 #endif
-  if constexpr (SS > 1) {
+  if constexpr (ACC) {
+    AccumulateEpilogue<SS>(rp, acc, s_rgb, tile_id, strip, s_ss8);
+  } else if constexpr (SS > 1) {
     SupersampleEpilogue<SS>(rp, s_rgb, tile_id, strip, s_ss8);
   } else {
     const int px0 = (tile_id % rp.tiles_x) * kTile, py0 = strip * kTile + (int)(threadIdx.x >> 5) * 4;
@@ -731,31 +827,42 @@ void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles,
 void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_blocks, bool debug_build, cudaStream_t stream) {
   if (n_blocks <= 0) return;
   if (debug_build) {
-    RenderMega<true, false, 1><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr);
+    RenderMega<true, false, 1, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{});
   } else {
-    RenderMega<false, false, 1><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr);
+    RenderMega<false, false, 1, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{});
   }
 }
 
-template <int SS>
-void LaunchBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const dim3 &grid, bool debug_build, cudaStream_t stream) {
+template <int SS, bool ACC>
+void LaunchBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const dim3 &grid, bool debug_build,
+                 cudaStream_t stream) {
   if (debug_build) {
-    RenderMega<true, true, SS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views);
+    RenderMega<true, true, SS, ACC><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc);
   } else {
-    RenderMega<false, true, SS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views);
+    RenderMega<false, true, SS, ACC><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc);
+  }
+}
+
+template <bool ACC>
+void LaunchBatchSS(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const dim3 &grid,
+                   int samples_per_axis, bool debug_build, cudaStream_t stream) {
+  switch (samples_per_axis) {
+    case 1: LaunchBatch<1, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
+    case 2: LaunchBatch<2, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
+    case 4: LaunchBatch<4, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
+    case 8: LaunchBatch<8, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
+    default: break;  // (the host API admits 1, 2, 4 and 8 only)
   }
 }
 
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
-                           int samples_per_axis, bool debug_build, cudaStream_t stream) {
+                           int samples_per_axis, const AccumParams &acc, bool debug_build, cudaStream_t stream) {
   if (tiles_per_view <= 0 || n_views <= 0) return;
   const dim3 grid((unsigned)tiles_per_view, (unsigned)n_views);
-  switch (samples_per_axis) {
-    case 1: LaunchBatch<1>(sc, rp, views, grid, debug_build, stream); break;
-    case 2: LaunchBatch<2>(sc, rp, views, grid, debug_build, stream); break;
-    case 4: LaunchBatch<4>(sc, rp, views, grid, debug_build, stream); break;
-    case 8: LaunchBatch<8>(sc, rp, views, grid, debug_build, stream); break;
-    default: break;  // (the host API admits 1, 2, 4 and 8 only)
+  if (acc.subframes > 1) {
+    LaunchBatchSS<true>(sc, rp, views, acc, grid, samples_per_axis, debug_build, stream);
+  } else {
+    LaunchBatchSS<false>(sc, rp, views, acc, grid, samples_per_axis, debug_build, stream);
   }
 }
 

@@ -1,7 +1,7 @@
 """Throughput of batches (mtb_render_batch) against one call per frame, on the C3 scene (two lights, depth 5) and its
 orbit yaw = C3 yaw + 2 degrees * k.
 
-    python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3] [--supersample | --debug-planes]
+    python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3] [--supersample | --debug-planes | --subframes]
 
 480x270, 64 frames: (a) one render_chunk per frame, megakernel forced; (b) one render_chunk per frame, automatic
 pipeline choice (after the 13 frames it needs to decide); (c) render_batch in batches of 1, 4, 16, 64.
@@ -26,6 +26,13 @@ views at 480x270 and 8 at 1920x1080, each with neither, with debug, with taps an
 render_chunk(debug=True) per frame (megakernel).  Per mode: median kernel_ms per call (summed over the calls of a
 pass for render_chunk), frames/s end to end, Mrays/s and the bytes copied back per view; whether the RGB equals that of
 the batch without planes, and whether the planes of the first and the last view equal render_chunk's.
+
+--subframes measures accumulated batches (render_batch(..., subframes=k)): output view f of the orbit is the mean of k
+sub-frames at yaw + 2 degrees * (f + j / k).  Shapes: 16 outputs x k = 8 at 480x270 (s = 1), 4 x k = 4 at 1920x1080
+(s = 1) and 16 x k = 4 at 480x270 with s = 4.  Each against the plain batch of the same sub-frames at the same s (the
+same rays; kernel time), and against the way a caller has to do it without the feature: render_batch of the sub-frames
+at s*W x s*H plus the mean in numpy (frames/s end to end).  Per mode: median kernel_ms per call over --reps calls,
+Mrays/s, output frames/s, and whether the output equals the numpy mean of the sub-frames.
 """
 import argparse
 import hashlib
@@ -188,6 +195,59 @@ def supersample(mt, files, cfg, reps):
     return dict(shape="C3 orbit, %d views" % n, modes=recs, work_per_ray=work)
 
 
+def _accum_mean(frames, k, s):
+    """(n_out * k, s*H, s*W, 3) -> (n_out, H, W, 3): the rounded mean of the k * s * s samples of every output channel."""
+    n_out, sh, sw = frames.shape[0] // k, frames.shape[1], frames.shape[2]
+    sums = frames.reshape(n_out, k, sh // s, s, sw // s, s, 3).sum(axis=(1, 3, 5), dtype=np.uint32)
+    n = k * s * s
+    return ((sums + n // 2) // n).astype(np.uint8)
+
+
+def subframes(mt, files, cfg, reps):
+    """The --subframes measurements (see the module docstring)."""
+    groups = []
+    for n_out, k, w, h, s in ((16, 8, 480, 270, 1), (4, 4, cfg["width"], cfg["height"], 1), (16, 4, 480, 270, 4)):
+        cams = [c for f in range(n_out) for c in _orbit_subframes(files.camera, f, k)]
+        out = np.zeros((n_out, h, w, 3), np.uint8)
+        walls, kms, rays = _timed_calls(lambda: mt.render_batch(cams, w, h, out=out, samples_per_axis=s, subframes=k)["stats"], reps)
+        got = out.copy()
+        hi = np.zeros((n_out * k, s * h, s * w, 3), np.uint8)
+        mt.render_batch(cams, s * w, s * h, out=hi)
+        want = _accum_mean(hi, k, s)
+        equal = bool(np.array_equal(got, want))
+        recs = [_ss_record("render_batch %d x %d subframes, %dx%d, s = %d" % (n_out, k, w, h, s), n_out, w, h, s, walls, kms, rays, equal)]
+        plain = np.zeros((n_out * k, h, w, 3), np.uint8)
+        walls, kms_p, rays_p = _timed_calls(lambda: mt.render_batch(cams, w, h, out=plain, samples_per_axis=s)["stats"], reps)
+        base_kms = statistics.median(kms_p)
+        recs.append(_ss_record("render_batch %d views (the sub-frames), %dx%d, s = %d" % (n_out * k, w, h, s), n_out * k, w, h, s, walls, kms_p,
+                               rays_p, None))
+
+        def hi_then_mean():
+            st = mt.render_batch(cams, s * w, s * h, out=hi)["stats"]
+            out[...] = _accum_mean(hi, k, s)
+            return st
+        walls, kms_h, rays_h = _timed_calls(hi_then_mean, reps)
+        recs.append(_ss_record("render_batch %d views at %dx%d + numpy mean" % (n_out * k, s * w, s * h), n_out, w, h, s, walls, kms_h, rays_h,
+                               bool(np.array_equal(out, want))))
+        for r in recs:
+            r["equals_numpy_mean"] = r.pop("equals_block_mean_of_1080p")
+        recs[0]["kernel_ms_over_plain_batch"] = round(statistics.median(kms) / base_kms, 4)
+        print("accumulated / plain kernel time: x%.4f" % recs[0]["kernel_ms_over_plain_batch"], file=sys.stderr, flush=True)
+        groups.append(dict(shape="C3 orbit, %d outputs x %d subframes at %dx%d, %d samples per axis" % (n_out, k, w, h, s), outputs=n_out,
+                           subframes=k, modes=recs))
+    return groups
+
+
+def _orbit_subframes(cam, f, k):
+    """The k sub-frames of output frame f of the orbit: yaw + 2 degrees * (f + j / k)."""
+    out = []
+    for j in range(k):
+        c = list(cam)
+        c[4] += 2.0 * f + 2.0 * j / k
+        out.append(tuple(c))
+    return out
+
+
 PLANE_KEYS = ("debug", "sig_hits", "sig_shadow", "n_rays")
 
 
@@ -258,6 +318,7 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--supersample", action="store_true")
     ap.add_argument("--debug-planes", action="store_true")
+    ap.add_argument("--subframes", action="store_true")
     args = ap.parse_args()
     devices = [int(x) for x in args.devices.split(",")]
     files, cfg = scenegen.generate_config("C3", os.environ.get("MTB_SCENE_DIR", "/tmp/mtb_scenes"))
@@ -276,6 +337,14 @@ def main():
         modes = [r for g in doc["debug_planes"] for r in g["modes"]]
         if not all(r.get("rgb_equals_no_planes", True) and r.get("planes_equal_render_chunk", True) for r in modes):
             sys.exit("a batch with planes differs from the batch without planes or from render_chunk")
+        return
+
+    if args.subframes:
+        doc["subframes"] = subframes(mt, files, cfg, args.reps)
+        mt.close()
+        _emit(doc, args.out)
+        if not all(r["equals_numpy_mean"] is not False for g in doc["subframes"] for r in g["modes"]):
+            sys.exit("an accumulated batch differs from the numpy mean of its sub-frames")
         return
 
     if args.supersample:

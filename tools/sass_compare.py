@@ -4,10 +4,12 @@
 
 Compiles csrc/megakernel.cu of both trees for sm_100a with the library's flags (no GPU needed), dumps the SASS with
 cuobjdump and compares the instruction listings of RenderMega<DBG, BATCH> (RenderMega<DBG, BATCH, 1> in a tree with
-the supersampled batch) for DBG and BATCH = false and true.  A tree from before the batch form only has the single-view
-kernel, RenderMega<DBG>, which is then compared with BATCH = false alone.  Also prints ptxas' registers / stack / spill
-figures of every RenderMega instantiation, the supersampled ones (SS = 2, 4, 8) included.  Exit status 0 when the
-listings are identical.
+the supersampled batch, RenderMega<DBG, BATCH, 1, false> in a tree with the accumulated batch) for DBG and BATCH = false
+and true, and those of the supersampled batch, RenderMega<DBG, true, SS> (SS = 2, 4, 8), wherever the old tree has it.
+A tree from before the batch form only has the single-view kernel, RenderMega<DBG>, which is then compared with
+BATCH = false alone.  Also prints ptxas' registers / stack / spill figures of every RenderMega instantiation, the
+supersampled (SS = 2, 4, 8) and accumulating (ACC = true) ones included.  Exit status 0 when the listings are
+identical.
 """
 import os
 import re
@@ -48,9 +50,13 @@ def _functions(sass):
     return funcs
 
 
-def _instantiation(funcs, dbg, batch):
-    """(name, code) of RenderMega<dbg, batch> (<dbg, batch, 1>; <dbg> stands for <dbg, false>), or None."""
-    patterns = [r"RenderMegaILb%dELb%dE(Li1E)?EEv" % (dbg, batch)] + ([r"RenderMegaILb%dEEEv" % dbg] if not batch else [])
+def _instantiation(funcs, dbg, batch, ss=1):
+    """(name, code) of RenderMega<dbg, batch, ss> (<dbg, batch> for ss = 1 without the SS parameter, <..., false> with
+    the ACC parameter; <dbg> stands for <dbg, false>), or None."""
+    if ss == 1:
+        patterns = [r"RenderMegaILb%dELb%dE(Li1E(Lb0E)?)?EEv" % (dbg, batch)] + ([r"RenderMegaILb%dEEEv" % dbg] if not batch else [])
+    else:
+        patterns = [r"RenderMegaILb%dELb%dELi%dE(Lb0E)?EEv" % (dbg, batch, ss)]
     for name, code in funcs.items():
         if any(re.search(p, name) for p in patterns):
             return name, code
@@ -71,21 +77,21 @@ def main():
         for name, fig in _ptxas_figures(log).items():
             print("%s %s %s" % (label, re.search(r"RenderMega\w*?E(?=EvN)", name).group(0), fig))
     old_f, new_f = _functions(old_sass), _functions(new_sass)
-    for batch in (0, 1):
+    for batch, ss in ((0, 1), (1, 1), (1, 2), (1, 4), (1, 8)):
         for dbg in (0, 1):
-            old, new = _instantiation(old_f, dbg, batch), _instantiation(new_f, dbg, batch)
+            old, new = _instantiation(old_f, dbg, batch, ss), _instantiation(new_f, dbg, batch, ss)
             if new is None:
-                raise SystemExit("no RenderMega<%d, %d> in the listing of %s" % (dbg, batch, new_tree))
+                raise SystemExit("no RenderMega<%d, %d, %d> in the listing of %s" % (dbg, batch, ss, new_tree))
             if old is None:
                 if not batch:
                     raise SystemExit("no single-view RenderMega<%d> in the listing of %s" % (dbg, old_tree))
-                print("RenderMega<DBG=%d, BATCH=1>: not in %s" % (dbg, old_tree))
+                print("RenderMega<DBG=%d, BATCH=1, SS=%d>: not in %s" % (dbg, ss, old_tree))
                 continue
             (on, oc), (nn, nc) = old, new
             equal = oc == nc
             same &= equal
-            print("RenderMega<DBG=%d, BATCH=%d>: %d vs %d instructions, %s" % (dbg, batch, len(oc), len(nc),
-                                                                             "identical" if equal else "DIFFERENT"))
+            print("RenderMega<DBG=%d, BATCH=%d, SS=%d>: %d vs %d instructions, %s" % (dbg, batch, ss, len(oc), len(nc),
+                                                                                    "identical" if equal else "DIFFERENT"))
             if not equal:
                 for i, (a, b) in enumerate(zip(oc, nc)):
                     if a != b:
