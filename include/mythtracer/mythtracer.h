@@ -204,6 +204,16 @@ class MythTracer {
                           const std::vector<std::vector<Light>> *lights, uint8_t *pinned_out) {
     return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, pinned_out, nullptr, false);
   }
+  // Batches left in device memory (mtb_render_batch_device): the bytes of the overloads above, written to d_rgb, DEVICE
+  // memory of the context's device 0 (cams.size() / subframes * w * h * 3 bytes), and ordered on `stream` (a
+  // cudaStream_t of device 0; nullptr = the context's own stream): the batch starts after the work queued there before
+  // the call, and work queued there afterwards sees the frames.  Returns once the work is queued.  RGB only: the planes
+  // of a batch in device memory come from the C ABI.
+  bool RayTraceBatchDevice(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
+                           const std::vector<std::vector<Light>> *lights, void *d_rgb, void *stream) {
+    return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, static_cast<uint8_t *>(d_rgb), nullptr, false,
+                       true, stream);
+  }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
   static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
     return static_cast<uint8_t *>(mtb_host_alloc((size_t)image_width * image_height * 3 * (size_t)n_frames));
@@ -219,7 +229,8 @@ class MythTracer {
 
  private:
   bool RenderBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
-                   const std::vector<std::vector<Light>> *lights, uint8_t *out, mtb_debug *dbg, bool synchronous) {
+                   const std::vector<std::vector<Light>> *lights, uint8_t *out, mtb_debug *dbg, bool synchronous, bool device = false,
+                   void *stream = nullptr) {
     if (!was_scene_finalized) {
       puts("Finalizing tree.");
       if (!scene.tree.Finalize(&scene.materials, &scene.textures)) return false;
@@ -252,16 +263,21 @@ class MythTracer {
     const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
     mtb_stats stats;
     int rc;
-    if (subframes != 1) {
+    if (subframes != 1 || device) {
       if (subframes < 1 || cams.size() % (size_t)subframes != 0) {
         fprintf(stderr, "error: %zu cameras are not a whole number of output views of %d subframes\n", cams.size(), subframes);
         return false;
       }
       const int32_t n_out = (int32_t)(cams.size() / (size_t)subframes);
-      rc = synchronous ? mtb_render_batch_accum(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
-                                                max_recursion_level, out, &stats)
-                       : mtb_render_batch_accum_async(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height,
-                                                      samples_per_axis, max_recursion_level, out);
+      if (device) {
+        rc = mtb_render_batch_device(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
+                                     max_recursion_level, out, nullptr, nullptr, stream, nullptr);
+      } else {
+        rc = synchronous ? mtb_render_batch_accum(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
+                                                  max_recursion_level, out, &stats)
+                         : mtb_render_batch_accum_async(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height,
+                                                        samples_per_axis, max_recursion_level, out);
+      }
     } else {
       // (samples_per_axis = 1: mtb_render_batch_ss is mtb_render_batch; dbg = NULL: mtb_render_batch_debug is mtb_render_batch_ss)
       rc = synchronous ? mtb_render_batch_debug(ctx, mcams.data(), (int32_t)mcams.size(), lp, n_lights, image_width, image_height,

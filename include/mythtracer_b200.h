@@ -315,6 +315,31 @@ int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32
                                  const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis,
                                  int max_depth, uint8_t *rgb_out);
 
+/* Batches into DEVICE memory: every batch form above, with its outputs left in HBM of device 0 and the work ordered on
+ * the caller's stream, for a consumer on the GPU (a torch model, object-id planes as segmentation masks, a second pass
+ * over the hit points) that would otherwise copy the outputs to the host and upload them again.  The bytes written are
+ * exactly those of the host form with the same arguments:
+ *   subframes == 1, no plane:    mtb_render_batch_ss (samples_per_axis = 1: mtb_render_batch);
+ *   subframes == 1, any plane:   mtb_render_batch_debug (planes on the sample grid, view-major);
+ *   subframes > 1:               mtb_render_batch_accum (planes are refused, as there).
+ * Argument rules, limits and the partition rule are those of the host forms; cams and lights are HOST memory and may
+ * be reused as soon as the call returns.  d_rgb (n_out * image_h * image_w * 3 bytes, any alignment) must not be NULL;
+ * d_dbg, d_taps and each pointer inside d_taps may be NULL.  Every output pointer must be device memory of the context's
+ * device 0, d_dbg and the sig_* planes 8-byte aligned and n_rays 4-byte aligned; anything else (host memory, pageable or
+ * pinned; memory of another device; misaligned planes) is MTB_ERR_ARG, before anything is queued.
+ *
+ * stream: a cudaStream_t of device 0 (NULL = the context's own stream).  The batch starts after all work queued on it
+ * before the call, and work queued on it after the call sees the finished outputs of every device, so a caching
+ * allocator (torch's) reuses an output dropped after the call only for work ordered after the batch.  stats == NULL:
+ * the call returns once its work is queued, with no host synchronisation (it may still wait for its own streams when a
+ * per-device buffer grows); stats != NULL: it waits for the batch and fills stats as the host forms do.  The call
+ * uploads view records from host memory, so it cannot be captured into a CUDA graph: a capturing stream is
+ * MTB_ERR_ARG.  With several devices, device 0 renders straight into the caller's buffers and every other device
+ * renders its slice into its own and copies it over with one device-to-device copy per output, on its own stream. */
+int mtb_render_batch_device(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
+                            int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, void *d_rgb,
+                            mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream, mtb_stats *stats);
+
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the
  * context has one device.  This is the entry bench.py times for the HBM-resident figure. */

@@ -80,7 +80,7 @@ EXPORTED_SYMBOLS = [
     "mtb_render_chunk_device", "mtb_render_chunk_async", "mtb_wait", "mtb_host_alloc", "mtb_host_free", "mtb_read_counters", "mtb_launch_count", "mtb_pipeline_in_use", "mtb_intersect_rays", "mtb_camera_sensor", "mtb_version",
     "mtb_frame_create", "mtb_frame_open", "mtb_frame_release", "mtb_frame_read", "mtb_load_timing", "mtb_hybrid_share",
     "mtb_render_batch", "mtb_render_batch_async", "mtb_render_batch_ss", "mtb_render_batch_ss_async", "mtb_render_batch_debug",
-    "mtb_render_batch_accum", "mtb_render_batch_accum_async",
+    "mtb_render_batch_accum", "mtb_render_batch_accum_async", "mtb_render_batch_device",
 ]
 
 
@@ -139,6 +139,7 @@ def load_library():
     lib.mtb_render_batch_debug.argtypes = [vp, vp, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp]
     lib.mtb_render_batch_accum.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp]
     lib.mtb_render_batch_accum_async.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp]
+    lib.mtb_render_batch_device.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp, vp]
     lib.mtb_read_counters.argtypes = [vp, vp]
     lib.mtb_pipeline_in_use.argtypes = [vp, vp, vp]
     lib.mtb_launch_count.argtypes = [vp]
@@ -320,6 +321,7 @@ class MythTracer:
         if rc != MTB_OK:
             raise MythTracerError("mtb_create failed: %s" % self._lib.mtb_last_error(None).decode())
         self.max_depth = max_depth
+        self._device0 = None if host_only else (int(dev_arr[0]) if n else 0)  # where render_batch(device=True) leaves its outputs
         self._scene = Scene(self)
         self._flags = 0
         if flags:
@@ -470,7 +472,7 @@ class MythTracer:
         return res
 
     def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None, samples_per_axis: int = 1,
-                     debug: bool = False, taps: bool = False, subframes: int = 1):
+                     debug: bool = False, taps: bool = False, subframes: int = 1, device: bool = False):
         """mtb_render_batch: len(cameras) whole frames in one launch per device, at depth self.max_depth.
 
         lights: None (every view uses GetScene().lights) or one list of Light per view, all of the same length.
@@ -487,7 +489,18 @@ class MythTracer:
         cameras (and lights, if given) hold k sub-frames per output view, output-major, and output view v is the
         rounded mean of all k*s*s samples of sub-frames v*k .. v*k + k-1.  rgb then has shape (len(cameras) / k,
         height, width, 3) and the stats are those of the sub-frames.  debug and taps are refused with k > 1: render the
-        sub-frames with render_batch(..., debug=True) for their planes."""
+        sub-frames with render_batch(..., debug=True) for their planes.
+
+        device: True leaves every output in device memory (mtb_render_batch_device): the same bytes as device=False, as
+        torch tensors on cuda:<devices[0]>, queued on torch.cuda.current_stream() of that device; the call returns
+        without synchronising, and work queued on that stream afterwards sees the finished outputs.  rgb is uint8
+        (n_out, height, width, 3); with debug, `debug` is the raw uint8 (n, s*height, s*width, 32) buffer of mtb_debug
+        records and line_no (int32) and points (float64, last axis 3) are views of it; with taps, sig_hits and sig_shadow
+        are torch.uint64 and n_rays torch.uint32.  out, if given, is a C-contiguous uint8 CUDA tensor of that shape on
+        that device.  stats is None and last_stats is left alone.  torch is imported only here."""
+        if not isinstance(device, (bool, np.bool_)):
+            raise MythTracerError("render_batch: device must be True or False (got %r)" % (device,))
+        device = bool(device)
         ss = samples_per_axis
         if isinstance(ss, bool) or not isinstance(ss, (int, np.integer)) or ss not in (1, 2, 4, 8):
             raise MythTracerError("render_batch: samples_per_axis must be 1, 2, 4 or 8 (got %r)" % (ss,))
@@ -511,7 +524,11 @@ class MythTracer:
         for i, c in enumerate(cams):
             cam_arr[i] = c.as_array()
         light_arr, n_lights = None, 0
-        if lights is None:
+        if lights is None and device:
+            # the scene's lights for every view, passed with the call: pushing them to the context would wait for its streams
+            n_lights = len(self._scene.lights)
+            light_arr = _lights_array(list(self._scene.lights) * len(cams)) if n_lights else np.zeros(1, LIGHT_DTYPE)
+        elif lights is None:
             self._push_lights()
         else:
             lights = list(lights)
@@ -525,9 +542,13 @@ class MythTracer:
             light_arr = _lights_array([l for ls in lights for l in ls]) if n_lights else np.zeros(1, LIGHT_DTYPE)
         n_out = len(cams) // k
         shape = (n_out, height, width, 3)
+        if device:
+            return self._render_batch_device(cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps)
         if out is None:
             rgb = np.zeros(shape, np.uint8)
         else:
+            if not isinstance(out, np.ndarray):
+                raise MythTracerError("render_batch: out must be a numpy array (got %s; a torch tensor needs device=True)" % type(out).__name__)
             if out.shape != shape or out.dtype != np.uint8 or not out.flags["C_CONTIGUOUS"]:
                 raise MythTracerError("render_batch: out must be a C-contiguous uint8 array of shape %s" % (shape,))
             rgb = out
@@ -562,6 +583,50 @@ class MythTracer:
         res["rgb"] = rgb
         res["stats"] = {k: stats[k].item() for k in STATS_DTYPE.names}
         self.last_stats = res["stats"]
+        return res
+
+    def _render_batch_device(self, cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps):
+        """render_batch(..., device=True) once the arguments shared with the host form are checked."""
+        try:
+            import torch
+        except ImportError as e:
+            raise MythTracerError("render_batch: device=True needs torch (%s)" % e)
+        shape = (n_out, height, width, 3)
+        where = torch.device("cuda", self._device0 if self._device0 is not None else 0)
+        if out is not None and not (isinstance(out, torch.Tensor) and out.dtype == torch.uint8 and tuple(out.shape) == shape and
+                                    out.is_contiguous() and out.device == where):
+            raise MythTracerError("render_batch: with device=True, out must be a C-contiguous uint8 torch tensor of shape %s on %s (got %s)" % (
+                shape, where, "%s %s on %s" % (out.dtype, tuple(out.shape), out.device) if isinstance(out, torch.Tensor) else type(out).__name__))
+        n_cams = len(cam_arr)
+        if self._device0 is None:  # host-only context: the library refuses the call (there is no CPU fallback)
+            self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
+                                                          self.max_depth, None, None, None, None, None), "mtb_render_batch_device")
+        stream = torch.cuda.current_stream(where).cuda_stream
+        # torch's default stream is the legacy default stream (handle 0), which the C ABI spells cudaStreamLegacy: a NULL
+        # stream there means the context's own stream
+        handle = ctypes.c_void_p(stream if stream != 0 else 1)
+        rgb = out if out is not None else torch.empty(shape, dtype=torch.uint8, device=where)
+        res = {}
+        dbg, tap_ptr = None, None
+        plane = (n_cams, ss * height, ss * width)
+        if debug:
+            dbg = torch.empty(plane + (DEBUG_DTYPE.itemsize,), dtype=torch.uint8, device=where)
+        if taps:
+            res["sig_hits"] = torch.empty(plane, dtype=torch.uint64, device=where)
+            res["sig_shadow"] = torch.empty(plane, dtype=torch.uint64, device=where)
+            res["n_rays"] = torch.empty(plane, dtype=torch.uint32, device=where)
+            tap_struct = _TapsStruct(res["sig_hits"].data_ptr(), res["sig_shadow"].data_ptr(), res["n_rays"].data_ptr())
+            tap_ptr = ctypes.cast(ctypes.pointer(tap_struct), ctypes.c_void_p)
+        self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
+                                                      self.max_depth, ctypes.c_void_p(rgb.data_ptr()),
+                                                      None if dbg is None else ctypes.c_void_p(dbg.data_ptr()), tap_ptr, handle, None),
+                    "mtb_render_batch_device")
+        res["rgb"] = rgb
+        if debug:
+            res["debug"] = dbg
+            res["line_no"] = dbg.view(torch.int32)[..., 0]
+            res["points"] = dbg.view(torch.float64)[..., 1:]
+        res["stats"] = None
         return res
 
     def render_device(self, camera, image_w, image_h, d_rgb_ptr: int, stream: int = 0, chunk=None):

@@ -117,6 +117,9 @@ struct DeviceState {
   // accumulated batches: the channel sums of this device's output views and the arrival counters of their tiles
   DeviceBuffer<uint32_t> batch_sum, batch_arrive;
   cudaEvent_t ev_batch_start = nullptr, ev_batch_stop = nullptr;
+  // batches into device memory (mtb_render_batch_device): device 0's ev_batch_caller marks the caller's stream at the
+  // call, every device's ev_batch_done its own stream after its last operation of the batch
+  cudaEvent_t ev_batch_caller = nullptr, ev_batch_done = nullptr;
   // intersect scratch
   DeviceBuffer<double> q_origins, q_dirs, q_t, q_point;
   DeviceBuffer<int32_t> q_tri;
@@ -143,7 +146,9 @@ struct DeviceState {
     batch_sum.Free(); batch_arrive.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
     if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
-    ev_batch_start = ev_batch_stop = nullptr;
+    if (ev_batch_caller != nullptr) cudaEventDestroy(ev_batch_caller);
+    if (ev_batch_done != nullptr) cudaEventDestroy(ev_batch_done);
+    ev_batch_start = ev_batch_stop = ev_batch_caller = ev_batch_done = nullptr;
     q_origins.Free(); q_dirs.Free(); q_t.Free(); q_point.Free(); q_tri.Free();
     wf_act_point.Free(); wf_act_dir.Free(); wf_act_color.Free(); wf_act_coef.Free(); wf_act_refl.Free(); wf_act_refr.Free();
     wf_act_mtl.Free(); wf_act_pixel.Free(); wf_act_info.Free(); wf_act_path.Free(); wf_ctrl.Free(); wf_act_ready.Free(); wf_qctl.Free();
@@ -795,10 +800,37 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 // subframes k > 1 (accumulated views, no planes): cams and lights hold k sub-frames per output view, output-major, and
 // output view v is the rounded mean of the k * ss * ss samples of sub-frames v*k .. v*k + k-1; n_out counts output
 // views.  Device g renders a contiguous range of output views with all their sub-frames.  k = 1: n_out views as above.
+// device_out: rgb_host, dbg_host and the taps are DEVICE memory of device 0 instead (mtb_render_batch_device), and the
+// batch is ordered on user_stream (NULL: device 0's own stream): it starts after the work queued there before the call,
+// and work queued there after the call sees every device's outputs.  Device 0 renders straight into the caller's
+// buffers; every other device renders into its own and copies its slice over with one copy per output.
 constexpr int64_t kMaxSampleSide = 65536;  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
+
+// mtb_render_batch_device: `p` (nullable unless `name` is d_rgb) must be device memory of `device` with `align`-byte alignment.
+int CheckDeviceOutput(mtb_context *ctx, const void *p, const char *name, int device, uintptr_t align) {
+  if (p == nullptr) return MTB_OK;
+  if ((reinterpret_cast<uintptr_t>(p) & (align - 1u)) != 0u) {
+    ctx->err = std::string(name) + " must be " + std::to_string(align) + "-byte aligned";
+    return MTB_ERR_ARG;
+  }
+  cudaPointerAttributes attr;
+  const cudaError_t e = cudaPointerGetAttributes(&attr, p);
+  cudaGetLastError();
+  if (e != cudaSuccess || attr.type != cudaMemoryTypeDevice) {
+    ctx->err = std::string(name) + " is not device memory (host memory, pageable or pinned, is refused: use the host forms)";
+    return MTB_ERR_ARG;
+  }
+  if (attr.device != device) {
+    ctx->err = std::string(name) + " is memory of device " + std::to_string(attr.device) + ", not of the context's device 0 (" +
+               std::to_string(device) + ")";
+    return MTB_ERR_ARG;
+  }
+  return MTB_OK;
+}
+
 int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
                     int image_w, int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps,
-                    mtb_stats *stats, bool synchronous) {
+                    mtb_stats *stats, bool synchronous, bool device_out = false, cudaStream_t user_stream = nullptr) {
   const auto wall0 = std::chrono::steady_clock::now();
   if (ctx == nullptr) return MTB_ERR_ARG;
   if (ctx->dev.empty()) {
@@ -810,7 +842,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
     return MTB_ERR_ARG;
   }
   if (cams == nullptr || rgb_host == nullptr) {
-    ctx->err = cams == nullptr ? "cams is NULL" : "rgb_out is NULL";
+    ctx->err = cams == nullptr ? "cams is NULL" : (device_out ? "d_rgb is NULL" : "rgb_out is NULL");
     return MTB_ERR_ARG;
   }
   if (subframes < 1) {
@@ -856,6 +888,30 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
   const int n_dev = (int)ctx->dev.size();
   const int tiles_x = (grid_w + 7) / 8, tiles_per_view = tiles_x * ((grid_h + 7) / 8);
   const bool accum = k > 1;
+  if (accum && (dbg_host != nullptr || hits_host != nullptr || shadow_host != nullptr || rays_host != nullptr)) {
+    ctx->err = "there are no debug or tap planes of accumulated views (subframes > 1): render the sub-frames for their planes";
+    return MTB_ERR_ARG;
+  }
+  // The caller's stream and buffers are checked before anything is queued.  The call uploads view records from host
+  // memory and may wait for its own streams when a buffer grows, so it cannot be captured into a graph.
+  cudaStream_t s_caller = nullptr;
+  if (device_out) {
+    const int dev0 = ctx->dev[0].device;
+    MTB_CUDA(ctx, cudaSetDevice(dev0));
+    s_caller = user_stream != nullptr ? user_stream : ctx->dev[0].stream;
+    cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
+    MTB_CUDA(ctx, cudaStreamIsCapturing(s_caller, &capture));
+    if (capture != cudaStreamCaptureStatusNone) {
+      ctx->err = "stream is being captured into a CUDA graph: mtb_render_batch_device cannot be captured";
+      return MTB_ERR_ARG;
+    }
+    int rc = CheckDeviceOutput(ctx, rgb_host, "d_rgb", dev0, 1);
+    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, dbg_host, "d_dbg", dev0, 8);
+    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, hits_host, "d_taps->sig_hits", dev0, 8);
+    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, shadow_host, "d_taps->sig_shadow", dev0, 8);
+    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, rays_host, "d_taps->n_rays", dev0, 4);
+    if (rc != MTB_OK) return rc;
+  }
 
   // per-view records and the views' lights, view-major (the context's lights repeated when the caller passes none)
   const int32_t nl = lights != nullptr ? n_lights : (int32_t)ctx->lights.size();
@@ -881,7 +937,8 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
   // take the second way: their epilogue stores single bytes, and a direct store of those into mapped host memory has
   // not been measured against the copy (which moves 1/ss^2 of the samples' bytes).
   uint8_t *host_direct = nullptr;
-  if (ss == 1 && !accum && n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 && (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
+  if (!device_out && ss == 1 && !accum && n_dev == 1 && !ctx->no_host_store && (image_w & 7) == 0 &&
+      (reinterpret_cast<uintptr_t>(rgb_host) & 7u) == 0u) {
     MTB_CUDA(ctx, cudaSetDevice(ctx->dev[0].device));
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer != nullptr) {
@@ -902,14 +959,18 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
       MTB_CUDA(ctx, cudaEventCreate(&d.ev_batch_start));
       MTB_CUDA(ctx, cudaEventCreate(&d.ev_batch_stop));
     }
+    if (device_out && d.ev_batch_done == nullptr) MTB_CUDA(ctx, cudaEventCreateWithFlags(&d.ev_batch_done, cudaEventDisableTiming));
+    // Device 0 of a batch into device memory stores straight into the caller's buffers.  The other devices render into
+    // their own, as for host outputs, and copy from there: a caller's allocation may have no peer mapping.
+    const bool direct = device_out && g == 0;
     // Everything below is ordered on d.stream: a batch queued behind another one overwrites the records only after the
     // earlier launch has read them.  A buffer that has to grow is freed and reallocated, so the earlier work that may
     // still read it is waited for first.
-    const size_t n_rgb = host_direct != nullptr ? 0 : (size_t)count_out * npx * 3;
+    const size_t n_rgb = host_direct != nullptr || direct ? 0 : (size_t)count_out * npx * 3;
     const size_t n_lt = (size_t)count * nl;
     const size_t n_plane = (size_t)count * gpx;
     const size_t n_sum = accum ? (size_t)count_out * npx * 3 : 0, n_arrive = accum ? (size_t)count_out * tiles_per_view * 2 : 0;
-    auto grows = [n_plane](const void *host, size_t have) { return host != nullptr && n_plane > have; };
+    auto grows = [n_plane, direct](const void *host, size_t have) { return !direct && host != nullptr && n_plane > have; };
     if ((size_t)count > d.batch_views.count || n_lt > d.batch_lights.count || n_rgb > d.batch_rgb.count ||
         grows(dbg_host, d.batch_dbg.count) || grows(hits_host, d.batch_sig_hits.count) || grows(shadow_host, d.batch_sig_shadow.count) ||
         grows(rays_host, d.batch_n_rays.count) || n_sum > d.batch_sum.count || n_arrive > d.batch_arrive.count) {
@@ -922,7 +983,12 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
     sc.lights = d.batch_lights.ptr;
     sc.n_lights = nl;
     mtb::RenderParams p = rp;  // (planes NULL unless this batch asks for them)
-    p.rgb = host_direct != nullptr ? host_direct + (size_t)first * npx * 3 : d.batch_rgb.ptr;
+    const size_t at = (size_t)first * gpx;
+    if (direct) {
+      p.rgb = rgb_host + (size_t)first_out * npx * 3;
+    } else {
+      p.rgb = host_direct != nullptr ? host_direct + (size_t)first * npx * 3 : d.batch_rgb.ptr;
+    }
     mtb::AccumParams acc{nullptr, nullptr, k};
     if (accum) {
       // (cleared on the stream before every launch: a call queued behind another one of a different shape starts from 0)
@@ -933,53 +999,81 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
       acc.sum = d.batch_sum.ptr;
       acc.arrive = d.batch_arrive.ptr;
     }
-    if (dbg_host != nullptr) {
-      MTB_CUDA(ctx, d.batch_dbg.Reserve(n_plane));
-      p.dbg = d.batch_dbg.ptr;
-    }
-    if (hits_host != nullptr) {
-      MTB_CUDA(ctx, d.batch_sig_hits.Reserve(n_plane));
-      p.sig_hits = d.batch_sig_hits.ptr;
-    }
-    if (shadow_host != nullptr) {
-      MTB_CUDA(ctx, d.batch_sig_shadow.Reserve(n_plane));
-      p.sig_shadow = d.batch_sig_shadow.ptr;
-    }
-    if (rays_host != nullptr) {
-      MTB_CUDA(ctx, d.batch_n_rays.Reserve(n_plane));
-      p.n_rays = d.batch_n_rays.ptr;
+    if (direct) {
+      if (dbg_host != nullptr) p.dbg = dbg_host + at;
+      if (hits_host != nullptr) p.sig_hits = hits_host + at;
+      if (shadow_host != nullptr) p.sig_shadow = shadow_host + at;
+      if (rays_host != nullptr) p.n_rays = rays_host + at;
+    } else {
+      if (dbg_host != nullptr) {
+        MTB_CUDA(ctx, d.batch_dbg.Reserve(n_plane));
+        p.dbg = d.batch_dbg.ptr;
+      }
+      if (hits_host != nullptr) {
+        MTB_CUDA(ctx, d.batch_sig_hits.Reserve(n_plane));
+        p.sig_hits = d.batch_sig_hits.ptr;
+      }
+      if (shadow_host != nullptr) {
+        MTB_CUDA(ctx, d.batch_sig_shadow.Reserve(n_plane));
+        p.sig_shadow = d.batch_sig_shadow.ptr;
+      }
+      if (rays_host != nullptr) {
+        MTB_CUDA(ctx, d.batch_n_rays.Reserve(n_plane));
+        p.n_rays = d.batch_n_rays.ptr;
+      }
     }
     MTB_CUDA(ctx, d.counters.Reserve(mtb::kNumCounters));
     p.counters = d.counters.ptr;
     if (stats != nullptr || synchronous) {
       MTB_CUDA(ctx, cudaMemsetAsync(d.counters.ptr, 0, mtb::kNumCounters * sizeof(unsigned long long), s));
     }
+    // (after the uploads: they never wait behind the caller's work)
+    if (device_out) MTB_CUDA(ctx, cudaStreamWaitEvent(s, ctx->dev[0].ev_batch_caller, 0));
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_start, s));
     mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, acc, debug_build, s);
     ctx->launches++;
     MTB_CUDA(ctx, cudaGetLastError());
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_stop, s));
-    if (host_direct == nullptr) {
-      MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first_out * npx * 3, d.batch_rgb.ptr, (size_t)count_out * npx * 3, cudaMemcpyDeviceToHost, s));
+    if (!direct) {
+      // device outputs: a copy from device g to device 0 (peer copy, or staged when there is no peer access)
+      const cudaMemcpyKind kind = device_out ? cudaMemcpyDefault : cudaMemcpyDeviceToHost;
+      if (host_direct == nullptr) {
+        MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first_out * npx * 3, d.batch_rgb.ptr, (size_t)count_out * npx * 3, kind, s));
+      }
+      if (dbg_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(dbg_host + at, p.dbg, n_plane * sizeof(mtb_debug), kind, s));
+      if (hits_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(hits_host + at, p.sig_hits, n_plane * 8, kind, s));
+      if (shadow_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(shadow_host + at, p.sig_shadow, n_plane * 8, kind, s));
+      if (rays_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(rays_host + at, p.n_rays, n_plane * 4, kind, s));
     }
-    const size_t at = (size_t)first * gpx;
-    if (dbg_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(dbg_host + at, p.dbg, n_plane * sizeof(mtb_debug), cudaMemcpyDeviceToHost, s));
-    if (hits_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(hits_host + at, p.sig_hits, n_plane * 8, cudaMemcpyDeviceToHost, s));
-    if (shadow_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(shadow_host + at, p.sig_shadow, n_plane * 8, cudaMemcpyDeviceToHost, s));
-    if (rays_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(rays_host + at, p.n_rays, n_plane * 4, cudaMemcpyDeviceToHost, s));
+    if (device_out) MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_done, s));
     return MTB_OK;
   };
+  if (device_out) {
+    // every device's stream waits for the caller's stream as it is at the call (device 0's event, recorded before any
+    // device queues its launch)
+    DeviceState &d0 = ctx->dev[0];
+    MTB_CUDA(ctx, cudaSetDevice(d0.device));
+    if (d0.ev_batch_caller == nullptr) MTB_CUDA(ctx, cudaEventCreateWithFlags(&d0.ev_batch_caller, cudaEventDisableTiming));
+    MTB_CUDA(ctx, cudaEventRecord(d0.ev_batch_caller, s_caller));
+  }
+  std::vector<int> rcs((size_t)n_dev, MTB_OK);
   if (n_dev == 1) {
-    const int rc = launch_on_device(0);
-    if (rc != MTB_OK) return rc;
+    rcs[0] = launch_on_device(0);
   } else {
-    std::vector<int> rcs((size_t)n_dev, MTB_OK);
     std::vector<std::thread> workers;
     for (int g = 0; g < n_dev; g++) workers.emplace_back([&, g]() { rcs[(size_t)g] = launch_on_device(g); });
     for (std::thread &t : workers) t.join();
-    for (int rc : rcs) {
-      if (rc != MTB_OK) return rc;
+  }
+  if (device_out) {
+    // ... and the caller's stream waits for every device's last operation: work queued there after the call (and a
+    // caching allocator that hands the outputs' memory to such work) sees the finished outputs
+    MTB_CUDA(ctx, cudaSetDevice(ctx->dev[0].device));
+    for (int g = 0; g < n_dev && g < n_out; g++) {
+      if (rcs[(size_t)g] == MTB_OK) MTB_CUDA(ctx, cudaStreamWaitEvent(s_caller, ctx->dev[(size_t)g].ev_batch_done, 0));
     }
+  }
+  for (int rc : rcs) {
+    if (rc != MTB_OK) return rc;
   }
   if (!synchronous && stats == nullptr) return MTB_OK;
 
@@ -1373,6 +1467,13 @@ int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32
                                  int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
   return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
                          nullptr, false);
+}
+
+int mtb_render_batch_device(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
+                            int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, void *d_rgb, mtb_debug *d_dbg,
+                            const mtb_taps *d_taps, void *stream, mtb_stats *stats) {
+  return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
+                         static_cast<uint8_t *>(d_rgb), d_dbg, d_taps, stats, false, true, static_cast<cudaStream_t>(stream));
 }
 
 int mtb_wait(mtb_context *ctx) {

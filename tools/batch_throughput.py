@@ -1,7 +1,8 @@
 """Throughput of batches (mtb_render_batch) against one call per frame, on the C3 scene (two lights, depth 5) and its
 orbit yaw = C3 yaw + 2 degrees * k.
 
-    python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3] [--supersample | --debug-planes | --subframes]
+    python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3]
+                                     [--supersample | --debug-planes | --subframes | --device-output]
 
 480x270, 64 frames: (a) one render_chunk per frame, megakernel forced; (b) one render_chunk per frame, automatic
 pipeline choice (after the 13 frames it needs to decide); (c) render_batch in batches of 1, 4, 16, 64.
@@ -33,6 +34,14 @@ sub-frames at yaw + 2 degrees * (f + j / k).  Shapes: 16 outputs x k = 8 at 480x
 same rays; kernel time), and against the way a caller has to do it without the feature: render_batch of the sub-frames
 at s*W x s*H plus the mean in numpy (frames/s end to end).  Per mode: median kernel_ms per call over --reps calls,
 Mrays/s, output frames/s, and whether the output equals the numpy mean of the sub-frames.
+
+--device-output measures batches that leave their outputs in device memory (render_batch(..., device=True),
+mtb_render_batch_device) against the same batch into host memory: 64 views at 480x270; the same with debug and taps;
+16 views at 480x270 with s = 4; 4 outputs x k = 4 sub-frames at 1920x1080.  Per row: frames/s end to end of both forms
+(median of --reps calls; the host form is synchronous, the device form is timed with a host clock around the call and
+torch.cuda.synchronize()), the median kernel_ms per call of both (CUDA events of the library: the device form's come from
+mtb_render_batch_device called with stats, in calls of their own), the bytes the host form copies back per output, and
+whether the device outputs, copied back, equal the host outputs byte for byte (RGB and every plane).
 """
 import argparse
 import hashlib
@@ -251,6 +260,88 @@ def _orbit_subframes(cam, f, k):
 PLANE_KEYS = ("debug", "sig_hits", "sig_shadow", "n_rays")
 
 
+def _walls(fn, reps):
+    """Host wall time of each of `reps` calls of fn() after one warm-up call."""
+    fn()
+    walls = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        fn()
+        walls.append(time.perf_counter() - t0)
+    return walls
+
+
+def _device_kernel_ms(mt, cams, n_out, k, w, h, s, planes, reps):
+    """kernel_ms of mtb_render_batch_device with stats (the call then waits for its batch), into fresh CUDA tensors, on
+    the context's lights: median over `reps` calls after one warm-up call."""
+    import ctypes
+
+    import torch
+
+    from mythtracer_b200 import api
+    cam_arr = np.zeros(len(cams), api.CAMERA_DTYPE)
+    for i, c in enumerate(cams):
+        cam_arr[i] = api.Camera.from_tuple(c).as_array()
+    rgb = torch.empty((n_out, h, w, 3), dtype=torch.uint8, device="cuda:%d" % mt._device0)
+    plane = len(cams) * s * s * w * h
+    dbg = torch.empty(plane * 32 if planes else 0, dtype=torch.uint8, device=rgb.device)
+    tap = torch.empty(plane * 20 if planes else 0, dtype=torch.uint8, device=rgb.device)
+    taps = api._TapsStruct(tap.data_ptr(), tap.data_ptr() + 8 * plane, tap.data_ptr() + 16 * plane) if planes else None
+    stats = np.zeros((), api.STATS_DTYPE)
+    kms = []
+    for rep in range(reps + 1):
+        rc = mt._lib.mtb_render_batch_device(mt._ctx, cam_arr.ctypes.data_as(ctypes.c_void_p), n_out, k, None, 0, w, h, s, mt.max_depth,
+                                             ctypes.c_void_p(rgb.data_ptr()), ctypes.c_void_p(dbg.data_ptr()) if planes else None,
+                                             ctypes.cast(ctypes.pointer(taps), ctypes.c_void_p) if planes else None, None,
+                                             stats.ctypes.data_as(ctypes.c_void_p))
+        mt._check(rc, "mtb_render_batch_device")
+        if rep > 0:
+            kms.append(float(stats["kernel_ms"]))
+    return kms
+
+
+def device_output(mt, files, cfg, reps):
+    """The --device-output measurements (see the module docstring)."""
+    import torch
+    rows = []
+    W, H = cfg["width"], cfg["height"]
+    for n_out, k, w, h, s, planes in ((64, 1, 480, 270, 1, False), (64, 1, 480, 270, 1, True), (16, 1, 480, 270, 4, False),
+                                      (4, 4, W, H, 1, False)):
+        cams = [c for f in range(n_out) for c in _orbit_subframes(files.camera, f, k)]
+        kw = dict(samples_per_axis=s, subframes=k, debug=planes, taps=planes)
+        host, dev = {}, {}
+
+        def host_call():
+            host.update(mt.render_batch(cams, w, h, **kw))
+            return host["stats"]
+        walls_h, kms_h, rays = _timed_calls(host_call, reps)
+
+        def device_call():
+            dev.update(mt.render_batch(cams, w, h, device=True, **kw))
+            torch.cuda.synchronize()
+        walls_d = _walls(device_call, reps)
+        kms_d = _device_kernel_ms(mt, cams, n_out, k, w, h, s, planes, reps)
+        equal = bool(np.array_equal(dev["rgb"].cpu().numpy(), host["rgb"]))
+        if planes:
+            equal &= dev["debug"].cpu().numpy().tobytes() == host["debug"].tobytes()
+            equal &= all(np.array_equal(dev[key].cpu().numpy(), host[key]) for key in ("sig_hits", "sig_shadow", "n_rays"))
+        wh, wd = statistics.median(walls_h), statistics.median(walls_d)
+        name = "%d x %dx%d, s = %d%s%s" % (n_out, w, h, s, ", k = %d" % k if k > 1 else "", ", debug + taps" if planes else "")
+        rec = dict(mode=name, outputs=n_out, subframes=k, width=w, height=h, samples_per_axis=s, debug=planes, taps=planes, rays=rays,
+                   host_frames_per_s=round(n_out / wh, 1), device_frames_per_s=round(n_out / wd, 1),
+                   host_kernel_ms=round(statistics.median(kms_h), 3), device_kernel_ms=round(statistics.median(kms_d), 3),
+                   host_wall_s_all=[round(x, 4) for x in walls_h], device_wall_s_all=[round(x, 4) for x in walls_d],
+                   host_kernel_ms_all=[round(x, 3) for x in kms_h], device_kernel_ms_all=[round(x, 3) for x in kms_d],
+                   host_bytes_copied_per_output=w * h * 3 + (k * s * s * w * h * (32 + 20) if planes else 0), device_equals_host=equal)
+        print("%-40s host %8.1f frames/s  device %8.1f frames/s  kernel %8.3f / %8.3f ms  %s" % (
+            name, rec["host_frames_per_s"], rec["device_frames_per_s"], rec["host_kernel_ms"], rec["device_kernel_ms"],
+            "equal" if equal else "DIFFERENT"), file=sys.stderr, flush=True)
+        rows.append(rec)
+        host.clear()
+        dev.clear()
+    return rows
+
+
 def debug_planes(mt, files, cfg, reps):
     """The --debug-planes measurements (see the module docstring)."""
     groups = []
@@ -319,6 +410,7 @@ def main():
     ap.add_argument("--supersample", action="store_true")
     ap.add_argument("--debug-planes", action="store_true")
     ap.add_argument("--subframes", action="store_true")
+    ap.add_argument("--device-output", action="store_true")
     args = ap.parse_args()
     devices = [int(x) for x in args.devices.split(",")]
     files, cfg = scenegen.generate_config("C3", os.environ.get("MTB_SCENE_DIR", "/tmp/mtb_scenes"))
@@ -337,6 +429,14 @@ def main():
         modes = [r for g in doc["debug_planes"] for r in g["modes"]]
         if not all(r.get("rgb_equals_no_planes", True) and r.get("planes_equal_render_chunk", True) for r in modes):
             sys.exit("a batch with planes differs from the batch without planes or from render_chunk")
+        return
+
+    if args.device_output:
+        doc["device_output"] = device_output(mt, files, cfg, args.reps)
+        mt.close()
+        _emit(doc, args.out)
+        if not all(r["device_equals_host"] for r in doc["device_output"]):
+            sys.exit("a batch into device memory differs from the same batch into host memory")
         return
 
     if args.subframes:
