@@ -129,29 +129,22 @@ typedef struct {
 #define MTB_FLAG_QUEUE 8192u     /* force the queue pipeline: the wavefront as ONE persistent kernel over a single device-side ray queue (all levels) */
 #define MTB_FLAG_WAVEFRONT 4u    /* the same as MTB_FLAG_QUEUE: the queue pipeline is the wavefront's only form */
 #define MTB_FLAG_EXACT_OCTREE 128u /* every regular ray walks the octree in the reference's recursion order (no certified fast traversal) */
-/* Retired forms (all bit-identical, all measured slower on B200; DESIGN.md sections 5 and 6 keep the numbers).  The
- * bits are still accepted and ignored, so callers that set them keep working. */
+/* Retired forms (all bit-identical, all measured slower on B200; DESIGN.md sections 5, 6 and 11 keep the numbers).
+ * The bits are still accepted and ignored, so callers that set them keep working. */
 #define MTB_FLAG_HYBRID 2048u     /* was: hybrid frames, the most expensive tiles through the level-by-level wavefront, the rest through the megakernel */
 #define MTB_FLAG_RAY_SORT 8u      /* was: wavefront, counting-sort every queue by origin cell + direction octant */
 #define MTB_FLAG_PACKING 256u     /* was: megakernel, block-level ray packing on 16x8 tiles */
 #define MTB_FLAG_RESUME 1024u     /* was: megakernel, suspendable walks */
 #define MTB_FLAG_WARP_SYNC 512u   /* was: megakernel, forced warp re-convergence in front of every traversal */
 #define MTB_FLAG_PERSISTENT 64u   /* was: megakernel, persistent warps drawing pixels from a counter */
+#define MTB_FLAG_PAIR_RAYS 16384u /* was: mtb_intersect_rays, rays 2i and 2i+1 walked in lock step by one thread */
+#define MTB_FLAG_CHAIN_RAYS 32768u /* was: mtb_intersect_rays, rays 2i and 2i+1 walked back to back in one node loop */
 /* Scene BVH built ON THE DEVICE (PLOC over the reference boxes, csrc/device_build.cu; SURVEY section 8 f1) instead of
  * on the host threads (binned SAH).  Measured on B200, C3: the device build takes ~20-50 ms against 165 ms on 24 host
  * cores (time to first frame 0.31 s vs 0.39 s), but its trees cost 12 % more box tests per ray (frame 10.2 vs 9.17 ms):
  * the right choice for a scene that is rendered a few times, the wrong one for an animation - hence opt-in.  The
  * rendered bytes are the same either way. */
 #define MTB_FLAG_DEVICE_BVH 4096u
-/* Two rays per lane (measurement aid): mtb_intersect_rays walks rays 2i and 2i+1 in ONE thread - two independent
- * node-load chains in flight per lane (csrc/device_core.cuh, Trace2).  Results are identical to the one-ray-per-lane
- * form; measured on B200 with the shadow rays of the C3 frame it is 6 % SLOWER (DESIGN.md section 11), so the
- * renderers do not use it. */
-#define MTB_FLAG_PAIR_RAYS 16384u
-/* Chained rays (measurement aid): mtb_intersect_rays walks rays 2i and 2i+1 in one thread, BACK TO BACK inside one node
- * loop (csrc/device_core.cuh, TraceChain); with MTB_FLAG_PAIR_RAYS also set: the same two rays by two ordinary calls,
- * the baseline of that comparison.  Results are identical to the one-ray-per-thread form. */
-#define MTB_FLAG_CHAIN_RAYS 32768u
 #define MTB_FLAG_NO_TILE_ORDER 32u /* megakernel: always launch tiles in scanline order (A/B of the cost-aware launch order) */
 
 /* ---- life cycle -------------------------------------------------------------------------------- */

@@ -1579,8 +1579,7 @@ int mtb_intersect_rays(mtb_context *ctx, int64_t n, const double *origins, const
   ip.point = d.q_point.ptr;
   ip.counters = d.counters.ptr;
   MTB_CUDA(ctx, cudaEventRecord(d.ev_start, d.stream));
-  mtb::LaunchIntersect(d.scene, ip, (ctx->flags & MTB_FLAG_COUNT_WORK) != 0,
-                       ((ctx->flags & MTB_FLAG_PAIR_RAYS) != 0 ? 1 : 0) + ((ctx->flags & MTB_FLAG_CHAIN_RAYS) != 0 ? 2 : 0), d.stream);
+  mtb::LaunchIntersect(d.scene, ip, (ctx->flags & MTB_FLAG_COUNT_WORK) != 0, d.stream);
   ctx->launches++;
   MTB_CUDA(ctx, cudaGetLastError());
   MTB_CUDA(ctx, cudaEventRecord(d.ev_stop, d.stream));

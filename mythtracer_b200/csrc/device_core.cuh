@@ -534,12 +534,6 @@ struct TriVerts {
   double2 a, b, c, d;
   double v22;
 };
-__device__ __forceinline__ TriVerts LoadVerts(const double *vert) {
-  TriVerts v;
-  v.a = Ld2(vert + 0), v.b = Ld2(vert + 2), v.c = Ld2(vert + 4), v.d = Ld2(vert + 6);
-  v.v22 = __ldg(vert + 8);
-  return v;
-}
 __device__ __forceinline__ bool MollerTrumboreBound(const TriVerts &tv, const Ray &r, double *t_out, double *e_out) {
   const D3 v0 = Mk(tv.a.x, tv.a.y, tv.b.x), v1 = Mk(tv.b.y, tv.c.x, tv.c.y), v2 = Mk(tv.d.x, tv.d.y, tv.v22);
   const D3 e1 = Sub(v1, v0);
@@ -583,81 +577,43 @@ __device__ __forceinline__ bool MollerTrumboreBound(const TriVerts &tv, const Ra
 // ray and the 6 of the best hit alive across it made the register allocator spill and rematerialise inside the loop
 // (3 local loads + 3 F2F + 3 DSETP per node visit under the 64-register cap).
 //
-// Where the twelve doubles live is a build option (measured A/B in DESIGN.md section 5):
-//   MTB_SMEM_RAY = 1  shared memory, laid out [field][thread] (conflict-free 64-bit accesses).  ncu on the
-//                     local-memory form: the leaf reloads were 44 % of the kernel's local-memory bytes, half of them
-//                     missed L1 (the per-SM working set of 1024 threads' local memory is larger than L1) and went to
-//                     L2 next to the BVH nodes.
-//   MTB_SMEM_RAY = 0  a local struct whose address escapes through MTB_FAST_BARRIER, so nothing of it stays in
-//                     registers between two leaf visits.
-#ifndef MTB_SMEM_RAY
-#define MTB_SMEM_RAY 1
-#endif
-#ifndef MTB_LEAF_PRELOAD
-#define MTB_LEAF_PRELOAD 1
-#endif
-#ifndef MTB_LD256
-#define MTB_LD256 1
-#endif
-// Traversal stack of TraceFast.  An entry is 64 bits: conservative entry distance (FP32 bits) << 32 | child
-// reference.  Short-stack form (north star item 3): the first MTB_SMEM_STACK entries of every thread live in shared
-// memory, laid out [entry][thread]; only deeper entries go to the thread's local array.  MTB_SMEM_STACK = 0 keeps
-// the whole stack in local memory (measured: 8.93 vs 9.06 ms on C3 for 8 shared entries - the carve-out costs L1).
-#ifndef MTB_SMEM_STACK
-#define MTB_SMEM_STACK 0
-#endif
+// The twelve doubles live in shared memory, laid out [field][thread] (conflict-free 64-bit accesses).  ncu on the
+// local-memory form: the leaf reloads were 44 % of the kernel's local-memory bytes, half of them missed L1 (the per-SM
+// working set of 1024 threads' local memory is larger than L1) and went to L2 next to the BVH nodes.  The best hit
+// (kFmT, kFmE, kFmLo2) is touched by only 0.5 accepted hits per ray, but keeping it in local memory instead, so that
+// sixteen 64-thread blocks fit a smaller shared-memory carve-out, measured neutral (DESIGN.md section 5, row "best hit
+// (t, e, lo2) in local memory"): L1 capacity is not what the walk waits for.
+//
+// Fields: o.xyz, d.xyz, inv.xyz, best t, its error bound e, lo2 = min (t - e) over all other accepted hits.
 enum FastField { kFmO = 0, kFmD = 3, kFmInv = 6, kFmT = 9, kFmE = 10, kFmLo2 = 11, kFmWords = 12 };
+// MTB_FAST_BARRIER: a compiler barrier whose operand is the address of a per-ray local FastMem.  Nothing reads or
+// writes the struct (the fields are in shared memory), but dropping the operand changes the code ptxas generates for
+// every kernel that traces, so the struct stays as the barrier's anchor.
 struct alignas(16) FastMem {
-  double w[kFmWords];  // o.xyz, d.xyz, inv.xyz, best t, its error bound e, lo2 = min (t - e) over all other accepted hits
+  double w[kFmWords];
 };
 #define MTB_FAST_BARRIER(m) asm volatile("" : : "l"(m) : "memory")
 
 // Per-thread handles of the fast traversal's scratch memory.
 struct FastCtx {
-  unsigned stack_base;  // shared-space address of this thread's stack column (entry k at + k * stride_bytes)
-  unsigned ray_base;    // shared-space address of this thread's FastMem column (field f at + f * stride_bytes)
-  int stride_bytes;     // threads per block * 8
+  unsigned ray_base;  // shared-space address of this thread's column of the fields (field f at + f * stride_bytes)
+  int stride_bytes;   // threads per block * 8
 };
-#if MTB_SMEM_STACK > 0 || MTB_SMEM_RAY
-#define MTB_DECLARE_FAST_CTX(threads)                                                                         \
-  __shared__ unsigned long long s_fast_scratch[(MTB_SMEM_STACK + (MTB_SMEM_RAY ? kFmSharedWords : 0)) * (threads)]; \
-  const unsigned fast_base__ = (unsigned)__cvta_generic_to_shared(s_fast_scratch + threadIdx.x);              \
-  const FastCtx fctx{fast_base__, fast_base__ + (unsigned)(MTB_SMEM_STACK * (threads) * 8), (threads) * 8}
-#else
-#define MTB_DECLARE_FAST_CTX(threads) const FastCtx fctx{0u, 0u, 0}
-#endif
+#define MTB_DECLARE_FAST_CTX(threads)                                                            \
+  __shared__ unsigned long long s_fast_scratch[kFmWords * (threads)];                            \
+  const FastCtx fctx{(unsigned)__cvta_generic_to_shared(s_fast_scratch + threadIdx.x), (threads) * 8}
 
-// kFmO .. kFmInv are read at every leaf visit and live in shared memory (MTB_SMEM_RAY).  The best hit (kFmT, kFmE,
-// kFmLo2) is touched by 0.5 accepted hits per ray; MTB_SMEM_HIT = 0 keeps it in the thread's local FastMem instead, so
-// that nine shared words per thread let sixteen 64-thread blocks fit the 100 KB shared-memory configuration instead of
-// the 132 KB one (32 KB more L1).  Measured on B200 at 16 blocks per SM: C3 8.92 vs 8.86 ms, C5 49.6 vs 49.3 with all
-// twelve words shared - L1 capacity is not what the walk waits for - so the default stays 1.  `field` is a constant at
-// every call site.
-#ifndef MTB_SMEM_HIT
-#define MTB_SMEM_HIT 1
-#endif
-constexpr int kFmSharedWords = MTB_SMEM_HIT ? (int)kFmWords : (int)kFmT;
-__device__ __forceinline__ double FmLoad(const FastCtx &fc, const FastMem *m, int field) {
-#if MTB_SMEM_RAY
-  if (MTB_SMEM_HIT || field < kFmT) {
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(fc.ray_base + (unsigned)(field * fc.stride_bytes)));
-    return v;
-  }
-#endif
-  return m->w[field];
+// `field` is a constant at every call site.
+__device__ __forceinline__ double FmLoad(const FastCtx &fc, int field) {
+  double v;
+  asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(fc.ray_base + (unsigned)(field * fc.stride_bytes)));
+  return v;
 }
-__device__ __forceinline__ void FmStore(const FastCtx &fc, FastMem *m, int field, double v) {
-#if MTB_SMEM_RAY
-  if (MTB_SMEM_HIT || field < kFmT) {
-    asm volatile("st.shared.f64 [%0], %1;" : : "r"(fc.ray_base + (unsigned)(field * fc.stride_bytes)), "d"(v));
-    return;
-  }
-#endif
-  m->w[field] = v;
+__device__ __forceinline__ void FmStore(const FastCtx &fc, int field, double v) {
+  asm volatile("st.shared.f64 [%0], %1;" : : "r"(fc.ray_base + (unsigned)(field * fc.stride_bytes)), "d"(v));
 }
-__device__ __forceinline__ D3 FmLoad3(const FastCtx &fc, const FastMem *m, int field) {
-  return Mk(FmLoad(fc, m, field), FmLoad(fc, m, field + 1), FmLoad(fc, m, field + 2));
+__device__ __forceinline__ D3 FmLoad3(const FastCtx &fc, int field) {
+  return Mk(FmLoad(fc, field), FmLoad(fc, field + 1), FmLoad(fc, field + 2));
 }
 
 struct FastRay {
@@ -668,10 +624,10 @@ struct FastRay {
 // origin and inverse direction (loaded once per leaf visit); the direction is fetched when the pre-test passes.
 // *slot / *prune are the canonical slot of the best hit so far (-1: none) and the FP32 pruning distance.
 template <bool DBG>
-__device__ __forceinline__ void TestSlotFast(const SlotRec *rec, Ray &r, const FastCtx &fc, FastMem *m, int *slot, float *prune,
+__device__ __forceinline__ void TestSlotFast(const SlotRec *rec, Ray &r, const FastCtx &fc, int *slot, float *prune,
                                              unsigned long long *cnt) {
-#if MTB_LD256 && MTB_LEAF_PRELOAD
-  // the whole 128-byte record (box, vertices, ids) in four 256-bit loads: one memory round trip per candidate
+  // the whole 128-byte record (box, vertices, ids) in four 256-bit loads: one memory round trip per candidate instead
+  // of two for the 58 % of the candidates that pass the pre-test
   double2 b0, b1, b2;
   TriVerts tv;
   double ids_word;
@@ -681,41 +637,26 @@ __device__ __forceinline__ void TestSlotFast(const SlotRec *rec, Ray &r, const F
     asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(tv.b.x), "=d"(tv.b.y), "=d"(tv.c.x), "=d"(tv.c.y) : "l"(reinterpret_cast<const char *>(rec) + 64));
     asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(tv.d.x), "=d"(tv.d.y), "=d"(tv.v22), "=d"(ids_word) : "l"(reinterpret_cast<const char *>(rec) + 96));
   }
-#else
-  const double2 b0 = Ld2(rec->box + 0), b1 = Ld2(rec->box + 2), b2 = Ld2(rec->box + 4);
-#if MTB_LEAF_PRELOAD
-  // the vertices travel with the box (same 128-byte record): one memory round trip per candidate instead of two
-  // for the 58 % of the candidates that pass the pre-test
-  const TriVerts tv = LoadVerts(rec->vert);
-#endif
-#endif
   Count<DBG>(cnt, kTriAabb);
   double unused;
   if (!SlabRegular(b0.x, b0.y, b1.x, b1.y, b2.x, b2.y, r, &unused)) return;  // primitive_triangle.cc:85-108
   Count<DBG>(cnt, kMt);
-  r.d = FmLoad3(fc, m, kFmD);
-#if !MTB_LEAF_PRELOAD
-  const TriVerts tv = LoadVerts(rec->vert);
-#endif
+  r.d = FmLoad3(fc, kFmD);
   double t, e;
   if (!MollerTrumboreBound(tv, r, &t, &e)) return;
   Count<DBG>(cnt, kHit);
-#if MTB_LD256 && MTB_LEAF_PRELOAD
   const int canon = __double2hiint(ids_word);  // SlotRec: tri (low word), canon (high word) behind the vertices
-#else
-  const int canon = __ldg(&rec->canon);
-#endif
   if (canon == *slot) return;  // the best hit itself, met again through another of its references (spatial splits)
   if (*slot >= 0) {
-    const double bt = FmLoad(fc, m, kFmT), lo2 = FmLoad(fc, m, kFmLo2);
+    const double bt = FmLoad(fc, kFmT), lo2 = FmLoad(fc, kFmLo2);
     if (!(t < bt)) {
-      FmStore(fc, m, kFmLo2, fmin(lo2, t - e));
+      FmStore(fc, kFmLo2, fmin(lo2, t - e));
       return;
     }
-    FmStore(fc, m, kFmLo2, fmin(lo2, bt - FmLoad(fc, m, kFmE)));
+    FmStore(fc, kFmLo2, fmin(lo2, bt - FmLoad(fc, kFmE)));
   }
-  FmStore(fc, m, kFmT, t);
-  FmStore(fc, m, kFmE, e);
+  FmStore(fc, kFmT, t);
+  FmStore(fc, kFmE, e);
   *slot = canon;
   *prune = fminf(*prune, __double2float_ru(t + 2.0 * e + t * 0x1p-20));
 }
@@ -763,32 +704,6 @@ __device__ __forceinline__ float LimitPrune(const DeviceScene &sc, const D3 &d, 
   return __double2float_ru(t_limit + 2.0 * m + t_limit * 0x1p-20);
 }
 
-constexpr int kFastLocalStack = kFastStack - MTB_SMEM_STACK;
-
-__device__ __forceinline__ void FastPush(const FastCtx &fc, unsigned long long *local, int sp, unsigned long long v) {
-#if MTB_SMEM_STACK > 0
-  if (sp < MTB_SMEM_STACK) {
-    asm volatile("st.shared.u64 [%0], %1;" : : "r"(fc.stack_base + (unsigned)(sp * fc.stride_bytes)), "l"(v));
-  } else {
-    local[sp - MTB_SMEM_STACK] = v;
-  }
-#else
-  local[sp] = v;
-#endif
-}
-__device__ __forceinline__ unsigned long long FastPop(const FastCtx &fc, const unsigned long long *local, int sp) {
-#if MTB_SMEM_STACK > 0
-  if (sp < MTB_SMEM_STACK) {
-    unsigned long long v;
-    asm volatile("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(fc.stack_base + (unsigned)(sp * fc.stride_bytes)));
-    return v;
-  }
-  return local[sp - MTB_SMEM_STACK];
-#else
-  return local[sp];
-#endif
-}
-
 // Closing stated edge case (a) of round 1 (DESIGN.md section 4).  The recursion stops at the first child, in
 // entry-distance order, that returns a hit (octtree.cc:244-246).  Octants have disjoint interiors, so along a regular
 // ray an octant B that is entered AFTER a sibling A is entered only when A has been left: a hit in A cannot be
@@ -800,10 +715,10 @@ __device__ __forceinline__ unsigned long long FastPop(const FastCtx &fc, const u
 // that HOLDS the winning triangle is measured with the reference's own FP64 slab arithmetic, and a passage shorter
 // than 2^-40 relative (keys carry ~2^-52) hands the ray to the exact recursion.  The test ray of round 1
 // (o = (7,7,3), d = (-1,-1,-1/8) through the edge x = y = 4 of a [0,8]^3 root) is such a ray.
-__device__ __forceinline__ bool DegeneratePassage(const DeviceScene &sc, int slot, const FastCtx &fc, const FastMem *m) {
+__device__ __forceinline__ bool DegeneratePassage(const DeviceScene &sc, int slot, const FastCtx &fc) {
   Ray r;
-  r.o = FmLoad3(fc, m, kFmO);
-  r.inv = FmLoad3(fc, m, kFmInv);
+  r.o = FmLoad3(fc, kFmO);
+  r.inv = FmLoad3(fc, kFmInv);
   r.sx = r.inv.x < 0.0;
   r.sy = r.inv.y < 0.0;
   r.sz = r.inv.z < 0.0;
@@ -820,23 +735,17 @@ __device__ __forceinline__ bool DegeneratePassage(const DeviceScene &sc, int slo
 
 // The FP64 ray has been stored by the caller (fields kFmO .. kFmInv); `prune0` = LimitPrune.  Returns the canonical
 // slot of the closest accepted hit (-1: none) with its distance in *t_out.
-#ifndef MTB_PREFETCH_KIDS
-#define MTB_PREFETCH_KIDS 0
-#endif
-#ifndef MTB_SPEC_LEAF
-#define MTB_SPEC_LEAF 0
-#endif
-#ifndef MTB_RAY_RELOAD
-#define MTB_RAY_RELOAD 1
-#endif
 template <bool DBG>
 __device__ __forceinline__ int TraceFast(const DeviceScene &sc, FastMem *m, const FastRay &r_in, float prune0, double *t_out, bool *ambiguous,
                                          unsigned long long *cnt, const FastCtx &fc) {
-  unsigned long long stack[kFastLocalStack];
+  // Traversal stack, in the thread's local memory.  An entry is 64 bits: conservative entry distance (FP32 bits) << 32 |
+  // child reference, so a pop can discard a subtree behind the pruning distance without touching its node.  Its first
+  // entries in shared memory measured slower: the carve-out costs L1 (DESIGN.md section 5, row "first 8 stack entries").
+  unsigned long long stack[kFastStack];
   int sp = 0;
   int slot = -1;
   float prune = prune0;
-  FmStore(fc, m, kFmLo2, CUDART_INF);
+  FmStore(fc, kFmLo2, CUDART_INF);
   int node = 0;
   unsigned visits = 0;  // (counting build only)
   // next subtree from the stack that still starts in front of the pruning distance; kFastExit when there is none
@@ -844,17 +753,13 @@ __device__ __forceinline__ int TraceFast(const DeviceScene &sc, FastMem *m, cons
   do {                                                                   \
     node = kFastExit;                                                    \
     while (sp > 0) {                                                     \
-      const unsigned long long top__ = FastPop(fc, stack, --sp);         \
+      const unsigned long long top__ = stack[--sp];                      \
       if (__uint_as_float((unsigned)(top__ >> 32)) <= prune) {           \
         node = (int)(unsigned)top__;                                     \
         break;                                                           \
       }                                                                  \
     }                                                                    \
   } while (0)
-#if MTB_SPEC_LEAF
-  int pend = kFastExit;  // a leaf that was reached but not tested yet (kFastExit: none)
-#endif
-#if MTB_RAY_RELOAD
   // The FP32 ray is only needed in the node loop, the leaf tests in between are where the register pressure peaks
   // (FP64 Moller-Trumbore).  Left to itself ptxas keeps the six floats "live" across the leaf phase by spilling them and
   // puts the reloads INSIDE the node loop (three LDL per node visit at 64 registers).  So the live range is split by
@@ -862,16 +767,10 @@ __device__ __forceinline__ int TraceFast(const DeviceScene &sc, FastMem *m, cons
   // barrier of the leaf phase (memory clobber) forces exactly that.
   const FastRay *r_mem = &r_in;
   asm volatile("" : "+l"(r_mem) : : "memory");
-#else
-  const FastRay &r = r_in;
-#endif
   for (;;) {
-#if MTB_RAY_RELOAD
     const FastRay r = *r_mem;
-#endif
     while (node >= 0) {
       if (DBG) visits++;
-#if MTB_LD256
       // one 64-byte node = two 256-bit loads (LDG.E.256, new with sm_100): half the L1 requests / wavefronts of four
       // 128-bit loads when the lanes of a warp are at different nodes
       float4 q0, q1, q2;
@@ -888,23 +787,13 @@ __device__ __forceinline__ int TraceFast(const DeviceScene &sc, FastMem *m, cons
         kids.x = __float_as_int(w8);
         kids.y = __float_as_int(w9);
       }
-#else
-      const float4 *q = reinterpret_cast<const float4 *>(sc.gnodes + node);
-      const int2 kids = __ldg(reinterpret_cast<const int2 *>(q + 3));
-      const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2);
-#endif
-#if MTB_PREFETCH_KIDS
-      // the next node of the walk is one of the two children: start both fetches now, the box tests take ~100 cycles
-      if (kids.x >= 0) asm volatile("prefetch.global.L1 [%0];" : : "l"(sc.gnodes + kids.x));
-      if (kids.y >= 0) asm volatile("prefetch.global.L1 [%0];" : : "l"(sc.gnodes + kids.y));
-#endif
       Count<DBG>(cnt, kBvh, 2);
       float tl, tr;
       const bool hl = FastBox(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, r, prune, &tl);
       const bool hr = FastBox(q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, r, prune, &tr);
       if (hl && hr) {
         const bool right_first = tr < tl;
-        FastPush(fc, stack, sp++, ((unsigned long long)__float_as_uint(right_first ? tl : tr) << 32) | (unsigned)(right_first ? kids.x : kids.y));
+        stack[sp++] = ((unsigned long long)__float_as_uint(right_first ? tl : tr) << 32) | (unsigned)(right_first ? kids.x : kids.y);
         node = right_first ? kids.y : kids.x;
       } else if (hl) {
         node = kids.x;
@@ -913,45 +802,18 @@ __device__ __forceinline__ int TraceFast(const DeviceScene &sc, FastMem *m, cons
       } else {
         MTB_FAST_POP();
       }
-#if MTB_SPEC_LEAF
-      // Speculative walk (Aila & Laine): the first leaf a lane reaches is parked and the lane keeps walking - the other
-      // lanes of the warp are still in this loop anyway - until it reaches a second leaf or runs out of nodes.  The
-      // parked leaf has not lowered the pruning distance yet, so the lane may visit nodes it would have skipped; which
-      // candidates are EVALUATED before the search ends can change, which triangle wins cannot (section 4: every
-      // accepted hit is exact, a pruned subtree starts behind t* + 2 e*).
-      if (node < 0 && node != kFastExit && pend == kFastExit) {
-        pend = node;
-        MTB_FAST_POP();
-      }
-#endif
     }
-#if MTB_SPEC_LEAF
-    if (node == kFastExit && pend == kFastExit) break;
-#else
     if (node == kFastExit) break;
-#endif
     {
       MTB_FAST_BARRIER(m);
       Ray rr;  // FP64 origin and inverse direction: once per leaf visit
-      rr.o = FmLoad3(fc, m, kFmO);
-      rr.inv = FmLoad3(fc, m, kFmInv);
+      rr.o = FmLoad3(fc, kFmO);
+      rr.inv = FmLoad3(fc, kFmInv);
       rr.sx = rr.inv.x < 0.0;
       rr.sy = rr.inv.y < 0.0;
       rr.sz = rr.inv.z < 0.0;
-#if MTB_SPEC_LEAF
-      // the parked leaf first (it was reached first), then the one the walk stopped at
-#pragma unroll 1
-      for (int k = 0; k < 2; k++) {
-        const int lf = k == 0 ? pend : node;
-        if (lf == kFastExit) continue;
-        const unsigned leaf = ~(unsigned)lf;
-        for (unsigned s = leaf >> 3, e = s + (leaf & 7u); s < e; s++) TestSlotFast<DBG>(sc.gslots + s, rr, fc, m, &slot, &prune, cnt);
-      }
-      pend = kFastExit;
-#else
       const unsigned leaf = ~(unsigned)node;
-      for (unsigned s = leaf >> 3, e = s + (leaf & 7u); s < e; s++) TestSlotFast<DBG>(sc.gslots + s, rr, fc, m, &slot, &prune, cnt);
-#endif
+      for (unsigned s = leaf >> 3, e = s + (leaf & 7u); s < e; s++) TestSlotFast<DBG>(sc.gslots + s, rr, fc, &slot, &prune, cnt);
       MTB_FAST_BARRIER(m);
     }
     MTB_FAST_POP();
@@ -964,8 +826,8 @@ __device__ __forceinline__ int TraceFast(const DeviceScene &sc, FastMem *m, cons
   bool amb = false;
   if (slot >= 0) {
     MTB_FAST_BARRIER(m);
-    const double t = FmLoad(fc, m, kFmT);
-    amb = FmLoad(fc, m, kFmLo2) <= t + FmLoad(fc, m, kFmE) || DegeneratePassage(sc, slot, fc, m);
+    const double t = FmLoad(fc, kFmT);
+    amb = FmLoad(fc, kFmLo2) <= t + FmLoad(fc, kFmE) || DegeneratePassage(sc, slot, fc);
     *t_out = t;
   }
   *ambiguous = amb;
@@ -1032,9 +894,9 @@ __device__ __forceinline__ int Trace(const DeviceScene &sc, const D3 &o, const D
     const double ai_max = fmax(fmax(fabs(inv.x), fabs(inv.y)), fabs(inv.z));
     const double ai_min = fmin(fmin(fabs(inv.x), fabs(inv.y)), fabs(inv.z));
     fast = regular && sc.gnodes != nullptr && R > 0.0f && ao <= 8.0 * (double)R && ai_max <= 0x1p100 && ai_min >= 0x1p-100;
-    FmStore(fc, &mem, kFmO + 0, o.x), FmStore(fc, &mem, kFmO + 1, o.y), FmStore(fc, &mem, kFmO + 2, o.z);
-    FmStore(fc, &mem, kFmD + 0, d.x), FmStore(fc, &mem, kFmD + 1, d.y), FmStore(fc, &mem, kFmD + 2, d.z);
-    FmStore(fc, &mem, kFmInv + 0, inv.x), FmStore(fc, &mem, kFmInv + 1, inv.y), FmStore(fc, &mem, kFmInv + 2, inv.z);
+    FmStore(fc, kFmO + 0, o.x), FmStore(fc, kFmO + 1, o.y), FmStore(fc, kFmO + 2, o.z);
+    FmStore(fc, kFmD + 0, d.x), FmStore(fc, kFmD + 1, d.y), FmStore(fc, kFmD + 2, d.z);
+    FmStore(fc, kFmInv + 0, inv.x), FmStore(fc, kFmInv + 1, inv.y), FmStore(fc, kFmInv + 2, inv.z);
     fr.ix = (float)inv.x;
     fr.iy = (float)inv.y;
     fr.iz = (float)inv.z;
@@ -1054,312 +916,8 @@ __device__ __forceinline__ int Trace(const DeviceScene &sc, const D3 &o, const D
     Count<DBG>(cnt, kFallback);
   }
   MTB_FAST_BARRIER(&mem);
-  return TraceExactCold<DBG>(sc, FmLoad3(fc, &mem, kFmO), FmLoad3(fc, &mem, kFmD), t_out, cnt);
+  return TraceExactCold<DBG>(sc, FmLoad3(fc, kFmO), FmLoad3(fc, kFmD), t_out, cnt);
 }
-
-// ---------------------------------------------------------------------------------------------------
-// Two rays per lane.  The fast traversal is latency-bound (DESIGN.md section 5: a walk is a chain of dependent node
-// loads, half of them served by L2, with ~24 warps per SM to hide them), so a lane that walks TWO independent rays in
-// one loop - both node loads are issued before either is consumed - doubles the loads in flight per warp for ~20
-// registers.  The two rays are independent queries (the shadow segments of one hit towards two lights; two rays of a
-// batch): each keeps its own stack (local memory), its own FP64 scratch column (shared memory) and its own best hit,
-// and is answered exactly as Trace() would answer it alone - same candidates, same exact tests, same certification,
-// same fallback to the exact recursion.
-// ---------------------------------------------------------------------------------------------------
-#define MTB_DECLARE_FAST_CTX2(threads)                                                             \
-  __shared__ unsigned long long s_fast_scratch[2 * kFmSharedWords * (threads)];                    \
-  const unsigned fast_base__ = (unsigned)__cvta_generic_to_shared(s_fast_scratch + threadIdx.x);   \
-  const FastCtx fctx{0u, fast_base__, (threads) * 8};                                              \
-  const FastCtx fctx_b{0u, fast_base__ + (unsigned)(kFmSharedWords * (threads) * 8), (threads) * 8}
-
-struct PairQuery {
-  bool active;     // in: there is a ray
-  bool fast;       // (internal) the ray is inside the fast traversal's model
-  double t_limit;  // in: as Trace()
-  int slot;        // out: canonical slot of the hit, -1: none
-  double t;        // out
-};
-
-// Ray set-up of Trace(): stores the FP64 ray into the scratch column `fc`, returns the FP32 ray and the pruning limit.
-__device__ __forceinline__ bool FastSetup(const DeviceScene &sc, const D3 &o, const D3 &d, double t_limit, const FastCtx &fc, FastMem *m,
-                                          FastRay *fr, float *prune0) {
-  const D3 inv = Mk(1.0 / d.x, 1.0 / d.y, 1.0 / d.z);
-  const bool regular = isfinite(inv.x) && isfinite(inv.y) && isfinite(inv.z) && inv.x != 0.0 && inv.y != 0.0 && inv.z != 0.0 &&
-                       isfinite(o.x) && isfinite(o.y) && isfinite(o.z);
-  const float R = sc.cull_radius;
-  const double ao = fmax(fmax(fabs(o.x), fabs(o.y)), fabs(o.z));
-  const double ai_max = fmax(fmax(fabs(inv.x), fabs(inv.y)), fabs(inv.z));
-  const double ai_min = fmin(fmin(fabs(inv.x), fabs(inv.y)), fabs(inv.z));
-  const bool fast = regular && sc.gnodes != nullptr && R > 0.0f && ao <= 8.0 * (double)R && ai_max <= 0x1p100 && ai_min >= 0x1p-100;
-  FmStore(fc, nullptr, kFmO + 0, o.x), FmStore(fc, nullptr, kFmO + 1, o.y), FmStore(fc, nullptr, kFmO + 2, o.z);
-  FmStore(fc, nullptr, kFmD + 0, d.x), FmStore(fc, nullptr, kFmD + 1, d.y), FmStore(fc, nullptr, kFmD + 2, d.z);
-  FmStore(fc, nullptr, kFmInv + 0, inv.x), FmStore(fc, nullptr, kFmInv + 1, inv.y), FmStore(fc, nullptr, kFmInv + 2, inv.z);
-  FmStore(fc, m, kFmLo2, CUDART_INF);
-  fr->ix = (float)inv.x;
-  fr->iy = (float)inv.y;
-  fr->iz = (float)inv.z;
-  fr->nox = -((float)o.x * fr->ix);
-  fr->noy = -((float)o.y * fr->iy);
-  fr->noz = -((float)o.z * fr->iz);
-  *prune0 = LimitPrune(sc, d, t_limit);
-  return fast;
-}
-
-#if MTB_SMEM_RAY && MTB_LD256 && MTB_SMEM_STACK == 0
-template <bool DBG>
-__device__ __forceinline__ void Trace2(const DeviceScene &sc, const D3 &oa, const D3 &da, const D3 &ob, const D3 &db, PairQuery *qa,
-                                       PairQuery *qb, unsigned long long *cnt, const FastCtx &fca, const FastCtx &fcb) {
-  FastRay ra, rb;
-  float prune_a = 0.f, prune_b = 0.f;
-  qa->slot = qb->slot = -1;
-  FastMem mem_a, mem_b;  // best hit of each walk (MTB_SMEM_HIT = 0)
-  qa->fast = qa->active && FastSetup(sc, oa, da, qa->t_limit, fca, &mem_a, &ra, &prune_a);
-  qb->fast = qb->active && FastSetup(sc, ob, db, qb->t_limit, fcb, &mem_b, &rb, &prune_b);
-  if (qa->active) Count<DBG>(cnt, kRays);
-  if (qb->active) Count<DBG>(cnt, kRays);
-  unsigned long long stack_a[kFastLocalStack], stack_b[kFastLocalStack];
-  int sp_a = 0, sp_b = 0, slot_a = -1, slot_b = -1;
-  int node_a = qa->fast ? 0 : kFastExit, node_b = qb->fast ? 0 : kFastExit;
-  asm volatile("" ::: "memory");
-  // one step of one walk: the two child boxes of the loaded node against the ray, nearer child first
-#define MTB_PAIR_STEP(node, q0, q1, q2, kx, ky, r, prune, stack, sp)                                                          \
-  do {                                                                                                                        \
-    Count<DBG>(cnt, kBvh, 2);                                                                                                 \
-    float tl__, tr__;                                                                                                         \
-    const bool hl__ = FastBox(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, r, prune, &tl__);                                           \
-    const bool hr__ = FastBox(q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, r, prune, &tr__);                                           \
-    if (hl__ && hr__) {                                                                                                       \
-      const bool rf__ = tr__ < tl__;                                                                                          \
-      stack[sp++] = ((unsigned long long)__float_as_uint(rf__ ? tl__ : tr__) << 32) | (unsigned)(rf__ ? kx : ky);             \
-      node = rf__ ? ky : kx;                                                                                                  \
-    } else if (hl__) {                                                                                                        \
-      node = kx;                                                                                                              \
-    } else if (hr__) {                                                                                                        \
-      node = ky;                                                                                                              \
-    } else {                                                                                                                  \
-      node = kFastExit;                                                                                                       \
-      while (sp > 0) {                                                                                                        \
-        const unsigned long long top__ = stack[--sp];                                                                         \
-        if (__uint_as_float((unsigned)(top__ >> 32)) <= prune) {                                                              \
-          node = (int)(unsigned)top__;                                                                                        \
-          break;                                                                                                              \
-        }                                                                                                                     \
-      }                                                                                                                       \
-    }                                                                                                                         \
-  } while (0)
-#define MTB_PAIR_LOAD(node, q0, q1, q2, kx, ky)                                                                               \
-  float4 q0, q1, q2;                                                                                                          \
-  int kx, ky;                                                                                                                 \
-  {                                                                                                                           \
-    const Bvh2Node *np__ = sc.gnodes + (node >= 0 ? node : 0);                                                                \
-    float w8__, w9__, w10__, w11__;                                                                                           \
-    asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"                                                       \
-                 : "=f"(q0.x), "=f"(q0.y), "=f"(q0.z), "=f"(q0.w), "=f"(q1.x), "=f"(q1.y), "=f"(q1.z), "=f"(q1.w)             \
-                 : "l"(np__));                                                                                                \
-    asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"                                                       \
-                 : "=f"(q2.x), "=f"(q2.y), "=f"(q2.z), "=f"(q2.w), "=f"(w8__), "=f"(w9__), "=f"(w10__), "=f"(w11__)           \
-                 : "l"(reinterpret_cast<const char *>(np__) + 32));                                                           \
-    kx = __float_as_int(w8__);                                                                                                \
-    ky = __float_as_int(w9__);                                                                                                \
-  }
-  for (;;) {
-    while (node_a >= 0 || node_b >= 0) {
-      // both loads leave before either result is needed
-      MTB_PAIR_LOAD(node_a, a0, a1, a2, akx, aky);
-      MTB_PAIR_LOAD(node_b, b0, b1, b2, bkx, bky);
-      if (node_a >= 0) MTB_PAIR_STEP(node_a, a0, a1, a2, akx, aky, ra, prune_a, stack_a, sp_a);
-      if (node_b >= 0) MTB_PAIR_STEP(node_b, b0, b1, b2, bkx, bky, rb, prune_b, stack_b, sp_b);
-    }
-    if (node_a == kFastExit && node_b == kFastExit) break;
-    // leaves: one instance of the exact tests serves both walks (k selects the scratch column and the state)
-#pragma unroll 1
-    for (int k = 0; k < 2; k++) {
-      const int lf = k == 0 ? node_a : node_b;
-      if (lf == kFastExit) continue;
-      FastCtx fck = fca;
-      if (k) fck.ray_base = fcb.ray_base;
-      int slot = k == 0 ? slot_a : slot_b;
-      float prune = k == 0 ? prune_a : prune_b;
-      Ray rr;
-      rr.o = FmLoad3(fck, nullptr, kFmO);
-      rr.inv = FmLoad3(fck, nullptr, kFmInv);
-      rr.sx = rr.inv.x < 0.0;
-      rr.sy = rr.inv.y < 0.0;
-      rr.sz = rr.inv.z < 0.0;
-      const unsigned leaf = ~(unsigned)lf;
-      FastMem *mk = k == 0 ? &mem_a : &mem_b;
-      MTB_FAST_BARRIER(mk);
-      for (unsigned s = leaf >> 3, e = s + (leaf & 7u); s < e; s++) TestSlotFast<DBG>(sc.gslots + s, rr, fck, mk, &slot, &prune, cnt);
-      MTB_FAST_BARRIER(mk);
-      int node = kFastExit;
-      if (k == 0) {
-        slot_a = slot, prune_a = prune;
-        while (sp_a > 0) {
-          const unsigned long long top = stack_a[--sp_a];
-          if (__uint_as_float((unsigned)(top >> 32)) <= prune) {
-            node = (int)(unsigned)top;
-            break;
-          }
-        }
-        node_a = node;
-      } else {
-        slot_b = slot, prune_b = prune;
-        while (sp_b > 0) {
-          const unsigned long long top = stack_b[--sp_b];
-          if (__uint_as_float((unsigned)(top >> 32)) <= prune) {
-            node = (int)(unsigned)top;
-            break;
-          }
-        }
-        node_b = node;
-      }
-    }
-  }
-#undef MTB_PAIR_STEP
-#undef MTB_PAIR_LOAD
-  asm volatile("" ::: "memory");
-  // certification and fallback, per ray, as in TraceFast / Trace
-#pragma unroll 1
-  for (int k = 0; k < 2; k++) {
-    PairQuery *q = k == 0 ? qa : qb;
-    if (!q->active) continue;
-    const FastCtx &fck = k == 0 ? fca : fcb;
-    const int slot = k == 0 ? slot_a : slot_b;
-    bool exact = !q->fast;
-    const FastMem *mk = k == 0 ? &mem_a : &mem_b;
-    if (q->fast && slot >= 0) {
-      const double t = FmLoad(fck, mk, kFmT);
-      exact = FmLoad(fck, mk, kFmLo2) <= t + FmLoad(fck, mk, kFmE) || DegeneratePassage(sc, slot, fck, mk);
-      q->t = t;
-    }
-    if (!exact) {
-      Count<DBG>(cnt, kFast);
-      q->slot = slot;
-    } else {
-      if (q->fast) Count<DBG>(cnt, kFallback);
-      q->slot = TraceExactCold<DBG>(sc, FmLoad3(fck, nullptr, kFmO), FmLoad3(fck, nullptr, kFmD), &q->t, cnt);
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------
-// A CHAIN of rays per lane.  A warp's Trace iteration lasts as long as the longest walk of its 32 lanes (mean 34 node
-// visits, per-warp maximum ~80: hence 14 of 32 lanes active).  When a lane has several independent queries at hand -
-// the first shadow segments of one hit towards all lights - it can walk them back to back INSIDE one node loop, so
-// that the warp waits for max(len0 + len1) over its lanes instead of max(len0) + max(len1).  Each ray is answered
-// exactly as Trace() answers it (same candidates, exact tests, certification, fallback to the exact recursion).
-// ---------------------------------------------------------------------------------------------------
-struct ChainRay {
-  double o[3], d[3];
-  double t_limit;  // in
-  double t;        // out
-  int slot;        // out: canonical slot, -1: none
-  int pad_;
-};
-
-template <bool DBG>
-__device__ __forceinline__ void TraceChain(const DeviceScene &sc, ChainRay *rays, int n, unsigned long long *cnt, const FastCtx &fc) {
-  constexpr int kNeedsExact = -2;
-  FastMem mem;
-  FastRay fr_store;
-  const FastRay *r_mem = &fr_store;
-  asm volatile("" : "+l"(r_mem) : : "memory");
-  unsigned long long stack[kFastLocalStack];
-  int sp = 0, slot = -1, node = kFastExit, k = -1;
-  float prune = 0.f;
-  for (;;) {
-    if (node == kFastExit) {
-      if (k >= 0) {  // ray k is finished: certify it (TraceFast's epilogue)
-        bool amb = false;
-        if (slot >= 0) {
-          MTB_FAST_BARRIER(&mem);
-          const double t = FmLoad(fc, &mem, kFmT);
-          amb = FmLoad(fc, &mem, kFmLo2) <= t + FmLoad(fc, &mem, kFmE) || DegeneratePassage(sc, slot, fc, &mem);
-          rays[k].t = t;
-        }
-        rays[k].slot = amb ? kNeedsExact : slot;
-        Count<DBG>(cnt, amb ? kFallback : kFast);
-      }
-      bool fast = false;
-      while (!fast && ++k < n) {  // next ray of the chain that the fast traversal can answer
-        Count<DBG>(cnt, kRays);
-        fast = FastSetup(sc, Load3(rays[k].o), Load3(rays[k].d), rays[k].t_limit, fc, &mem, &fr_store, &prune);
-        if (!fast) rays[k].slot = kNeedsExact;
-      }
-      if (!fast) break;
-      sp = 0;
-      slot = -1;
-      node = 0;
-      MTB_FAST_BARRIER(&mem);
-    }
-    const FastRay r = *r_mem;
-    while (node >= 0) {
-      float4 q0, q1, q2;
-      int2 kids;
-      {
-        const Bvh2Node *np_ = sc.gnodes + node;
-        float w8, w9, w10, w11;
-        asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=f"(q0.x), "=f"(q0.y), "=f"(q0.z), "=f"(q0.w), "=f"(q1.x), "=f"(q1.y), "=f"(q1.z), "=f"(q1.w)
-                     : "l"(np_));
-        asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=f"(q2.x), "=f"(q2.y), "=f"(q2.z), "=f"(q2.w), "=f"(w8), "=f"(w9), "=f"(w10), "=f"(w11)
-                     : "l"(reinterpret_cast<const char *>(np_) + 32));
-        kids.x = __float_as_int(w8);
-        kids.y = __float_as_int(w9);
-      }
-      Count<DBG>(cnt, kBvh, 2);
-      float tl, tr;
-      const bool hl = FastBox(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, r, prune, &tl);
-      const bool hr = FastBox(q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, r, prune, &tr);
-      if (hl && hr) {
-        const bool right_first = tr < tl;
-        stack[sp++] = ((unsigned long long)__float_as_uint(right_first ? tl : tr) << 32) | (unsigned)(right_first ? kids.x : kids.y);
-        node = right_first ? kids.y : kids.x;
-      } else if (hl) {
-        node = kids.x;
-      } else if (hr) {
-        node = kids.y;
-      } else {
-        node = kFastExit;
-        while (sp > 0) {
-          const unsigned long long top = stack[--sp];
-          if (__uint_as_float((unsigned)(top >> 32)) <= prune) {
-            node = (int)(unsigned)top;
-            break;
-          }
-        }
-      }
-    }
-    if (node == kFastExit) continue;
-    {
-      MTB_FAST_BARRIER(&mem);
-      Ray rr;
-      rr.o = FmLoad3(fc, &mem, kFmO);
-      rr.inv = FmLoad3(fc, &mem, kFmInv);
-      rr.sx = rr.inv.x < 0.0;
-      rr.sy = rr.inv.y < 0.0;
-      rr.sz = rr.inv.z < 0.0;
-      const unsigned leaf = ~(unsigned)node;
-      for (unsigned s = leaf >> 3, e = s + (leaf & 7u); s < e; s++) TestSlotFast<DBG>(sc.gslots + s, rr, fc, &mem, &slot, &prune, cnt);
-      MTB_FAST_BARRIER(&mem);
-    }
-    node = kFastExit;
-    while (sp > 0) {
-      const unsigned long long top = stack[--sp];
-      if (__uint_as_float((unsigned)(top >> 32)) <= prune) {
-        node = (int)(unsigned)top;
-        break;
-      }
-    }
-  }
-  // rays the fast traversal did not answer or could not certify: the exact recursion, one by one
-#pragma unroll 1
-  for (int i = 0; i < n; i++) {
-    if (rays[i].slot == kNeedsExact) rays[i].slot = TraceExactCold<DBG>(sc, Load3(rays[i].o), Load3(rays[i].d), &rays[i].t, cnt);
-  }
-}
-#endif
 
 // ---------------------------------------------------------------------------------------------------
 // shading helpers

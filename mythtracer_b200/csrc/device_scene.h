@@ -143,6 +143,6 @@ void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_block
 // must be NULL.  k = 1: the batches above.
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
                            int samples_per_axis, const AccumParams &acc, bool debug_build, cudaStream_t stream);
-void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, int mode, cudaStream_t stream);  // mode 0: one ray per thread, 1: two rays per lane (Trace2), 2: chain (TraceChain), 3: two calls
+void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, cudaStream_t stream);  // one ray per thread
 
 }  // namespace mtb

@@ -59,13 +59,10 @@ __device__ __forceinline__ void St3(double *p, const D3 &v) {
 // Retired launch forms of round 1, all bit-identical and all measured slower on B200 (DESIGN.md section 5):
 // persistent lane refill, block-level ray packing, forced warp re-convergence, suspendable walks.
 // ---------------------------------------------------------------------------------------------------
-#ifndef MTB_BLOCK_EPILOGUE
-#define MTB_BLOCK_EPILOGUE 0
-#endif
 #ifndef MTB_MEGA_MIN_BLOCKS
 // Blocks per SM = registers per thread.  The frame time falls with every warp in flight as long as the node loop of
 // TraceFast stays free of spill code (B200, C3, ms): 10 blocks (96 registers) 10.50, 12 (80) 9.66, 14 (72) 9.07 - and,
-// once the FP32 ray's live range was split by hand (MTB_RAY_RELOAD, device_core.cuh) and the small per-pixel integers
+// once the FP32 ray's live range was split by hand (TraceFast, device_core.cuh) and the small per-pixel integers
 // moved into PixelState, so that 64 registers no longer put reloads into the node loop - 16 (64) 8.88, 18 (56) 9.00,
 // 20 (48) 9.14.
 #define MTB_MEGA_MIN_BLOCKS 16
@@ -561,12 +558,8 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
   // ---- the warp's half of the tile (4 rows of 24 bytes) leaves as aligned 8-byte stores when the layout allows it.
   // Warp-level on purpose: with a block-wide barrier here the warp that finishes first kept its slot on the SM until
   // the other one was done (ncu: 9 % of all warp samples sat in that barrier); now it exits and a warp of the next
-  // tile takes its registers. ----
-#if MTB_BLOCK_EPILOGUE
-  __syncthreads();  // (A/B of the warp-level epilogue)
-#else
+  // tile takes its registers (DESIGN.md section 5, the warp-level epilogue row). ----
   __syncwarp();
-#endif
   if constexpr (ACC) {
     AccumulateEpilogue<SS>(rp, acc, s_rgb, tile_id, strip, s_ss8);
   } else if constexpr (SS > 1) {
@@ -642,116 +635,6 @@ __global__ void __launch_bounds__(128) IntersectKernel(DeviceScene sc, Intersect
         ip.point[i * 3 + 0] = p.x;
         ip.point[i * 3 + 1] = p.y;
         ip.point[i * 3 + 2] = p.z;
-      }
-    }
-  }
-  if (DBG && ip.counters != nullptr) {
-    for (int k = 0; k < kNumCounters; k++) {
-      unsigned long long v = cnt[k];
-      for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
-      if ((threadIdx.x & 31u) == 0u && v != 0ull) atomicAdd(ip.counters + k, v);
-    }
-  }
-}
-
-// The same query, two rays per thread (rays 2i and 2i + 1): Trace2, device_core.cuh.
-template <bool DBG>
-__global__ void __launch_bounds__(64) IntersectPairKernel(DeviceScene sc, IntersectParams ip) {
-  MTB_DECLARE_FAST_CTX2(64);
-  const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 2;
-  unsigned long long cnt_store[DBG ? kNumCounters : 1];
-  unsigned long long *cnt = cnt_store;
-  if (DBG) {
-    for (int k = 0; k < kNumCounters; k++) cnt[k] = 0;
-  }
-  if (i < ip.n) {
-    PairQuery qa, qb;
-    qa.active = true;
-    qb.active = i + 1 < ip.n;
-    qa.t_limit = qb.t_limit = CUDART_INF;
-    const int64_t j = qb.active ? i + 1 : i;
-    Trace2<DBG>(sc, Load3(ip.origins + i * 3), Load3(ip.dirs + i * 3), Load3(ip.origins + j * 3), Load3(ip.dirs + j * 3), &qa, &qb, cnt, fctx, fctx_b);
-#pragma unroll 1
-    for (int k = 0; k < 2; k++) {
-      const PairQuery &q = k == 0 ? qa : qb;
-      if (!q.active) continue;
-      const int64_t r = i + k;
-      if (q.slot < 0) {
-        ip.tri_index[r] = -1;
-        if (ip.t != nullptr) ip.t[r] = CUDART_NAN;
-        if (ip.point != nullptr) ip.point[r * 3 + 0] = ip.point[r * 3 + 1] = ip.point[r * 3 + 2] = CUDART_NAN;
-      } else {
-        ip.tri_index[r] = sc.slots[q.slot].tri;
-        if (ip.t != nullptr) ip.t[r] = q.t;
-        if (ip.point != nullptr) {
-          const D3 p = Add(Load3(ip.origins + r * 3), MulS(Load3(ip.dirs + r * 3), q.t));
-          ip.point[r * 3 + 0] = p.x;
-          ip.point[r * 3 + 1] = p.y;
-          ip.point[r * 3 + 2] = p.z;
-        }
-      }
-    }
-  }
-  if (DBG && ip.counters != nullptr) {
-    for (int k = 0; k < kNumCounters; k++) {
-      unsigned long long v = cnt[k];
-      for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
-      if ((threadIdx.x & 31u) == 0u && v != 0ull) atomicAdd(ip.counters + k, v);
-    }
-  }
-}
-
-// Rays 2i and 2i + 1 by one thread: CHAINED = back to back inside one node loop (TraceChain), else by two ordinary
-// Trace calls (the warp reconverges in between) - the A/B of chaining, same threads, same rays.
-template <bool DBG, bool CHAINED>
-__global__ void __launch_bounds__(64) IntersectChainKernel(DeviceScene sc, IntersectParams ip) {
-  MTB_DECLARE_FAST_CTX(64);
-  const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 2;
-  unsigned long long cnt_store[DBG ? kNumCounters : 1];
-  unsigned long long *cnt = cnt_store;
-  if (DBG) {
-    for (int k = 0; k < kNumCounters; k++) cnt[k] = 0;
-  }
-  if (i < ip.n) {
-    ChainRay rays[2];
-    const int n = i + 1 < ip.n ? 2 : 1;
-    for (int k = 0; k < n; k++) {
-      for (int a = 0; a < 3; a++) {
-        rays[k].o[a] = ip.origins[(i + k) * 3 + a];
-        rays[k].d[a] = ip.dirs[(i + k) * 3 + a];
-      }
-      rays[k].t_limit = CUDART_INF;
-      rays[k].slot = -1;
-      rays[k].t = 0.0;
-    }
-    if (CHAINED) {
-      ChainRay *rp = rays;
-      asm volatile("" : "+l"(rp) : : "memory");
-      TraceChain<DBG>(sc, rp, n, cnt, fctx);
-      asm volatile("" : : "l"(rp) : "memory");
-    } else {
-#pragma unroll 1
-      for (int k = 0; k < n; k++) {
-        rays[k].slot = Trace<DBG>(sc, Load3(rays[k].o), Load3(rays[k].d), CUDART_INF, &rays[k].t, cnt, fctx);
-        __syncwarp();
-      }
-    }
-#pragma unroll 1
-    for (int k = 0; k < n; k++) {
-      const int64_t r = i + k;
-      if (rays[k].slot < 0) {
-        ip.tri_index[r] = -1;
-        if (ip.t != nullptr) ip.t[r] = CUDART_NAN;
-        if (ip.point != nullptr) ip.point[r * 3 + 0] = ip.point[r * 3 + 1] = ip.point[r * 3 + 2] = CUDART_NAN;
-      } else {
-        ip.tri_index[r] = sc.slots[rays[k].slot].tri;
-        if (ip.t != nullptr) ip.t[r] = rays[k].t;
-        if (ip.point != nullptr) {
-          const D3 p = Add(Load3(rays[k].o), MulS(Load3(rays[k].d), rays[k].t));
-          ip.point[r * 3 + 0] = p.x;
-          ip.point[r * 3 + 1] = p.y;
-          ip.point[r * 3 + 2] = p.z;
-        }
       }
     }
   }
@@ -866,27 +749,8 @@ void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const 
   }
 }
 
-void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, int mode, cudaStream_t stream) {
+void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, cudaStream_t stream) {
   if (ip.n <= 0) return;
-  const int pair_blocks = (int)(((ip.n + 1) / 2 + 63) / 64);
-  if (mode == 1) {
-    if (debug_build) {
-      IntersectPairKernel<true><<<pair_blocks, 64, 0, stream>>>(sc, ip);
-    } else {
-      IntersectPairKernel<false><<<pair_blocks, 64, 0, stream>>>(sc, ip);
-    }
-    return;
-  }
-  if (mode >= 2) {
-    if (debug_build) {
-      if (mode == 2) IntersectChainKernel<true, true><<<pair_blocks, 64, 0, stream>>>(sc, ip);
-      else IntersectChainKernel<true, false><<<pair_blocks, 64, 0, stream>>>(sc, ip);
-    } else {
-      if (mode == 2) IntersectChainKernel<false, true><<<pair_blocks, 64, 0, stream>>>(sc, ip);
-      else IntersectChainKernel<false, false><<<pair_blocks, 64, 0, stream>>>(sc, ip);
-    }
-    return;
-  }
   const int blocks = (int)((ip.n + 127) / 128);
   if (debug_build) {
     IntersectKernel<true><<<blocks, 128, 0, stream>>>(sc, ip);

@@ -696,9 +696,10 @@ def test_sibling_entry_tie_on_the_device(product_lib, oracle_mod):
         mt.close()
 
 
-def test_two_rays_per_lane_gives_the_same_answers(product_lib, oracle_mod, scene_dir):
-    """MTB_FLAG_PAIR_RAYS (Trace2: one thread walks rays 2i and 2i+1 in one loop) and MTB_FLAG_CHAIN_RAYS against the oracle: random rays,
-    axis-parallel ones (literal path), rays from outside, and an odd count (the last thread has one ray)."""
+def test_retired_pair_and_chain_flags_change_nothing(product_lib, oracle_mod, scene_dir):
+    """MTB_FLAG_PAIR_RAYS and MTB_FLAG_CHAIN_RAYS (retired two-rays-per-thread forms of mtb_intersect_rays) are accepted and
+    ignored: the answers match the oracle and, with the integer stats, the same call without the two bits.  Random rays,
+    axis-parallel ones (literal path), rays from outside, and an odd count."""
     from mythtracer_b200 import MTB_FLAG_CHAIN_RAYS, MTB_FLAG_COUNT_WORK, MTB_FLAG_PAIR_RAYS
     files, cfg = scenes.config_scene("C2", scene_dir, scale=0.2)
     mt, orc = _load_pair(product_lib, oracle_mod, files, 3)
@@ -709,7 +710,10 @@ def test_two_rays_per_lane_gives_the_same_answers(product_lib, oracle_mod, scene
     cpu = orc.intersect(o, d)
     hit = cpu["tri"] >= 0
     assert hit.sum() > 5000
-    # (MTB_FLAG_CHAIN_RAYS: the two rays of a thread back to back inside one node loop, TraceChain; both flags: by two calls)
+    plain = {}
+    for flags in (0, MTB_FLAG_COUNT_WORK):
+        mt.set_flags(flags)
+        plain[flags] = mt.intersect_rays(o, d, want_stats=True)
     for flags in (MTB_FLAG_PAIR_RAYS, MTB_FLAG_PAIR_RAYS | MTB_FLAG_COUNT_WORK, MTB_FLAG_CHAIN_RAYS, MTB_FLAG_CHAIN_RAYS | MTB_FLAG_COUNT_WORK,
                   MTB_FLAG_CHAIN_RAYS | MTB_FLAG_PAIR_RAYS):
         mt.set_flags(flags)
@@ -720,3 +724,7 @@ def test_two_rays_per_lane_gives_the_same_answers(product_lib, oracle_mod, scene
         assert np.isnan(gpu["t"][~hit]).all()
         if flags & MTB_FLAG_COUNT_WORK:
             assert gpu["stats"]["rays"] == len(o) and gpu["stats"]["n_literal"] >= 1000
+        ref = plain[flags & MTB_FLAG_COUNT_WORK]
+        for k in ("tri", "t", "point"):
+            assert np.array_equal(gpu[k], ref[k], equal_nan=True), (flags, k)
+        assert {k: v for k, v in gpu["stats"].items() if isinstance(v, int)} == {k: v for k, v in ref["stats"].items() if isinstance(v, int)}, flags

@@ -10,7 +10,7 @@ out = []
 for name in names:
     files, cfg = scenegen.generate_config(name, "/tmp/mtb_scenes")
     for mode in modes:
-        base_flags = {"bvh": 16, "nobvh": MTB_FLAG_NO_LIST_BVH | 16, "auto": 0, "noorder": 16 | 32, "persist": 16 | 64, "exact": 16 | 128, "pack": 16 | 256, "sync": 16 | 512, "resume": 16 | 1024, "devbvh": 16 | 4096, "queue": 8192}.get(mode, 0)
+        base_flags = {"bvh": 16, "nobvh": MTB_FLAG_NO_LIST_BVH | 16, "auto": 0, "noorder": 16 | 32, "exact": 16 | 128, "devbvh": 16 | 4096, "queue": 8192}.get(mode, 0)
         mt = MythTracer(max_depth=cfg["depth"], flags=base_flags)
         t0 = time.time(); assert mt.LoadObj(files.obj_path); t_load = time.time() - t0
         mt.GetScene().lights = [Light.from_tuple(l) for l in files.lights]

@@ -1,102 +1,107 @@
-"""Compares the SASS of the megakernel of two source trees, ignoring symbol names.
+"""Compares the SASS of every kernel of the megakernel and wavefront sources of two source trees.
 
     python tools/sass_compare.py OLD_TREE [NEW_TREE]      (NEW_TREE defaults to this repository)
 
-Compiles csrc/megakernel.cu of both trees for sm_100a with the library's flags (no GPU needed), dumps the SASS with
-cuobjdump and compares the instruction listings of RenderMega<DBG, BATCH> (RenderMega<DBG, BATCH, 1> in a tree with
-the supersampled batch, RenderMega<DBG, BATCH, 1, false> in a tree with the accumulated batch) for DBG and BATCH = false
-and true, and those of the supersampled batch, RenderMega<DBG, true, SS> (SS = 2, 4, 8), wherever the old tree has it.
-A tree from before the batch form only has the single-view kernel, RenderMega<DBG>, which is then compared with
-BATCH = false alone.  Also prints ptxas' registers / stack / spill figures of every RenderMega instantiation, the
-supersampled (SS = 2, 4, 8) and accumulating (ACC = true) ones included.  Exit status 0 when the listings are
-identical.
+Compiles csrc/megakernel.cu and csrc/wavefront.cu of both trees for sm_100a with the library's flags (no GPU needed),
+dumps the SASS with cuobjdump and compares the instruction listings of every kernel by name.  Kernels are matched by
+their demangled names: a mangled name contains a per-file hash of the anonymous namespace, which changes whenever the
+file's content does.  Prints ptxas' registers / stack / spill figures of every kernel in both trees.  A kernel that
+only the old tree has is listed as removed, one that only the new tree has as added; neither is a difference.  Exit
+status 0 when every kernel of both trees has the same instruction listing and the same ptxas figures.
 """
 import os
 import re
+import shutil
 import subprocess
 import sys
 import tempfile
+from concurrent.futures import ThreadPoolExecutor
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from mythtracer_b200.build import NVCC_FLAGS  # noqa: E402
 
+SOURCES = ("megakernel.cu", "wavefront.cu")
+NVCC = os.environ.get("NVCC", "nvcc")
 
-def _compile(tree, out_dir):
-    cubin = os.path.join(out_dir, "mega.cubin")
-    nvcc = os.environ.get("NVCC", "nvcc")
-    res = subprocess.run([nvcc] + NVCC_FLAGS + ["-Xptxas", "-v", "-I", os.path.join(tree, "include"), "-I",
-                                                os.path.join(tree, "mythtracer_b200", "csrc"), "-cubin", "-o", cubin,
-                                                os.path.join(tree, "mythtracer_b200", "csrc", "megakernel.cu")],
+
+def _compile(tree, src, out_dir):
+    """(ptxas log, SASS listing) of csrc/<src> of `tree`, or None when the tree has no such file."""
+    path = os.path.join(tree, "mythtracer_b200", "csrc", src)
+    if not os.path.exists(path):
+        return None
+    cubin = os.path.join(out_dir, src + ".cubin")
+    res = subprocess.run([NVCC] + NVCC_FLAGS + ["-Xptxas", "-v", "-I", os.path.join(tree, "include"), "-I",
+                                                os.path.dirname(path), "-cubin", "-o", cubin, path],
                          capture_output=True, text=True, check=True)
     sass = subprocess.run(["cuobjdump", "-sass", cubin], capture_output=True, text=True, check=True).stdout
     return res.stderr, sass
 
 
-def _ptxas_figures(log):
-    out = {}
-    for m in re.finditer(r"Function properties for (\S*RenderMega\S*)\n\s*(\d+) bytes stack frame, (\d+) bytes spill stores, "
-                         r"(\d+) bytes spill loads\n.*?Used (\d+) registers", log):
-        out[m.group(1)] = dict(stack=int(m.group(2)), spill_stores=int(m.group(3)), spill_loads=int(m.group(4)), registers=int(m.group(5)))
-    return out
+def _demangle(names):
+    filt = os.path.join(os.path.dirname(shutil.which(NVCC) or NVCC), "cu++filt")
+    out = subprocess.run([filt if os.path.exists(filt) else "cu++filt"] + names, capture_output=True, text=True,
+                         check=True).stdout.splitlines()
+    return dict(zip(names, out))
 
 
-def _functions(sass):
-    """{mangled name: [instruction text]} without addresses and encodings."""
-    funcs = {}
+def _short(demangled):
+    """RenderMega<false, true, 8, false> for void mtb::<unnamed>::RenderMega<(bool)0, (bool)1, (int)8, (bool)0>(...)."""
+    name = re.sub(r"\(bool\)([01])", lambda m: "true" if m.group(1) == "1" else "false", demangled).replace("(int)", "")
+    return re.sub(r"^void |\(.*$", "", name).replace("mtb::<unnamed>::", "")
+
+
+def _kernels(log, sass):
+    """{demangled name: (ptxas figures, [instruction text])}: listings without addresses and encodings."""
+    figures = {}
+    for m in re.finditer(r"Compiling entry function '(\S+)'.*?\n.*?Function properties for \1\n\s*(\d+) bytes stack frame, "
+                         r"(\d+) bytes spill stores, (\d+) bytes spill loads\n.*?Used (\d+) registers", log):
+        figures[m.group(1)] = "%s registers, %s B stack, %s / %s B spill stores / loads" % (m.group(5), m.group(2), m.group(3),
+                                                                                            m.group(4))
+    code = {}
     for block in sass.split("Function : ")[1:]:
         name, body = block.split("\n", 1)
-        funcs[name.strip()] = [m.group(1).strip() for m in re.finditer(r"/\*[0-9a-f]{4,}\*/\s*(.*?)\s*;", body)]
-    return funcs
-
-
-def _instantiation(funcs, dbg, batch, ss=1):
-    """(name, code) of RenderMega<dbg, batch, ss> (<dbg, batch> for ss = 1 without the SS parameter, <..., false> with
-    the ACC parameter; <dbg> stands for <dbg, false>), or None."""
-    if ss == 1:
-        patterns = [r"RenderMegaILb%dELb%dE(Li1E(Lb0E)?)?EEv" % (dbg, batch)] + ([r"RenderMegaILb%dEEEv" % dbg] if not batch else [])
-    else:
-        patterns = [r"RenderMegaILb%dELb%dELi%dE(Lb0E)?EEv" % (dbg, batch, ss)]
-    for name, code in funcs.items():
-        if any(re.search(p, name) for p in patterns):
-            return name, code
-    return None
+        code[name.strip()] = [m.group(1).strip() for m in re.finditer(r"/\*[0-9a-f]{4,}\*/\s*(.*?)\s*;", body)]
+    missing = sorted(set(code) - set(figures))
+    if missing:
+        raise SystemExit("no ptxas figures for the kernel(s) %s" % ", ".join(missing))
+    names = _demangle(sorted(code))
+    return {names[n]: (figures[n], c) for n, c in code.items()}
 
 
 def main():
     if len(sys.argv) < 2:
         raise SystemExit(__doc__)
     old_tree, new_tree = sys.argv[1], sys.argv[2] if len(sys.argv) > 2 else ROOT
+    jobs = [(tree, src) for src in SOURCES for tree in (old_tree, new_tree)]
+    with tempfile.TemporaryDirectory() as tmp, ThreadPoolExecutor(len(jobs)) as pool:
+        dirs = [os.path.join(tmp, str(i)) for i in range(len(jobs))]
+        for d in dirs:
+            os.makedirs(d)
+        results = list(pool.map(lambda job, d: _compile(job[0], job[1], d), jobs, dirs))
     same = True
-    with tempfile.TemporaryDirectory() as tmp:
-        os.makedirs(os.path.join(tmp, "old"))
-        os.makedirs(os.path.join(tmp, "new"))
-        old_log, old_sass = _compile(old_tree, os.path.join(tmp, "old"))
-        new_log, new_sass = _compile(new_tree, os.path.join(tmp, "new"))
-    for label, log in (("old", old_log), ("new", new_log)):
-        for name, fig in _ptxas_figures(log).items():
-            print("%s %s %s" % (label, re.search(r"RenderMega\w*?E(?=EvN)", name).group(0), fig))
-    old_f, new_f = _functions(old_sass), _functions(new_sass)
-    for batch, ss in ((0, 1), (1, 1), (1, 2), (1, 4), (1, 8)):
-        for dbg in (0, 1):
-            old, new = _instantiation(old_f, dbg, batch, ss), _instantiation(new_f, dbg, batch, ss)
-            if new is None:
-                raise SystemExit("no RenderMega<%d, %d, %d> in the listing of %s" % (dbg, batch, ss, new_tree))
-            if old is None:
-                if not batch:
-                    raise SystemExit("no single-view RenderMega<%d> in the listing of %s" % (dbg, old_tree))
-                print("RenderMega<DBG=%d, BATCH=1, SS=%d>: not in %s" % (dbg, ss, old_tree))
+    for k, src in enumerate(SOURCES):
+        old_res, new_res = results[2 * k], results[2 * k + 1]
+        if new_res is None:
+            raise SystemExit("no %s in %s" % (src, new_tree))
+        old, new = _kernels(*old_res) if old_res else {}, _kernels(*new_res)
+        print("%s:" % src)
+        for name in sorted(set(old) | set(new), key=_short):
+            if name not in new:
+                print("  %s: removed (old: %s)" % (_short(name), old[name][0]))
                 continue
-            (on, oc), (nn, nc) = old, new
-            equal = oc == nc
+            if name not in old:
+                print("  %s: added (new: %s)" % (_short(name), new[name][0]))
+                continue
+            (of, oc), (nf, nc) = old[name], new[name]
+            equal = oc == nc and of == nf
             same &= equal
-            print("RenderMega<DBG=%d, BATCH=%d, SS=%d>: %d vs %d instructions, %s" % (dbg, batch, ss, len(oc), len(nc),
-                                                                                    "identical" if equal else "DIFFERENT"))
-            if not equal:
-                for i, (a, b) in enumerate(zip(oc, nc)):
-                    if a != b:
-                        print("  first difference at instruction %d: %s | %s" % (i, a, b))
-                        break
+            print("  %s: %d vs %d instructions, %s" % (_short(name), len(oc), len(nc), "identical" if equal else "DIFFERENT"))
+            print("    old: %s\n    new: %s" % (of, nf))
+            if oc != nc:
+                i = next((i for i, (a, b) in enumerate(zip(oc, nc)) if a != b), min(len(oc), len(nc)))
+                print("    first difference at instruction %d: %s | %s" % (i, oc[i] if i < len(oc) else "(end)",
+                                                                           nc[i] if i < len(nc) else "(end)"))
     sys.exit(0 if same else 1)
 
 
