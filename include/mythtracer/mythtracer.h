@@ -214,6 +214,19 @@ class MythTracer {
     return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, static_cast<uint8_t *>(d_rgb), nullptr, false,
                        true, stream);
   }
+  // Depth of field (mtb_render_batch_lens): the accumulated batch above with one thin-lens sample (u, v,
+  // focus_distance) per camera.  Camera i's primary rays start at its origin moved by u along the image's right and v
+  // along its down direction, and pass through the points where its pinhole rays meet the focal plane at
+  // focus_distance; k lens points spread over an aperture, averaged as sub-frames, give depth of field.  A centred
+  // sample (0, 0, f) is the pinhole ray.  lenses.size() must equal cams.size().
+  bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
+                     const std::vector<mtb_lens> &lenses, const std::vector<std::vector<Light>> *lights, uint8_t *out) {
+    if (lenses.size() != cams.size()) {
+      fprintf(stderr, "error: %zu lens samples for %zu cameras (one per camera)\n", lenses.size(), cams.size());
+      return false;
+    }
+    return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, out, nullptr, true, false, nullptr, lenses.data());
+  }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
   static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
     return static_cast<uint8_t *>(mtb_host_alloc((size_t)image_width * image_height * 3 * (size_t)n_frames));
@@ -230,7 +243,7 @@ class MythTracer {
  private:
   bool RenderBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
                    const std::vector<std::vector<Light>> *lights, uint8_t *out, mtb_debug *dbg, bool synchronous, bool device = false,
-                   void *stream = nullptr) {
+                   void *stream = nullptr, const mtb_lens *lenses = nullptr) {
     if (!was_scene_finalized) {
       puts("Finalizing tree.");
       if (!scene.tree.Finalize(&scene.materials, &scene.textures)) return false;
@@ -263,13 +276,16 @@ class MythTracer {
     const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
     mtb_stats stats;
     int rc;
-    if (subframes != 1 || device) {
+    if (subframes != 1 || device || lenses != nullptr) {
       if (subframes < 1 || cams.size() % (size_t)subframes != 0) {
         fprintf(stderr, "error: %zu cameras are not a whole number of output views of %d subframes\n", cams.size(), subframes);
         return false;
       }
       const int32_t n_out = (int32_t)(cams.size() / (size_t)subframes);
-      if (device) {
+      if (lenses != nullptr) {
+        rc = mtb_render_batch_lens(ctx, mcams.data(), lenses, n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
+                                   max_recursion_level, out, nullptr, nullptr, &stats);
+      } else if (device) {
         rc = mtb_render_batch_device(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
                                      max_recursion_level, out, nullptr, nullptr, stream, nullptr);
       } else {

@@ -88,6 +88,13 @@ typedef struct {
   uint32_t *n_rays;     /* chunk_w*chunk_h, may be NULL */
 } mtb_taps;
 
+/* Thin-lens sample of one sub-frame of mtb_render_batch_lens: the lens point (u, v) in world units, u along the image's
+ * right and v along its down direction, and the distance of the focal plane from the camera origin along its normal. */
+typedef struct {
+  double u, v;
+  double focus_distance;
+} mtb_lens;
+
 /* Work done by one render / intersect call.  Counters other than `rays..refract` are only filled by the
  * counting build of the kernels (MTB_FLAG_COUNT_WORK), which is slower and never timed. */
 typedef struct {
@@ -332,6 +339,40 @@ int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32
 int mtb_render_batch_device(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
                             int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, void *d_rgb,
                             mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream, mtb_stats *stats);
+
+/* Depth of field: the batch forms with a thin-lens sample per sub-frame.  With S = start_point, Dy = delta_scanline,
+ * Dx = delta_pixel of the sensor of sub-frame u at (s*image_w) x (s*image_h) (mtb_camera_sensor), O its origin and
+ * (u, v, f) = lenses[u], every operation in FP64 and in the order written (Cross, Dot, Normalized of the reference's
+ * math3d.h), once per sub-frame:
+ *     n  = Normalized(Cross(Dy, Dx));  if Dot(n, S) < 0: n = -n          focal-plane normal
+ *     ex = Normalized(Dx)                                                 image right
+ *     ey = Cross(n, ex);               if Dot(ey, Dy) < 0: ey = -ey        image down
+ *     L  = ex * u + ey * v                                                lens point, relative to O
+ * and for sample (X, Y) of its sample grid, with d = Normalized(S + Dy * Y + Dx * X) the pinhole direction:
+ *     u == 0 and v == 0:   origin O,      direction d                     (the pinhole ray)
+ *     otherwise:           t = f / Dot(d, n);  origin O + L,  direction Normalized(d * t - L)
+ * Every ray of a sub-frame passes through the same focal plane, at distance f from O along n: that plane is in focus,
+ * and the mean over sub-frames with lens points spread over an aperture blurs everything in front of it and behind
+ * it.  The sample is the reference's TraceRay of that primary ray at depth max_depth (reflection, refraction, shadows
+ * and quantisation unchanged), and the output bytes are those of mtb_render_batch_accum over these samples (the
+ * rounded mean of the k*s*s quantised samples of an output pixel; k = 1: the sub-frame itself).  The library chooses no
+ * samples: the aperture shape, the sample pattern and the focus are the caller's.
+ *
+ * lenses: one entry per camera (n_out * subframes), HOST memory.  Planes (dbg_out, taps) are those of
+ * mtb_render_batch_debug for the lens rays and only available with subframes == 1.  Every argument rule of
+ * mtb_render_batch_debug / mtb_render_batch_accum applies; in addition each of these is MTB_ERR_ARG, before anything is
+ * queued: lenses == NULL (the pinhole forms are the other entry points); u, v or focus_distance not finite, or
+ * focus_distance <= 0; a sub-frame whose four sample-grid corner directions c do not all satisfy Dot(n, c) > 0 (a
+ * degenerate view, such as aov 0, or an aov of about 180 degrees), which also makes t finite and positive for every
+ * sample.  Synchronous. */
+int mtb_render_batch_lens(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes,
+                          const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                          uint8_t *rgb_out, mtb_debug *dbg_out, const mtb_taps *taps, mtb_stats *stats);
+/* The same into DEVICE memory: the contract of mtb_render_batch_device (pointer and stream checks, stream ordering,
+ * the split over devices) with the lens samples and rules of mtb_render_batch_lens. */
+int mtb_render_batch_lens_device(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes,
+                                 const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                                 void *d_rgb, mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream, mtb_stats *stats);
 
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the

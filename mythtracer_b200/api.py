@@ -80,7 +80,8 @@ EXPORTED_SYMBOLS = [
     "mtb_render_chunk_device", "mtb_render_chunk_async", "mtb_wait", "mtb_host_alloc", "mtb_host_free", "mtb_read_counters", "mtb_launch_count", "mtb_pipeline_in_use", "mtb_intersect_rays", "mtb_camera_sensor", "mtb_version",
     "mtb_frame_create", "mtb_frame_open", "mtb_frame_release", "mtb_frame_read", "mtb_load_timing", "mtb_hybrid_share",
     "mtb_render_batch", "mtb_render_batch_async", "mtb_render_batch_ss", "mtb_render_batch_ss_async", "mtb_render_batch_debug",
-    "mtb_render_batch_accum", "mtb_render_batch_accum_async", "mtb_render_batch_device",
+    "mtb_render_batch_accum", "mtb_render_batch_accum_async", "mtb_render_batch_device", "mtb_render_batch_lens",
+    "mtb_render_batch_lens_device",
 ]
 
 
@@ -140,6 +141,9 @@ def load_library():
     lib.mtb_render_batch_accum.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp]
     lib.mtb_render_batch_accum_async.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp]
     lib.mtb_render_batch_device.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp, vp]
+    lib.mtb_render_batch_lens.argtypes = [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp]
+    lib.mtb_render_batch_lens_device.argtypes = [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp,
+                                                 vp, vp, vp]
     lib.mtb_read_counters.argtypes = [vp, vp]
     lib.mtb_pipeline_in_use.argtypes = [vp, vp, vp]
     lib.mtb_launch_count.argtypes = [vp]
@@ -222,6 +226,24 @@ def _lights_array(lights) -> np.ndarray:
         arr[i]["position"], arr[i]["ambient"] = l.position, l.ambient
         arr[i]["diffuse"], arr[i]["specular"] = l.diffuse, l.specular
     return arr
+
+
+def _lens_array(lenses, n_cams: int) -> np.ndarray:
+    """render_batch's lenses as the (n_cams, 3) float64 array of mtb_lens records (u, v, focus_distance)."""
+    if isinstance(lenses, (str, bytes)):
+        raise MythTracerError("render_batch: lenses must be a sequence of (u, v, focus_distance) or a float64 array (got %r)" % (lenses,))
+    try:
+        arr = np.array(lenses, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise MythTracerError("render_batch: lenses must hold numbers (u, v, focus_distance): %s" % e)
+    if arr.shape != (n_cams, 3):
+        raise MythTracerError("render_batch: lenses must have shape (%d, 3), one (u, v, focus_distance) per camera (got %s)" % (
+            n_cams, arr.shape))
+    if not np.isfinite(arr).all():
+        raise MythTracerError("render_batch: every lens u, v and focus_distance must be finite")
+    if not (arr[:, 2] > 0).all():
+        raise MythTracerError("render_batch: every lens focus_distance must be > 0")
+    return np.ascontiguousarray(arr)
 
 
 @dataclass
@@ -472,7 +494,7 @@ class MythTracer:
         return res
 
     def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None, samples_per_axis: int = 1,
-                     debug: bool = False, taps: bool = False, subframes: int = 1, device: bool = False):
+                     debug: bool = False, taps: bool = False, subframes: int = 1, device: bool = False, lenses=None):
         """mtb_render_batch: len(cameras) whole frames in one launch per device, at depth self.max_depth.
 
         lights: None (every view uses GetScene().lights) or one list of Light per view, all of the same length.
@@ -497,7 +519,15 @@ class MythTracer:
         (n_out, height, width, 3); with debug, `debug` is the raw uint8 (n, s*height, s*width, 32) buffer of mtb_debug
         records and line_no (int32) and points (float64, last axis 3) are views of it; with taps, sig_hits and sig_shadow
         are torch.uint64 and n_rays torch.uint32.  out, if given, is a C-contiguous uint8 CUDA tensor of that shape on
-        that device.  stats is None and last_stats is left alone.  torch is imported only here."""
+        that device.  stats is None and last_stats is left alone.  torch is imported only here.
+
+        lenses: None (pinhole views) or one thin-lens sample (u, v, focus_distance) per camera, as a sequence or a
+        float64 array of shape (len(cameras), 3): depth of field through mtb_render_batch_lens (device=True:
+        mtb_render_batch_lens_device).  Camera u's primary rays start at its origin + u * right + v * down and pass
+        through the points where its pinhole rays meet the plane at focus_distance along the view axis; with subframes
+        k > 1 an output view is the mean of its k sub-frames, so k lens points spread over an aperture give depth of field
+        (include/mythtracer_b200.h has the exact formula).  A centred sample (0, 0, f) is the pinhole ray.  Everything
+        else (samples_per_axis, subframes, lights, debug, taps, device, out) is as without lenses."""
         if not isinstance(device, (bool, np.bool_)):
             raise MythTracerError("render_batch: device must be True or False (got %r)" % (device,))
         device = bool(device)
@@ -520,6 +550,7 @@ class MythTracer:
             raise MythTracerError("render_batch: no cameras")
         if len(cams) % k != 0:
             raise MythTracerError("render_batch: %d cameras are not a whole number of output views of %d subframes" % (len(cams), k))
+        lens_arr = None if lenses is None else _lens_array(lenses, len(cams))
         cam_arr = np.zeros(len(cams), CAMERA_DTYPE)
         for i, c in enumerate(cams):
             cam_arr[i] = c.as_array()
@@ -543,7 +574,7 @@ class MythTracer:
         n_out = len(cams) // k
         shape = (n_out, height, width, 3)
         if device:
-            return self._render_batch_device(cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps)
+            return self._render_batch_device(cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps, lens_arr)
         if out is None:
             rgb = np.zeros(shape, np.uint8)
         else:
@@ -554,23 +585,24 @@ class MythTracer:
             rgb = out
         stats = np.zeros((), STATS_DTYPE)
         res = {}
+        dbg, tap_ptr = None, None
         if debug or taps:
             plane = (len(cams), ss * height, ss * width)
             dbg = np.zeros(plane, DEBUG_DTYPE) if debug else None
-            tap_ptr = None
             if taps:
                 res["sig_hits"] = np.zeros(plane, np.uint64)
                 res["sig_shadow"] = np.zeros(plane, np.uint64)
                 res["n_rays"] = np.zeros(plane, np.uint32)
                 tap_struct = _TapsStruct(res["sig_hits"].ctypes.data, res["sig_shadow"].ctypes.data, res["n_rays"].ctypes.data)
                 tap_ptr = ctypes.cast(ctypes.pointer(tap_struct), ctypes.c_void_p)
+        if lens_arr is not None:
+            self._check(self._lib.mtb_render_batch_lens(self._ctx, _ptr(cam_arr), _ptr(lens_arr), n_out, k, _ptr(light_arr), n_lights, width,
+                                                        height, ss, self.max_depth, _ptr(rgb), _ptr(dbg), tap_ptr, _ptr(stats)),
+                        "mtb_render_batch_lens")
+        elif debug or taps:
             self._check(self._lib.mtb_render_batch_debug(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
                                                          ss, self.max_depth, _ptr(rgb), _ptr(dbg), tap_ptr, _ptr(stats)),
                         "mtb_render_batch_debug")
-            if debug:
-                res["debug"] = dbg
-                res["line_no"] = dbg["line_no"]
-                res["points"] = dbg["point"]
         elif k > 1:
             self._check(self._lib.mtb_render_batch_accum(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height,
                                                          ss, self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch_accum")
@@ -580,12 +612,16 @@ class MythTracer:
         else:
             self._check(self._lib.mtb_render_batch_ss(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
                                                       ss, self.max_depth, _ptr(rgb), _ptr(stats)), "mtb_render_batch_ss")
+        if debug:
+            res["debug"] = dbg
+            res["line_no"] = dbg["line_no"]
+            res["points"] = dbg["point"]
         res["rgb"] = rgb
         res["stats"] = {k: stats[k].item() for k in STATS_DTYPE.names}
         self.last_stats = res["stats"]
         return res
 
-    def _render_batch_device(self, cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps):
+    def _render_batch_device(self, cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps, lens_arr=None):
         """render_batch(..., device=True) once the arguments shared with the host form are checked."""
         try:
             import torch
@@ -598,6 +634,10 @@ class MythTracer:
             raise MythTracerError("render_batch: with device=True, out must be a C-contiguous uint8 torch tensor of shape %s on %s (got %s)" % (
                 shape, where, "%s %s on %s" % (out.dtype, tuple(out.shape), out.device) if isinstance(out, torch.Tensor) else type(out).__name__))
         n_cams = len(cam_arr)
+        if self._device0 is None and lens_arr is not None:  # host-only context: the library refuses the call (no CPU fallback)
+            self._check(self._lib.mtb_render_batch_lens_device(self._ctx, _ptr(cam_arr), _ptr(lens_arr), n_out, k, _ptr(light_arr), n_lights,
+                                                               width, height, ss, self.max_depth, None, None, None, None, None),
+                        "mtb_render_batch_lens_device")
         if self._device0 is None:  # host-only context: the library refuses the call (there is no CPU fallback)
             self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
                                                           self.max_depth, None, None, None, None, None), "mtb_render_batch_device")
@@ -617,10 +657,14 @@ class MythTracer:
             res["n_rays"] = torch.empty(plane, dtype=torch.uint32, device=where)
             tap_struct = _TapsStruct(res["sig_hits"].data_ptr(), res["sig_shadow"].data_ptr(), res["n_rays"].data_ptr())
             tap_ptr = ctypes.cast(ctypes.pointer(tap_struct), ctypes.c_void_p)
-        self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
-                                                      self.max_depth, ctypes.c_void_p(rgb.data_ptr()),
-                                                      None if dbg is None else ctypes.c_void_p(dbg.data_ptr()), tap_ptr, handle, None),
-                    "mtb_render_batch_device")
+        d_rgb, d_dbg = ctypes.c_void_p(rgb.data_ptr()), None if dbg is None else ctypes.c_void_p(dbg.data_ptr())
+        if lens_arr is not None:
+            self._check(self._lib.mtb_render_batch_lens_device(self._ctx, _ptr(cam_arr), _ptr(lens_arr), n_out, k, _ptr(light_arr), n_lights,
+                                                               width, height, ss, self.max_depth, d_rgb, d_dbg, tap_ptr, handle, None),
+                        "mtb_render_batch_lens_device")
+        else:
+            self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
+                                                          self.max_depth, d_rgb, d_dbg, tap_ptr, handle, None), "mtb_render_batch_device")
         res["rgb"] = rgb
         if debug:
             res["debug"] = dbg

@@ -109,6 +109,7 @@ struct DeviceState {
   // tap planes of those views (only when a batch asks for them), and the events that time them (the single-frame
   // events steer the automatic pipeline choice and are left alone)
   DeviceBuffer<mtb::ViewRec> batch_views;
+  DeviceBuffer<mtb::LensRec> batch_lens;  // thin-lens batches: one record per sub-frame of this device
   DeviceBuffer<mtb_light> batch_lights;
   DeviceBuffer<uint8_t> batch_rgb;
   DeviceBuffer<mtb_debug> batch_dbg;
@@ -142,7 +143,7 @@ struct DeviceState {
     nodes.Free(); slots.Free(); shade.Free(); bvh.Free(); gnodes.Free(); gslots.Free(); list_order.Free(); slot_node.Free(); leaf_ref.Free(); ref_slot.Free(); materials.Free();
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
     counters.Free(); tile_cost.Free(); tile_order.Free();
-    batch_views.Free(); batch_lights.Free(); batch_rgb.Free(); batch_dbg.Free(); batch_sig_hits.Free(); batch_sig_shadow.Free(); batch_n_rays.Free();
+    batch_views.Free(); batch_lens.Free(); batch_lights.Free(); batch_rgb.Free(); batch_dbg.Free(); batch_sig_hits.Free(); batch_sig_shadow.Free(); batch_n_rays.Free();
     batch_sum.Free(); batch_arrive.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
     if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
@@ -804,7 +805,64 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 // batch is ordered on user_stream (NULL: device 0's own stream): it starts after the work queued there before the call,
 // and work queued there after the call sees every device's outputs.  Device 0 renders straight into the caller's
 // buffers; every other device renders into its own and copies its slice over with one copy per output.
-constexpr int64_t kMaxSampleSide = 65536;  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
+// lenses (nullable): one thin-lens sample per sub-frame (mtb_render_batch_lens); the kernel makes each sub-frame's
+// primary rays from its LensRec.  NULL: pinhole views, exactly as without the argument.
+constexpr int64_t kMaxSampleSide = 65536;
+
+// Host restatement of the FP64 vector operations of device_core.cuh, in the same evaluation order (the library is built
+// with -ffp-contract=off), for the thin-lens records.
+struct H3 {
+  double x, y, z;
+};
+H3 HAdd(const H3 &a, const H3 &b) { return H3{a.x + b.x, a.y + b.y, a.z + b.z}; }
+H3 HMulS(const H3 &a, double s) { return H3{a.x * s, a.y * s, a.z * s}; }
+H3 HNeg(const H3 &a) { return H3{-a.x, -a.y, -a.z}; }
+double HDot(const H3 &a, const H3 &b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
+H3 HCross(const H3 &t, const H3 &a) { return H3{t.y * a.z - t.z * a.y, t.z * a.x - t.x * a.z, t.x * a.y - t.y * a.x}; }
+H3 HNormalized(const H3 &a) {
+  const double l = std::sqrt(a.x * a.x + a.y * a.y + a.z * a.z);
+  return H3{a.x / l, a.y / l, a.z / l};
+}
+
+// The LensRec of one sub-frame from its lens sample and its sensor (start_point S, delta_scanline Dy, delta_pixel Dx of
+// the grid_w x grid_h sample grid); MTB_ERR_ARG with ctx->err when the sample or the view cannot make thin-lens rays.
+int MakeLensRec(mtb_context *ctx, const mtb_lens &ln, const double sensor[9], int grid_w, int grid_h, int32_t u, mtb::LensRec *out) {
+  const std::string at = "lenses[" + std::to_string(u) + "]";
+  if (!std::isfinite(ln.u) || !std::isfinite(ln.v) || !std::isfinite(ln.focus_distance)) {
+    ctx->err = at + ": u, v and focus_distance must be finite";
+    return MTB_ERR_ARG;
+  }
+  if (!(ln.focus_distance > 0.0)) {
+    ctx->err = at + ": focus_distance must be > 0";
+    return MTB_ERR_ARG;
+  }
+  const H3 S{sensor[0], sensor[1], sensor[2]}, Dy{sensor[3], sensor[4], sensor[5]}, Dx{sensor[6], sensor[7], sensor[8]};
+  H3 n = HNormalized(HCross(Dy, Dx));  // focal-plane normal, facing the sensor
+  if (HDot(n, S) < 0) n = HNeg(n);
+  // every sample direction must point into the half-space in front of the focal plane (t finite and positive): the
+  // directions of a view are a convex bilinear fan, so its four corners decide
+  for (int c = 0; c < 4; c++) {
+    const double X = (c & 1) ? (double)(grid_w - 1) : 0.0, Y = (c & 2) ? (double)(grid_h - 1) : 0.0;
+    const H3 corner = HNormalized(HAdd(HAdd(S, HMulS(Dy, Y)), HMulS(Dx, X)));
+    if (!(HDot(n, corner) > 0)) {
+      ctx->err = at + ": the sub-frame's corner rays do not all face its focal plane (a degenerate view, such as aov 0 or about 180)";
+      return MTB_ERR_ARG;
+    }
+  }
+  const H3 ex = HNormalized(Dx);  // image right
+  H3 ey = HCross(n, ex);          // image down
+  if (HDot(ey, Dy) < 0) ey = HNeg(ey);
+  const H3 L = HAdd(HMulS(ex, ln.u), HMulS(ey, ln.v));
+  out->shift[0] = L.x;
+  out->shift[1] = L.y;
+  out->shift[2] = L.z;
+  out->axis[0] = n.x;
+  out->axis[1] = n.y;
+  out->axis[2] = n.z;
+  out->focus = ln.focus_distance;
+  out->centred = ln.u == 0.0 && ln.v == 0.0 ? 1u : 0u;
+  return MTB_OK;
+}  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
 
 // mtb_render_batch_device: `p` (nullable unless `name` is d_rgb) must be device memory of `device` with `align`-byte alignment.
 int CheckDeviceOutput(mtb_context *ctx, const void *p, const char *name, int device, uintptr_t align) {
@@ -828,7 +886,7 @@ int CheckDeviceOutput(mtb_context *ctx, const void *p, const char *name, int dev
   return MTB_OK;
 }
 
-int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
+int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
                     int image_w, int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps,
                     mtb_stats *stats, bool synchronous, bool device_out = false, cudaStream_t user_stream = nullptr) {
   const auto wall0 = std::chrono::steady_clock::now();
@@ -923,6 +981,11 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
     const mtb_light *src = lights != nullptr ? lights + (size_t)v * nl : ctx->lights.data();
     if (nl > 0) std::copy(src, src + nl, view_lights.begin() + (size_t)v * nl);
   }
+  std::vector<mtb::LensRec> lens_recs(lenses != nullptr ? (size_t)n_views : 0);
+  for (int32_t v = 0; v < n_views && lenses != nullptr; v++) {
+    const int rc = MakeLensRec(ctx, lenses[v], views[(size_t)v].sensor, grid_w, grid_h, v, &lens_recs[(size_t)v]);
+    if (rc != MTB_OK) return rc;
+  }
 
   mtb::RenderParams rp;
   memset(&rp, 0, sizeof(rp));
@@ -971,12 +1034,14 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
     const size_t n_plane = (size_t)count * gpx;
     const size_t n_sum = accum ? (size_t)count_out * npx * 3 : 0, n_arrive = accum ? (size_t)count_out * tiles_per_view * 2 : 0;
     auto grows = [n_plane, direct](const void *host, size_t have) { return !direct && host != nullptr && n_plane > have; };
-    if ((size_t)count > d.batch_views.count || n_lt > d.batch_lights.count || n_rgb > d.batch_rgb.count ||
+    if ((size_t)count > d.batch_views.count || (lenses != nullptr && (size_t)count > d.batch_lens.count) || n_lt > d.batch_lights.count ||
+        n_rgb > d.batch_rgb.count ||
         grows(dbg_host, d.batch_dbg.count) || grows(hits_host, d.batch_sig_hits.count) || grows(shadow_host, d.batch_sig_shadow.count) ||
         grows(rays_host, d.batch_n_rays.count) || n_sum > d.batch_sum.count || n_arrive > d.batch_arrive.count) {
       MTB_CUDA(ctx, cudaStreamSynchronize(s));
     }
     MTB_CUDA(ctx, d.batch_views.Upload(views.data() + first, (size_t)count, s));
+    if (lenses != nullptr) MTB_CUDA(ctx, d.batch_lens.Upload(lens_recs.data() + first, (size_t)count, s));
     MTB_CUDA(ctx, d.batch_lights.Upload(view_lights.data() + (size_t)first * nl, n_lt, s));
     if (n_rgb > 0) MTB_CUDA(ctx, d.batch_rgb.Reserve(n_rgb));
     mtb::DeviceScene sc = d.scene;
@@ -1030,7 +1095,8 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int
     // (after the uploads: they never wait behind the caller's work)
     if (device_out) MTB_CUDA(ctx, cudaStreamWaitEvent(s, ctx->dev[0].ev_batch_caller, 0));
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_start, s));
-    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, acc, debug_build, s);
+    mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, acc, lenses != nullptr ? d.batch_lens.ptr : nullptr,
+                               debug_build, s);
     ctx->launches++;
     MTB_CUDA(ctx, cudaGetLastError());
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_stop, s));
@@ -1432,47 +1498,69 @@ int mtb_render_chunk_async(mtb_context *ctx, const mtb_camera *cam, int image_w,
 
 int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                      int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
+  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                         int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
+  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                               int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_debug(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_debug *dbg_out,
                            const mtb_taps *taps, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
+  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
                          true);
 }
 
 int mtb_render_batch_accum(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
+  return RenderBatchImpl(ctx, cams, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
                          stats, true);
 }
 
 int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
                                  int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
+  return RenderBatchImpl(ctx, cams, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
                          nullptr, false);
 }
 
 int mtb_render_batch_device(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
                             int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, void *d_rgb, mtb_debug *d_dbg,
                             const mtb_taps *d_taps, void *stream, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
+  return RenderBatchImpl(ctx, cams, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
+                         static_cast<uint8_t *>(d_rgb), d_dbg, d_taps, stats, false, true, static_cast<cudaStream_t>(stream));
+}
+
+int mtb_render_batch_lens(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes,
+                          const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                          uint8_t *rgb_out, mtb_debug *dbg_out, const mtb_taps *taps, mtb_stats *stats) {
+  if (ctx != nullptr && lenses == nullptr) {
+    ctx->err = "lenses is NULL (pinhole views: mtb_render_batch_debug / mtb_render_batch_accum)";
+    return MTB_ERR_ARG;
+  }
+  return RenderBatchImpl(ctx, cams, lenses, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out,
+                         dbg_out, taps, stats, true);
+}
+
+int mtb_render_batch_lens_device(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes,
+                                 const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                                 void *d_rgb, mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream, mtb_stats *stats) {
+  if (ctx != nullptr && lenses == nullptr) {
+    ctx->err = "lenses is NULL (pinhole views: mtb_render_batch_device)";
+    return MTB_ERR_ARG;
+  }
+  return RenderBatchImpl(ctx, cams, lenses, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
                          static_cast<uint8_t *>(d_rgb), d_dbg, d_taps, stats, false, true, static_cast<cudaStream_t>(stream));
 }
 

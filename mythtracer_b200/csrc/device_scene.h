@@ -79,6 +79,16 @@ struct AccumParams {
   int32_t subframes;   // k; 1: no accumulation (sum and arrive unused)
 };
 
+// Thin-lens sample of one grid row (sub-frame) of a batch launch, from mtb_lens on the host (RenderBatchImpl).  The
+// primary ray of sample (X, Y), with d the pinhole direction of that sample and O the view's origin, starts at O + shift
+// and points along Normalized(d * (focus / Dot(d, axis)) - shift).  centred != 0 (u = v = 0): the pinhole ray itself.
+struct LensRec {
+  double shift[3];  // L: the lens point relative to O
+  double axis[3];   // n: unit normal of the focal plane, facing the sensor
+  double focus;     // focus_distance along n
+  uint32_t centred;
+};
+
 struct IntersectParams {
   int64_t n;
   const double *origins, *dirs;
@@ -141,8 +151,10 @@ void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_block
 // view u above, and output view v = u / k (W x H, at rp.rgb + v * W * H * 3) is the rounded mean of the k * s * s
 // samples of its sub-frames, summed in acc.sum (zeroed by the caller, with acc.arrive, before the launch).  The planes
 // must be NULL.  k = 1: the batches above.
+// lens (device memory, nullable): one LensRec per grid row (sub-frame); the primary rays of row u are those of lens[u].
+// NULL: pinhole views, the kernels above.
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
-                           int samples_per_axis, const AccumParams &acc, bool debug_build, cudaStream_t stream);
+                           int samples_per_axis, const AccumParams &acc, const LensRec *lens, bool debug_build, cudaStream_t stream);
 void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, cudaStream_t stream);  // one ray per thread
 
 }  // namespace mtb

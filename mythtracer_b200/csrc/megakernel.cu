@@ -246,12 +246,15 @@ __device__ __forceinline__ void AccumulateEpilogue(const RenderParams &rp, const
 // start at v * chunk_w * chunk_h (PlaneIndex).  Without BATCH, `views` is unused and every `BATCH ? :`
 // folds away: the single-view kernels compile to the code they had before the batch form existed.  SS > 1 (BATCH only):
 // the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.  ACC (BATCH only): the
-// accumulated batch, see AccumulateEpilogue; `acc` is unused without it.
-template <bool DBG, bool BATCH, int SS, bool ACC>
+// accumulated batch, see AccumulateEpilogue; `acc` is unused without it.  LENS (BATCH only): thin-lens views, the
+// primary ray of grid row u starts on the lens point of lens[u] and passes through the focal-plane point of the pinhole
+// ray (LensRec); `lens` is unused without it, and only the primary ray differs.
+template <bool DBG, bool BATCH, int SS, bool ACC, bool LENS>
 __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(DeviceScene sc, RenderParams rp, const ViewRec *views,
-                                                                                 AccumParams acc) {
+                                                                                 AccumParams acc, const LensRec *lens) {
   static_assert(SS == 1 || (BATCH && (SS == 2 || SS == 4 || SS == 8)), "supersampling is a batch form with 2, 4 or 8 samples per axis");
   static_assert(!ACC || BATCH, "accumulation is a batch form");
+  static_assert(!LENS || BATCH, "thin-lens views are a batch form");
   MTB_DECLARE_FAST_CTX(kBlockThreads);
   // (SS = 8: 7 more words behind the samples for the epilogue's counter and partial sums)
   __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3 + (SS == 8 ? 7 * 4 : 0)];
@@ -294,8 +297,24 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
     {  // Sensor::GetRay (camera.cc:65-69) with full-image pixel coordinates (mythtracer.cc:298)
       const double *sensor = BATCH ? views[blockIdx.y].sensor : rp.sensor;
       const D3 start = Load3(sensor), d_scan = Load3(sensor + 3), d_pixel = Load3(sensor + 6);
-      St3(st.m_o, Load3(BATCH ? views[blockIdx.y].origin : rp.origin));
-      St3(st.m_d, Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px)))));
+      if constexpr (LENS) {
+        // thin lens (LensRec): from O + L towards the point where the pinhole ray d meets the focal plane, O + d * t
+        const D3 o = Load3(views[blockIdx.y].origin);
+        const D3 d = Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px))));
+        const LensRec &ln = lens[blockIdx.y];
+        if (ln.centred != 0u) {
+          St3(st.m_o, o);
+          St3(st.m_d, d);
+        } else {
+          const D3 shift = Load3(ln.shift);
+          const double t = ln.focus / Dot(d, Load3(ln.axis));
+          St3(st.m_o, Add(o, shift));
+          St3(st.m_d, Normalized(Sub(MulS(d, t), shift)));
+        }
+      } else {
+        St3(st.m_o, Load3(BATCH ? views[blockIdx.y].origin : rp.origin));
+        St3(st.m_d, Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px)))));
+      }
       st.coef = 1.0;
       st.path = 1ull;
       st.sig_hits = 0ull;
@@ -710,42 +729,48 @@ void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles,
 void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_blocks, bool debug_build, cudaStream_t stream) {
   if (n_blocks <= 0) return;
   if (debug_build) {
-    RenderMega<true, false, 1, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{});
+    RenderMega<true, false, 1, false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{}, nullptr);
   } else {
-    RenderMega<false, false, 1, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{});
+    RenderMega<false, false, 1, false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{}, nullptr);
   }
 }
 
-template <int SS, bool ACC>
-void LaunchBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const dim3 &grid, bool debug_build,
-                 cudaStream_t stream) {
+template <int SS, bool ACC, bool LENS>
+void LaunchBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const LensRec *lens,
+                 const dim3 &grid, bool debug_build, cudaStream_t stream) {
   if (debug_build) {
-    RenderMega<true, true, SS, ACC><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc);
+    RenderMega<true, true, SS, ACC, LENS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens);
   } else {
-    RenderMega<false, true, SS, ACC><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc);
+    RenderMega<false, true, SS, ACC, LENS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens);
   }
 }
 
-template <bool ACC>
-void LaunchBatchSS(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const dim3 &grid,
-                   int samples_per_axis, bool debug_build, cudaStream_t stream) {
+template <bool ACC, bool LENS>
+void LaunchBatchSS(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const LensRec *lens,
+                   const dim3 &grid, int samples_per_axis, bool debug_build, cudaStream_t stream) {
   switch (samples_per_axis) {
-    case 1: LaunchBatch<1, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
-    case 2: LaunchBatch<2, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
-    case 4: LaunchBatch<4, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
-    case 8: LaunchBatch<8, ACC>(sc, rp, views, acc, grid, debug_build, stream); break;
+    case 1: LaunchBatch<1, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
+    case 2: LaunchBatch<2, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
+    case 4: LaunchBatch<4, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
+    case 8: LaunchBatch<8, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
     default: break;  // (the host API admits 1, 2, 4 and 8 only)
   }
 }
 
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
-                           int samples_per_axis, const AccumParams &acc, bool debug_build, cudaStream_t stream) {
+                           int samples_per_axis, const AccumParams &acc, const LensRec *lens, bool debug_build, cudaStream_t stream) {
   if (tiles_per_view <= 0 || n_views <= 0) return;
   const dim3 grid((unsigned)tiles_per_view, (unsigned)n_views);
   if (acc.subframes > 1) {
-    LaunchBatchSS<true>(sc, rp, views, acc, grid, samples_per_axis, debug_build, stream);
+    if (lens != nullptr) {
+      LaunchBatchSS<true, true>(sc, rp, views, acc, lens, grid, samples_per_axis, debug_build, stream);
+    } else {
+      LaunchBatchSS<true, false>(sc, rp, views, acc, nullptr, grid, samples_per_axis, debug_build, stream);
+    }
+  } else if (lens != nullptr) {
+    LaunchBatchSS<false, true>(sc, rp, views, acc, lens, grid, samples_per_axis, debug_build, stream);
   } else {
-    LaunchBatchSS<false>(sc, rp, views, acc, grid, samples_per_axis, debug_build, stream);
+    LaunchBatchSS<false, false>(sc, rp, views, acc, nullptr, grid, samples_per_axis, debug_build, stream);
   }
 }
 

@@ -2,7 +2,7 @@
 orbit yaw = C3 yaw + 2 degrees * k.
 
     python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3]
-                                     [--supersample | --debug-planes | --subframes | --device-output]
+                                     [--supersample | --debug-planes | --subframes | --device-output | --lens]
 
 480x270, 64 frames: (a) one render_chunk per frame, megakernel forced; (b) one render_chunk per frame, automatic
 pipeline choice (after the 13 frames it needs to decide); (c) render_batch in batches of 1, 4, 16, 64.
@@ -42,6 +42,13 @@ mtb_render_batch_device) against the same batch into host memory: 64 views at 48
 torch.cuda.synchronize()), the median kernel_ms per call of both (CUDA events of the library: the device form's come from
 mtb_render_batch_device called with stats, in calls of their own), the bytes the host form copies back per output, and
 whether the device outputs, copied back, equal the host outputs byte for byte (RGB and every plane).
+
+--lens measures thin-lens batches (render_batch(..., lenses=...), mtb_render_batch_lens): 16 outputs x k = 8 at 480x270
+and 4 x k = 4 at 1920x1080, both on the orbit sub-frames of --subframes.  Three modes per shape, timed in turn in every
+pass: the accumulated batch without lenses; the same with centred lens samples (0, 0, f), which trace the same rays
+(its output must equal the first's); and a disc aperture (seeded concentric-disc samples of radius 4 focused at 150),
+which traces different rays.  Per mode: median kernel_ms per call over --reps passes, Mrays/s, output frames/s, and the
+kernel time over that of the batch without lenses.
 """
 import argparse
 import hashlib
@@ -247,6 +254,55 @@ def subframes(mt, files, cfg, reps):
     return groups
 
 
+def _disc_lenses(n, radius, focus, seed):
+    """n seeded thin-lens samples (u, v, focus) on a disc of `radius` (Shirley-Chiu concentric mapping)."""
+    out = []
+    for a, b in 2.0 * np.random.default_rng(seed).random((n, 2)) - 1.0:
+        if abs(a) > abs(b):
+            r, phi = a, np.pi / 4 * (b / a)
+        elif b != 0.0:
+            r, phi = b, np.pi / 2 - np.pi / 4 * (a / b)
+        else:
+            r, phi = 0.0, 0.0
+        out.append((radius * r * np.cos(phi), radius * r * np.sin(phi), focus))
+    return np.array(out)
+
+
+def lens(mt, files, cfg, reps):
+    """The --lens measurements (see the module docstring)."""
+    groups = []
+    for n_out, k, w, h in ((16, 8, 480, 270), (4, 4, cfg["width"], cfg["height"])):
+        cams = [c for f in range(n_out) for c in _orbit_subframes(files.camera, f, k)]
+        modes = (("render_batch %d x %d subframes, no lenses" % (n_out, k), None),
+                 ("render_batch %d x %d subframes, centred lens samples" % (n_out, k), np.array([(0.0, 0.0, 150.0)] * len(cams))),
+                 ("render_batch %d x %d subframes, disc aperture r = 4, focus 150" % (n_out, k), _disc_lenses(len(cams), 4.0, 150.0, 7)))
+        outs = [np.zeros((n_out, h, w, 3), np.uint8) for _ in modes]
+        call = [lambda i=i: mt.render_batch(cams, w, h, out=outs[i], subframes=k, lenses=modes[i][1])["stats"] for i in range(len(modes))]
+        for c in call:
+            c()  # warm-up of this shape
+        walls, kms, rays = [[] for _ in modes], [[] for _ in modes], [0] * len(modes)
+        for _ in range(reps):  # the modes alternate within every pass
+            for i, c in enumerate(call):
+                t0 = time.perf_counter()
+                st = c()
+                walls[i].append(time.perf_counter() - t0)
+                kms[i].append(st["kernel_ms"])
+                rays[i] = st["rays"]
+        base = statistics.median(kms[0])
+        recs = []
+        for i, (name, _) in enumerate(modes):
+            rec = _ss_record(name, n_out, w, h, 1, walls[i], kms[i], rays[i], None)
+            rec.pop("equals_block_mean_of_1080p")
+            rec["kernel_ms_over_no_lenses"] = round(statistics.median(kms[i]) / base, 4)
+            recs.append(rec)
+        recs[1]["equals_no_lenses"] = bool(np.array_equal(outs[1], outs[0]))
+        recs[2]["differs_from_no_lenses"] = not np.array_equal(outs[2], outs[0])
+        print("centred / no lenses kernel time: x%.4f, disc / no lenses: x%.4f" % (recs[1]["kernel_ms_over_no_lenses"],
+                                                                                 recs[2]["kernel_ms_over_no_lenses"]), file=sys.stderr, flush=True)
+        groups.append(dict(shape="C3 orbit, %d outputs x %d subframes at %dx%d" % (n_out, k, w, h), outputs=n_out, subframes=k, modes=recs))
+    return groups
+
+
 def _orbit_subframes(cam, f, k):
     """The k sub-frames of output frame f of the orbit: yaw + 2 degrees * (f + j / k)."""
     out = []
@@ -411,6 +467,7 @@ def main():
     ap.add_argument("--debug-planes", action="store_true")
     ap.add_argument("--subframes", action="store_true")
     ap.add_argument("--device-output", action="store_true")
+    ap.add_argument("--lens", action="store_true")
     args = ap.parse_args()
     devices = [int(x) for x in args.devices.split(",")]
     files, cfg = scenegen.generate_config("C3", os.environ.get("MTB_SCENE_DIR", "/tmp/mtb_scenes"))
@@ -437,6 +494,14 @@ def main():
         _emit(doc, args.out)
         if not all(r["device_equals_host"] for r in doc["device_output"]):
             sys.exit("a batch into device memory differs from the same batch into host memory")
+        return
+
+    if args.lens:
+        doc["lens"] = lens(mt, files, cfg, args.reps)
+        mt.close()
+        _emit(doc, args.out)
+        if not all(g["modes"][1]["equals_no_lenses"] for g in doc["lens"]):
+            sys.exit("centred lens samples differ from the batch without lenses")
         return
 
     if args.subframes:

@@ -51,8 +51,14 @@ def _short(demangled):
     return re.sub(r"^void |\(.*$", "", name).replace("mtb::<unnamed>::", "")
 
 
+def _key(demangled):
+    """The name a kernel is matched by: its short name, with RenderMega's LENS parameter dropped when it is false, so
+    that RenderMega<a, b, c, d, false> of a tree with thin-lens views meets RenderMega<a, b, c, d> of one without."""
+    return re.sub(r"^(RenderMega<[^,<>]+, [^,<>]+, [^,<>]+, [^,<>]+), false>$", r"\1>", _short(demangled))
+
+
 def _kernels(log, sass):
-    """{demangled name: (ptxas figures, [instruction text])}: listings without addresses and encodings."""
+    """{_key name: (ptxas figures, [instruction text])}: listings without addresses and encodings."""
     figures = {}
     for m in re.finditer(r"Compiling entry function '(\S+)'.*?\n.*?Function properties for \1\n\s*(\d+) bytes stack frame, "
                          r"(\d+) bytes spill stores, (\d+) bytes spill loads\n.*?Used (\d+) registers", log):
@@ -66,7 +72,7 @@ def _kernels(log, sass):
     if missing:
         raise SystemExit("no ptxas figures for the kernel(s) %s" % ", ".join(missing))
     names = _demangle(sorted(code))
-    return {names[n]: (figures[n], c) for n, c in code.items()}
+    return {_key(names[n]): (figures[n], c) for n, c in code.items()}
 
 
 def main():
@@ -86,17 +92,17 @@ def main():
             raise SystemExit("no %s in %s" % (src, new_tree))
         old, new = _kernels(*old_res) if old_res else {}, _kernels(*new_res)
         print("%s:" % src)
-        for name in sorted(set(old) | set(new), key=_short):
+        for name in sorted(set(old) | set(new)):
             if name not in new:
-                print("  %s: removed (old: %s)" % (_short(name), old[name][0]))
+                print("  %s: removed (old: %s)" % (name, old[name][0]))
                 continue
             if name not in old:
-                print("  %s: added (new: %s)" % (_short(name), new[name][0]))
+                print("  %s: added (new: %s)" % (name, new[name][0]))
                 continue
             (of, oc), (nf, nc) = old[name], new[name]
             equal = oc == nc and of == nf
             same &= equal
-            print("  %s: %d vs %d instructions, %s" % (_short(name), len(oc), len(nc), "identical" if equal else "DIFFERENT"))
+            print("  %s: %d vs %d instructions, %s" % (name, len(oc), len(nc), "identical" if equal else "DIFFERENT"))
             print("    old: %s\n    new: %s" % (of, nf))
             if oc != nc:
                 i = next((i for i, (a, b) in enumerate(zip(oc, nc)) if a != b), min(len(oc), len(nc)))
