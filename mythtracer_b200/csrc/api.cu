@@ -63,6 +63,8 @@ struct DeviceBuffer {
   }
 };
 
+constexpr int kBatchPlanes = 4;  // the optional outputs of a batch: debug info, sig_hits, sig_shadow, n_rays
+
 struct DeviceState {
   int device = 0;
   int sm_count = 148;
@@ -112,9 +114,7 @@ struct DeviceState {
   DeviceBuffer<mtb::LensRec> batch_lens;  // thin-lens batches: one record per sub-frame of this device
   DeviceBuffer<mtb_light> batch_lights;
   DeviceBuffer<uint8_t> batch_rgb;
-  DeviceBuffer<mtb_debug> batch_dbg;
-  DeviceBuffer<uint64_t> batch_sig_hits, batch_sig_shadow;
-  DeviceBuffer<uint32_t> batch_n_rays;
+  DeviceBuffer<uint8_t> batch_planes[kBatchPlanes];  // bytes of the debug and tap planes, in BatchPlane order
   // accumulated batches: the channel sums of this device's output views and the arrival counters of their tiles
   DeviceBuffer<uint32_t> batch_sum, batch_arrive;
   cudaEvent_t ev_batch_start = nullptr, ev_batch_stop = nullptr;
@@ -143,7 +143,8 @@ struct DeviceState {
     nodes.Free(); slots.Free(); shade.Free(); bvh.Free(); gnodes.Free(); gslots.Free(); list_order.Free(); slot_node.Free(); leaf_ref.Free(); ref_slot.Free(); materials.Free();
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
     counters.Free(); tile_cost.Free(); tile_order.Free();
-    batch_views.Free(); batch_lens.Free(); batch_lights.Free(); batch_rgb.Free(); batch_dbg.Free(); batch_sig_hits.Free(); batch_sig_shadow.Free(); batch_n_rays.Free();
+    batch_views.Free(); batch_lens.Free(); batch_lights.Free(); batch_rgb.Free();
+    for (DeviceBuffer<uint8_t> &b : batch_planes) b.Free();
     batch_sum.Free(); batch_arrive.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
     if (ev_batch_stop != nullptr) cudaEventDestroy(ev_batch_stop);
@@ -437,6 +438,51 @@ void FillStats(const unsigned long long *c, mtb_stats *s) {
   s->n_long512_visits = c[mtb::kLongVisits512];
 }
 
+// rcs[g] = launch(g) for every device g: one host thread per device when there are several (launching a frame is a
+// few dozen driver calls per device; in parallel the devices start together).
+template <class F>
+std::vector<int> OnEveryDevice(int n_dev, const F &launch) {
+  std::vector<int> rcs((size_t)n_dev, MTB_OK);
+  if (n_dev == 1) {
+    rcs[0] = launch(0);
+  } else {
+    std::vector<std::thread> workers;
+    for (int g = 0; g < n_dev; g++) workers.emplace_back([&, g]() { rcs[(size_t)g] = launch(g); });
+    for (std::thread &t : workers) t.join();
+  }
+  return rcs;
+}
+
+// Waits for the stream of each of devices 0 .. n_dev - 1 (device 0: stream0 unless it is NULL) and, with stats, fills
+// them: the devices' counters summed, kernel_ms the slowest device's time from its event `start` to `stop` (the devices
+// run concurrently), total_ms the time since wall0.
+int WaitAndFillStats(mtb_context *ctx, int n_dev, cudaStream_t stream0, cudaEvent_t DeviceState::*start, cudaEvent_t DeviceState::*stop,
+                     std::chrono::steady_clock::time_point wall0, mtb_stats *stats) {
+  unsigned long long total[mtb::kNumCounters];
+  memset(total, 0, sizeof(total));
+  double kernel_ms = 0.0;
+  for (int g = 0; g < n_dev; g++) {
+    DeviceState &d = ctx->dev[(size_t)g];
+    MTB_CUDA(ctx, cudaSetDevice(d.device));
+    cudaStream_t s = (g == 0 && stream0 != nullptr) ? stream0 : d.stream;
+    MTB_CUDA(ctx, cudaStreamSynchronize(s));
+    if (stats == nullptr) continue;
+    unsigned long long c[mtb::kNumCounters];
+    MTB_CUDA(ctx, cudaMemcpy(c, d.counters.ptr, sizeof(c), cudaMemcpyDeviceToHost));
+    for (int i = 0; i < mtb::kNumCounters; i++) total[i] += c[i];
+    float ms = 0.f;
+    MTB_CUDA(ctx, cudaEventElapsedTime(&ms, d.*start, d.*stop));
+    if (ms > kernel_ms) kernel_ms = ms;
+  }
+  if (stats != nullptr) {
+    memset(stats, 0, sizeof(*stats));
+    FillStats(total, stats);
+    stats->kernel_ms = kernel_ms;
+    stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
+  }
+  return MTB_OK;
+}
+
 struct StripPlan {
   int n_strips = 0;   // strips of 8 rows in the chunk
   int owners = 1;     // part_count * n_devices
@@ -616,8 +662,7 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
   std::vector<char> peer_store((size_t)n_dev, 0);
   for (int g = 1; g < n_dev; g++) peer_store[(size_t)g] = ctx->dev[(size_t)g].peer_store_dev0 && d_rgb_user == nullptr && !ctx->no_peer_store;
 
-  // ---- launch on every device: one host thread per device when there are several (launching a frame is a few
-  // dozen driver calls per device; in parallel the devices start together) ----
+  // ---- launch on every device ----
   auto launch_on_device = [&](int g) -> int {
     DeviceState &d = ctx->dev[g];
     MTB_CUDA(ctx, cudaSetDevice(d.device));
@@ -717,17 +762,8 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
     MTB_CUDA(ctx, cudaEventRecord(d.ev_stop, s));
     return MTB_OK;
   };
-  if (n_dev == 1) {
-    const int rc = launch_on_device(0);
+  for (int rc : OnEveryDevice(n_dev, launch_on_device)) {
     if (rc != MTB_OK) return rc;
-  } else {
-    std::vector<int> rcs((size_t)n_dev, MTB_OK);
-    std::vector<std::thread> workers;
-    for (int g = 0; g < n_dev; g++) workers.emplace_back([&, g]() { rcs[(size_t)g] = launch_on_device(g); });
-    for (std::thread &t : workers) t.join();
-    for (int rc : rcs) {
-      if (rc != MTB_OK) return rc;
-    }
   }
 
   // ---- gather on device 0 (peer copies), then device -> host ----
@@ -766,28 +802,8 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
   if (!synchronous && stats == nullptr) return MTB_OK;
 
   MTB_CUDA(ctx, cudaStreamSynchronize(s0));
-  if (stats != nullptr) {
-    unsigned long long total[mtb::kNumCounters];
-    memset(total, 0, sizeof(total));
-    double kernel_ms = 0.0;
-    for (int g = 0; g < n_dev; g++) {
-      DeviceState &d = ctx->dev[g];
-      MTB_CUDA(ctx, cudaSetDevice(d.device));
-      cudaStream_t s = (g == 0 && user_stream != nullptr) ? user_stream : d.stream;
-      MTB_CUDA(ctx, cudaStreamSynchronize(s));
-      unsigned long long c[mtb::kNumCounters];
-      MTB_CUDA(ctx, cudaMemcpy(c, d.counters.ptr, sizeof(c), cudaMemcpyDeviceToHost));
-      for (int i = 0; i < mtb::kNumCounters; i++) total[i] += c[i];
-      float ms = 0.f;
-      MTB_CUDA(ctx, cudaEventElapsedTime(&ms, d.ev_start, d.ev_stop));
-      if (ms > kernel_ms) kernel_ms = ms;  // devices run concurrently: the frame takes the slowest
-    }
-    memset(stats, 0, sizeof(*stats));
-    FillStats(total, stats);
-    stats->kernel_ms = kernel_ms;
-    stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
-  }
-  return MTB_OK;
+  if (stats == nullptr) return MTB_OK;
+  return WaitAndFillStats(ctx, n_dev, user_stream, &DeviceState::ev_start, &DeviceState::ev_stop, wall0, stats);
 }
 
 // A batch: n_views whole frames of one scene, one camera and one light set per view.  Always the megakernel, in one
@@ -886,6 +902,15 @@ int CheckDeviceOutput(mtb_context *ctx, const void *p, const char *name, int dev
   return MTB_OK;
 }
 
+// An optional output plane of a batch (RenderBatchImpl): one entry per sample of every view, view-major.
+struct BatchPlane {
+  uint8_t *out;       // the caller's plane (NULL: not asked for)
+  size_t elem;        // bytes per entry
+  uintptr_t align;    // required alignment of a device output (mtb_render_batch_device)
+  const char *name;   // in error text
+  void (*feed)(mtb::RenderParams &p, uint8_t *plane);  // sets the RenderParams field the plane is rendered through
+};
+
 int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
                     int image_w, int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps,
                     mtb_stats *stats, bool synchronous, bool device_out = false, cudaStream_t user_stream = nullptr) {
@@ -939,14 +964,23 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
   const size_t npx = (size_t)image_w * image_h;  // output pixels of a view
   const int grid_w = image_w * ss, grid_h = image_h * ss;  // its sample grid (the view itself when ss = 1)
   const size_t gpx = (size_t)grid_w * grid_h;              // entries of each of its debug / tap planes
-  uint64_t *const hits_host = taps != nullptr ? taps->sig_hits : nullptr;
-  uint64_t *const shadow_host = taps != nullptr ? taps->sig_shadow : nullptr;
-  uint32_t *const rays_host = taps != nullptr ? taps->n_rays : nullptr;
+  // (kBatchPlanes entries, in the order of the device buffers' batch_planes)
+  const BatchPlane planes[] = {
+      {reinterpret_cast<uint8_t *>(dbg_host), sizeof(mtb_debug), 8, "d_dbg",
+       [](mtb::RenderParams &p, uint8_t *b) { p.dbg = reinterpret_cast<mtb_debug *>(b); }},
+      {reinterpret_cast<uint8_t *>(taps != nullptr ? taps->sig_hits : nullptr), 8, 8, "d_taps->sig_hits",
+       [](mtb::RenderParams &p, uint8_t *b) { p.sig_hits = reinterpret_cast<uint64_t *>(b); }},
+      {reinterpret_cast<uint8_t *>(taps != nullptr ? taps->sig_shadow : nullptr), 8, 8, "d_taps->sig_shadow",
+       [](mtb::RenderParams &p, uint8_t *b) { p.sig_shadow = reinterpret_cast<uint64_t *>(b); }},
+      {reinterpret_cast<uint8_t *>(taps != nullptr ? taps->n_rays : nullptr), 4, 4, "d_taps->n_rays",
+       [](mtb::RenderParams &p, uint8_t *b) { p.n_rays = reinterpret_cast<uint32_t *>(b); }},
+  };
+  static_assert(sizeof(planes) / sizeof(planes[0]) == kBatchPlanes, "one entry per batch plane");
   const bool debug_build = (ctx->flags & MTB_FLAG_COUNT_WORK) != 0;
   const int n_dev = (int)ctx->dev.size();
   const int tiles_x = (grid_w + 7) / 8, tiles_per_view = tiles_x * ((grid_h + 7) / 8);
   const bool accum = k > 1;
-  if (accum && (dbg_host != nullptr || hits_host != nullptr || shadow_host != nullptr || rays_host != nullptr)) {
+  if (accum && std::any_of(std::begin(planes), std::end(planes), [](const BatchPlane &pl) { return pl.out != nullptr; })) {
     ctx->err = "there are no debug or tap planes of accumulated views (subframes > 1): render the sub-frames for their planes";
     return MTB_ERR_ARG;
   }
@@ -964,10 +998,9 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
       return MTB_ERR_ARG;
     }
     int rc = CheckDeviceOutput(ctx, rgb_host, "d_rgb", dev0, 1);
-    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, dbg_host, "d_dbg", dev0, 8);
-    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, hits_host, "d_taps->sig_hits", dev0, 8);
-    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, shadow_host, "d_taps->sig_shadow", dev0, 8);
-    if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, rays_host, "d_taps->n_rays", dev0, 4);
+    for (const BatchPlane &pl : planes) {
+      if (rc == MTB_OK) rc = CheckDeviceOutput(ctx, pl.out, pl.name, dev0, pl.align);
+    }
     if (rc != MTB_OK) return rc;
   }
 
@@ -1033,11 +1066,12 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
     const size_t n_lt = (size_t)count * nl;
     const size_t n_plane = (size_t)count * gpx;
     const size_t n_sum = accum ? (size_t)count_out * npx * 3 : 0, n_arrive = accum ? (size_t)count_out * tiles_per_view * 2 : 0;
-    auto grows = [n_plane, direct](const void *host, size_t have) { return !direct && host != nullptr && n_plane > have; };
+    bool planes_grow = false;
+    for (int i = 0; i < kBatchPlanes; i++) {
+      planes_grow |= !direct && planes[i].out != nullptr && n_plane * planes[i].elem > d.batch_planes[i].count;
+    }
     if ((size_t)count > d.batch_views.count || (lenses != nullptr && (size_t)count > d.batch_lens.count) || n_lt > d.batch_lights.count ||
-        n_rgb > d.batch_rgb.count ||
-        grows(dbg_host, d.batch_dbg.count) || grows(hits_host, d.batch_sig_hits.count) || grows(shadow_host, d.batch_sig_shadow.count) ||
-        grows(rays_host, d.batch_n_rays.count) || n_sum > d.batch_sum.count || n_arrive > d.batch_arrive.count) {
+        n_rgb > d.batch_rgb.count || planes_grow || n_sum > d.batch_sum.count || n_arrive > d.batch_arrive.count) {
       MTB_CUDA(ctx, cudaStreamSynchronize(s));
     }
     MTB_CUDA(ctx, d.batch_views.Upload(views.data() + first, (size_t)count, s));
@@ -1064,27 +1098,13 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
       acc.sum = d.batch_sum.ptr;
       acc.arrive = d.batch_arrive.ptr;
     }
-    if (direct) {
-      if (dbg_host != nullptr) p.dbg = dbg_host + at;
-      if (hits_host != nullptr) p.sig_hits = hits_host + at;
-      if (shadow_host != nullptr) p.sig_shadow = shadow_host + at;
-      if (rays_host != nullptr) p.n_rays = rays_host + at;
-    } else {
-      if (dbg_host != nullptr) {
-        MTB_CUDA(ctx, d.batch_dbg.Reserve(n_plane));
-        p.dbg = d.batch_dbg.ptr;
-      }
-      if (hits_host != nullptr) {
-        MTB_CUDA(ctx, d.batch_sig_hits.Reserve(n_plane));
-        p.sig_hits = d.batch_sig_hits.ptr;
-      }
-      if (shadow_host != nullptr) {
-        MTB_CUDA(ctx, d.batch_sig_shadow.Reserve(n_plane));
-        p.sig_shadow = d.batch_sig_shadow.ptr;
-      }
-      if (rays_host != nullptr) {
-        MTB_CUDA(ctx, d.batch_n_rays.Reserve(n_plane));
-        p.n_rays = d.batch_n_rays.ptr;
+    for (int i = 0; i < kBatchPlanes; i++) {
+      if (planes[i].out == nullptr) continue;
+      if (direct) {
+        planes[i].feed(p, planes[i].out + at * planes[i].elem);
+      } else {
+        MTB_CUDA(ctx, d.batch_planes[i].Reserve(n_plane * planes[i].elem));
+        planes[i].feed(p, d.batch_planes[i].ptr);
       }
     }
     MTB_CUDA(ctx, d.counters.Reserve(mtb::kNumCounters));
@@ -1106,10 +1126,10 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
       if (host_direct == nullptr) {
         MTB_CUDA(ctx, cudaMemcpyAsync(rgb_host + (size_t)first_out * npx * 3, d.batch_rgb.ptr, (size_t)count_out * npx * 3, kind, s));
       }
-      if (dbg_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(dbg_host + at, p.dbg, n_plane * sizeof(mtb_debug), kind, s));
-      if (hits_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(hits_host + at, p.sig_hits, n_plane * 8, kind, s));
-      if (shadow_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(shadow_host + at, p.sig_shadow, n_plane * 8, kind, s));
-      if (rays_host != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(rays_host + at, p.n_rays, n_plane * 4, kind, s));
+      for (int i = 0; i < kBatchPlanes; i++) {
+        const BatchPlane &pl = planes[i];
+        if (pl.out != nullptr) MTB_CUDA(ctx, cudaMemcpyAsync(pl.out + at * pl.elem, d.batch_planes[i].ptr, n_plane * pl.elem, kind, s));
+      }
     }
     if (device_out) MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_done, s));
     return MTB_OK;
@@ -1122,14 +1142,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
     if (d0.ev_batch_caller == nullptr) MTB_CUDA(ctx, cudaEventCreateWithFlags(&d0.ev_batch_caller, cudaEventDisableTiming));
     MTB_CUDA(ctx, cudaEventRecord(d0.ev_batch_caller, s_caller));
   }
-  std::vector<int> rcs((size_t)n_dev, MTB_OK);
-  if (n_dev == 1) {
-    rcs[0] = launch_on_device(0);
-  } else {
-    std::vector<std::thread> workers;
-    for (int g = 0; g < n_dev; g++) workers.emplace_back([&, g]() { rcs[(size_t)g] = launch_on_device(g); });
-    for (std::thread &t : workers) t.join();
-  }
+  const std::vector<int> rcs = OnEveryDevice(n_dev, launch_on_device);
   if (device_out) {
     // ... and the caller's stream waits for every device's last operation: work queued there after the call (and a
     // caching allocator that hands the outputs' memory to such work) sees the finished outputs
@@ -1142,29 +1155,8 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
     if (rc != MTB_OK) return rc;
   }
   if (!synchronous && stats == nullptr) return MTB_OK;
-
-  unsigned long long total[mtb::kNumCounters];
-  memset(total, 0, sizeof(total));
-  double kernel_ms = 0.0;
-  for (int g = 0; g < n_dev && g < n_out; g++) {
-    DeviceState &d = ctx->dev[(size_t)g];
-    MTB_CUDA(ctx, cudaSetDevice(d.device));
-    MTB_CUDA(ctx, cudaStreamSynchronize(d.stream));
-    if (stats == nullptr) continue;
-    unsigned long long c[mtb::kNumCounters];
-    MTB_CUDA(ctx, cudaMemcpy(c, d.counters.ptr, sizeof(c), cudaMemcpyDeviceToHost));
-    for (int i = 0; i < mtb::kNumCounters; i++) total[i] += c[i];
-    float ms = 0.f;
-    MTB_CUDA(ctx, cudaEventElapsedTime(&ms, d.ev_batch_start, d.ev_batch_stop));
-    if (ms > kernel_ms) kernel_ms = ms;  // devices run concurrently: the batch takes the slowest
-  }
-  if (stats != nullptr) {
-    memset(stats, 0, sizeof(*stats));
-    FillStats(total, stats);
-    stats->kernel_ms = kernel_ms;
-    stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
-  }
-  return MTB_OK;
+  // (only the devices that rendered: the others have no events of this batch)
+  return WaitAndFillStats(ctx, std::min(n_dev, n_out), nullptr, &DeviceState::ev_batch_start, &DeviceState::ev_batch_stop, wall0, stats);
 }
 
 }  // namespace

@@ -71,6 +71,11 @@ __device__ __forceinline__ D3 Normalized(const D3 &a) {
   return Mk(a.x / l, a.y / l, a.z / l);
 }
 __device__ __forceinline__ D3 Load3(const double *p) { return Mk(p[0], p[1], p[2]); }
+__device__ __forceinline__ void Store3(double *p, const D3 &v) {
+  p[0] = v.x;
+  p[1] = v.y;
+  p[2] = v.z;
+}
 
 // std::min / std::max of libstdc++ (NaN behaviour is contract, SURVEY.md appendix A.7)
 __device__ __forceinline__ double SMin(double a, double b) { return (b < a) ? b : a; }

@@ -1,4 +1,6 @@
 // RenderMega (per-pixel megakernel) and the batched intersect kernel; see device_core.cuh for the traversal.
+#include <type_traits>
+
 #include "device_core.cuh"
 
 namespace mtb {
@@ -41,13 +43,6 @@ struct alignas(16) PixelState {
 };
 #define MTB_STATE_BARRIER() asm volatile("" : : "l"(&st) : "memory")
 
-__device__ __forceinline__ D3 Ld3(const double *p) { return Mk(p[0], p[1], p[2]); }
-__device__ __forceinline__ void St3(double *p, const D3 &v) {
-  p[0] = v.x;
-  p[1] = v.y;
-  p[2] = v.z;
-}
-
 // ---------------------------------------------------------------------------------------------------
 // RenderMega: one thread = one pixel = the whole TraceRay recursion, evaluated in the reference's
 // post-order so that colour sums associate identically.  Every loop iteration issues exactly one
@@ -89,23 +84,38 @@ __device__ __forceinline__ size_t PlaneIndex(const RenderParams &rp, int px, int
   return (BATCH ? (size_t)blockIdx.y * rp.chunk_w * rp.chunk_h : 0) + (size_t)py * rp.chunk_w + px;
 }
 
-// Supersampled batch (SS = 2, 4, 8 samples per axis): the tile is a tile of the (SS*W) x (SS*H) sample grid (rp.chunk_w
-// x rp.chunk_h), every thread traces one sample exactly as a pixel of that frame, and the epilogue writes the
-// (8/SS)^2 output pixels of the tile, each the rounded mean of its SS x SS quantised samples, to view-major W x H frames.
-// W = chunk_w / SS: the sample grid's sides are multiples of SS, so an output pixel inside the frame has all its samples
-// live, and its SS x SS block never straddles a tile (SS divides 8).
+// Averaged batch: the output pixel is the rounded mean of n quantised samples.
 //
-// SS = 2 and 4: a warp (8x4 samples) holds whole blocks, so the sum stays warp-level like the plain epilogue.
+// Supersampled (SS = 2, 4, 8 samples per axis): the tile is a tile of the (SS*W) x (SS*H) sample grid (rp.chunk_w x
+// rp.chunk_h), every thread traces one sample exactly as a pixel of that frame, and the epilogue writes the (8/SS)^2
+// output pixels of the tile, each the mean of its SS x SS samples, to view-major W x H frames.  W = chunk_w / SS: the
+// sample grid's sides are multiples of SS, so an output pixel inside the frame has all its samples live, and its SS x SS
+// block never straddles a tile (SS divides 8).
+//
+// Accumulated (ACC, SS = 1, 2, 4, 8): block row u traces sub-frame u of output view v = u / k exactly as view u of a
+// batch, and the output pixel is the mean of all k * SS * SS samples of its k sub-frames.  Every warp adds the
+// per-output-channel sums of its half tile (SS = 8: the warp that finishes second, for the whole tile) into acc.sum of
+// view v, fences, and bumps the arrival counter of (v, tile, warp half).  The warp whose arrival is the k-th reads the
+// completed sums from L2 and stores the bytes.  The sums are integers, so the bytes do not depend on the order in which
+// the sub-frames finish.
+//
+// No block barrier after the trace, for the reason of the plain epilogue (RenderMega).  SS = 1, 2 and 4: a warp (8x4
+// samples) holds whole blocks, so the sum stays warp-level like the plain epilogue.
 // SS = 8: the one output pixel of a tile spans both warps.  Each warp reduces its 32 samples with shuffles; the warp
-// that finishes first leaves its partial sums in shared memory and exits, the last one adds them and stores the pixel.
+// that finishes first leaves its partial sums in shared memory and exits, the last one adds them and finishes the pixel.
 // A block barrier there instead holds the first warp's slot until the other is done: 1.3 % more kernel time for 16 C3
 // views at 240x135 (B200, DESIGN.md section 13).
-template <int SS>
-__device__ __forceinline__ void SupersampleEpilogue(const RenderParams &rp, const unsigned char *s_rgb, int tile_id, int strip,
-                                                    unsigned *s_ss8) {
+template <int SS, bool ACC>
+__device__ __forceinline__ void AverageEpilogue(const RenderParams &rp, const AccumParams &acc, const unsigned char *s_rgb, int tile_id,
+                                                int strip, unsigned *s_ss8) {
   const int out_w = rp.chunk_w / SS, out_h = rp.chunk_h / SS;
-  uint8_t *frame = rp.rgb + (size_t)blockIdx.y * out_w * out_h * 3;
+  const unsigned view = ACC ? blockIdx.y / (unsigned)acc.subframes : blockIdx.y;
+  const size_t view_base = (size_t)view * out_w * out_h * 3;
+  uint32_t *const sum = acc.sum + view_base;
+  uint8_t *const frame = rp.rgb + view_base;
   const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  const unsigned n = (ACC ? (unsigned)acc.subframes : 1u) * (SS * SS);
+  uint32_t *const arrive = acc.arrive + ((size_t)view * gridDim.x + tile_id) * 2;
   if constexpr (SS == 8) {
     // the tile is one output pixel, and every sample of it is live (tiles_x = W, 8 rows of tiles per output row)
     const unsigned char *mine = s_rgb + threadIdx.x * 3;
@@ -117,87 +127,33 @@ __device__ __forceinline__ void SupersampleEpilogue(const RenderParams &rp, cons
     }
     // s_ss8: [0] warps done (zeroed before the trace), [1 + 3 * warp ..] that warp's three sums
     volatile unsigned *part = s_ss8 + 1;
-    if (lane == 0u) {
-      part[warp * 3 + 0] = r;
-      part[warp * 3 + 1] = g;
-      part[warp * 3 + 2] = b;
-      __threadfence_block();
-      if (atomicAdd(s_ss8, 1u) == 1u) {  // the other warp's sums are in place
-        __threadfence_block();
-        const unsigned o = (warp ^ 1u) * 3;
-        uint8_t *dst = frame + (size_t)tile_id * 3;  // tile (x, y) = output pixel (x, y): tiles_x = out_w
-        dst[0] = (uint8_t)((r + part[o + 0] + 32u) >> 6);
-        dst[1] = (uint8_t)((g + part[o + 1] + 32u) >> 6);
-        dst[2] = (uint8_t)((b + part[o + 2] + 32u) >> 6);
-      }
-    }
-  } else {
-    // this warp's 8x4 samples = (8/SS) x (4/SS) output pixels; one lane per output channel
-    constexpr int kCols = kTile / SS, kRows = 4 / SS;
-    if (lane >= (unsigned)(kCols * kRows * 3)) return;
-    const int k = (int)lane / 3, c = (int)lane % 3, i = k % kCols, j = k / kCols;
-    const int ox = (tile_id % rp.tiles_x) * kCols + i, oy = (strip * kTile + (int)warp * 4) / SS + j;
-    if (ox >= out_w || oy >= out_h) return;
-    const unsigned char *src = s_rgb + warp * (4 * kTile * 3) + (j * SS * kTile + i * SS) * 3 + c;
-    unsigned sum = 0;
-#pragma unroll
-    for (int a = 0; a < SS; a++) {
-#pragma unroll
-      for (int b = 0; b < SS; b++) sum += src[(a * kTile + b) * 3];
-    }
-    frame[((size_t)oy * out_w + ox) * 3 + c] = (uint8_t)((sum + SS * SS / 2) / (SS * SS));
-  }
-}
-
-// Accumulated batch (ACC, SS = 1, 2, 4, 8): block row u traces sub-frame u of output view v = u / k exactly as view u of
-// a batch, and the output pixel is the rounded mean of all k * SS * SS quantised samples of its k sub-frames.  Every
-// warp adds the per-output-channel sums of its half tile (formed as SupersampleEpilogue forms them; SS = 8: by the
-// warp that finishes second, for the whole tile) into acc.sum of view v, fences, and bumps the arrival counter of
-// (v, tile, warp half).  The warp whose arrival is the k-th reads the completed sums from L2 and stores the bytes.  The
-// sums are integers, so the bytes do not depend on the order in which the sub-frames finish.  No block barrier after
-// the trace, for the reason of the plain epilogue.
-template <int SS>
-__device__ __forceinline__ void AccumulateEpilogue(const RenderParams &rp, const AccumParams &acc, const unsigned char *s_rgb, int tile_id,
-                                                   int strip, unsigned *s_ss8) {
-  const int out_w = rp.chunk_w / SS, out_h = rp.chunk_h / SS;
-  const unsigned view = blockIdx.y / (unsigned)acc.subframes;
-  const size_t view_base = (size_t)view * out_w * out_h * 3;
-  uint32_t *const sum = acc.sum + view_base;
-  uint8_t *const frame = rp.rgb + view_base;
-  const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-  const unsigned n = (unsigned)acc.subframes * (SS * SS);
-  uint32_t *const arrive = acc.arrive + ((size_t)view * gridDim.x + tile_id) * 2;
-  if constexpr (SS == 8) {
-    // as SupersampleEpilogue: the warp that finishes second holds the tile's (= the output pixel's) three sums in lane 0
-    const unsigned char *mine = s_rgb + threadIdx.x * 3;
-    unsigned r = mine[0], g = mine[1], b = mine[2];
-    for (int off = 16; off > 0; off >>= 1) {
-      r += __shfl_down_sync(0xffffffffu, r, off);
-      g += __shfl_down_sync(0xffffffffu, g, off);
-      b += __shfl_down_sync(0xffffffffu, b, off);
-    }
-    volatile unsigned *part = s_ss8 + 1;
     if (lane != 0u) return;
     part[warp * 3 + 0] = r;
     part[warp * 3 + 1] = g;
     part[warp * 3 + 2] = b;
     __threadfence_block();
-    if (atomicAdd(s_ss8, 1u) != 1u) return;
+    if (atomicAdd(s_ss8, 1u) != 1u) return;  // the other warp's sums are not in place yet
     __threadfence_block();
     const unsigned o = (warp ^ 1u) * 3;
-    uint32_t *dst = sum + (size_t)tile_id * 3;  // tile (x, y) = output pixel (x, y)
-    atomicAdd(dst + 0, r + part[o + 0]);
-    atomicAdd(dst + 1, g + part[o + 1]);
-    atomicAdd(dst + 2, b + part[o + 2]);
-    __threadfence();
-    if (atomicAdd(arrive, 1u) != (unsigned)acc.subframes - 1u) return;
-    __threadfence();
-    for (int c = 0; c < 3; c++) frame[(size_t)tile_id * 3 + c] = (uint8_t)((__ldcg(dst + c) + n / 2) / n);
+    const size_t at = (size_t)tile_id * 3;  // tile (x, y) = output pixel (x, y): tiles_x = out_w
+    if constexpr (ACC) {
+      atomicAdd(sum + at + 0, r + part[o + 0]);
+      atomicAdd(sum + at + 1, g + part[o + 1]);
+      atomicAdd(sum + at + 2, b + part[o + 2]);
+      __threadfence();
+      if (atomicAdd(arrive, 1u) != (unsigned)acc.subframes - 1u) return;
+      __threadfence();
+      for (int c = 0; c < 3; c++) frame[at + c] = (uint8_t)((__ldcg(sum + at + c) + n / 2) / n);
+    } else {
+      frame[at + 0] = (uint8_t)((r + part[o + 0] + n / 2) / n);
+      frame[at + 1] = (uint8_t)((g + part[o + 1] + n / 2) / n);
+      frame[at + 2] = (uint8_t)((b + part[o + 2] + n / 2) / n);
+    }
   } else {
     // the output channels this lane owns: SS = 1, the 3 of its own pixel; SS = 2, 4, one of the warp's (8/SS) x (4/SS)
     // output pixels (lane = 3 * pixel + channel)
     constexpr int kPer = SS == 1 ? 3 : 1;
-    long long at = -1;  // this lane's first channel in the view's sums; -1: none
+    long long at = -1;  // this lane's first channel in the view's frame; -1: none
     unsigned val[kPer];
     if constexpr (SS == 1) {
       const int tx = (int)(threadIdx.x & 7u), ty = (int)(threadIdx.x >> 3);
@@ -225,17 +181,20 @@ __device__ __forceinline__ void AccumulateEpilogue(const RenderParams &rp, const
         }
       }
     }
-    if (at >= 0) {
-      for (int c = 0; c < kPer; c++) atomicAdd(sum + at + c, val[c]);
+    if (at < 0 && !ACC) return;  // (an accumulating lane without a channel still takes part in the warp's arrival)
+    if constexpr (ACC) {
+      if (at >= 0) {
+        for (int c = 0; c < kPer; c++) atomicAdd(sum + at + c, val[c]);
+      }
+      __threadfence();
+      __syncwarp();
+      unsigned last = 0u;
+      if (lane == 0u) last = atomicAdd(arrive + warp, 1u) == (unsigned)acc.subframes - 1u ? 1u : 0u;
+      if (__shfl_sync(0xffffffffu, last, 0) == 0u) return;
+      __threadfence();
     }
-    __threadfence();
-    __syncwarp();
-    unsigned last = 0u;
-    if (lane == 0u) last = atomicAdd(arrive + warp, 1u) == (unsigned)acc.subframes - 1u ? 1u : 0u;
-    if (__shfl_sync(0xffffffffu, last, 0) == 0u) return;
-    __threadfence();
     if (at >= 0) {
-      for (int c = 0; c < kPer; c++) frame[at + c] = (uint8_t)((__ldcg(sum + at + c) + n / 2) / n);
+      for (int c = 0; c < kPer; c++) frame[at + c] = (uint8_t)(((ACC ? __ldcg(sum + at + c) : val[c]) + n / 2) / n);
     }
   }
 }
@@ -245,8 +204,8 @@ __device__ __forceinline__ void AccumulateEpilogue(const RenderParams &rp, const
 // tile_cost and run_if; its debug and tap planes (NULL unless the caller asked for them) are view-major, view v's entries
 // start at v * chunk_w * chunk_h (PlaneIndex).  Without BATCH, `views` is unused and every `BATCH ? :`
 // folds away: the single-view kernels compile to the code they had before the batch form existed.  SS > 1 (BATCH only):
-// the supersampled batch, see SupersampleEpilogue; with SS = 1 every `SS` branch folds away.  ACC (BATCH only): the
-// accumulated batch, see AccumulateEpilogue; `acc` is unused without it.  LENS (BATCH only): thin-lens views, the
+// the supersampled batch, see AverageEpilogue; with SS = 1 every `SS` branch folds away.  ACC (BATCH only): the
+// accumulated batch, see AverageEpilogue; `acc` is unused without it.  LENS (BATCH only): thin-lens views, the
 // primary ray of grid row u starts on the lens point of lens[u] and passes through the focal-plane point of the pinhole
 // ray (LensRec); `lens` is unused without it, and only the primary ray differs.
 template <bool DBG, bool BATCH, int SS, bool ACC, bool LENS>
@@ -303,17 +262,17 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         const D3 d = Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px))));
         const LensRec &ln = lens[blockIdx.y];
         if (ln.centred != 0u) {
-          St3(st.m_o, o);
-          St3(st.m_d, d);
+          Store3(st.m_o, o);
+          Store3(st.m_d, d);
         } else {
           const D3 shift = Load3(ln.shift);
           const double t = ln.focus / Dot(d, Load3(ln.axis));
-          St3(st.m_o, Add(o, shift));
-          St3(st.m_d, Normalized(Sub(MulS(d, t), shift)));
+          Store3(st.m_o, Add(o, shift));
+          Store3(st.m_d, Normalized(Sub(MulS(d, t), shift)));
         }
       } else {
-        St3(st.m_o, Load3(BATCH ? views[blockIdx.y].origin : rp.origin));
-        St3(st.m_d, Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px)))));
+        Store3(st.m_o, Load3(BATCH ? views[blockIdx.y].origin : rp.origin));
+        Store3(st.m_d, Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px)))));
       }
       st.coef = 1.0;
       st.path = 1ull;
@@ -329,15 +288,15 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         D3 to, td;
         double limit = CUDART_INF;
         if (flags & kShadowMode) {
-          const D3 seg = Ld3(st.seg_start);
-          td = Ld3(st.ldir);
+          const D3 seg = Load3(st.seg_start);
+          td = Load3(st.ldir);
           to = Add(seg, MulS(td, 0.00001));                                    // mythtracer.cc:95-99
           limit = Dist(seg, Load3(ViewLights<BATCH>(sc)[st.li].position));  // mythtracer.cc:101-102
           st.light_distance = limit;
           Count<DBG>(cnt, kShadow);
         } else {
-          to = Ld3(st.m_o);
-          td = Ld3(st.m_d);
+          to = Load3(st.m_o);
+          td = Load3(st.m_d);
         }
         MTB_STATE_BARRIER();
         slot = Trace<DBG>(sc, to, td, limit, &t, cnt, fctx);
@@ -359,27 +318,27 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
           // mtl is dereferenced unconditionally upstream (mythtracer.cc:121); a missing material acts opaque
           const double str = smtl >= 0 ? __ldg(&sc.materials[smtl].transparency) : 0.0;
           if (str == 0.0) {
-            St3(st.power, Mk(0.0, 0.0, 0.0));
+            Store3(st.power, Mk(0.0, 0.0, 0.0));
             flags |= kInShadow;
             light_done = true;
           } else {
-            D3 power = Ld3(st.power);
+            D3 power = Load3(st.power);
             if (!(flags & kThrough)) {  // light_power *= Tf * Tr (mythtracer.cc:129-132)
               const D3 tf = Load3(sc.materials[smtl].transmission_filter);
               power = MulV(power, MulS(tf, str));
-              St3(st.power, power);
+              Store3(st.power, power);
             }
             flags ^= kThrough;
-            const D3 ldir = Ld3(st.ldir);
-            const D3 to = Add(Ld3(st.seg_start), MulS(ldir, 0.00001));
+            const D3 ldir = Load3(st.ldir);
+            const D3 to = Add(Load3(st.seg_start), MulS(ldir, 0.00001));
             const D3 hit_point = Add(to, MulS(ldir, t));                 // primitive_triangle.cc:141
             const D3 seg_start = Add(hit_point, MulS(ldir, 0.0000001));  // mythtracer.cc:137
-            St3(st.seg_start, seg_start);
-            const D3 P = Ld3(st.P);
+            Store3(st.seg_start, seg_start);
+            const D3 P = Load3(st.P);
             if (SqrDist(P, seg_start) > SqrDist(P, Load3(ViewLights<BATCH>(sc)[st.li].position))) {  // mythtracer.cc:141-145
               light_done = true;
             } else if (power.x <= 0.001 && power.y <= 0.001 && power.z <= 0.001) {
-              St3(st.power, Mk(0.0, 0.0, 0.0));
+              Store3(st.power, Mk(0.0, 0.0, 0.0));
               flags |= kInShadow;
               light_done = true;
             }
@@ -395,20 +354,20 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
           st.sig_shadow += Mix64(st.path, 2ull + (unsigned long long)st.li, (in_shadow ? 1ull : 0ull) | ((unsigned long long)st.segments << 1));
         }
         const D3 lamb = Load3(lt->ambient);
-        D3 power = Ld3(st.power);
+        D3 power = Load3(st.power);
         power.x = SMax(power.x, lamb.x);
         power.y = SMax(power.y, lamb.y);
         power.z = SMax(power.z, lamb.z);
-        const D3 surface = Ld3(st.surface);
-        D3 color = Ld3(st.color);
-        color = Add(color, MulV(MulV(MulS(MulV(Load3(m->diffuse), surface), Dot(Ld3(st.normal), Ld3(st.ldir))), Load3(lt->diffuse)), power));
+        const D3 surface = Load3(st.surface);
+        D3 color = Load3(st.color);
+        color = Add(color, MulV(MulV(MulS(MulV(Load3(m->diffuse), surface), Dot(Load3(st.normal), Load3(st.ldir))), Load3(lt->diffuse)), power));
         if (!in_shadow) {
-          const double refl_dot = Dot(Neg(Ld3(st.m_d)), Ld3(st.reflected));
+          const double refl_dot = Dot(Neg(Load3(st.m_d)), Load3(st.reflected));
           if (refl_dot > 0) {
             color = Add(color, MulV(MulS(MulV(Load3(m->specular), surface), pow(refl_dot, m->specular_exp)), Load3(lt->specular)));
           }
         }
-        St3(st.color, color);
+        Store3(st.color, color);
         st.li++;
       } else {
         // ---- result of a primary / reflection / refraction ray (mythtracer.cc:13-76) ----
@@ -423,8 +382,8 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         } else {
           const ShadeRec *sh = sc.shade + slot;
           const SlotRec *sr = sc.slots + slot;
-          const D3 m_d = Ld3(st.m_d);
-          const D3 P = Add(Ld3(st.m_o), MulS(m_d, t));
+          const D3 m_d = Load3(st.m_d);
+          const D3 P = Add(Load3(st.m_o), MulS(m_d, t));
           const int line_no = __ldg(&sh->line_no);
           if (st.level == 0 && rp.dbg != nullptr) {
             mtb_debug *dbg = rp.dbg + PlaneIndex<BATCH>(rp, px, py);
@@ -460,12 +419,12 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
               const double v = (sh->uv[1] * w.n0 + sh->uv[3] * w.n1 + sh->uv[5] * w.n2) / w.n;
               surface = MulV(surface, SampleTexture(sc.tex_atlas, tex, sc.texture_dim[tex], u, v));
             }
-            St3(st.P, P);
-            St3(st.normal, normal);
-            St3(st.surface, surface);
+            Store3(st.P, P);
+            Store3(st.normal, normal);
+            Store3(st.surface, surface);
             // ray.direction - normal * (2 * ray.direction.Dot(normal)) (mythtracer.cc:68-69)
-            St3(st.reflected, Sub(m_d, MulS(normal, 2 * Dot(normal, m_d))));
-            St3(st.color, Mk(0.0, 0.0, 0.0));
+            Store3(st.reflected, Sub(m_d, MulS(normal, 2 * Dot(normal, m_d))));
+            Store3(st.color, Mk(0.0, 0.0, 0.0));
             st.li = 0;
           }
         }
@@ -475,11 +434,11 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         if (st.li < sc.n_lights) {
           // ---- start the shadow walk of light li (mythtracer.cc:79-94) ----
           const mtb_light *lt = ViewLights<BATCH>(sc) + st.li;
-          const D3 P = Ld3(st.P);
-          St3(st.ldir, Normalized(Sub(Load3(lt->position), P)));
-          St3(st.color, Add(Ld3(st.color), MulV(Load3(lt->ambient), Ld3(st.surface))));  // mythtracer.cc:83-84
-          St3(st.power, Mk(1.0, 1.0, 1.0));
-          St3(st.seg_start, P);
+          const D3 P = Load3(st.P);
+          Store3(st.ldir, Normalized(Sub(Load3(lt->position), P)));
+          Store3(st.color, Add(Load3(st.color), MulV(Load3(lt->ambient), Load3(st.surface))));  // mythtracer.cc:83-84
+          Store3(st.power, Mk(1.0, 1.0, 1.0));
+          Store3(st.seg_start, P);
           flags = (flags & kInObject) | kShadowMode;  // in_shadow = through = false
           st.segments = 0;
           continue;
@@ -493,11 +452,11 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         const bool do_reflect = st.level < rp.max_depth && refl > 0.0 && coef > 0.01 && !in_object;
         const bool do_refract = st.level < rp.max_depth && tr > 0.0;
         if (do_reflect || do_refract) {
-          const D3 P = Ld3(st.P), m_d = Ld3(st.m_d);
+          const D3 P = Load3(st.P), m_d = Load3(st.m_d);
           ShadeFrame &f = frames[sp];
-          St3(f.color, Ld3(st.color));
-          St3(f.point, P);
-          St3(f.dir, m_d);
+          Store3(f.color, Load3(st.color));
+          Store3(f.point, P);
+          Store3(f.dir, m_d);
           f.coef = coef;
           f.path = st.path;
           f.material = st.material;
@@ -508,22 +467,22 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
           st.level++;
           if (do_reflect) {
             Count<DBG>(cnt, kReflect);
-            const D3 reflected = Ld3(st.reflected);
-            St3(st.m_o, Add(P, MulS(reflected, 0.0001)));  // mythtracer.cc:70-75
-            St3(st.m_d, reflected);
+            const D3 reflected = Load3(st.reflected);
+            Store3(st.m_o, Add(P, MulS(reflected, 0.0001)));  // mythtracer.cc:70-75
+            Store3(st.m_d, reflected);
             st.coef = coef * refl;
             st.path = st.path * 2ull;
           } else {
             Count<DBG>(cnt, kRefract);
             const D3 rdir = Normalized(m_d);           // mythtracer.cc:208-212
-            St3(st.m_o, Add(P, MulS(rdir, 0.00001)));  // mythtracer.cc:214-218
-            St3(st.m_d, rdir);
+            Store3(st.m_o, Add(P, MulS(rdir, 0.00001)));  // mythtracer.cc:214-218
+            Store3(st.m_d, rdir);
             flags ^= kInObject;
             st.path = st.path * 2ull + 1ull;
           }
           continue;
         }
-        ret = Ld3(st.color);
+        ret = Load3(st.color);
       }
 
       // ---- an activation returned `ret`: fold it into suspended parents (mythtracer.cc:185-189,220-224) ----
@@ -536,14 +495,14 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         ShadeFrame &f = frames[sp - 1];
         const mtb_material *m = sc.materials + f.material;
         if (f.stage == 0) {
-          const D3 c = Add(Ld3(f.color), MulS(ret, m->reflectance));
+          const D3 c = Add(Load3(f.color), MulS(ret, m->reflectance));
           if (f.do_refract) {
-            St3(f.color, c);
+            Store3(f.color, c);
             f.stage = 1;
             Count<DBG>(cnt, kRefract);
-            const D3 rdir = Normalized(Ld3(f.dir));
-            St3(st.m_o, Add(Ld3(f.point), MulS(rdir, 0.00001)));
-            St3(st.m_d, rdir);
+            const D3 rdir = Normalized(Load3(f.dir));
+            Store3(st.m_o, Add(Load3(f.point), MulS(rdir, 0.00001)));
+            Store3(st.m_d, rdir);
             flags = f.in_object != 0 ? 0u : kInObject;  // in_object toggled; not in a shadow walk
             st.coef = f.coef;
             st.path = f.path * 2ull + 1ull;
@@ -554,7 +513,7 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
           sp--;
         } else {
           // (c * Tf) * Tr (mythtracer.cc:224)
-          ret = Add(Ld3(f.color), MulS(MulV(ret, Load3(m->transmission_filter)), m->transparency));
+          ret = Add(Load3(f.color), MulS(MulV(ret, Load3(m->transmission_filter)), m->transparency));
           sp--;
         }
       }
@@ -579,10 +538,8 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
   // the other one was done (ncu: 9 % of all warp samples sat in that barrier); now it exits and a warp of the next
   // tile takes its registers (DESIGN.md section 5, the warp-level epilogue row). ----
   __syncwarp();
-  if constexpr (ACC) {
-    AccumulateEpilogue<SS>(rp, acc, s_rgb, tile_id, strip, s_ss8);
-  } else if constexpr (SS > 1) {
-    SupersampleEpilogue<SS>(rp, s_rgb, tile_id, strip, s_ss8);
+  if constexpr (ACC || SS > 1) {
+    AverageEpilogue<SS, ACC>(rp, acc, s_rgb, tile_id, strip, s_ss8);
   } else {
     const int px0 = (tile_id % rp.tiles_x) * kTile, py0 = strip * kTile + (int)(threadIdx.x >> 5) * 4;
     const unsigned lane = threadIdx.x & 31u;
@@ -612,6 +569,8 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
     for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
     if ((threadIdx.x & 31u) == 0u) atomicAdd(rp.tile_cost + tile_id, v);
   }
+  // (FlushCounters of wavefront.cu does the same; called here instead, it reschedules the single-frame kernels: 8 more
+  // instructions in RenderMega<false, false, 1, false, false>)
   if (DBG && rp.counters != nullptr) {
     for (int i = 0; i < kNumCounters; i++) {
       unsigned long long v = cnt[i];
@@ -735,43 +694,38 @@ void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_block
   }
 }
 
-template <int SS, bool ACC, bool LENS>
-void LaunchBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const LensRec *lens,
-                 const dim3 &grid, bool debug_build, cudaStream_t stream) {
-  if (debug_build) {
-    RenderMega<true, true, SS, ACC, LENS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens);
+// Calls f(std::true_type{}) or f(std::false_type{}): a run-time flag as a template argument.
+template <class F>
+void WithBool(bool b, const F &f) {
+  if (b) {
+    f(std::true_type{});
   } else {
-    RenderMega<false, true, SS, ACC, LENS><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens);
+    f(std::false_type{});
   }
 }
 
-template <bool ACC, bool LENS>
-void LaunchBatchSS(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, const AccumParams &acc, const LensRec *lens,
-                   const dim3 &grid, int samples_per_axis, bool debug_build, cudaStream_t stream) {
-  switch (samples_per_axis) {
-    case 1: LaunchBatch<1, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
-    case 2: LaunchBatch<2, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
-    case 4: LaunchBatch<4, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
-    case 8: LaunchBatch<8, ACC, LENS>(sc, rp, views, acc, lens, grid, debug_build, stream); break;
-    default: break;  // (the host API admits 1, 2, 4 and 8 only)
-  }
-}
-
+// One of the 32 batch kernels: DBG x SS (1, 2, 4, 8) x ACC x LENS.
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
                            int samples_per_axis, const AccumParams &acc, const LensRec *lens, bool debug_build, cudaStream_t stream) {
   if (tiles_per_view <= 0 || n_views <= 0) return;
   const dim3 grid((unsigned)tiles_per_view, (unsigned)n_views);
-  if (acc.subframes > 1) {
-    if (lens != nullptr) {
-      LaunchBatchSS<true, true>(sc, rp, views, acc, lens, grid, samples_per_axis, debug_build, stream);
-    } else {
-      LaunchBatchSS<true, false>(sc, rp, views, acc, nullptr, grid, samples_per_axis, debug_build, stream);
-    }
-  } else if (lens != nullptr) {
-    LaunchBatchSS<false, true>(sc, rp, views, acc, lens, grid, samples_per_axis, debug_build, stream);
-  } else {
-    LaunchBatchSS<false, false>(sc, rp, views, acc, nullptr, grid, samples_per_axis, debug_build, stream);
-  }
+  WithBool(debug_build, [&](auto dbg) {
+    WithBool(acc.subframes > 1, [&](auto accum) {
+      WithBool(lens != nullptr, [&](auto thin_lens) {
+        const auto launch = [&](auto ss) {
+          RenderMega<decltype(dbg)::value, true, decltype(ss)::value, decltype(accum)::value, decltype(thin_lens)::value>
+              <<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens);
+        };
+        switch (samples_per_axis) {
+          case 1: launch(std::integral_constant<int, 1>{}); break;
+          case 2: launch(std::integral_constant<int, 2>{}); break;
+          case 4: launch(std::integral_constant<int, 4>{}); break;
+          case 8: launch(std::integral_constant<int, 8>{}); break;
+          default: break;  // (the host API admits 1, 2, 4 and 8 only)
+        }
+      });
+    });
+  });
 }
 
 void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, cudaStream_t stream) {

@@ -20,12 +20,6 @@
 namespace mtb {
 namespace {
 
-__device__ __forceinline__ void Store3(double *p, const D3 &v) {
-  p[0] = v.x;
-  p[1] = v.y;
-  p[2] = v.z;
-}
-
 template <bool DBG>
 __device__ __forceinline__ void FlushCounters(unsigned long long *cnt, unsigned long long *global, unsigned n_rays) {
   if (global == nullptr) return;
