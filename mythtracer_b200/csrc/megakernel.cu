@@ -59,7 +59,8 @@ struct alignas(16) PixelState {
 // TraceFast stays free of spill code (B200, C3, ms): 10 blocks (96 registers) 10.50, 12 (80) 9.66, 14 (72) 9.07 - and,
 // once the FP32 ray's live range was split by hand (TraceFast, device_core.cuh) and the small per-pixel integers
 // moved into PixelState, so that 64 registers no longer put reloads into the node loop - 16 (64) 8.88, 18 (56) 9.00,
-// 20 (48) 9.14.
+// 20 (48) 9.14.  With the leaf's FP64 ray read from shared memory at each use (fewer leaf spills below 64 registers;
+// DESIGN.md section 5): 16 8.83, 20 8.83, 24 (40) 9.32 - the optimum is not set by the leaf spills alone.
 #define MTB_MEGA_MIN_BLOCKS 16
 #endif
 
@@ -208,8 +209,13 @@ __device__ __forceinline__ void AverageEpilogue(const RenderParams &rp, const Ac
 // accumulated batch, see AverageEpilogue; `acc` is unused without it.  LENS (BATCH only): thin-lens views, the
 // primary ray of grid row u starts on the lens point of lens[u] and passes through the focal-plane point of the pinhole
 // ray (LensRec); `lens` is unused without it, and only the primary ray differs.
+// `sc` is __grid_constant__: the exact traversals take it by reference (TraceExactCold is not inlined), and a plain
+// by-value parameter whose address is taken is copied to local memory at kernel start (112 B), after which the scene
+// pointers (nodes, leaf records, shading records, materials, lights) are loaded from that copy.  A grid constant's
+// address points at the parameter bank itself, so the fields are constant-bank operands: C3 8.86 ->
+// 8.56 ms, C5 49.1 -> 47.7 ms, C4 7.73-7.79 -> 7.59-7.61 ms (B200, 1000 W, 1965 MHz max SM clock; DESIGN.md section 5).
 template <bool DBG, bool BATCH, int SS, bool ACC, bool LENS>
-__global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(DeviceScene sc, RenderParams rp, const ViewRec *views,
+__global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(const __grid_constant__ DeviceScene sc, RenderParams rp, const ViewRec *views,
                                                                                  AccumParams acc, const LensRec *lens) {
   static_assert(SS == 1 || (BATCH && (SS == 2 || SS == 4 || SS == 8)), "supersampling is a batch form with 2, 4 or 8 samples per axis");
   static_assert(!ACC || BATCH, "accumulation is a batch form");
@@ -587,7 +593,7 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
 
 // Batched OctTree::IntersectRay (octtree.cc:26-40), one ray per thread.
 template <bool DBG>
-__global__ void __launch_bounds__(128) IntersectKernel(DeviceScene sc, IntersectParams ip) {
+__global__ void __launch_bounds__(128) IntersectKernel(const __grid_constant__ DeviceScene sc, IntersectParams ip) {
   MTB_DECLARE_FAST_CTX(128);
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long cnt_store[DBG ? kNumCounters : 1];

@@ -102,8 +102,9 @@ __global__ void WfQueueBegin(WfBuffers wf, int slots) {
   if (i < kQWords) wf.qctl[i] = (i == kQTail || i == kQPending) ? (uint32_t)slots : 0u;
 }
 
+// (`sc` is __grid_constant__ for the reason given at RenderMega: no local copy of the scene record.)
 template <bool DBG>
-__global__ void __launch_bounds__(kBlockThreads, MTB_QUEUE_MIN_BLOCKS) WfQueue(DeviceScene sc, RenderParams rp, WfBuffers wf, int slots, unsigned epoch) {
+__global__ void __launch_bounds__(kBlockThreads, MTB_QUEUE_MIN_BLOCKS) WfQueue(const __grid_constant__ DeviceScene sc, RenderParams rp, WfBuffers wf, int slots, unsigned epoch) {
   MTB_DECLARE_FAST_CTX(kBlockThreads);
   unsigned long long cnt_store[DBG ? kNumCounters : 1];
   unsigned long long *cnt = cnt_store;
@@ -493,7 +494,7 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_QUEUE_MIN_BLOCKS) WfQueue(D
 // Per-pixel fold of the activation tree in the reference's order - parent += child * Refl, then
 // parent += (child * Tf) * Tr (mythtracer.cc:185-189, 220-224), children before parents - followed by V3DtoRGB
 // (mythtracer.cc:235-241).  One block = one 8x8 tile (slots pos * 64 ..), written like RenderMega writes its tiles.
-__global__ void __launch_bounds__(kBlockThreads) WfResolveTree(DeviceScene sc, RenderParams rp, WfBuffers wf, int slots) {
+__global__ void __launch_bounds__(kBlockThreads) WfResolveTree(const __grid_constant__ DeviceScene sc, RenderParams rp, WfBuffers wf, int slots) {
   __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3];
   if (wf.ctrl[0] != 0u) return;
   const int tile = (int)blockIdx.x, root = tile * 64 + (int)threadIdx.x;
