@@ -227,6 +227,19 @@ class MythTracer {
     }
     return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, out, nullptr, true, false, nullptr, lenses.data());
   }
+  // Panoramas (mtb_render_batch_pano): the accumulated batch above with every camera rendering an h_fov x v_fov degree
+  // longitude / latitude grid around its origin, turned by its pitch, yaw and roll (its aov is ignored); (360, 180) is a
+  // full equirectangular panorama.  eye_offsets: empty (all 0) or one per camera, the distance each column's origin
+  // moves along its tangent; -IPD/2 and +IPD/2 give the two eyes of an omni-directional stereo pair.
+  bool RayTraceBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams, double h_fov,
+                     double v_fov, const std::vector<double> &eye_offsets, const std::vector<std::vector<Light>> *lights, uint8_t *out) {
+    if (!eye_offsets.empty() && eye_offsets.size() != cams.size()) {
+      fprintf(stderr, "error: %zu eye offsets for %zu cameras (one per camera, or none)\n", eye_offsets.size(), cams.size());
+      return false;
+    }
+    const Panorama pano{h_fov, v_fov, eye_offsets.empty() ? nullptr : eye_offsets.data()};
+    return RenderBatch(image_width, image_height, samples_per_axis, subframes, cams, lights, out, nullptr, true, false, nullptr, nullptr, &pano);
+  }
   bool Wait() { return mtb_wait(scene.tree.context()) == MTB_OK; }
   static uint8_t *AllocFrames(int image_width, int image_height, int n_frames) {
     return static_cast<uint8_t *>(mtb_host_alloc((size_t)image_width * image_height * 3 * (size_t)n_frames));
@@ -241,9 +254,13 @@ class MythTracer {
   mtb_stats last_stats{};
 
  private:
+  struct Panorama {
+    double h_fov, v_fov;
+    const double *eye_offsets;
+  };
   bool RenderBatch(int image_width, int image_height, int samples_per_axis, int subframes, const std::vector<Camera> &cams,
                    const std::vector<std::vector<Light>> *lights, uint8_t *out, mtb_debug *dbg, bool synchronous, bool device = false,
-                   void *stream = nullptr, const mtb_lens *lenses = nullptr) {
+                   void *stream = nullptr, const mtb_lens *lenses = nullptr, const Panorama *pano = nullptr) {
     if (!was_scene_finalized) {
       puts("Finalizing tree.");
       if (!scene.tree.Finalize(&scene.materials, &scene.textures)) return false;
@@ -276,7 +293,7 @@ class MythTracer {
     const mtb_light *lp = lights == nullptr ? nullptr : reinterpret_cast<const mtb_light *>(flat.data());
     mtb_stats stats;
     int rc;
-    if (subframes != 1 || device || lenses != nullptr) {
+    if (subframes != 1 || device || lenses != nullptr || pano != nullptr) {
       if (subframes < 1 || cams.size() % (size_t)subframes != 0) {
         fprintf(stderr, "error: %zu cameras are not a whole number of output views of %d subframes\n", cams.size(), subframes);
         return false;
@@ -285,6 +302,9 @@ class MythTracer {
       if (lenses != nullptr) {
         rc = mtb_render_batch_lens(ctx, mcams.data(), lenses, n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
                                    max_recursion_level, out, nullptr, nullptr, &stats);
+      } else if (pano != nullptr) {
+        rc = mtb_render_batch_pano(ctx, mcams.data(), pano->eye_offsets, n_out, subframes, pano->h_fov, pano->v_fov, lp, n_lights, image_width,
+                                   image_height, samples_per_axis, max_recursion_level, out, nullptr, nullptr, &stats);
       } else if (device) {
         rc = mtb_render_batch_device(ctx, mcams.data(), n_out, subframes, lp, n_lights, image_width, image_height, samples_per_axis,
                                      max_recursion_level, out, nullptr, nullptr, stream, nullptr);

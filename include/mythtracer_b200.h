@@ -374,6 +374,42 @@ int mtb_render_batch_lens_device(mtb_context *ctx, const mtb_camera *cams, const
                                  const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
                                  void *d_rgb, mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream, mtb_stats *stats);
 
+/* Panoramas: the batch forms with a longitude / latitude sample grid instead of the pinhole sensor, for equirectangular
+ * and omni-directional stereo (ODS) views.  Each camera's origin, pitch, yaw and roll are used and its aov is ignored.
+ * With Wg x Hg = (s*image_w) x (s*image_h) the sample grid, every operation in FP64 and in the order written
+ * (compiled with --fmad=false / -ffp-contract=off), once per call, for column X < Wg and row Y < Hg:
+ *     lon_X = ((double)(2X + 1 - Wg) / (double)(2 Wg)) * (h_fov * (M_PI / 180.0))      positive = right
+ *     lat_Y = ((double)(Hg - 2Y - 1) / (double)(2 Hg)) * (v_fov * (M_PI / 180.0))      positive = up
+ *     cl_X = cos(lon_X), sl_X = sin(lon_X), cp_Y = cos(lat_Y), sp_Y = sin(lat_Y)       (the C library's cos / sin)
+ * once per sub-frame u, with aim = Mul(Mul(RotY(yaw), RotX(pitch)), RotZ(roll)) the rotation of mtb_camera_sensor:
+ *     F = Apply(aim, (0, 0, 1)),  R = Apply(aim, (-1, 0, 0)),  U = Apply(aim, (0, 1, 0))
+ * (R points along the pinhole sensor's delta_pixel and U against its delta_scanline), and per sample (X, Y), with O the
+ * camera's origin and e = eye_offsets[u]:
+ *     h      = F * cl_X + R * sl_X
+ *     d      = Normalized(h * cp_Y + U * sp_Y)
+ *     origin = O + (R * cl_X - F * sl_X) * e            (e == 0: O itself)
+ * The sample is the reference's TraceRay of (origin, d) at depth max_depth, and the output bytes are those of
+ * mtb_render_batch_accum over these samples (the rounded mean of the k*s*s quantised samples of an output pixel; k = 1:
+ * the sub-frame itself).  h_fov = 360 and v_fov = 180 give a full equirectangular panorama whose left and right edges
+ * meet without a seam; e = -IPD/2 and +IPD/2 give the left and right eye of an ODS pair, the eye displaced along each
+ * column's tangent.  The library chooses no field of view, eye distance or sample pattern.  mtb_panorama_rays returns
+ * the rays of one sub-frame.
+ *
+ * eye_offsets: NULL (all 0) or one entry per camera (n_out * subframes), HOST memory.  Planes (dbg_out, taps) are those
+ * of mtb_render_batch_debug for the panorama rays and only available with subframes == 1.  Every argument rule of
+ * mtb_render_batch_debug / mtb_render_batch_accum applies; in addition each of these is MTB_ERR_ARG, before anything is
+ * queued (also on a host-only context): h_fov not finite or outside (0, 360]; v_fov not finite or outside (0, 180]; an
+ * eye offset that is not finite.  Synchronous. */
+int mtb_render_batch_pano(mtb_context *ctx, const mtb_camera *cams, const double *eye_offsets, int32_t n_out, int32_t subframes, double h_fov,
+                          double v_fov, const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                          uint8_t *rgb_out, mtb_debug *dbg_out, const mtb_taps *taps, mtb_stats *stats);
+/* The same into DEVICE memory: the contract of mtb_render_batch_device (pointer and stream checks, stream ordering,
+ * the split over devices) with the panorama arguments and rules of mtb_render_batch_pano. */
+int mtb_render_batch_pano_device(mtb_context *ctx, const mtb_camera *cams, const double *eye_offsets, int32_t n_out, int32_t subframes,
+                                 double h_fov, double v_fov, const mtb_light *lights, int32_t n_lights, int image_w, int image_h,
+                                 int samples_per_axis, int max_depth, void *d_rgb, mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream,
+                                 mtb_stats *stats);
+
 /* Same render, result left in DEVICE memory of device 0 (d_rgb: chunk_w*chunk_h*3 bytes); enqueued on
  * `stream` (a cudaStream_t of device 0; NULL = the context's own stream) without synchronising when the
  * context has one device.  This is the entry bench.py times for the HBM-resident figure. */
@@ -418,6 +454,13 @@ int mtb_intersect_rays(mtb_context *ctx, int64_t n, const double *origins, const
 
 /* Camera::GetSensor (camera.cc:17-63): start_point, delta_scanline, delta_pixel (9 doubles), host side. */
 int mtb_camera_sensor(const mtb_camera *cam, int image_w, int image_h, double out9[9]);
+
+/* The primary rays of one panorama sub-frame of mtb_render_batch_pano (its contract, bit for bit) on a grid_w x grid_h
+ * sample grid, host side: origins (nullable) and dirs are grid_h * grid_w * 3 doubles, row-major, sample (X, Y) at
+ * (Y * grid_w + X) * 3.  MTB_ERR_ARG for a NULL cam or dirs, a grid side outside 1..65536, and the h_fov, v_fov and
+ * eye_offset rules of mtb_render_batch_pano.  Needs no context and no device. */
+int mtb_panorama_rays(const mtb_camera *cam, int grid_w, int grid_h, double h_fov, double v_fov, double eye_offset, double *origins,
+                      double *dirs);
 
 const char *mtb_version(void);
 

@@ -20,6 +20,7 @@ without a CUDA device raises.
 from __future__ import annotations
 
 import ctypes
+import math
 import os
 from dataclasses import dataclass, field
 from typing import List, Optional, Sequence
@@ -81,7 +82,7 @@ EXPORTED_SYMBOLS = [
     "mtb_frame_create", "mtb_frame_open", "mtb_frame_release", "mtb_frame_read", "mtb_load_timing", "mtb_hybrid_share",
     "mtb_render_batch", "mtb_render_batch_async", "mtb_render_batch_ss", "mtb_render_batch_ss_async", "mtb_render_batch_debug",
     "mtb_render_batch_accum", "mtb_render_batch_accum_async", "mtb_render_batch_device", "mtb_render_batch_lens",
-    "mtb_render_batch_lens_device",
+    "mtb_render_batch_lens_device", "mtb_render_batch_pano", "mtb_render_batch_pano_device", "mtb_panorama_rays",
 ]
 
 
@@ -144,6 +145,12 @@ def load_library():
     lib.mtb_render_batch_lens.argtypes = [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp, vp, vp]
     lib.mtb_render_batch_lens_device.argtypes = [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp,
                                                  vp, vp, vp]
+    f64 = ctypes.c_double
+    lib.mtb_render_batch_pano.argtypes = [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, f64, f64, vp, ctypes.c_int32, i32, i32, i32, i32, vp, vp,
+                                          vp, vp]
+    lib.mtb_render_batch_pano_device.argtypes = [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, f64, f64, vp, ctypes.c_int32, i32, i32, i32, i32,
+                                                 vp, vp, vp, vp, vp]
+    lib.mtb_panorama_rays.argtypes = [vp, i32, i32, f64, f64, f64, vp, vp]
     lib.mtb_read_counters.argtypes = [vp, vp]
     lib.mtb_pipeline_in_use.argtypes = [vp, vp, vp]
     lib.mtb_launch_count.argtypes = [vp]
@@ -244,6 +251,55 @@ def _lens_array(lenses, n_cams: int) -> np.ndarray:
     if not (arr[:, 2] > 0).all():
         raise MythTracerError("render_batch: every lens focus_distance must be > 0")
     return np.ascontiguousarray(arr)
+
+
+def _fov_pair(h_fov, v_fov, who: str):
+    """(h_fov, v_fov) as floats, checked against the rules of mtb_render_batch_pano."""
+    for name, value, top in (("h_fov", h_fov, 360.0), ("v_fov", v_fov, 180.0)):
+        if isinstance(value, (bool, np.bool_)) or not isinstance(value, (int, float, np.integer, np.floating)):
+            raise MythTracerError("%s: %s must be a number of degrees (got %r)" % (who, name, value))
+        if not (math.isfinite(value) and 0.0 < value <= top):
+            raise MythTracerError("%s: %s must be finite and in (0, %g] degrees (got %r)" % (who, name, top, value))
+    return float(h_fov), float(v_fov)
+
+
+def _panorama_args(panorama, eye_offsets, n_cams: int):
+    """render_batch's panorama and eye_offsets as (h_fov, v_fov, float64 array of n_cams eye offsets or None)."""
+    if isinstance(panorama, (str, bytes)) or not isinstance(panorama, (tuple, list, np.ndarray)) or len(panorama) != 2:
+        raise MythTracerError("render_batch: panorama must be a pair (h_fov, v_fov) in degrees (got %r)" % (panorama,))
+    h_fov, v_fov = _fov_pair(panorama[0], panorama[1], "render_batch")
+    if eye_offsets is None:
+        return h_fov, v_fov, None
+    if isinstance(eye_offsets, (str, bytes)):
+        raise MythTracerError("render_batch: eye_offsets must be a sequence of numbers or a float64 array (got %r)" % (eye_offsets,))
+    try:
+        eye = np.array(eye_offsets, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise MythTracerError("render_batch: eye_offsets must hold numbers: %s" % e)
+    if eye.shape != (n_cams,):
+        raise MythTracerError("render_batch: eye_offsets must have shape (%d,), one per camera (got %s)" % (n_cams, eye.shape))
+    if not np.isfinite(eye).all():
+        raise MythTracerError("render_batch: every eye offset must be finite")
+    return h_fov, v_fov, np.ascontiguousarray(eye)
+
+
+def panorama_rays(camera, w: int, h: int, h_fov: float, v_fov: float, eye_offset: float = 0.0):
+    """mtb_panorama_rays: the primary rays (origins, dirs), each a (h, w, 3) float64 array, of one sub-frame of a
+    panorama batch on a w x h sample grid (render_batch(..., panorama=(h_fov, v_fov), eye_offsets=...) at
+    samples_per_axis s traces those of the (s*width) x (s*height) grid).  Host side: needs no context and no GPU."""
+    cam = camera if isinstance(camera, Camera) else Camera.from_tuple(camera)
+    for name, n in (("w", w), ("h", h)):
+        if isinstance(n, (bool, np.bool_)) or not isinstance(n, (int, np.integer)) or not 1 <= n <= 65536:
+            raise MythTracerError("panorama_rays: %s must be an int in 1..65536 (got %r)" % (name, n))
+    h_fov, v_fov = _fov_pair(h_fov, v_fov, "panorama_rays")
+    if isinstance(eye_offset, (bool, np.bool_)) or not isinstance(eye_offset, (int, float, np.integer, np.floating)) or not math.isfinite(eye_offset):
+        raise MythTracerError("panorama_rays: eye_offset must be a finite number (got %r)" % (eye_offset,))
+    origins = np.zeros((int(h), int(w), 3))
+    dirs = np.zeros((int(h), int(w), 3))
+    rc = load_library().mtb_panorama_rays(_ptr(cam.as_array()), int(w), int(h), h_fov, v_fov, float(eye_offset), _ptr(origins), _ptr(dirs))
+    if rc != MTB_OK:
+        raise MythTracerError("mtb_panorama_rays refused its arguments")
+    return origins, dirs
 
 
 @dataclass
@@ -494,7 +550,8 @@ class MythTracer:
         return res
 
     def render_batch(self, cameras, width: int, height: int, lights=None, out: Optional[np.ndarray] = None, samples_per_axis: int = 1,
-                     debug: bool = False, taps: bool = False, subframes: int = 1, device: bool = False, lenses=None):
+                     debug: bool = False, taps: bool = False, subframes: int = 1, device: bool = False, lenses=None, panorama=None,
+                     eye_offsets=None):
         """mtb_render_batch: len(cameras) whole frames in one launch per device, at depth self.max_depth.
 
         lights: None (every view uses GetScene().lights) or one list of Light per view, all of the same length.
@@ -527,7 +584,16 @@ class MythTracer:
         through the points where its pinhole rays meet the plane at focus_distance along the view axis; with subframes
         k > 1 an output view is the mean of its k sub-frames, so k lens points spread over an aperture give depth of field
         (include/mythtracer_b200.h has the exact formula).  A centred sample (0, 0, f) is the pinhole ray.  Everything
-        else (samples_per_axis, subframes, lights, debug, taps, device, out) is as without lenses."""
+        else (samples_per_axis, subframes, lights, debug, taps, device, out) is as without lenses.
+
+        panorama: None (pinhole views) or (h_fov, v_fov) in degrees, h_fov in (0, 360] and v_fov in (0, 180], for the
+        whole call: every camera renders a longitude / latitude grid around its origin, turned by its pitch, yaw and roll
+        (its aov is ignored), through mtb_render_batch_pano (device=True: mtb_render_batch_pano_device).  (360, 180) is a
+        full equirectangular panorama.  eye_offsets: None (all 0) or one number per camera, as a sequence or a float64
+        array of shape (len(cameras),); a non-zero e moves the origin of every column by e along its tangent, so -IPD/2
+        and +IPD/2 give the two eyes of an omni-directional stereo pair.  panorama_rays() returns the rays of one camera
+        (include/mythtracer_b200.h has the exact formula).  Not with lenses.  Everything else (samples_per_axis,
+        subframes, lights, debug, taps, device, out) is as without a panorama."""
         if not isinstance(device, (bool, np.bool_)):
             raise MythTracerError("render_batch: device must be True or False (got %r)" % (device,))
         device = bool(device)
@@ -551,6 +617,11 @@ class MythTracer:
         if len(cams) % k != 0:
             raise MythTracerError("render_batch: %d cameras are not a whole number of output views of %d subframes" % (len(cams), k))
         lens_arr = None if lenses is None else _lens_array(lenses, len(cams))
+        if panorama is None and eye_offsets is not None:
+            raise MythTracerError("render_batch: eye_offsets need a panorama (panorama=(h_fov, v_fov))")
+        if panorama is not None and lenses is not None:
+            raise MythTracerError("render_batch: panorama and lenses cannot be combined (a panorama has no thin-lens form)")
+        pano = None if panorama is None else _panorama_args(panorama, eye_offsets, len(cams))
         cam_arr = np.zeros(len(cams), CAMERA_DTYPE)
         for i, c in enumerate(cams):
             cam_arr[i] = c.as_array()
@@ -574,7 +645,7 @@ class MythTracer:
         n_out = len(cams) // k
         shape = (n_out, height, width, 3)
         if device:
-            return self._render_batch_device(cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps, lens_arr)
+            return self._render_batch_device(cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps, lens_arr, pano)
         if out is None:
             rgb = np.zeros(shape, np.uint8)
         else:
@@ -599,6 +670,10 @@ class MythTracer:
             self._check(self._lib.mtb_render_batch_lens(self._ctx, _ptr(cam_arr), _ptr(lens_arr), n_out, k, _ptr(light_arr), n_lights, width,
                                                         height, ss, self.max_depth, _ptr(rgb), _ptr(dbg), tap_ptr, _ptr(stats)),
                         "mtb_render_batch_lens")
+        elif pano is not None:
+            self._check(self._lib.mtb_render_batch_pano(self._ctx, _ptr(cam_arr), _ptr(pano[2]), n_out, k, pano[0], pano[1], _ptr(light_arr),
+                                                        n_lights, width, height, ss, self.max_depth, _ptr(rgb), _ptr(dbg), tap_ptr, _ptr(stats)),
+                        "mtb_render_batch_pano")
         elif debug or taps:
             self._check(self._lib.mtb_render_batch_debug(self._ctx, _ptr(cam_arr), len(cams), _ptr(light_arr), n_lights, width, height,
                                                          ss, self.max_depth, _ptr(rgb), _ptr(dbg), tap_ptr, _ptr(stats)),
@@ -621,7 +696,7 @@ class MythTracer:
         self.last_stats = res["stats"]
         return res
 
-    def _render_batch_device(self, cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps, lens_arr=None):
+    def _render_batch_device(self, cam_arr, n_out, k, light_arr, n_lights, width, height, ss, out, debug, taps, lens_arr=None, pano=None):
         """render_batch(..., device=True) once the arguments shared with the host form are checked."""
         try:
             import torch
@@ -638,6 +713,10 @@ class MythTracer:
             self._check(self._lib.mtb_render_batch_lens_device(self._ctx, _ptr(cam_arr), _ptr(lens_arr), n_out, k, _ptr(light_arr), n_lights,
                                                                width, height, ss, self.max_depth, None, None, None, None, None),
                         "mtb_render_batch_lens_device")
+        if self._device0 is None and pano is not None:
+            self._check(self._lib.mtb_render_batch_pano_device(self._ctx, _ptr(cam_arr), _ptr(pano[2]), n_out, k, pano[0], pano[1], _ptr(light_arr),
+                                                               n_lights, width, height, ss, self.max_depth, None, None, None, None, None),
+                        "mtb_render_batch_pano_device")
         if self._device0 is None:  # host-only context: the library refuses the call (there is no CPU fallback)
             self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
                                                           self.max_depth, None, None, None, None, None), "mtb_render_batch_device")
@@ -662,6 +741,10 @@ class MythTracer:
             self._check(self._lib.mtb_render_batch_lens_device(self._ctx, _ptr(cam_arr), _ptr(lens_arr), n_out, k, _ptr(light_arr), n_lights,
                                                                width, height, ss, self.max_depth, d_rgb, d_dbg, tap_ptr, handle, None),
                         "mtb_render_batch_lens_device")
+        elif pano is not None:
+            self._check(self._lib.mtb_render_batch_pano_device(self._ctx, _ptr(cam_arr), _ptr(pano[2]), n_out, k, pano[0], pano[1], _ptr(light_arr),
+                                                               n_lights, width, height, ss, self.max_depth, d_rgb, d_dbg, tap_ptr, handle, None),
+                        "mtb_render_batch_pano_device")
         else:
             self._check(self._lib.mtb_render_batch_device(self._ctx, _ptr(cam_arr), n_out, k, _ptr(light_arr), n_lights, width, height, ss,
                                                           self.max_depth, d_rgb, d_dbg, tap_ptr, handle, None), "mtb_render_batch_device")

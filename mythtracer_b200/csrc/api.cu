@@ -112,6 +112,9 @@ struct DeviceState {
   // events steer the automatic pipeline choice and are left alone)
   DeviceBuffer<mtb::ViewRec> batch_views;
   DeviceBuffer<mtb::LensRec> batch_lens;  // thin-lens batches: one record per sub-frame of this device
+  // panorama batches: one record per sub-frame of this device, and the call's longitude and latitude tables
+  DeviceBuffer<mtb::PanoRec> batch_pano;
+  DeviceBuffer<double> batch_pano_tab;
   DeviceBuffer<mtb_light> batch_lights;
   DeviceBuffer<uint8_t> batch_rgb;
   DeviceBuffer<uint8_t> batch_planes[kBatchPlanes];  // bytes of the debug and tap planes, in BatchPlane order
@@ -143,7 +146,7 @@ struct DeviceState {
     nodes.Free(); slots.Free(); shade.Free(); bvh.Free(); gnodes.Free(); gslots.Free(); list_order.Free(); slot_node.Free(); leaf_ref.Free(); ref_slot.Free(); materials.Free();
     tex_dims.Free(); lights.Free(); rgb.Free(); dbg.Free(); sig_hits.Free(); sig_shadow.Free(); n_rays.Free();
     counters.Free(); tile_cost.Free(); tile_order.Free();
-    batch_views.Free(); batch_lens.Free(); batch_lights.Free(); batch_rgb.Free();
+    batch_views.Free(); batch_lens.Free(); batch_pano.Free(); batch_pano_tab.Free(); batch_lights.Free(); batch_rgb.Free();
     for (DeviceBuffer<uint8_t> &b : batch_planes) b.Free();
     batch_sum.Free(); batch_arrive.Free();
     if (ev_batch_start != nullptr) cudaEventDestroy(ev_batch_start);
@@ -823,14 +826,17 @@ int RenderImpl(mtb_context *ctx, const mtb_camera *cam, int image_w, int image_h
 // buffers; every other device renders into its own and copies its slice over with one copy per output.
 // lenses (nullable): one thin-lens sample per sub-frame (mtb_render_batch_lens); the kernel makes each sub-frame's
 // primary rays from its LensRec.  NULL: pinhole views, exactly as without the argument.
+// pano (nullable, never with lenses; checked by CheckPanorama): panoramas (mtb_render_batch_pano); each device uploads
+// the PanoRec of its sub-frames and the call's longitude / latitude tables.  NULL: the views above.
 constexpr int64_t kMaxSampleSide = 65536;
 
 // Host restatement of the FP64 vector operations of device_core.cuh, in the same evaluation order (the library is built
-// with -ffp-contract=off), for the thin-lens records.
+// with -ffp-contract=off), for the thin-lens records and the panorama rays.
 struct H3 {
   double x, y, z;
 };
 H3 HAdd(const H3 &a, const H3 &b) { return H3{a.x + b.x, a.y + b.y, a.z + b.z}; }
+H3 HSub(const H3 &a, const H3 &b) { return H3{a.x - b.x, a.y - b.y, a.z - b.z}; }
 H3 HMulS(const H3 &a, double s) { return H3{a.x * s, a.y * s, a.z * s}; }
 H3 HNeg(const H3 &a) { return H3{-a.x, -a.y, -a.z}; }
 double HDot(const H3 &a, const H3 &b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
@@ -880,6 +886,63 @@ int MakeLensRec(mtb_context *ctx, const mtb_lens &ln, const double sensor[9], in
   return MTB_OK;
 }  // (keeps the tiles of a view's sample grid, 2^26, well inside int32)
 
+// A panorama batch (mtb_render_batch_pano): the call's fields of view in degrees and one eye offset per sub-frame
+// (eye_offsets NULL: all 0).
+struct Panorama {
+  double h_fov, v_fov;
+  const double *eye_offsets;
+};
+
+// The panorama rules of mtb_render_batch_pano: MTB_ERR_ARG, with the reason in ctx->err when there is a context.  The eye
+// offsets are read only when n_out and subframes pass the batch rules (RenderBatchImpl refuses the others).
+int CheckPanorama(mtb_context *ctx, double h_fov, double v_fov, const double *eye_offsets, int32_t n_out, int32_t subframes) {
+  std::string err;
+  if (!std::isfinite(h_fov) || !(h_fov > 0.0 && h_fov <= 360.0)) {
+    err = "h_fov must be finite and in (0, 360] degrees";
+  } else if (!std::isfinite(v_fov) || !(v_fov > 0.0 && v_fov <= 180.0)) {
+    err = "v_fov must be finite and in (0, 180] degrees";
+  } else if (eye_offsets != nullptr && n_out >= 1 && subframes >= 1 && (int64_t)n_out * subframes <= 65535) {
+    for (int32_t u = 0; u < n_out * subframes && err.empty(); u++) {
+      if (!std::isfinite(eye_offsets[u])) err = "eye_offsets[" + std::to_string(u) + "] must be finite";
+    }
+  }
+  if (err.empty()) return MTB_OK;
+  if (ctx != nullptr) ctx->err = err;
+  return MTB_ERR_ARG;
+}
+
+// The {cos, sin} tables of a grid_w x grid_h panorama: the grid_w longitudes, then the grid_h latitudes, in the FP64
+// order of the contract (include/mythtracer_b200.h).  cos and sin are separate calls of the C library's functions, the
+// ones a restatement calls per entry.
+std::vector<double> PanoramaTables(int grid_w, int grid_h, double h_fov, double v_fov) {
+  std::vector<double> tab(2 * ((size_t)grid_w + (size_t)grid_h));
+  const double h_rad = h_fov * (M_PI / 180.0), v_rad = v_fov * (M_PI / 180.0);
+  double *lat = tab.data() + 2 * (size_t)grid_w;
+  for (int X = 0; X < grid_w; X++) tab[2 * (size_t)X] = std::cos(((double)(2 * X + 1 - grid_w) / (double)(2 * grid_w)) * h_rad);
+  for (int X = 0; X < grid_w; X++) tab[2 * (size_t)X + 1] = std::sin(((double)(2 * X + 1 - grid_w) / (double)(2 * grid_w)) * h_rad);
+  for (int Y = 0; Y < grid_h; Y++) lat[2 * (size_t)Y] = std::cos(((double)(grid_h - 2 * Y - 1) / (double)(2 * grid_h)) * v_rad);
+  for (int Y = 0; Y < grid_h; Y++) lat[2 * (size_t)Y + 1] = std::sin(((double)(grid_h - 2 * Y - 1) / (double)(2 * grid_h)) * v_rad);
+  return tab;
+}
+
+mtb::PanoRec MakePanoRec(const mtb_camera &cam, double eye) {
+  mtb::PanoRec r;
+  mtb::ComputePanoramaBasis(cam, r.forward, r.right, r.up);
+  r.eye = eye;
+  return r;
+}
+
+// The primary ray of the sample with table entries lon = {cl, sl}, lat = {cp, sp}: RenderMega's panorama block on the
+// host (the same operations in the same order).
+void PanoramaRay(const mtb::PanoRec &r, const double origin[3], const double lon[2], const double lat[2], double o[3], double d[3]) {
+  const H3 F{r.forward[0], r.forward[1], r.forward[2]}, R{r.right[0], r.right[1], r.right[2]}, U{r.up[0], r.up[1], r.up[2]};
+  const H3 dir = HNormalized(HAdd(HMulS(HAdd(HMulS(F, lon[0]), HMulS(R, lon[1])), lat[0]), HMulS(U, lat[1])));
+  H3 org{origin[0], origin[1], origin[2]};
+  if (r.eye != 0.0) org = HAdd(org, HMulS(HSub(HMulS(R, lon[0]), HMulS(F, lon[1])), r.eye));
+  o[0] = org.x, o[1] = org.y, o[2] = org.z;
+  d[0] = dir.x, d[1] = dir.y, d[2] = dir.z;
+}
+
 // mtb_render_batch_device: `p` (nullable unless `name` is d_rgb) must be device memory of `device` with `align`-byte alignment.
 int CheckDeviceOutput(mtb_context *ctx, const void *p, const char *name, int device, uintptr_t align) {
   if (p == nullptr) return MTB_OK;
@@ -911,7 +974,7 @@ struct BatchPlane {
   void (*feed)(mtb::RenderParams &p, uint8_t *plane);  // sets the RenderParams field the plane is rendered through
 };
 
-int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
+int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *lenses, const Panorama *pano, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
                     int image_w, int image_h, int ss, int max_depth, uint8_t *rgb_host, mtb_debug *dbg_host, const mtb_taps *taps,
                     mtb_stats *stats, bool synchronous, bool device_out = false, cudaStream_t user_stream = nullptr) {
   const auto wall0 = std::chrono::steady_clock::now();
@@ -1019,6 +1082,11 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
     const int rc = MakeLensRec(ctx, lenses[v], views[(size_t)v].sensor, grid_w, grid_h, v, &lens_recs[(size_t)v]);
     if (rc != MTB_OK) return rc;
   }
+  std::vector<mtb::PanoRec> pano_recs(pano != nullptr ? (size_t)n_views : 0);
+  for (int32_t v = 0; v < n_views && pano != nullptr; v++) {
+    pano_recs[(size_t)v] = MakePanoRec(cams[v], pano->eye_offsets != nullptr ? pano->eye_offsets[v] : 0.0);
+  }
+  const std::vector<double> pano_tab = pano != nullptr ? PanoramaTables(grid_w, grid_h, pano->h_fov, pano->v_fov) : std::vector<double>();
 
   mtb::RenderParams rp;
   memset(&rp, 0, sizeof(rp));
@@ -1070,12 +1138,19 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
     for (int i = 0; i < kBatchPlanes; i++) {
       planes_grow |= !direct && planes[i].out != nullptr && n_plane * planes[i].elem > d.batch_planes[i].count;
     }
-    if ((size_t)count > d.batch_views.count || (lenses != nullptr && (size_t)count > d.batch_lens.count) || n_lt > d.batch_lights.count ||
+    if ((size_t)count > d.batch_views.count || (lenses != nullptr && (size_t)count > d.batch_lens.count) ||
+        (pano != nullptr && ((size_t)count > d.batch_pano.count || pano_tab.size() > d.batch_pano_tab.count)) || n_lt > d.batch_lights.count ||
         n_rgb > d.batch_rgb.count || planes_grow || n_sum > d.batch_sum.count || n_arrive > d.batch_arrive.count) {
       MTB_CUDA(ctx, cudaStreamSynchronize(s));
     }
     MTB_CUDA(ctx, d.batch_views.Upload(views.data() + first, (size_t)count, s));
     if (lenses != nullptr) MTB_CUDA(ctx, d.batch_lens.Upload(lens_recs.data() + first, (size_t)count, s));
+    mtb::PanoParams pp{};
+    if (pano != nullptr) {
+      MTB_CUDA(ctx, d.batch_pano.Upload(pano_recs.data() + first, (size_t)count, s));
+      MTB_CUDA(ctx, d.batch_pano_tab.Upload(pano_tab.data(), pano_tab.size(), s));
+      pp = mtb::PanoParams{d.batch_pano.ptr, d.batch_pano_tab.ptr, d.batch_pano_tab.ptr + 2 * (size_t)grid_w};
+    }
     MTB_CUDA(ctx, d.batch_lights.Upload(view_lights.data() + (size_t)first * nl, n_lt, s));
     if (n_rgb > 0) MTB_CUDA(ctx, d.batch_rgb.Reserve(n_rgb));
     mtb::DeviceScene sc = d.scene;
@@ -1116,7 +1191,7 @@ int RenderBatchImpl(mtb_context *ctx, const mtb_camera *cams, const mtb_lens *le
     if (device_out) MTB_CUDA(ctx, cudaStreamWaitEvent(s, ctx->dev[0].ev_batch_caller, 0));
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_start, s));
     mtb::LaunchRenderMegaBatch(sc, p, d.batch_views.ptr, tiles_per_view, count, ss, acc, lenses != nullptr ? d.batch_lens.ptr : nullptr,
-                               debug_build, s);
+                               pp, debug_build, s);
     ctx->launches++;
     MTB_CUDA(ctx, cudaGetLastError());
     MTB_CUDA(ctx, cudaEventRecord(d.ev_batch_stop, s));
@@ -1490,47 +1565,47 @@ int mtb_render_chunk_async(mtb_context *ctx, const mtb_camera *cam, int image_w,
 
 int mtb_render_batch(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                      int image_h, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_views, 1, lights, n_lights, image_w, image_h, 1, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_ss(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights, int image_w,
                         int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, stats, true);
 }
 
 int mtb_render_batch_ss_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                               int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr, nullptr, false);
 }
 
 int mtb_render_batch_debug(mtb_context *ctx, const mtb_camera *cams, int32_t n_views, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_debug *dbg_out,
                            const mtb_taps *taps, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_views, 1, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, dbg_out, taps, stats,
                          true);
 }
 
 int mtb_render_batch_accum(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights, int32_t n_lights,
                            int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
                          stats, true);
 }
 
 int mtb_render_batch_accum_async(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
                                  int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, uint8_t *rgb_out) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out, nullptr, nullptr,
                          nullptr, false);
 }
 
 int mtb_render_batch_device(mtb_context *ctx, const mtb_camera *cams, int32_t n_out, int32_t subframes, const mtb_light *lights,
                             int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth, void *d_rgb, mtb_debug *d_dbg,
                             const mtb_taps *d_taps, void *stream, mtb_stats *stats) {
-  return RenderBatchImpl(ctx, cams, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
+  return RenderBatchImpl(ctx, cams, nullptr, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
                          static_cast<uint8_t *>(d_rgb), d_dbg, d_taps, stats, false, true, static_cast<cudaStream_t>(stream));
 }
 
@@ -1541,7 +1616,7 @@ int mtb_render_batch_lens(mtb_context *ctx, const mtb_camera *cams, const mtb_le
     ctx->err = "lenses is NULL (pinhole views: mtb_render_batch_debug / mtb_render_batch_accum)";
     return MTB_ERR_ARG;
   }
-  return RenderBatchImpl(ctx, cams, lenses, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out,
+  return RenderBatchImpl(ctx, cams, lenses, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out,
                          dbg_out, taps, stats, true);
 }
 
@@ -1552,7 +1627,30 @@ int mtb_render_batch_lens_device(mtb_context *ctx, const mtb_camera *cams, const
     ctx->err = "lenses is NULL (pinhole views: mtb_render_batch_device)";
     return MTB_ERR_ARG;
   }
-  return RenderBatchImpl(ctx, cams, lenses, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
+  return RenderBatchImpl(ctx, cams, lenses, nullptr, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
+                         static_cast<uint8_t *>(d_rgb), d_dbg, d_taps, stats, false, true, static_cast<cudaStream_t>(stream));
+}
+
+int mtb_render_batch_pano(mtb_context *ctx, const mtb_camera *cams, const double *eye_offsets, int32_t n_out, int32_t subframes, double h_fov,
+                          double v_fov, const mtb_light *lights, int32_t n_lights, int image_w, int image_h, int samples_per_axis, int max_depth,
+                          uint8_t *rgb_out, mtb_debug *dbg_out, const mtb_taps *taps, mtb_stats *stats) {
+  if (ctx == nullptr) return MTB_ERR_ARG;
+  const int rc = CheckPanorama(ctx, h_fov, v_fov, eye_offsets, n_out, subframes);
+  if (rc != MTB_OK) return rc;
+  const Panorama pano{h_fov, v_fov, eye_offsets};
+  return RenderBatchImpl(ctx, cams, nullptr, &pano, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth, rgb_out,
+                         dbg_out, taps, stats, true);
+}
+
+int mtb_render_batch_pano_device(mtb_context *ctx, const mtb_camera *cams, const double *eye_offsets, int32_t n_out, int32_t subframes,
+                                 double h_fov, double v_fov, const mtb_light *lights, int32_t n_lights, int image_w, int image_h,
+                                 int samples_per_axis, int max_depth, void *d_rgb, mtb_debug *d_dbg, const mtb_taps *d_taps, void *stream,
+                                 mtb_stats *stats) {
+  if (ctx == nullptr) return MTB_ERR_ARG;
+  const int rc = CheckPanorama(ctx, h_fov, v_fov, eye_offsets, n_out, subframes);
+  if (rc != MTB_OK) return rc;
+  const Panorama pano{h_fov, v_fov, eye_offsets};
+  return RenderBatchImpl(ctx, cams, nullptr, &pano, n_out, subframes, lights, n_lights, image_w, image_h, samples_per_axis, max_depth,
                          static_cast<uint8_t *>(d_rgb), d_dbg, d_taps, stats, false, true, static_cast<cudaStream_t>(stream));
 }
 
@@ -1748,6 +1846,23 @@ int mtb_frame_read(mtb_context *ctx, const void *d_ptr, size_t offset, size_t by
 int mtb_camera_sensor(const mtb_camera *cam, int image_w, int image_h, double out9[9]) {
   if (cam == nullptr || out9 == nullptr || image_w <= 0 || image_h <= 0) return MTB_ERR_ARG;
   mtb::ComputeSensor(*cam, image_w, image_h, out9);
+  return MTB_OK;
+}
+
+int mtb_panorama_rays(const mtb_camera *cam, int grid_w, int grid_h, double h_fov, double v_fov, double eye_offset, double *origins,
+                      double *dirs) {
+  if (cam == nullptr || dirs == nullptr || grid_w <= 0 || grid_h <= 0 || grid_w > kMaxSampleSide || grid_h > kMaxSampleSide) return MTB_ERR_ARG;
+  if (CheckPanorama(nullptr, h_fov, v_fov, &eye_offset, 1, 1) != MTB_OK) return MTB_ERR_ARG;
+  const std::vector<double> tab = PanoramaTables(grid_w, grid_h, h_fov, v_fov);
+  const mtb::PanoRec rec = MakePanoRec(*cam, eye_offset);
+  const double *lat = tab.data() + 2 * (size_t)grid_w;
+  double o[3];
+  for (int Y = 0; Y < grid_h; Y++) {
+    for (int X = 0; X < grid_w; X++) {
+      const size_t i = ((size_t)Y * grid_w + X) * 3;
+      PanoramaRay(rec, cam->origin, &tab[2 * (size_t)X], &lat[2 * (size_t)Y], origins != nullptr ? origins + i : o, dirs + i);
+    }
+  }
   return MTB_OK;
 }
 

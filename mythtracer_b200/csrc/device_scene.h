@@ -89,6 +89,22 @@ struct LensRec {
   uint32_t centred;
 };
 
+// Panorama of one grid row (sub-frame) of a batch launch, from the camera and eye offset on the host
+// (RenderBatchImpl).  With {cl, sl} = lon[X] and {cp, sp} = lat[Y], sample (X, Y) is traced along
+// Normalized((forward * cl + right * sl) * cp + up * sp) from O, or from O + (right * cl - forward * sl) * eye when
+// eye != 0 (O the view's origin).
+struct PanoRec {
+  double forward[3], right[3], up[3];  // the camera's basis (ComputePanoramaBasis)
+  double eye;                          // e: the offset along the column's tangent
+};
+
+// The panorama of a batch launch: one PanoRec per grid row, and the {cos, sin} tables of the sample grid's longitudes
+// (one per column) and latitudes (one per row), each entry 16-byte aligned.  rec == NULL: no panorama.
+struct PanoParams {
+  const PanoRec *rec;
+  const double *lon, *lat;
+};
+
 struct IntersectParams {
   int64_t n;
   const double *origins, *dirs;
@@ -153,8 +169,11 @@ void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_block
 // must be NULL.  k = 1: the batches above.
 // lens (device memory, nullable): one LensRec per grid row (sub-frame); the primary rays of row u are those of lens[u].
 // NULL: pinhole views, the kernels above.
+// pano.rec (device memory, nullable, never with lens): panoramas; the primary rays of row u are those of pano.rec[u] and
+// the launch's longitude / latitude tables (views[u].sensor is unused).  NULL: the kernels above.
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
-                           int samples_per_axis, const AccumParams &acc, const LensRec *lens, bool debug_build, cudaStream_t stream);
+                           int samples_per_axis, const AccumParams &acc, const LensRec *lens, const PanoParams &pano, bool debug_build,
+                           cudaStream_t stream);
 void LaunchIntersect(const DeviceScene &sc, const IntersectParams &ip, bool debug_build, cudaStream_t stream);  // one ray per thread
 
 }  // namespace mtb

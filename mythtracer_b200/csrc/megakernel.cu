@@ -208,18 +208,22 @@ __device__ __forceinline__ void AverageEpilogue(const RenderParams &rp, const Ac
 // the supersampled batch, see AverageEpilogue; with SS = 1 every `SS` branch folds away.  ACC (BATCH only): the
 // accumulated batch, see AverageEpilogue; `acc` is unused without it.  LENS (BATCH only): thin-lens views, the
 // primary ray of grid row u starts on the lens point of lens[u] and passes through the focal-plane point of the pinhole
-// ray (LensRec); `lens` is unused without it, and only the primary ray differs.
+// ray (LensRec); `lens` is unused without it, and only the primary ray differs.  PANO (BATCH only, never with LENS):
+// panoramas, the primary ray of sample (X, Y) of grid row u is made from pano.rec[u] and the {cos, sin} entries
+// pano.lon[X] and pano.lat[Y] with + * / sqrt only (PanoRec; the host computes the trigonometry, so the rays match
+// its restatement bit for bit); `pano` is unused without it, and only the primary ray differs.
 // `sc` is __grid_constant__: the exact traversals take it by reference (TraceExactCold is not inlined), and a plain
 // by-value parameter whose address is taken is copied to local memory at kernel start (112 B), after which the scene
 // pointers (nodes, leaf records, shading records, materials, lights) are loaded from that copy.  A grid constant's
 // address points at the parameter bank itself, so the fields are constant-bank operands: C3 8.86 ->
 // 8.56 ms, C5 49.1 -> 47.7 ms, C4 7.73-7.79 -> 7.59-7.61 ms (B200, 1000 W, 1965 MHz max SM clock; DESIGN.md section 5).
-template <bool DBG, bool BATCH, int SS, bool ACC, bool LENS>
+template <bool DBG, bool BATCH, int SS, bool ACC, bool LENS, bool PANO>
 __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega(const __grid_constant__ DeviceScene sc, RenderParams rp, const ViewRec *views,
-                                                                                 AccumParams acc, const LensRec *lens) {
+                                                                                 AccumParams acc, const LensRec *lens, PanoParams pano) {
   static_assert(SS == 1 || (BATCH && (SS == 2 || SS == 4 || SS == 8)), "supersampling is a batch form with 2, 4 or 8 samples per axis");
   static_assert(!ACC || BATCH, "accumulation is a batch form");
   static_assert(!LENS || BATCH, "thin-lens views are a batch form");
+  static_assert(!PANO || (BATCH && !LENS), "panoramas are a batch form without thin lenses");
   MTB_DECLARE_FAST_CTX(kBlockThreads);
   // (SS = 8: 7 more words behind the samples for the epilogue's counter and partial sums)
   __shared__ __align__(8) unsigned char s_rgb[kTile * kTile * 3 + (SS == 8 ? 7 * 4 : 0)];
@@ -259,7 +263,15 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
     st.segments = 0;
     st.n_rays = 0;
 
-    {  // Sensor::GetRay (camera.cc:65-69) with full-image pixel coordinates (mythtracer.cc:298)
+    if constexpr (PANO) {  // panorama (PanoRec): longitude X and latitude Y of the sample grid, from the row's basis
+      const PanoRec &pr = pano.rec[blockIdx.y];
+      const double2 lon = reinterpret_cast<const double2 *>(pano.lon)[rp.chunk_x + px];  // {cos, sin}
+      const double2 lat = reinterpret_cast<const double2 *>(pano.lat)[rp.chunk_y + py];
+      const D3 fwd = Load3(pr.forward), right = Load3(pr.right);
+      Store3(st.m_d, Normalized(Add(MulS(Add(MulS(fwd, lon.x), MulS(right, lon.y)), lat.x), MulS(Load3(pr.up), lat.y))));
+      const D3 o = Load3(views[blockIdx.y].origin);
+      Store3(st.m_o, pr.eye == 0.0 ? o : Add(o, MulS(Sub(MulS(right, lon.x), MulS(fwd, lon.y)), pr.eye)));
+    } else {  // Sensor::GetRay (camera.cc:65-69) with full-image pixel coordinates (mythtracer.cc:298)
       const double *sensor = BATCH ? views[blockIdx.y].sensor : rp.sensor;
       const D3 start = Load3(sensor), d_scan = Load3(sensor + 3), d_pixel = Load3(sensor + 6);
       if constexpr (LENS) {
@@ -280,12 +292,12 @@ __global__ void __launch_bounds__(kBlockThreads, MTB_MEGA_MIN_BLOCKS) RenderMega
         Store3(st.m_o, Load3(BATCH ? views[blockIdx.y].origin : rp.origin));
         Store3(st.m_d, Normalized(Add(Add(start, MulS(d_scan, (double)(rp.chunk_y + py))), MulS(d_pixel, (double)(rp.chunk_x + px)))));
       }
-      st.coef = 1.0;
-      st.path = 1ull;
-      st.sig_hits = 0ull;
-      st.sig_shadow = 0ull;
-      Count<DBG>(cnt, kPrimary);
     }
+    st.coef = 1.0;
+    st.path = 1ull;
+    st.sig_hits = 0ull;
+    st.sig_shadow = 0ull;
+    Count<DBG>(cnt, kPrimary);
 
     for (;;) {
       int slot;
@@ -694,9 +706,9 @@ void LaunchBuildTileOrder(uint32_t *tile_cost, int32_t *tile_order, int n_tiles,
 void LaunchRenderMega(const DeviceScene &sc, const RenderParams &rp, int n_blocks, bool debug_build, cudaStream_t stream) {
   if (n_blocks <= 0) return;
   if (debug_build) {
-    RenderMega<true, false, 1, false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{}, nullptr);
+    RenderMega<true, false, 1, false, false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{}, nullptr, PanoParams{});
   } else {
-    RenderMega<false, false, 1, false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{}, nullptr);
+    RenderMega<false, false, 1, false, false, false><<<n_blocks, kBlockThreads, 0, stream>>>(sc, rp, nullptr, AccumParams{}, nullptr, PanoParams{});
   }
 }
 
@@ -710,17 +722,26 @@ void WithBool(bool b, const F &f) {
   }
 }
 
-// One of the 32 batch kernels: DBG x SS (1, 2, 4, 8) x ACC x LENS.
+// One of the 48 batch kernels: DBG x SS (1, 2, 4, 8) x ACC x primary ray (pinhole, thin lens, panorama).
 void LaunchRenderMegaBatch(const DeviceScene &sc, const RenderParams &rp, const ViewRec *views, int tiles_per_view, int n_views,
-                           int samples_per_axis, const AccumParams &acc, const LensRec *lens, bool debug_build, cudaStream_t stream) {
+                           int samples_per_axis, const AccumParams &acc, const LensRec *lens, const PanoParams &pano, bool debug_build,
+                           cudaStream_t stream) {
   if (tiles_per_view <= 0 || n_views <= 0) return;
   const dim3 grid((unsigned)tiles_per_view, (unsigned)n_views);
+  // f(lens, panorama) as two type flags, never both true
+  const auto with_primary_ray = [&](const auto &f) {
+    if (lens != nullptr) {
+      f(std::true_type{}, std::false_type{});
+    } else {
+      WithBool(pano.rec != nullptr, [&](auto panorama) { f(std::false_type{}, panorama); });
+    }
+  };
   WithBool(debug_build, [&](auto dbg) {
     WithBool(acc.subframes > 1, [&](auto accum) {
-      WithBool(lens != nullptr, [&](auto thin_lens) {
+      with_primary_ray([&](auto thin_lens, auto panorama) {
         const auto launch = [&](auto ss) {
-          RenderMega<decltype(dbg)::value, true, decltype(ss)::value, decltype(accum)::value, decltype(thin_lens)::value>
-              <<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens);
+          RenderMega<decltype(dbg)::value, true, decltype(ss)::value, decltype(accum)::value, decltype(thin_lens)::value,
+                     decltype(panorama)::value><<<grid, kBlockThreads, 0, stream>>>(sc, rp, views, acc, lens, pano);
         };
         switch (samples_per_axis) {
           case 1: launch(std::integral_constant<int, 1>{}); break;

@@ -1017,6 +1017,9 @@ Mat4 RotZ(double deg) {
   return Mat4{{{cos(a), -sin(a), 0.0, 0.0}, {sin(a), cos(a), 0.0, 0.0}, {0.0, 0.0, 1.0, 0.0}, {0.0, 0.0, 0.0, 1.0}}};
 }
 
+// The camera's rotation (camera.cc:48-51): the one matrix both the pinhole sensor and the panorama basis turn by.
+Mat4 Aim(const mtb_camera &cam) { return Mul(Mul(RotY(cam.yaw), RotX(cam.pitch)), RotZ(cam.roll)); }
+
 }  // namespace
 
 void ComputeSensor(const mtb_camera &cam, int image_w, int image_h, double out9[9]) {
@@ -1031,7 +1034,7 @@ void ComputeSensor(const mtb_camera &cam, int image_w, int image_h, double out9[
   Apply(corner_tl, fwd, tl);
   Apply(corner_tr, fwd, tr);
   Apply(corner_bl, fwd, bl);
-  const Mat4 aim = Mul(Mul(RotY(cam.yaw), RotX(cam.pitch)), RotZ(cam.roll));  // camera.cc:48-51
+  const Mat4 aim = Aim(cam);
   Apply(aim, tl, tl);
   Apply(aim, tr, tr);
   Apply(aim, bl, bl);
@@ -1040,6 +1043,14 @@ void ComputeSensor(const mtb_camera &cam, int image_w, int image_h, double out9[
     out9[3 + a] = (bl[a] - tl[a]) / double(image_h);  // delta_scanline
     out9[6 + a] = (tr[a] - tl[a]) / double(image_w);  // delta_pixel
   }
+}
+
+void ComputePanoramaBasis(const mtb_camera &cam, double forward[3], double right[3], double up[3]) {
+  const Mat4 aim = Aim(cam);
+  const double f[3] = {0.0, 0.0, 1.0}, r[3] = {-1.0, 0.0, 0.0}, u[3] = {0.0, 1.0, 0.0};
+  Apply(aim, f, forward);
+  Apply(aim, r, right);
+  Apply(aim, u, up);
 }
 
 }  // namespace mtb

@@ -127,6 +127,9 @@ int BuildFlatScene(const mtb_triangle *tris, int64_t n, bool use_list_bvh, Scene
 
 // Camera::GetSensor / Sensor::Reset (camera.cc:17-63): out9 = start_point, delta_scanline, delta_pixel.
 void ComputeSensor(const mtb_camera &cam, int image_w, int image_h, double out9[9]);
+// The panorama basis of a camera (mtb_render_batch_pano): aim (ComputeSensor's rotation) applied to (0, 0, 1),
+// (-1, 0, 0) and (0, 1, 0).  right points along the pinhole sensor's delta_pixel and up against its delta_scanline.
+void ComputePanoramaBasis(const mtb_camera &cam, double forward[3], double right[3], double up[3]);
 
 // ObjFileReader::ReadObjFile + MtlFileReader::ReadMtlFile (objreader.cc:201-274,472-549) + own decoders
 // for Texture::LoadFromFile (texture.cc:60-109; SDL2_image is not available offline).

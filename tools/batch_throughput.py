@@ -2,7 +2,7 @@
 orbit yaw = C3 yaw + 2 degrees * k.
 
     python tools/batch_throughput.py [--devices 0[,1,..]] [--out FILE] [--reps 3]
-                                     [--supersample | --debug-planes | --subframes | --device-output | --lens]
+                                     [--supersample | --debug-planes | --subframes | --device-output | --lens | --panorama]
 
 480x270, 64 frames: (a) one render_chunk per frame, megakernel forced; (b) one render_chunk per frame, automatic
 pipeline choice (after the 13 frames it needs to decide); (c) render_batch in batches of 1, 4, 16, 64.
@@ -49,6 +49,12 @@ pass: the accumulated batch without lenses; the same with centred lens samples (
 (its output must equal the first's); and a disc aperture (seeded concentric-disc samples of radius 4 focused at 150),
 which traces different rays.  Per mode: median kernel_ms per call over --reps passes, Mrays/s, output frames/s, and the
 kernel time over that of the batch without lenses.
+
+--panorama measures panorama batches (render_batch(..., panorama=(360, 180)), mtb_render_batch_pano) against pinhole
+batches of the same primary-ray count (same views, grid and s): 8 equirectangular C3 panoramas of the orbit at
+4096x2048; an omni-directional stereo pair from the C3 camera at 4096x2048 (eye offsets -/+0.032 x the scene's
+diagonal); 16 panoramas of the orbit at 1024x512 with s = 2.  Pinhole and panorama are timed in turn in every pass.  Per
+mode: median kernel_ms per call over --reps passes, Mrays/s, output frames/s, and the kernel time over the pinhole's.
 """
 import argparse
 import hashlib
@@ -303,6 +309,44 @@ def lens(mt, files, cfg, reps):
     return groups
 
 
+def panorama(mt, files, cfg, reps):
+    """The --panorama measurements (see the module docstring)."""
+    box = mt.scene_info()
+    scale = float(np.linalg.norm(np.array(box["aabb_max"]) - np.array(box["aabb_min"])))
+    groups = []
+    for title, n, w, h, s, eyes in (("8 equirectangular panoramas", 8, 4096, 2048, 1, None),
+                                    ("ODS stereo pair, e = -/+0.032 x scene diagonal", 2, 4096, 2048, 1, [-0.032 * scale, 0.032 * scale]),
+                                    ("16 panoramas, s = 2", 16, 1024, 512, 2, None)):
+        cams = _orbit(files.camera, n) if eyes is None else [files.camera] * n
+        modes = (("pinhole batch", {}), ("panorama 360 x 180", dict(panorama=(360.0, 180.0), eye_offsets=eyes)))
+        outs = [np.zeros((n, h, w, 3), np.uint8) for _ in modes]
+        call = [lambda i=i: mt.render_batch(cams, w, h, out=outs[i], samples_per_axis=s, **modes[i][1])["stats"] for i in range(len(modes))]
+        for c in call:
+            c()  # warm-up of this shape
+        walls, kms, rays = [[] for _ in modes], [[] for _ in modes], [0] * len(modes)
+        for _ in range(reps):  # the modes alternate within every pass
+            for i, c in enumerate(call):
+                t0 = time.perf_counter()
+                st = c()
+                walls[i].append(time.perf_counter() - t0)
+                kms[i].append(st["kernel_ms"])
+                rays[i] = st["rays"]
+        base = statistics.median(kms[0])
+        recs = []
+        for i, (name, _) in enumerate(modes):
+            rec = _ss_record(name, n, w, h, s, walls[i], kms[i], rays[i], None)
+            rec.pop("equals_block_mean_of_1080p")
+            rec["primary_rays"] = n * w * h * s * s
+            rec["kernel_ms_over_pinhole"] = round(statistics.median(kms[i]) / base, 4)
+            recs.append(rec)
+        recs[1]["differs_from_pinhole"] = not np.array_equal(outs[1], outs[0])
+        if eyes is not None:
+            recs[1]["eyes_differ"] = not np.array_equal(outs[1][0], outs[1][1])
+        print("%s: panorama / pinhole kernel time x%.4f" % (title, recs[1]["kernel_ms_over_pinhole"]), file=sys.stderr, flush=True)
+        groups.append(dict(shape="C3, %s at %dx%d" % (title, w, h), views=n, samples_per_axis=s, eye_offsets=eyes, modes=recs))
+    return groups
+
+
 def _orbit_subframes(cam, f, k):
     """The k sub-frames of output frame f of the orbit: yaw + 2 degrees * (f + j / k)."""
     out = []
@@ -468,6 +512,7 @@ def main():
     ap.add_argument("--subframes", action="store_true")
     ap.add_argument("--device-output", action="store_true")
     ap.add_argument("--lens", action="store_true")
+    ap.add_argument("--panorama", action="store_true")
     args = ap.parse_args()
     devices = [int(x) for x in args.devices.split(",")]
     files, cfg = scenegen.generate_config("C3", os.environ.get("MTB_SCENE_DIR", "/tmp/mtb_scenes"))
@@ -502,6 +547,14 @@ def main():
         _emit(doc, args.out)
         if not all(g["modes"][1]["equals_no_lenses"] for g in doc["lens"]):
             sys.exit("centred lens samples differ from the batch without lenses")
+        return
+
+    if args.panorama:
+        doc["panorama"] = panorama(mt, files, cfg, args.reps)
+        mt.close()
+        _emit(doc, args.out)
+        if not all(g["modes"][1]["differs_from_pinhole"] and g["modes"][1].get("eyes_differ", True) for g in doc["panorama"]):
+            sys.exit("a panorama gave the pinhole frames, or both eyes gave the same frame")
         return
 
     if args.subframes:

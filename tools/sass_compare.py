@@ -52,9 +52,12 @@ def _short(demangled):
 
 
 def _key(demangled):
-    """The name a kernel is matched by: its short name, with RenderMega's LENS parameter dropped when it is false, so
-    that RenderMega<a, b, c, d, false> of a tree with thin-lens views meets RenderMega<a, b, c, d> of one without."""
-    return re.sub(r"^(RenderMega<[^,<>]+, [^,<>]+, [^,<>]+, [^,<>]+), false>$", r"\1>", _short(demangled))
+    """The name a kernel is matched by: its short name, with RenderMega's trailing primary-ray parameters dropped while
+    they are false (PANO, then LENS), so that RenderMega<a, b, c, d, e, false> of a tree with panoramas meets
+    RenderMega<a, b, c, d, e> of one without, and RenderMega<a, b, c, d, false> meets RenderMega<a, b, c, d> of a tree
+    without thin-lens views."""
+    name = re.sub(r"^(RenderMega<[^,<>]+, [^,<>]+, [^,<>]+, [^,<>]+, [^,<>]+), false>$", r"\1>", _short(demangled))
+    return re.sub(r"^(RenderMega<[^,<>]+, [^,<>]+, [^,<>]+, [^,<>]+), false>$", r"\1>", name)
 
 
 def _kernels(log, sass):
